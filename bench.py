@@ -1,12 +1,18 @@
 #!/usr/bin/env python
 """Headline benchmark: movies/s for a 40x4096x4096 fp32 movie through estimate + correct.
 
-    python bench.py --gpus N --steps K --warmup W [--impl reference]
+    python bench.py --gpus N --steps K --warmup W [--impl reference] [--dump-outputs DIR]
 
 One "step" = one movie through ``motion_correct`` (whole-frame XC -> patch XC on the rigidly pre-shifted windows ->
 spline optimiser -> fused warp-and-sum).  At N > 1 (torchrun, one rank per GPU) every
 rank aligns its own movie (independent movies, no data-path collective: weak scaling) and the value
 is total movies / max-over-ranks device time.  Prints ONE JSON line (rank 0).
+
+``--dump-outputs DIR`` writes what the last timed step returned (rank 0) as ``DIR/<name>.npy``, float32, at most
+DUMP_BYTES in all.  Inputs and the optimiser's mini-batch order are seeded, so two builds run with the same arguments
+can be compared output for output.  Two runs of one build still differ a little: the optimiser accumulates in float
+atomics, so its field varies by about 4e-7 Angstrom, and next to the frame edge the sum is not continuous in the field
+(adding 1e-6 Angstrom to the field moved one edge pixel of the sum by 2.4; measured on a B200, 1000 W power limit).
 
 ``--impl reference`` times the CPU oracle (restatement of the reference's PyTorch path; the
 reference itself cannot be installed offline, see DESIGN.md) on a bounded sample of the workload.
@@ -17,6 +23,7 @@ from __future__ import annotations
 import argparse
 import json
 import os
+import random
 import subprocess
 import sys
 import threading
@@ -57,7 +64,33 @@ def parse_args():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-aten-baseline", action="store_true")
     ap.add_argument("--no-frame-split", action="store_true", help="skip the frame-split (one movie over N GPUs) sub-record at N > 1")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the outputs of the last timed step to DIR/<name>.npy")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    return args
+
+
+DUMP_BYTES = 64_000_000  # on disk, all files of --dump-outputs together
+NPY_HEADER = 4096  # more than any .npy header takes
+
+
+def dump_outputs(out_dir, arrays):
+    """Writes every array of ``arrays`` (name -> tensor, in order) as ``out_dir/<name>.npy`` in float32.  One that does
+    not fit what is left of DUMP_BYTES is replaced by a fixed, seeded sample of its elements (flattened, in index
+    order): the same positions on every run with the same arguments."""
+    import numpy as np
+
+    os.makedirs(out_dir, exist_ok=True)
+    left = DUMP_BYTES
+    for name, a in arrays.items():
+        a = a.detach().float().cpu().numpy()
+        if a.nbytes + NPY_HEADER > left:
+            keep = torch.randperm(a.size, generator=torch.Generator().manual_seed(0))[: (left - NPY_HEADER) // a.itemsize]
+            a = a.reshape(-1)[keep.sort().values.numpy()]
+        path = os.path.join(out_dir, name + ".npy")
+        np.save(path, a)
+        left -= os.path.getsize(path)
 
 
 # --------------------------------------------------------------------------------------------
@@ -483,6 +516,7 @@ def main():
     movie, _ = synthetic_movie_gpu(cfg["t"], cfg["h"], cfg["w"], 1000 + rank, dev)
 
     def step(m):
+        random.seed(0)  # the optimiser's mini-batch order: every step computes the same outputs
         return tmc.motion_correct(
             m, px, patch_sidelength=p, deformation_field_resolution=cfg["resolution"], n_iterations=iterations
         )
@@ -509,7 +543,7 @@ def main():
     barrier()
     start.record()
     for _ in range(args.steps):
-        step(movie)
+        total, field = step(movie)
     end.record()
     barrier()
     elapsed_ms = start.elapsed_time(end)
@@ -522,6 +556,9 @@ def main():
     if world > 1:
         dist.all_reduce(t_ms, op=dist.ReduceOp.MAX)
     max_ms = float(t_ms)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {"field": field, "frame_sum": total})
+    del total, field
 
     # ---- end to end through the public API with HOST buffers ----------------------------------
     # motion_correct_many: the public call for host-resident movies; it overlaps the H2D copy of the next movie

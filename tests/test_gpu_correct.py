@@ -104,15 +104,16 @@ def test_correct_motion_golden(dev, small):
     g, movie, px = small
     m = movie.to(dev)
     field = torch.as_tensor(g["field_344"]).to(dev)
-    assert rel_l2(tmc.correct_motion(m, field, px), g["correct_catmull"]) <= REL_L2
-    assert rel_l2(tmc.correct_motion(m, field, px, grid_type="bspline"), g["correct_bspline"]) <= REL_L2
+    # the corrected stacks are stored for every other row
+    assert rel_l2(tmc.correct_motion(m, field, px)[:, ::2], g["correct_catmull"]) <= REL_L2
+    assert rel_l2(tmc.correct_motion(m, field, px, grid_type="bspline")[:, ::2], g["correct_bspline"]) <= REL_L2
     f1 = torch.as_tensor(g["field_611"]).to(dev)
-    assert rel_l2(tmc.correct_motion(m, f1, px), g["correct_611_catmull"]) <= REL_L2
-    assert rel_l2(tmc.correct_motion_slow(m, field), g["correct_slow"]) <= REL_L2
+    assert rel_l2(tmc.correct_motion(m, f1, px)[:, ::2], g["correct_611_catmull"]) <= REL_L2
+    assert rel_l2(tmc.correct_motion_slow(m, field)[:, ::2], g["correct_slow"]) <= REL_L2
     new = torch.as_tensor(g["two_grids_new"]).to(dev)
-    assert rel_l2(tmc.correct_motion_two_grids(m, new, field, px, grad=False), g["correct_two_grids"]) <= REL_L2
+    assert rel_l2(tmc.correct_motion_two_grids(m, new, field, px, grad=False)[:, ::2], g["correct_two_grids"]) <= REL_L2
     s = tmc.correct_motion_sum(m, field, px, grid_type="bspline")
-    assert rel_l2(s, torch.as_tensor(g["correct_bspline"]).sum(dim=0)) <= REL_L2
+    assert rel_l2(s[::2], torch.as_tensor(g["correct_bspline"]).sum(dim=0)) <= REL_L2
 
 
 def test_zero_field_is_identity(dev):

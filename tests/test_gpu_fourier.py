@@ -183,8 +183,8 @@ def test_correct_motion_fast_golden(dev, golden_small):
     movie = torch.as_tensor(g["movie"]).to(dev)
     field = torch.as_tensor(g["field_611"]).to(dev)
     out = tmc.correct_motion_fast(movie, field)
-    want = torch.as_tensor(g["correct_fast"])
-    assert float(torch.linalg.norm(out.cpu() - want) / torch.linalg.norm(want)) <= 1e-4
+    want = torch.as_tensor(g["correct_fast"])  # every other row
+    assert float(torch.linalg.norm(out.cpu()[:, ::2] - want) / torch.linalg.norm(want)) <= 1e-4
     assert torch.equal(field.cpu(), torch.as_tensor(g["correct_fast_field_after"]))  # Q2: negated in place
     with pytest.raises(ValueError, match="Expected single patch deformation field"):
         tmc.correct_motion_fast(movie, torch.zeros((2, 6, 2, 2), device=dev))

@@ -38,7 +38,7 @@ def sum_samples(s):
     return {
         "sum_centre": s[h // 2 - 96 : h // 2 + 96, w // 2 - 96 : w // 2 + 96],
         "sum_corner": s[:96, :96],
-        "sum_rows": s[:: h // 16, :],
+        "sum_rows": s[:: h // (16 if h <= 4096 else 8), :],  # 8 rows of 8192^2: keeps each golden file under 1 MB
     }
 
 
@@ -151,5 +151,5 @@ def test_whole_frame_transforms(dev, n):
     out = tmc.correct_motion_fast(movie, shift)
     assert rel_l2(out[:, n // 2 - 64 : n // 2 + 64, n // 2 - 64 : n // 2 + 64], g["fast_centre"]) <= SUM_REL
     assert rel_l2(out[:, :64, :64], g["fast_corner"]) <= SUM_REL
-    assert rel_l2(out[:, :: n // 8, :], g["fast_rows"]) <= SUM_REL
+    assert rel_l2(out[:, :: n // (8 if n <= 4096 else 4), :], g["fast_rows"]) <= SUM_REL  # 4 rows of 8192^2 frames
     assert abs(float(torch.linalg.norm(out.double())) - float(g["fast_norm"])) <= SUM_REL * float(g["fast_norm"])

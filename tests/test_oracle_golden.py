@@ -72,14 +72,15 @@ def test_correction(small):
     g, movie, px, _ = small
     field = torch.as_tensor(g["field_344"])
     field1 = torch.as_tensor(g["field_611"])
-    close(rp.correct_motion(movie, field, px), g["correct_catmull"])
-    close(rp.correct_motion(movie, field, px, "bspline"), g["correct_bspline"])
-    close(rp.correct_motion(movie, field1, px), g["correct_611_catmull"])
+    # the corrected stacks are stored for every other row
+    close(rp.correct_motion(movie, field, px)[:, ::2], g["correct_catmull"])
+    close(rp.correct_motion(movie, field, px, "bspline")[:, ::2], g["correct_bspline"])
+    close(rp.correct_motion(movie, field1, px)[:, ::2], g["correct_611_catmull"])
     fast_in = field1.clone()
-    close(rp.correct_motion_fast(movie, fast_in), g["correct_fast"], 1e-5)
+    close(rp.correct_motion_fast(movie, fast_in)[:, ::2], g["correct_fast"], 1e-5)
     close(fast_in, g["correct_fast_field_after"])
-    close(rp.correct_motion_slow(movie, field), g["correct_slow"])
-    close(rp.correct_motion_two_grids(movie, torch.as_tensor(g["two_grids_new"]), field, px), g["correct_two_grids"])
+    close(rp.correct_motion_slow(movie, field)[:, ::2], g["correct_slow"])
+    close(rp.correct_motion_two_grids(movie, torch.as_tensor(g["two_grids_new"]), field, px)[:, ::2], g["correct_two_grids"])
     with pytest.raises(ValueError, match="Expected single patch deformation field"):
         rp.correct_motion_fast(movie, field.clone())
 
