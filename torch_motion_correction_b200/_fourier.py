@@ -219,6 +219,7 @@ class BandPlan:
 
 
 _tiles: dict = {}
+_self_paired: dict = {}
 
 
 def band_tiles(plan: "BandPlan") -> torch.Tensor:
@@ -236,6 +237,26 @@ def band_tiles(plan: "BandPlan") -> torch.Tensor:
         if hit.shape[0] == 0:
             hit = torch.zeros((1, 2), dtype=torch.int32, device=w.device)
         _tiles[key] = hit
+    return hit
+
+
+def self_paired_weight(plan: "BandPlan") -> bool:
+    """True if the pass band weights a bin that the real-space losses ("cc", "ncc") see only through its Hermitian
+    part: the Nyquist column kx = nx/2 (nx even), or the ky = -ny/2 bin of the DC column (ny even).  irfftn keeps
+    only the real part of those columns after its transform along y, so a fractional shift changes what the loss sees
+    there (csrc/optimizer.cu, header).  The generic loss kernels handle these bins; the tiled iteration does not.
+    Cached per plan geometry."""
+    key = plan.key
+    hit = _self_paired.get(key)
+    if hit is None:
+        w = plan.weight
+        live = torch.zeros((), dtype=torch.bool, device=w.device)
+        if plan.nx % 2 == 0 and plan.kx == plan.nx // 2 + 1:
+            live |= (w[:, -1] != 0).any()
+        if plan.ny % 2 == 0 and plan.ky == plan.ny and plan.ky_start == -(plan.ny // 2):
+            live |= w[0, 0] != 0
+        hit = bool(live)
+        _self_paired[key] = hit
     return hit
 
 

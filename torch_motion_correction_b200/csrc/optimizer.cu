@@ -15,6 +15,16 @@
 //   ncc_t = cc_t / sqrt((A_t / P + eps)(B_t + eps)),  B_t = (q - 2 p_t + A_t) / (P (T-1)^2)
 // and dL/ds_{t,y} = sum_f w (-c f_y) Im(S_t conj Z_t),  Z_t = (alpha_t + 2 beta) Sigma + sum_u alpha_u S_u,
 // alpha_t = dL/dp_t, beta = dL/dq, c f_y = fp32(-2 pi) f_y as the reference forms it.
+//
+// Self-paired columns ("cc" / "ncc" only).  The reference takes the real-space patches with irfftn, whose c2r step keeps
+// only the real part of the kx = 0 and (nx even) kx = nx/2 columns after the transform along y.  For a shift that is not
+// a whole number of pixels S_t is not Hermitian-consistent there (the Nyquist column, and the ky = -ny/2 bin of the DC
+// column when ny is even), so on those two columns the losses see H_t(ky) = (S_t(ky) + conj S_t(-ky mod ny)) / 2
+// instead of S_t: Sigma, p_t, q and A_t are formed from H_t, which makes A_t shift dependent there (the kernels add
+// A_t(H) - A_t(S) to the shift-independent norms every evaluation).  Because H_t(-ky) = conj H_t(ky), the gradient keeps
+// the form above with the raw S_t and Z_t built from H_t, plus 2 gamma_t H_t (gamma_t = dL/dA_t) on those columns.
+// The band box is symmetric in ky, so both bins of a pair lie in the same column of the box.  "mse" compares the
+// half spectra directly and uses S_t everywhere.
 #include "common.cuh"
 
 namespace {
@@ -37,6 +47,22 @@ __device__ __forceinline__ void bin_freqs(const BandGeom& g, int bin, float& cfy
   herm = (kx == 0 || 2 * kx == g.nx) ? 1.0f : 2.0f;
 }
 
+// box row of the bin (-ky mod ny, kx) that irfftn pairs with bin `bin` on a self-paired column (kx = 0, or kx = nx/2 with
+// nx even), -1 on every other column; the ky = -ny/2 bin (ny even) is its own partner
+__device__ __forceinline__ int partner_row(const BandGeom& g, int bin) {
+  const int kyb = bin / g.KX, kx = bin % g.KX;
+  if (kx != 0 && 2 * kx != g.nx) return -1;
+  int ky = g.ky_start + kyb;
+  ky = ((ky % g.ny) + g.ny) % g.ny;
+  if (ky >= (g.ny + 1) / 2) ky -= g.ny;
+  return 2 * ky == -g.ny ? kyb : -ky - g.ky_start;
+}
+
+// (S + conj S') / 2
+__device__ __forceinline__ float2 hermitian_part(float2 s, float2 s_partner) {
+  return make_float2(0.5f * (s.x + s_partner.x), 0.5f * (s.y - s_partner.y));
+}
+
 __device__ __forceinline__ float2 shifted(float2 fw, float cfy, float cfx, float sy, float sx) {
   const float ang = __fadd_rn(__fmul_rn(cfy, sy), __fmul_rn(cfx, sx));
   float s, c;
@@ -51,6 +77,9 @@ __device__ __forceinline__ void block_accumulate(double v, double* target, doubl
 }
 
 // A[g][t] = sum_f w |FW_t|^2 for both weightings: norms[(g*T + t)*2 + {0: w=1, 1: hermitian}]
+// (the shift-independent part: on the self-paired columns the "cc" / "ncc" kernels add A_t(H) - A_t(S) every
+// evaluation, see the header; the tiled kernel, which runs only when those columns carry no pass-band weight beyond
+// the Hermitian-consistent DC column, uses these norms as they are)
 __global__ void __launch_bounds__(kOptThreads)
 spectra_norms_kernel(const float2* __restrict__ spec, int T, int Tp, BandGeom geom, int frame_major,
                      double* __restrict__ norms) {
@@ -76,49 +105,91 @@ spectra_norms_kernel(const float2* __restrict__ spec, int T, int Tp, BandGeom ge
   }
 }
 
-// Sigma[g][bin], q[g] and p[g][t]
+// per-bin state of the generic kernels: the bin's frequency factors and weight, and (hermitian weighting, self-paired
+// column) the partner bin's offset and frequency factor, see the header
+struct BinState {
+  float cfy, cfx, w, pcfy;
+  int partner;  // bin index of the partner, -1: S_t is used as it is
+};
+
+__device__ __forceinline__ BinState bin_state(const BandGeom& geom, int bin, bool live, int hermitian) {
+  BinState b{0.f, 0.f, 0.f, 0.f, -1};
+  if (!live) return b;
+  float herm, pcfx;
+  bin_freqs(geom, bin, b.cfy, b.cfx, herm);
+  b.w = hermitian ? herm : 1.0f;
+  const int pr = hermitian ? partner_row(geom, bin) : -1;
+  if (pr >= 0) {
+    b.partner = pr * geom.KX + bin % geom.KX;
+    bin_freqs(geom, b.partner, b.pcfy, pcfx, herm);
+  }
+  return b;
+}
+
+// the spectrum the loss sees at frame t: S_t, or H_t on a self-paired column (s: the raw S_t)
+__device__ __forceinline__ float2 loss_spectrum(const float2* __restrict__ sp_t, int bin, const BinState& b, float2 s, float sy,
+                                                float sx) {
+  if (b.partner < 0) return s;
+  return hermitian_part(s, shifted(sp_t[b.partner - bin], b.pcfy, b.cfx, sy, sx));
+}
+
+// Sigma[g][bin], q[g], p[g][t] and (self-paired columns) dA[g][t] = A_t(H) - A_t(S)
 __global__ void __launch_bounds__(kOptThreads)
 loss_forward_kernel(const float2* __restrict__ spec, const float* __restrict__ shifts, int T, int Tp, BandGeom geom,
-                    int hermitian, float2* __restrict__ sigma, double* __restrict__ q, double* __restrict__ p) {
+                    int hermitian, float2* __restrict__ sigma, double* __restrict__ q, double* __restrict__ p,
+                    double* __restrict__ dA) {
   const int g = blockIdx.y;
   const int bins = geom.KY * geom.KX;
   const int bin = blockIdx.x * kOptThreads + threadIdx.x;
   const bool live = bin < bins;
-  float cfy = 0.f, cfx = 0.f, herm = 0.f;
-  if (live) bin_freqs(geom, bin, cfy, cfx, herm);
-  const float w = hermitian ? herm : (live ? 1.0f : 0.0f);
+  const BinState b = bin_state(geom, bin, live, hermitian);
   const float2* sp = spec + (long)g * Tp * bins + bin;
   const float* sh = shifts + (long)g * T * 2;
   float2 sum = make_float2(0.f, 0.f);
   if (live)
-    for (int t = 0; t < T; ++t) sum = cadd(sum, shifted(sp[(long)t * bins], cfy, cfx, __ldg(sh + 2 * t), __ldg(sh + 2 * t + 1)));
+    for (int t = 0; t < T; ++t) {
+      const float sy = __ldg(sh + 2 * t), sx = __ldg(sh + 2 * t + 1);
+      sum = cadd(sum, loss_spectrum(sp + (long)t * bins, bin, b, shifted(sp[(long)t * bins], b.cfy, b.cfx, sy, sx), sy, sx));
+    }
   if (live) sigma[(long)g * bins + bin] = sum;
   {
-    double v = live ? (double)w * ((double)sum.x * sum.x + (double)sum.y * sum.y) : 0.0;
+    double v = live ? (double)b.w * ((double)sum.x * sum.x + (double)sum.y * sum.y) : 0.0;
     v = warp_sum(v);
     if ((threadIdx.x & 31) == 0) atomicAdd(q + g, v);
   }
+  const bool paired = __any_sync(0xffffffffu, b.partner >= 0);
   for (int t = 0; t < T; ++t) {
-    double v = 0.0;
+    double v = 0.0, d = 0.0;
     if (live) {
-      const float2 s = shifted(sp[(long)t * bins], cfy, cfx, __ldg(sh + 2 * t), __ldg(sh + 2 * t + 1));
-      v = (double)w * ((double)s.x * sum.x + (double)s.y * sum.y);  // Re(S conj Sigma)
+      const float sy = __ldg(sh + 2 * t), sx = __ldg(sh + 2 * t + 1);
+      const float2 s = shifted(sp[(long)t * bins], b.cfy, b.cfx, sy, sx);
+      const float2 h = loss_spectrum(sp + (long)t * bins, bin, b, s, sy, sx);
+      v = (double)b.w * ((double)h.x * sum.x + (double)h.y * sum.y);  // Re(H conj Sigma)
+      if (b.partner >= 0)
+        d = (double)b.w * (((double)h.x * h.x + (double)h.y * h.y) - ((double)s.x * s.x + (double)s.y * s.y));
     }
     v = warp_sum(v);
     if ((threadIdx.x & 31) == 0) atomicAdd(p + (long)g * T + t, v);
+    if (paired) {
+      d = warp_sum(d);
+      if ((threadIdx.x & 31) == 0 && d != 0.0) atomicAdd(dA + (long)g * T + t, d);
+    }
   }
 }
 
 // loss_type: 0 mse, 1 cc, 2 ncc.  scale[g]: per-patch weight of the (mean-reduced) mini-batch loss.
-// Writes loss (+=), alpha[g][t], beta[g].  One thread per (g, t) pair is plenty.
+// A_t = norms + dA (hermitian weighting).  Writes loss (+=), alpha[g][t], beta[g], gamma[g][t] = dL/dA_t.
+// One thread per (g, t) pair is plenty.
 __global__ void loss_scalars_kernel(const double* __restrict__ norms, const double* __restrict__ q, const double* __restrict__ p,
-                                    const float* __restrict__ scale, int G, int T, int ph, int pw, int loss_type,
-                                    float* __restrict__ alpha, float* __restrict__ beta, double* __restrict__ loss) {
+                                    const double* __restrict__ dA, const float* __restrict__ scale, int G, int T, int ph, int pw,
+                                    int loss_type, float* __restrict__ alpha, float* __restrict__ beta, float* __restrict__ gamma,
+                                    double* __restrict__ loss) {
   const int g = blockIdx.x * blockDim.x + threadIdx.x;
   if (g >= G) return;
   const double sc = (double)scale[g];
   const double P = (double)ph * (double)pw;
   double l = 0.0, b = 0.0;
+  for (int t = 0; t < T; ++t) gamma[(long)g * T + t] = 0.f;
   if (T < 2 || sc == 0.0) {
     for (int t = 0; t < T; ++t) alpha[(long)g * T + t] = 0.f;
     beta[g] = 0.f;
@@ -136,16 +207,17 @@ __global__ void loss_scalars_kernel(const double* __restrict__ norms, const doub
   } else if (loss_type == 1) {
     const double k = 1.0 / (P * (T - 1));
     for (int t = 0; t < T; ++t) {
-      const double A = norms[((long)g * T + t) * 2 + 1];
+      const double A = norms[((long)g * T + t) * 2 + 1] + dA[(long)g * T + t];
       l += -sc * k * (p[(long)g * T + t] - A);
       alpha[(long)g * T + t] = (float)(-sc * k);
+      gamma[(long)g * T + t] = (float)(sc * k);
     }
   } else {
     const double eps = 1e-8;
     const double k = 1.0 / (P * (T - 1));
     const double kb = 1.0 / (P * (double)(T - 1) * (double)(T - 1));
     for (int t = 0; t < T; ++t) {
-      const double A = norms[((long)g * T + t) * 2 + 1];
+      const double A = norms[((long)g * T + t) * 2 + 1] + dA[(long)g * T + t];
       const double pt = p[(long)g * T + t];
       const double cc = k * (pt - A);
       const double X = A / P + eps;
@@ -157,6 +229,8 @@ __global__ void loss_scalars_kernel(const double* __restrict__ norms, const doub
       const double dB = -0.5 * ncc / B;
       alpha[(long)g * T + t] = (float)(-sc * (k / den + dB * (-2.0 * kb)));
       b += -sc * dB * kb;
+      // d ncc / d A_t = -k / den - ncc / (2 X) / P - ncc / (2 B) * kb
+      gamma[(long)g * T + t] = (float)(-sc * (-k / den - 0.5 * ncc / (X * P) + dB * kb));
     }
   }
   beta[g] = (float)b;
@@ -166,25 +240,26 @@ __global__ void loss_scalars_kernel(const double* __restrict__ norms, const doub
 // grad[g][t][2] += sum_f w (-c f) Im(S_t conj Z_t)
 __global__ void __launch_bounds__(kOptThreads)
 loss_backward_kernel(const float2* __restrict__ spec, const float* __restrict__ shifts, const float2* __restrict__ sigma,
-                     const float* __restrict__ alpha, const float* __restrict__ beta, int T, int Tp, BandGeom geom,
-                     int hermitian, int has_alpha, float* __restrict__ grad) {
+                     const float* __restrict__ alpha, const float* __restrict__ beta, const float* __restrict__ gamma, int T,
+                     int Tp, BandGeom geom, int hermitian, int has_alpha, float* __restrict__ grad) {
   const int g = blockIdx.y;
   const int bins = geom.KY * geom.KX;
   const int bin = blockIdx.x * kOptThreads + threadIdx.x;
   const bool live = bin < bins;
-  float cfy = 0.f, cfx = 0.f, herm = 0.f;
-  if (live) bin_freqs(geom, bin, cfy, cfx, herm);
-  const float w = hermitian ? herm : (live ? 1.0f : 0.0f);
+  const BinState b = bin_state(geom, bin, live, hermitian);
+  const float w = b.w, cfy = b.cfy, cfx = b.cfx;
   const float2* sp = spec + (long)g * Tp * bins + bin;
   const float* sh = shifts + (long)g * T * 2;
   const float* al = alpha + (long)g * T;
+  const float* ga = gamma + (long)g * T;
   const float be2 = 2.0f * __ldg(beta + g);
   float2 sum = make_float2(0.f, 0.f), wsum = make_float2(0.f, 0.f);
   if (live) {
     sum = sigma[(long)g * bins + bin];
     if (has_alpha)
       for (int t = 0; t < T; ++t) {
-        const float2 s = shifted(sp[(long)t * bins], cfy, cfx, __ldg(sh + 2 * t), __ldg(sh + 2 * t + 1));
+        const float sy = __ldg(sh + 2 * t), sx = __ldg(sh + 2 * t + 1);
+        const float2 s = loss_spectrum(sp + (long)t * bins, bin, b, shifted(sp[(long)t * bins], cfy, cfx, sy, sx), sy, sx);
         const float a = __ldg(al + t);
         wsum.x += a * s.x;
         wsum.y += a * s.y;
@@ -193,9 +268,16 @@ loss_backward_kernel(const float2* __restrict__ spec, const float* __restrict__ 
   for (int t = 0; t < T; ++t) {
     float gy = 0.f, gx = 0.f;
     if (live) {
-      const float2 s = shifted(sp[(long)t * bins], cfy, cfx, __ldg(sh + 2 * t), __ldg(sh + 2 * t + 1));
+      const float sy = __ldg(sh + 2 * t), sx = __ldg(sh + 2 * t + 1);
+      const float2 s = shifted(sp[(long)t * bins], cfy, cfx, sy, sx);
       const float a = (has_alpha ? __ldg(al + t) : 0.f) + be2;
-      const float2 z = make_float2(a * sum.x + wsum.x, a * sum.y + wsum.y);
+      float2 z = make_float2(a * sum.x + wsum.x, a * sum.y + wsum.y);
+      if (b.partner >= 0) {  // + 2 gamma_t H_t: A_t depends on the shift on this column
+        const float2 h = loss_spectrum(sp + (long)t * bins, bin, b, s, sy, sx);
+        const float g2 = 2.0f * __ldg(ga + t);
+        z.x += g2 * h.x;
+        z.y += g2 * h.y;
+      }
       const float im = s.y * z.x - s.x * z.y;  // Im(S conj Z)
       gy = -w * cfy * im;
       gx = -w * cfx * im;
@@ -236,6 +318,7 @@ __global__ void phase_tables_kernel(const float* __restrict__ shifts, int T, Ban
 }
 
 // q[g] += sum_f w |Sigma|^2 ; grad[g][t][:] += -2 b sum_f w (c f) Im(S_t conj Sigma)
+// ("cc" on a self-paired column: Sigma = sum_t H_t, q[g] -= A_t(H) - A_t(S), Im(S_t conj (Sigma - H_t)); see the header)
 // kFusedBins bins per thread amortise the per-frame warp reductions; UNROLL frames in flight hide load latency;
 // MINB CTAs/SM caps the registers (the first version ran at 168 registers, 17 % occupancy: profiles/r01_final_*)
 template <int kFusedBins, int UNROLL, int MINB>
@@ -256,7 +339,7 @@ loss_fused_kernel(const float2* __restrict__ spec, const float2* __restrict__ E,
   } else {
     b = -sc / ((float)ph * (float)pw * (float)(T - 1));
   }
-  int bin[kFusedBins], kyb[kFusedBins], kx[kFusedBins];
+  int bin[kFusedBins], kyb[kFusedBins], kx[kFusedBins], pyb[kFusedBins];
   float cfy[kFusedBins], cfx[kFusedBins], w[kFusedBins];
   float2 sum[kFusedBins];
 #pragma unroll
@@ -269,9 +352,11 @@ loss_fused_kernel(const float2* __restrict__ spec, const float2* __restrict__ E,
     w[i] = live ? (loss_type == 0 ? 1.0f : herm) : 0.0f;
     kyb[i] = bb / geom.KX;
     kx[i] = bb % geom.KX;
+    pyb[i] = live && loss_type != 0 ? partner_row(geom, bb) : -1;
     bin[i] = bb;
     sum[i] = make_float2(0.f, 0.f);
   }
+  double dq = 0.0;  // - sum_t (A_t(H) - A_t(S)) over this thread's self-paired bins
   const float2* sp = spec + (long)g * Tp * bins;
   const float2* Eg = E + (long)g * T * (geom.KY + geom.KX);
 #pragma unroll UNROLL
@@ -280,11 +365,18 @@ loss_fused_kernel(const float2* __restrict__ spec, const float2* __restrict__ E,
 #pragma unroll
     for (int i = 0; i < kFusedBins; ++i) {
       const float2 e = cmul(__ldg(Et + kyb[i]), __ldg(Et + geom.KY + kx[i]));
-      sum[i] = cadd(sum[i], cmul(__ldg(sp + (long)t * bins + bin[i]), e));
+      float2 s = cmul(__ldg(sp + (long)t * bins + bin[i]), e);
+      if (pyb[i] >= 0) {
+        const float2 ep = cmul(__ldg(Et + pyb[i]), __ldg(Et + geom.KY + kx[i]));
+        const float2 h = hermitian_part(s, cmul(__ldg(sp + (long)t * bins + pyb[i] * geom.KX + kx[i]), ep));
+        dq -= (double)w[i] * (((double)h.x * h.x + (double)h.y * h.y) - ((double)s.x * s.x + (double)s.y * s.y));
+        s = h;
+      }
+      sum[i] = cadd(sum[i], s);
     }
   }
   {
-    double v = 0.0;
+    double v = dq;
 #pragma unroll
     for (int i = 0; i < kFusedBins; ++i) v += (double)w[i] * ((double)sum[i].x * sum[i].x + (double)sum[i].y * sum[i].y);
     v = warp_sum(v);
@@ -299,7 +391,13 @@ loss_fused_kernel(const float2* __restrict__ spec, const float2* __restrict__ E,
     for (int i = 0; i < kFusedBins; ++i) {
       const float2 e = cmul(__ldg(Et + kyb[i]), __ldg(Et + geom.KY + kx[i]));
       const float2 s = cmul(__ldg(sp + (long)t * bins + bin[i]), e);
-      const float im = w[i] * (s.y * sum[i].x - s.x * sum[i].y);  // w Im(S conj Sigma)
+      float2 z = sum[i];
+      if (pyb[i] >= 0) {
+        const float2 ep = cmul(__ldg(Et + pyb[i]), __ldg(Et + geom.KY + kx[i]));
+        const float2 h = hermitian_part(s, cmul(__ldg(sp + (long)t * bins + pyb[i] * geom.KX + kx[i]), ep));
+        z = make_float2(z.x - h.x, z.y - h.y);
+      }
+      const float im = w[i] * (s.y * z.x - s.x * z.y);  // w Im(S conj Sigma)
       gy = fmaf(cfy[i], im, gy);
       gx = fmaf(cfx[i], im, gx);
     }
@@ -416,14 +514,14 @@ TMC_API int tmc_local_spectra_norms(const void* spec, int g, int t, int tp, int 
 //  patch_scale: (G) f32, or (n_iterations, G) when `iteration` (device int, nullable) selects the row -- this
 //  lets a captured CUDA graph replay the step with a different mini-batch weighting every iteration;
 //  workspace layout (floats): sigma 2*G*bins | phase tables 2*G*T*(KY+KX) | shifts 2*G*T | grad_shifts 2*G*T |
-//                             alpha G*T | beta G | then doubles q G | p G*T
+//                             alpha G*T | beta G | gamma G*T | then doubles q G | p G*T | dA G*T
 static long local_loss_workspace_floats(int g, int t, int ky_count, int kx_count) {
   long bins = (long)ky_count * kx_count;
-  long floats = 2 * g * bins + 2l * g * t * (ky_count + kx_count) + 2l * g * t + 2l * g * t + (long)g * t + g;
+  long floats = 2 * g * bins + 2l * g * t * (ky_count + kx_count) + 2l * g * t + 2l * g * t + (long)g * t + g + (long)g * t;
   return (floats + 1) & ~1l;
 }
 TMC_API long tmc_local_loss_workspace_bytes(int g, int t, int ky_count, int kx_count) {
-  return local_loss_workspace_floats(g, t, ky_count, kx_count) * 4 + 8l * (g + (long)g * t);
+  return local_loss_workspace_floats(g, t, ky_count, kx_count) * 4 + 8l * (g + 2l * g * t);
 }
 
 TMC_API int tmc_local_loss_grad(const void* spec, const double* norms, const float* eval_new, const float* eval_base,
@@ -443,10 +541,12 @@ TMC_API int tmc_local_loss_grad(const void* spec, const double* norms, const flo
   float* grad_shifts = shifts + 2l * g * t;
   float* alpha = grad_shifts + 2l * g * t;
   float* beta = alpha + (long)g * t;
+  float* gamma = beta + g;
   const long floats = local_loss_workspace_floats(g, t, ky_count, kx_count);
   double* q = (double*)(wf + floats);
   double* p = q + g;
-  TMC_CUDA(cudaMemsetAsync(q, 0, sizeof(double) * ((size_t)g + (size_t)g * t), stream));
+  double* dA = p + (long)g * t;
+  TMC_CUDA(cudaMemsetAsync(q, 0, sizeof(double) * ((size_t)g + 2 * (size_t)g * t), stream));
   TMC_CUDA(cudaMemsetAsync(grad_shifts, 0, sizeof(float) * 2 * (size_t)g * t, stream));
   TMC_CUDA(cudaMemsetAsync(loss, 0, sizeof(double), stream));
   const int n = t * g * 2;
@@ -473,9 +573,11 @@ TMC_API int tmc_local_loss_grad(const void* spec, const double* norms, const flo
   TMC_CHECK_ARG(iteration == nullptr, "local_loss_grad: the ncc path takes the per-iteration scale row directly");
   const int hermitian = loss_type != 0;
   dim3 grid(tmc_div_up(bins, kOptThreads), g);
-  loss_forward_kernel<<<grid, kOptThreads, 0, stream>>>((const float2*)spec, shifts, t, tp, geom, hermitian, sigma, q, p); tmc_count_launch();
-  loss_scalars_kernel<<<tmc_div_up(g, 64), 64, 0, stream>>>(norms, q, p, patch_scale, g, t, ny, nx, loss_type, alpha, beta, loss); tmc_count_launch();
-  loss_backward_kernel<<<grid, kOptThreads, 0, stream>>>((const float2*)spec, shifts, sigma, alpha, beta, t, tp, geom, hermitian,
+  loss_forward_kernel<<<grid, kOptThreads, 0, stream>>>((const float2*)spec, shifts, t, tp, geom, hermitian, sigma, q, p, dA);
+  tmc_count_launch();
+  loss_scalars_kernel<<<tmc_div_up(g, 64), 64, 0, stream>>>(norms, q, p, dA, patch_scale, g, t, ny, nx, loss_type, alpha, beta, gamma,
+                                                            loss); tmc_count_launch();
+  loss_backward_kernel<<<grid, kOptThreads, 0, stream>>>((const float2*)spec, shifts, sigma, alpha, beta, gamma, t, tp, geom, hermitian,
                                                         loss_type != 0, grad_shifts); tmc_count_launch();
   shifts_grad_to_eval_kernel<<<tmc_div_up(n, 128), 128, 0, stream>>>(grad_shifts, t, g, pixel_spacing, grad_eval); tmc_count_launch();
   TMC_CHECK_LAUNCH("tmc_local_loss_grad");

@@ -247,7 +247,7 @@ def estimate_patch_motion_frame_split(local_frames, pixel_spacing, frame_offset,
 def _make_patch_shard_problem(spec_sub, centres_norm_sub, base, kind, loss_code, px, t, ph, pw, resolution, plan, dev):
     """A ``LocalMotionProblem`` (estimate_motion_optimizer.py) for a subset of the patches with ALL frames, built from
     spectra ``spec_sub`` (G_r, tp, KY, KX) that are already on the device."""
-    from .estimate_motion_optimizer import FUSED_STEPS, LocalMotionProblem
+    from .estimate_motion_optimizer import LocalMotionProblem, fused_steps_apply
     from ._lib import query
 
     prob = LocalMotionProblem.__new__(LocalMotionProblem)
@@ -259,7 +259,7 @@ def _make_patch_shard_problem(spec_sub, centres_norm_sub, base, kind, loss_code,
     prob.base = base
     prob.plan = plan
     prob.tp = spec_sub.shape[1]
-    prob.fused = FUSED_STEPS and loss_code != 2 and bool(query("tmc_local_steps_supported", g, t, resolution[0], resolution[1] * resolution[2]))
+    prob.fused = fused_steps_apply(loss_code, g, t, resolution, plan)
     prob.frame_major = False  # (G, tp, KY, KX): patch-major
     prob.spec = spec_sub
     prob.norms = torch.empty((g, t, 2), dtype=torch.float64, device=dev)

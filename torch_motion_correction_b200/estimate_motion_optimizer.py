@@ -28,6 +28,16 @@ LOSS_TYPES = {"mse": 0, "cc": 1, "ncc": 2}
 FUSED_STEPS = os.environ.get("TMC_FUSED_STEPS", "1") != "0"
 
 
+def fused_steps_apply(loss_type: int, g: int, t: int, resolution, plan) -> bool:
+    """Whether the one-kernel iteration runs this problem: "mse" / "cc" at a size it supports, and for "cc" a band
+    without weight on the self-paired Nyquist bins (``_fourier.self_paired_weight``; the generic kernels take those)."""
+    if not FUSED_STEPS or loss_type == 2:
+        return False
+    if loss_type == 1 and _fourier.self_paired_weight(plan):
+        return False
+    return bool(query("tmc_local_steps_supported", g, t, resolution[0], resolution[1] * resolution[2]))
+
+
 def _setup_optimizer(optimizer_type: str, parameters, **kwargs: Any) -> torch.optim.Optimizer:
     """Same optimisers and defaults as the reference (estimate_motion_optimizer.py:513-608)."""
     name = optimizer_type.lower()
@@ -104,8 +114,7 @@ class LocalMotionProblem:
         self.plan = _fourier.BandPlan(ph, pw, dev, pixel_spacing, b_factor, frequency_range)
         mask, ylo, yhi = _fourier.soft_disc_mask((ph, pw), pw / 4, pw / 4, dev)  # quirk Q18: smoothing pw/4
         self.tp = 2 * ((t + 1) // 2)
-        self.fused = FUSED_STEPS and self.loss_type != 2 and bool(
-            query("tmc_local_steps_supported", self.g, t, self.resolution[0], self.resolution[1] * self.resolution[2]))
+        self.fused = fused_steps_apply(self.loss_type, self.g, t, self.resolution, self.plan)
         # frame-pair jobs; for the tiled path they are listed frame pair by frame pair, so the 50 %-overlapping patches of
         # a pair run back to back and every frame comes from HBM once (patch-major order re-read it 2.3x: ncu)
         self.frame_major = self.fused
