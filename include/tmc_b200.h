@@ -98,6 +98,12 @@ long tmc_warp_workspace_floats(int t, int w, int lh); /* t * 2 * (lh + 3) * w: x
 int tmc_warp_lattice(const float* image, int t, int h, int w, const float* lattice, int lh, int lw, float pixel_spacing,
                      const float* mean_std, float* out_stack, float* out_sum, int accumulate_sum, float* workspace,
                      tmc_stream_t stream);
+/* frame-weighted sums in one pass over the movie: out_sums (n_sums, h, w) = sum_f frame_weights[s][f] * (frame f warped as
+ * by tmc_warp_lattice), frame_weights (n_sums, t) f32.  At most 19 sums per call (3 plain sums + 2 x 8 low-rank dose
+ * components; split larger requests into passes); an all-ones row gives the out_sum of tmc_warp_lattice bit for bit.
+ * workspace: tmc_warp_workspace_floats(t, w, lh) floats. */
+int tmc_warp_lattice_sums(const float* image, int t, int h, int w, const float* lattice, int lh, int lw, float pixel_spacing,
+                          const float* frame_weights, int n_sums, float* out_sums, float* workspace, tmc_stream_t stream);
 /* backward of tmc_warp_lattice w.r.t. the lattice (correct_motion_two_grids, grad=True; correct_motion.py:256-317):
  * grad_out (t,h,w) -> grad_lattice (t,2,lh,lw).  workspace: 2 * tmc_warp_workspace_floats(t, w, lh) floats. */
 int tmc_warp_lattice_backward(const float* image, int t, int h, int w, const float* lattice, int lh, int lw,
@@ -132,6 +138,15 @@ int tmc_band_weights(int ny, int nx, int ky_count, int kx_count, int ky_start, f
 int tmc_dose_weighted_sum(const void* spec, int t, int ny, int nx, float pixel_size, float pre_exposure,
                           float dose_per_frame, float voltage_kv, int frame_offset, void* out, float* den2, int finalize,
                           tmc_stream_t stream);
+
+/* low-rank dose weighting (correct_motion_sums): the normalised weights w_t(k) = q_t(k) / sqrt(sum_t q_t(k)^2) depend on k
+ * only through x = 1 / N_e(k) and are approximated as sum_r U_r(t) v_r(x) with a worst L2 residual over t of 1e-6 (R <= 8
+ * for real exposures).  spec (n_spec, ny, nx/2+1) complex64: spectra of the weighted sums sum_t U_r(t) c_t; table
+ * (n_spec, n_table) f32: v_r of each plane on n_table uniform nodes of x in [0, x_max], linearly interpolated;
+ * plane_outputs (n_spec) int32: bit o set = the plane adds to output o.  out (n_out <= 3, ny, nx/2+1) complex64. */
+int tmc_dose_lowrank_combine(const void* spec, int n_spec, int ny, int nx, float pixel_size, float voltage_kv,
+                             const float* table, int n_table, float x_max, const int* plane_outputs, int n_out, void* out,
+                             tmc_stream_t stream);
 
 /* the same exposure filter q_frame / sqrt(sum_t q_t^2) applied per frame to the band-limited spectra of tmc_rfft2_band
  * (planes 2 job + {0, 1} belong to jobs[job].frame_a / frame_b): additive pre-filter of the patch cross-correlation

@@ -10,6 +10,7 @@ from .correct_motion import (
     correct_motion_fast,
     correct_motion_slow,
     correct_motion_sum,
+    correct_motion_sums,
     correct_motion_two_grids,
     get_pixel_shifts,
 )
@@ -43,6 +44,7 @@ __all__ = [
     "correct_motion_fast",
     "correct_motion_slow",
     "correct_motion_sum",
+    "correct_motion_sums",
     "get_pixel_shifts",
     "evaluate_deformation_field",
     "estimate_global_motion",

@@ -75,20 +75,28 @@ def _max_index_within(n: int, high: float) -> int:
     return int(ok[-1]) if len(ok) else -1
 
 
+def unsupported_lengths(ny: int, nx: int, full: bool) -> str | None:
+    """Why BandPlan(ny, nx, full=full) cannot be built, or None if it can (host query, no CUDA call)."""
+    for n in (ny, nx):
+        kind = query("tmc_fft_supported_length", n)
+        if kind == 0 or (full and kind != 1):
+            return (
+                f"transform length {n} is not supported: the sm_100a FFT kernels take powers of two in [16, 8192], "
+                f"arbitrary lengths up to 4096 and 2..8 times such a length (K3 5760 x 4092, super-resolution "
+                f"11520 x 8184); full-spectrum transforms (correct_motion_fast, dose_weight) of the latter stop at "
+                f"12158 (plus 12288 and 16384), the band-limited ones of the motion estimators at 32768"
+            )
+    return None
+
+
 class BandPlan:
     """Geometry + tables of one band-limited 2-D transform size."""
 
     def __init__(self, ny: int, nx: int, device: torch.device, pixel_spacing: float | None = None,
                  b_factor: float | None = None, frequency_range=None, full: bool = False):
-        for n in (ny, nx):
-            kind = query("tmc_fft_supported_length", n)
-            if kind == 0 or (full and kind != 1):
-                raise NotImplementedError(
-                    f"transform length {n} is not supported: the sm_100a FFT kernels take powers of two in [16, 8192], "
-                    f"arbitrary lengths up to 4096 and 2..8 times such a length (K3 5760 x 4092, super-resolution "
-                    f"11520 x 8184); full-spectrum transforms (correct_motion_fast, dose_weight) of the latter stop at "
-                    f"12158 (plus 12288 and 16384), the band-limited ones of the motion estimators at 32768"
-                )
+        msg = unsupported_lengths(ny, nx, full)
+        if msg:
+            raise NotImplementedError(msg)
         self.ny, self.nx, self.device = ny, nx, device
         self.tw_y, self.tw_x = twiddles(ny, device), twiddles(nx, device)
         if full:

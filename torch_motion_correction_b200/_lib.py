@@ -47,6 +47,7 @@ _SIGNATURES = {
     "tmc_spline_lattice": (I, [P, I, I, I, I, I, P, I, I, I, I, I, I, I, I, I, P, P, P]),
     "tmc_warp_workspace_floats": (L, [I, I, I]),
     "tmc_warp_lattice": (I, [P, I, I, I, P, I, I, F, P, P, P, I, P, P]),
+    "tmc_warp_lattice_sums": (I, [P, I, I, I, P, I, I, F, P, I, P, P, P]),
     "tmc_pixel_shifts": (I, [P, I, I, I, I, F, P, P]),
     "tmc_warp_lattice_backward": (I, [P, I, I, I, P, I, I, F, P, P, P, P]),
     "tmc_lattice_tyx": (I, [I, I, I, I, I, P, P]),
@@ -70,6 +71,7 @@ _SIGNATURES = {
     "tmc_band_weights": (I, [I, I, I, I, I, F, F, I, F, F, I, P, P]),
     "tmc_dose_filter_spectra": (I, [P, P, I, I, I, I, I, I, I, F, F, F, F, P, P]),
     "tmc_dose_weighted_sum": (I, [P, I, I, I, F, F, F, F, I, P, P, I, P]),
+    "tmc_dose_lowrank_combine": (I, [P, I, I, I, F, F, P, I, F, P, I, P, P]),
     "tmc_xc_postprocess": (I, [P, I, I, F, I, I, F, I, I, I, P, P, P]),
     "tmc_global_shifts_to_field": (I, [P, I, F, I, P, P]),
     "tmc_subtract_mean": (I, [P, L, P]),

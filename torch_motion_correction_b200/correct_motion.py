@@ -6,6 +6,7 @@ All arithmetic runs in hand-written sm_100a kernels behind the C ABI (``csrc/war
 
 from __future__ import annotations
 
+import numpy as np
 import torch
 
 from . import _ops
@@ -119,6 +120,140 @@ def correct_motion_sum(
         accumulate = False
     _ops.warp_lattice(movie, lattice, pixel_spacing, out_sum=out, accumulate_sum=accumulate)
     return out
+
+
+#: weighted sums per launch of tmc_warp_lattice_sums (larger requests run in passes over the movie)
+_MAX_SUMS_PER_PASS = 19
+#: bit of each dose-weighted output in the plane masks of tmc_dose_lowrank_combine
+_DOSE_OUTPUTS = ("dose_weighted", "dose_weighted_even", "dose_weighted_odd")
+
+
+def check_sums_arguments(shape, frame_range, dose_per_frame) -> tuple[int, int]:
+    """Validate the host-side arguments of correct_motion_sums (no CUDA call); returns (first, stop)."""
+    if len(shape) != 3:
+        raise ValueError(f"image must be (t, h, w), got {tuple(shape)}")
+    t, h, w = shape
+    first, stop = (0, t) if frame_range is None else (int(frame_range[0]), int(frame_range[1]))
+    if not 0 <= first < stop <= t:
+        raise ValueError(f"frame_range must satisfy 0 <= first < stop <= {t} frames, got {frame_range}")
+    if dose_per_frame is not None:
+        if not dose_per_frame > 0:
+            raise ValueError(f"dose_per_frame must be > 0, got {dose_per_frame}")
+        from ._fourier import unsupported_lengths
+
+        msg = unsupported_lengths(h, w, True)
+        if msg:
+            raise ValueError(msg)
+    return first, stop
+
+
+def warp_sums(movie, field, pixel_spacing, kind, frame_offset, total_frames, half_sets, lowrank, pixel_size=None,
+              voltage=300.0) -> dict:
+    """Frame sums of ``movie`` (frames frame_offset .. of a movie of total_frames) in one pass of the weighted-sum warp
+    (two or more beyond 19 sums), plus the low-rank dose-weighted sums of ``lowrank`` (exposure_filter_lowrank).  Every
+    output is linear in the frames, so sums over blocks of one movie add up to the sums over the movie."""
+    from . import _fourier
+    from ._lib import call, ptr, query, stream_ptr
+
+    dev = movie.device
+    t, h, w = movie.shape
+    frames = np.arange(frame_offset, frame_offset + t)
+    rows, names = [np.ones(t)], ["sum"]
+    if half_sets:
+        rows += [(frames % 2 == 0).astype(np.float64), (frames % 2 == 1).astype(np.float64)]
+        names += ["sum_even", "sum_odd"]
+    n_plain = len(rows)
+    dose_names, masks, tables = [], [], []
+    if lowrank is not None:
+        dose_names = list(_DOSE_OUTPUTS if half_sets else _DOSE_OUTPUTS[:1])
+        for name, g in lowrank.groups.items():
+            mask = {"all": 1, "even": 1 | 2, "odd": 1 | 4}[name]  # the half sets add up to the whole
+            local = g.frames - frame_offset
+            keep = (local >= 0) & (local < t)
+            for r in range(g.basis.shape[1]):
+                row = np.zeros(t)
+                row[local[keep]] = g.basis[keep, r]
+                rows.append(row)
+                masks.append(mask)
+                tables.append(g.table[r])
+    weights = torch.from_numpy(np.stack(rows).astype(np.float32)).to(dev)
+    n_sums = weights.shape[0]
+    gh, gw = field.shape[-2:]
+    lattice = _ops.spline_lattice(field, kind, t, 10 * gh, 10 * gw, frame_offset=frame_offset, total_frames=total_frames)
+    lh, lw = lattice.shape[-2:]
+    ws = torch.empty((query("tmc_warp_workspace_floats", t, w, lh),), dtype=torch.float32, device=dev)
+    sums = torch.empty((n_sums, h, w), dtype=torch.float32, device=dev)
+    with torch.cuda.device(dev):
+        for s0 in range(0, n_sums, _MAX_SUMS_PER_PASS):
+            n = min(_MAX_SUMS_PER_PASS, n_sums - s0)
+            call("tmc_warp_lattice_sums", ptr(movie), t, h, w, ptr(lattice), lh, lw, float(pixel_spacing),
+                 weights.data_ptr() + s0 * t * 4, n, sums.data_ptr() + s0 * h * w * 4, ptr(ws), stream_ptr(dev))
+    # the plain sums are copied out so that the dose planes' memory is freed with `sums`
+    plain = sums[:n_plain].clone() if n_sums > n_plain else sums
+    out = {name: plain[i] for i, name in enumerate(names)}
+    if dose_names:
+        n_planes = n_sums - n_plain
+        plan = _fourier.BandPlan(h, w, dev, full=True)
+        dw = torch.zeros((len(dose_names), h, w), dtype=torch.float32, device=dev)
+        if n_planes:  # no planes: this block holds none of the frames of the filter
+            spec = plan.forward(sums[n_plain:], None, None, 0, h, _fourier.frame_pair_jobs(n_planes, dev), job_mode=2)
+            table = torch.from_numpy(np.stack(tables).astype(np.float32)).to(dev)
+            plane_outputs = torch.tensor(masks, dtype=torch.int32).to(dev)
+            combined = torch.empty((len(dose_names), h, w // 2 + 1, 2), dtype=torch.float32, device=dev)
+            with torch.cuda.device(dev):
+                call("tmc_dose_lowrank_combine", ptr(spec), n_planes, h, w, float(pixel_size), float(voltage), ptr(table),
+                     table.shape[1], float(lowrank.x_max), ptr(plane_outputs), len(dose_names), ptr(combined),
+                     stream_ptr(dev))
+            del spec
+            plan.inverse_full(combined, dw)
+        out.update({name: dw[i] for i, name in enumerate(dose_names)})
+    return out
+
+
+def correct_motion_sums(
+    image: torch.Tensor,
+    deformation_grid: torch.Tensor,
+    pixel_spacing: float,
+    grid_type: str = "catmull_rom",
+    device: torch.device = None,
+    *,
+    dose_per_frame: float | None = None,
+    pre_exposure: float = 0.0,
+    voltage: float = 300.0,
+    half_sets: bool = False,
+    frame_range: tuple[int, int] | None = None,
+) -> dict[str, torch.Tensor]:
+    """Frame sums of the motion-corrected movie, never materialising the corrected stack: {name: (h, w) fp32}.
+
+    * ``"sum"``: ``correct_motion(...).sum(0)``, bit for bit the output of ``correct_motion_sum``;
+    * ``half_sets``: ``"sum_even"`` / ``"sum_odd"`` over the frames of even / odd (0-based, global) index -- the half
+      sets denoisers train on and resolution estimates compare;
+    * ``dose_per_frame`` (e/A^2): ``"dose_weighted"``, the sum ``dose_weight`` forms from the corrected stack (Grant &
+      Grigorieff exposure filter, N_t = pre_exposure + (t + 1) dose_per_frame for global frame index t, the same N_e and
+      200 kV scaling), and with ``half_sets`` also ``"dose_weighted_even"`` / ``"dose_weighted_odd"``.  The halves use
+      the normalisation of all included frames, so dose_weighted_even + dose_weighted_odd == dose_weighted.
+
+    The exposure weights are applied through a low-rank factorisation (``dose_weight.exposure_filter_lowrank``: worst
+    residual 1e-6 per frequency, R <= 8 components for real exposures): R frame-weighted sums formed while warping, R
+    full-frame transforms and one inverse per output, independent of the number of frames.
+
+    ``frame_range=(first, stop)`` restricts every sum to frames first .. stop - 1: only those frames are read, the field
+    is evaluated at their place in the whole movie, exposure still counts all earlier frames and the dose
+    normalisation runs over the included frames."""
+    first, stop = check_sums_arguments(image.shape, frame_range, dose_per_frame)
+    kind = grid_kind(grid_type)
+    dev = resolve_device(image, device)
+    total = image.shape[0]
+    movie = _movie(image[first:stop], dev)
+    field = _field(deformation_grid, dev)
+    lowrank = None
+    if dose_per_frame is not None:
+        from .dose_weight import exposure_filter_lowrank
+
+        h, w = movie.shape[-2:]
+        lowrank = exposure_filter_lowrank(h, w, pixel_spacing, range(first, stop), dose_per_frame, pre_exposure,
+                                          voltage, half_sets)
+    return warp_sums(movie, field, pixel_spacing, kind, first, total, half_sets, lowrank, pixel_spacing, voltage)
 
 
 def get_pixel_shifts(

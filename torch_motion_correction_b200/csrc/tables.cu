@@ -164,6 +164,48 @@ __global__ void dose_filter_spectra_kernel(float2* __restrict__ spec, const int*
   *z = make_float2(v.x * q, v.y * q);
 }
 
+// ---- low-rank dose weighting (dose_weight.exposure_filter_lowrank) -------------------------------------------------------
+// The normalised exposure weights w_t(k) = q_t(k) / sqrt(sum_t q_t(k)^2) depend on k only through x = 1 / N_e(k), and as a
+// (frames x x) matrix they have very low rank: w_t(k) ~= sum_r U_r(t) v_r(x(k)) to 1e-6 (L2 over t) with R <= 8 for real
+// exposures.  spec plane p holds the spectrum of the real-space sum sum_t U_r(t) c_t for one (group, r); table row p holds
+// v_r on a uniform grid of x in [0, x_max].  out[o][bin] = sum over the planes p with bit o of plane_outputs[p] of
+// lerp(table[p], x(k)) * spec[p][bin].  k as in dose_weighted_sum_kernel (same float operations, same N_e).
+constexpr int kMaxLowRankOutputs = 3;
+__global__ void dose_lowrank_combine_kernel(const float2* __restrict__ spec, int n_spec, int ny, int nx, float pixel_size,
+                                            float ne_scale, const float* __restrict__ table, int n_table, float x_max,
+                                            const int* __restrict__ plane_outputs, int n_out, float2* __restrict__ out) {
+  const int kxn = nx / 2 + 1;
+  const int kx = blockIdx.x * blockDim.x + threadIdx.x;
+  const int kyi = blockIdx.y;
+  if (kx >= kxn) return;
+  const int ky = kyi < (ny + 1) / 2 ? kyi : kyi - ny;
+  const float fy = __fmul_rn((float)ky, (float)(1.0 / (double)ny));
+  const float fx = __fmul_rn((float)kx, (float)(1.0 / (double)nx));
+  const float f = __fsqrt_rn(__fadd_rn(__fmul_rn(fy, fy), __fmul_rn(fx, fx)));
+  const float k = fmaxf(__fdiv_rn(f, pixel_size), 1e-10f);
+  const float ne = ne_scale * (0.24499f * powf(k, -1.6649f) + 2.8141f);
+  const float pos = fminf(fmaxf(__fdiv_rn(1.0f, ne) / x_max * (float)(n_table - 1), 0.f), (float)(n_table - 1));
+  const int i = min((int)pos, n_table - 2);
+  const float frac = pos - (float)i;
+  const long bins = (long)ny * kxn, bin = (long)kyi * kxn + kx;
+  float2 acc[kMaxLowRankOutputs];
+#pragma unroll
+  for (int o = 0; o < kMaxLowRankOutputs; ++o) acc[o] = make_float2(0.f, 0.f);
+  for (int p = 0; p < n_spec; ++p) {
+    const float* row = table + (long)p * n_table + i;
+    const float v = fmaf(frac, __ldg(row + 1) - __ldg(row), __ldg(row));
+    const float2 z = spec[p * bins + bin];
+    const int mask = __ldg(plane_outputs + p);
+#pragma unroll
+    for (int o = 0; o < kMaxLowRankOutputs; ++o)
+      if (mask & (1 << o)) {
+        acc[o].x = fmaf(v, z.x, acc[o].x);
+        acc[o].y = fmaf(v, z.y, acc[o].y);
+      }
+  }
+  for (int o = 0; o < n_out; ++o) out[o * bins + bin] = acc[o];
+}
+
 }  // namespace
 
 // Exposure filter of torch_fourier_filter.dose_weight_movie (SURVEY.md A.6) applied per frame to the band-limited
@@ -227,5 +269,26 @@ TMC_API int tmc_band_weights(int ny, int nx, int ky_count, int kx_count, int ky_
   band_weight_kernel<<<grid, 128, 0, stream>>>(ny, nx, ky_count, kx_count, ky_start, low, high, use_band, b_factor,
                                               pixel_size, use_envelope, weight); tmc_count_launch();
   TMC_CHECK_LAUNCH("tmc_band_weights");
+  return TMC_OK;
+}
+
+// spec (n_spec, ny, nx/2+1) complex64 -> out (n_out, ny, nx/2+1) complex64, see dose_lowrank_combine_kernel.  table
+// (n_spec, n_table) f32 and plane_outputs (n_spec) int32 (bit o: the plane adds to output o) are device arrays;
+// n_out <= 3; voltage_kv < 300 uses the 0.8 scaling of N_e.
+TMC_API int tmc_dose_lowrank_combine(const void* spec, int n_spec, int ny, int nx, float pixel_size, float voltage_kv,
+                                     const float* table, int n_table, float x_max, const int* plane_outputs, int n_out,
+                                     void* out, cudaStream_t stream) {
+  TMC_CHECK_ARG(spec && table && plane_outputs && out, "dose_lowrank_combine: null pointer");
+  TMC_CHECK_ARG(n_spec >= 1 && ny >= 1 && nx >= 2 && n_table >= 2, "dose_lowrank_combine: bad shape n_spec=%d ny=%d nx=%d "
+                "n_table=%d", n_spec, ny, nx, n_table);
+  TMC_CHECK_ARG(n_out >= 1 && n_out <= kMaxLowRankOutputs, "dose_lowrank_combine: n_out=%d outside [1, %d]", n_out,
+                kMaxLowRankOutputs);
+  TMC_CHECK_ARG(pixel_size > 0.f && x_max > 0.f, "dose_lowrank_combine: pixel_size and x_max must be > 0");
+  dim3 grid(tmc_div_up(nx / 2 + 1, 128), ny);
+  TMC_TIMED("dose_lowrank_combine_kernel", stream,
+            dose_lowrank_combine_kernel<<<grid, 128, 0, stream>>>((const float2*)spec, n_spec, ny, nx, pixel_size,
+                                                                 voltage_kv >= 300.f ? 1.0f : 0.8f, table, n_table, x_max,
+                                                                 plane_outputs, n_out, (float2*)out));
+  TMC_CHECK_LAUNCH("tmc_dose_lowrank_combine");
   return TMC_OK;
 }

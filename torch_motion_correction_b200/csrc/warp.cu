@@ -1,7 +1,8 @@
 // Deformation-field warp of a movie stack: per-pixel bicubic lookup of the per-frame shift
 // lattice (reflection padding) followed by a bicubic gather of the frame (border-clamped
 // taps, zero outside), either written as a (t,h,w) stack or accumulated over frames into one
-// (h,w) sum without materialising the warped stack.
+// (h,w) sum without materialising the warped stack, or accumulated into several frame-weighted (h,w) sums at once
+// (tmc_warp_lattice_sums: half-set and low-rank dose-weighted sums).
 //
 // Replaces the reference's correct_motion.py:81-185 (`_correct_frame`, `get_pixel_shifts`) and
 // torch_image_interpolation.sample_image_2d / F.grid_sample(bicubic, align_corners=True)
@@ -222,25 +223,89 @@ __device__ __noinline__ float warp_pixel_generic(const float* __restrict__ image
   return acc;
 }
 
+// ---- frame-weighted sums: out_sums[s] = sum_f weights[s][f] * warped frame f --------------------------------------------
+// Per sum, a thread keeps the accumulators of its kRows (= 4) pixels as one float4 in thread-private shared memory
+// (acc[s * stride]): up to kMaxSums of them would not fit the 128-register budget of the warp kernels.  With a weight of
+// exactly 1, fmaf(1, v, a) == a + v, so an all-ones row reproduces the plain frame sum bit for bit.
+constexpr int kMaxSums = 19;  // per launch (tmc_warp_lattice_sums); the caller splits larger requests into passes
+
+__device__ __forceinline__ void zero_sums(float4* acc, int stride, int n_sums) {
+  for (int s = 0; s < n_sums; ++s) acc[s * stride] = make_float4(0.f, 0.f, 0.f, 0.f);
+}
+__device__ __forceinline__ void accumulate_sums(float4* acc, int stride, const float* __restrict__ weights, int T, int f,
+                                                int n_sums, const float (&v)[4]) {
+  const float* wf = weights + f;
+  for (int s = 0; s < n_sums; ++s, wf += T, acc += stride) {
+    const float ws = __ldg(wf);
+    float4 a = *acc;
+    a.x = fmaf(ws, v[0], a.x);
+    a.y = fmaf(ws, v[1], a.y);
+    a.z = fmaf(ws, v[2], a.z);
+    a.w = fmaf(ws, v[3], a.w);
+    *acc = a;
+  }
+}
+__device__ __forceinline__ void store_sums(const float4* acc, int stride, int n_sums, float* __restrict__ out, int H, int W,
+                                           int x, int y_base, int y_end) {
+  for (int s = 0; s < n_sums; ++s) {
+    const float4 a = acc[s * stride];
+    const float v[4] = {a.x, a.y, a.z, a.w};
+#pragma unroll
+    for (int r = 0; r < 4; ++r)
+      if (y_base + r < y_end) out[((size_t)s * H + y_base + r) * W + x] = v[r];
+  }
+}
+
+// warp_pixel_generic for the weighted sums: acc points at the pixel's component of the thread's float4 of sum 0
+__device__ __noinline__ void warp_pixel_generic_sums(const float* __restrict__ image, int T, int H, int W,
+                                                     const float* __restrict__ rx, int lh, float inv_px,
+                                                     const float* __restrict__ weights, int n_sums, float* acc, int stride,
+                                                     int x, int y) {
+  const LatticeAxis a = lattice_axis(y, H, lh);
+  const size_t rx_plane = (size_t)(lh + kRxPad) * W;
+  for (int f = 0; f < T; ++f) {
+    const float* Ry = rx + (size_t)f * 2 * rx_plane + x + 2 * W;
+    const float* Rx = Ry + W;
+    float sy = a.w[0] * __ldg(Ry + (size_t)a.j[0] * 2 * W), sx = a.w[0] * __ldg(Rx + (size_t)a.j[0] * 2 * W);
+#pragma unroll
+    for (int k = 1; k < 4; ++k) {
+      sy = fmaf(a.w[k], __ldg(Ry + (size_t)a.j[k] * 2 * W), sy);
+      sx = fmaf(a.w[k], __ldg(Rx + (size_t)a.j[k] * 2 * W), sx);
+    }
+    const float cy = __fadd_rn((float)y, __fmul_rn(sy, inv_px));
+    const float cx = __fadd_rn((float)x, __fmul_rn(sx, inv_px));
+    const float v = gather_border(image + (size_t)f * H * W, H, W, cy, cx);
+    for (int s = 0; s < n_sums; ++s) acc[s * stride] = fmaf(__ldg(weights + (size_t)s * T + f), v, acc[s * stride]);
+  }
+}
+
 // Stage 2: one thread = kRows vertically adjacent output pixels of one column; the coordinate chain of a pixel
 // (Angstrom -> px, grid_sample round trip, cubic weights) runs on both axes at once as packed fp32x2 arithmetic
 // and the 8 lattice taps of a frame are shared by the thread's pixels.
 // measured alternatives on B200 (C2, fused sum): 4 rows per thread at 128 registers (2 CTAs per SM) 4.3 ms (4.1 ms with
 // the shared tap rows); capped at 80 registers (3 CTAs per SM) 5.4 ms (4.9 ms with shared tap rows); 2 rows per thread 4.6-4.8 ms; uncapped registers (1 CTA per SM) 6.2 ms;
 // prefetch.global.L2 of the next frame's rows +2 %
-template <bool WRITE_STACK, bool WRITE_SUM, bool NORMALISE>
+template <bool WRITE_STACK, bool WRITE_SUM, bool NORMALISE, bool WEIGHTED = false>
 #ifndef TMC_WARP_MINB
 #define TMC_WARP_MINB 2
 #endif
-__global__ void __launch_bounds__(kTileX* kTileYGroups, TMC_WARP_MINB)
+// (the weighted sums keep no sum in registers but load the weights: at 2 CTAs per SM they would spill, so 1)
+__global__ void __launch_bounds__(kTileX* kTileYGroups, WEIGHTED ? 1 : TMC_WARP_MINB)
 warp_lattice_kernel(const float* __restrict__ image, int T, int H, int W, const float* __restrict__ rx, int lh,
                     float pixel_spacing, const float* __restrict__ mean_std, float* __restrict__ out_stack,
-                    float* __restrict__ out_sum, int accumulate_sum, int x_begin, int x_end, int y_begin, int y_end) {
+                    float* __restrict__ out_sum, int accumulate_sum, int x_begin, int x_end, int y_begin, int y_end,
+                    const float* __restrict__ weights, int n_sums, float* __restrict__ out_sums) {
   // the launch covers the output rectangle [x_begin, x_end) x [y_begin, y_end)
   const int x = x_begin + blockIdx.x * kTileX + threadIdx.x;
   const int y_base = y_begin + (blockIdx.y * kTileYGroups + threadIdx.y) * kRows;
   if (x >= x_end || y_base >= y_end) return;
   const int y_last = y_end - 1;
+  // WEIGHTED: n_sums float4 accumulators per thread (dynamic shared memory, stride = threads per CTA)
+  static_assert(!WEIGHTED || (kRows == 4 && !WRITE_STACK && !WRITE_SUM && !NORMALISE), "weighted sums: 4 rows, no other output");
+  extern __shared__ float4 sums_smem[];
+  constexpr int kSumStride = kTileX * kTileYGroups;
+  float4* const sums_acc = sums_smem + threadIdx.y * kTileX + threadIdx.x;
+  if constexpr (WEIGHTED) zero_sums(sums_acc, kSumStride, n_sums);
 
   // lattice taps along y: rows of RX (offsets in floats) and duplicated weights per pixel
   int jy[4];
@@ -270,6 +335,13 @@ warp_lattice_kernel(const float* __restrict__ image, int T, int H, int W, const 
   for (int r = 0; r < kRows; ++r) acc[r] = 0.f;
   if (!same_cell) {
     // the rows of this thread straddle a lattice cell (warp-uniform, ~kRows in every H / lh rows)
+    if constexpr (WEIGHTED) {
+      for (int r = 0; r < kRows && y_base + r < y_end; ++r)
+        warp_pixel_generic_sums(image, T, H, W, rx, lh, 1.0f / pixel_spacing, weights, n_sums,
+                                reinterpret_cast<float*>(sums_acc) + r, 4 * kSumStride, x, y_base + r);
+      store_sums(sums_acc, kSumStride, n_sums, out_sums, H, W, x, y_base, y_end);
+      return;
+    }
     for (int r = 0; r < kRows; ++r) {
       const int y = y_base + r;
       if (y >= y_end) break;
@@ -404,7 +476,9 @@ warp_lattice_kernel(const float* __restrict__ image, int T, int H, int W, const 
         if (WRITE_SUM) acc[r] += o;
       }
     }
+    if constexpr (WEIGHTED) accumulate_sums(sums_acc, kSumStride, weights, T, f, n_sums, v);
   }
+  if constexpr (WEIGHTED) store_sums(sums_acc, kSumStride, n_sums, out_sums, H, W, x, y_base, y_end);
   if (WRITE_SUM) {
 #pragma unroll
     for (int r = 0; r < kRows; ++r) {
@@ -585,15 +659,11 @@ TMC_API long tmc_warp_workspace_floats(int t, int w, int lh) { return (long)t * 
 // (v - mean) / std applied to the warped value, zero outside); out_stack (t,h,w) nullable;
 // out_sum (h,w) nullable; accumulate_sum != 0 adds to out_sum; workspace:
 // tmc_warp_workspace_floats(t, w, lh) floats.
-TMC_API int tmc_warp_lattice(const float* image, int t, int h, int w, const float* lattice, int lh, int lw,
-                             float pixel_spacing, const float* mean_std, float* out_stack, float* out_sum,
-                             int accumulate_sum, float* workspace, cudaStream_t stream) {
-  TMC_CHECK_ARG(image && lattice && workspace, "warp_lattice: null pointer");
-  TMC_CHECK_ARG(out_stack || out_sum, "warp_lattice: need out_stack and/or out_sum");
-  TMC_CHECK_ARG(t >= 1 && h >= 2 && w >= 2 && lh >= 1 && lw >= 1, "warp_lattice: bad shape t=%d h=%d w=%d lattice=%dx%d", t,
-                h, w, lh, lw);
-  TMC_CHECK_ARG(pixel_spacing > 0.f, "warp_lattice: pixel_spacing must be > 0");
-  TMC_CHECK_ARG((long)(lh + kRxPad) * w < (1l << 31), "warp_lattice: lattice rows x width overflows int");
+// shared by tmc_warp_lattice and tmc_warp_lattice_sums (weights != nullptr: the weighted sums, arguments validated)
+static int warp_lattice_launch(const float* image, int t, int h, int w, const float* lattice, int lh, int lw,
+                               float pixel_spacing, const float* mean_std, float* out_stack, float* out_sum,
+                               int accumulate_sum, const float* weights, int n_sums, float* out_sums, float* workspace,
+                               cudaStream_t stream) {
   {
     // every thread sets up its column's taps once (two divisions) and then walks over rows: few, long-lived CTAs
     long rows = (long)t * 2 * (lh + kRxPad);
@@ -613,8 +683,9 @@ TMC_API int tmc_warp_lattice(const float* image, int t, int h, int w, const floa
     const bool ok = tma::make_map_3d(&img_map, image, (uint64_t)w, (uint64_t)h, (uint64_t)t, tma::kBoxW, tma::kBoxH, 1) &&
                     tma::make_map_3d(&rx_map, workspace, (uint64_t)w, 2, (uint64_t)t * (lh + kRxPad), tma::kTX, 2,
                                      (uint32_t)tma::staged_lattice_rows(h, lh));
-    if (ok) {
-      tma::Params prm;
+    if (ok && (!weights || (tma::kMaxSmemBytes - 128 - n_sums * tma::kConsumers * (int)sizeof(float4)) /
+                                   tma::stage_bytes_for(tma::staged_lattice_rows(h, lh)) >= 2)) {
+      tma::SumsParams prm;  // passed as tma::Params to all but the weighted instantiation
       prm.image = image;
       prm.T = t;
       prm.H = h;
@@ -624,11 +695,19 @@ TMC_API int tmc_warp_lattice(const float* image, int t, int h, int w, const floa
       prm.rx_rows = tma::staged_lattice_rows(h, lh);
       prm.stage_bytes = tma::stage_bytes_for(prm.rx_rows);
       prm.n_stages = tma::stages_for(prm.rx_rows);
+      prm.weights = weights;
+      prm.n_sums = n_sums;
+      prm.out_sums = out_sums;
+      prm.acc_bytes = weights ? n_sums * tma::kConsumers * (int)sizeof(float4) : 0;
+      if (weights) {  // the accumulators take shared memory from the ring
+        const int n = (tma::kMaxSmemBytes - 128 - prm.acc_bytes) / prm.stage_bytes;
+        if (n < prm.n_stages) prm.n_stages = n;
+      }
       if (const char* e = getenv("TMC_WARP_TMA_STAGES")) {  // experiment: shallower ring
         const int v = atoi(e);
         if (v >= 2 && v < prm.n_stages) prm.n_stages = v;
       }
-      const size_t smem_bytes = (size_t)prm.n_stages * prm.stage_bytes + 128;  // + alignment slack
+      const size_t smem_bytes = (size_t)prm.acc_bytes + (size_t)prm.n_stages * prm.stage_bytes + 128;  // + alignment slack
       prm.pixel_spacing = pixel_spacing;
       prm.mean_std = mean_std;
       prm.out_stack = out_stack;
@@ -653,7 +732,13 @@ TMC_API int tmc_warp_lattice(const float* image, int t, int h, int w, const floa
     tma::warp_tma_kernel<S, A, N><<<grid, tma::kThreads, smem_bytes, stream>>>(img_map, rx_map, prm);                         \
     tmc_timing_end("warp_tma_kernel", stream);                                                                               \
   }
-      if (s && a && n) LAUNCH_TMA(true, true, true)
+      if (weights) {
+        TMC_CUDA(cudaFuncSetAttribute(tma::warp_tma_kernel<false, false, false, true>,
+                                      cudaFuncAttributeMaxDynamicSharedMemorySize, tma::kMaxSmemBytes));
+        tmc_timing_begin(stream);
+        tma::warp_tma_kernel<false, false, false, true><<<grid, tma::kThreads, smem_bytes, stream>>>(img_map, rx_map, prm);
+        tmc_timing_end("warp_tma_kernel_sums", stream);
+      } else if (s && a && n) LAUNCH_TMA(true, true, true)
       else if (s && a) LAUNCH_TMA(true, true, false)
       else if (s && n) LAUNCH_TMA(true, false, true)
       else if (s) LAUNCH_TMA(true, false, false)
@@ -668,10 +753,21 @@ TMC_API int tmc_warp_lattice(const float* image, int t, int h, int w, const floa
   {
     dim3 block(kTileX, kTileYGroups);
     dim3 grid(tmc_div_up(w, kTileX), tmc_div_up(h, kTileYGroups * kRows));
+    if (weights) {
+      const int smem = n_sums * kTileX * kTileYGroups * (int)sizeof(float4);
+      TMC_CUDA(cudaFuncSetAttribute(warp_lattice_kernel<false, false, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                    smem));
+      TMC_TIMED("warp_lattice_kernel_sums", stream,
+                warp_lattice_kernel<false, false, false, true><<<grid, block, smem, stream>>>(
+                    image, t, h, w, workspace, lh, pixel_spacing, nullptr, nullptr, nullptr, 0, 0, w, 0, h, weights, n_sums,
+                    out_sums));
+      TMC_CHECK_LAUNCH("tmc_warp_lattice_sums");
+      return TMC_OK;
+    }
     tmc_timing_begin(stream);
 #define LAUNCH(S, A, N)                                                                                          \
   warp_lattice_kernel<S, A, N><<<grid, block, 0, stream>>>(image, t, h, w, workspace, lh, pixel_spacing, mean_std, \
-                                                           out_stack, out_sum, accumulate_sum, 0, w, 0, h)
+                                                           out_stack, out_sum, accumulate_sum, 0, w, 0, h, nullptr, 0, nullptr)
     if (s && a && n) LAUNCH(true, true, true);
     else if (s && a) LAUNCH(true, true, false);
     else if (s && n) LAUNCH(true, false, true);
@@ -684,6 +780,35 @@ TMC_API int tmc_warp_lattice(const float* image, int t, int h, int w, const floa
   }
   TMC_CHECK_LAUNCH("tmc_warp_lattice");
   return TMC_OK;
+}
+
+TMC_API int tmc_warp_lattice(const float* image, int t, int h, int w, const float* lattice, int lh, int lw,
+                             float pixel_spacing, const float* mean_std, float* out_stack, float* out_sum,
+                             int accumulate_sum, float* workspace, cudaStream_t stream) {
+  TMC_CHECK_ARG(image && lattice && workspace, "warp_lattice: null pointer");
+  TMC_CHECK_ARG(out_stack || out_sum, "warp_lattice: need out_stack and/or out_sum");
+  TMC_CHECK_ARG(t >= 1 && h >= 2 && w >= 2 && lh >= 1 && lw >= 1, "warp_lattice: bad shape t=%d h=%d w=%d lattice=%dx%d", t,
+                h, w, lh, lw);
+  TMC_CHECK_ARG(pixel_spacing > 0.f, "warp_lattice: pixel_spacing must be > 0");
+  TMC_CHECK_ARG((long)(lh + kRxPad) * w < (1l << 31), "warp_lattice: lattice rows x width overflows int");
+  return warp_lattice_launch(image, t, h, w, lattice, lh, lw, pixel_spacing, mean_std, out_stack, out_sum, accumulate_sum,
+                             nullptr, 0, nullptr, workspace, stream);
+}
+
+// out_sums (n_sums, h, w) = sum_f frame_weights[s][f] * (frame f warped as by tmc_warp_lattice); frame_weights (n_sums, t)
+// f32 device; 1 <= n_sums <= 19 (kMaxSums); workspace: tmc_warp_workspace_floats(t, w, lh) floats.
+TMC_API int tmc_warp_lattice_sums(const float* image, int t, int h, int w, const float* lattice, int lh, int lw,
+                                  float pixel_spacing, const float* frame_weights, int n_sums, float* out_sums,
+                                  float* workspace, cudaStream_t stream) {
+  TMC_CHECK_ARG(image && lattice && frame_weights && out_sums && workspace, "warp_lattice_sums: null pointer");
+  TMC_CHECK_ARG(n_sums >= 1 && n_sums <= kMaxSums, "warp_lattice_sums: n_sums=%d outside [1, %d] (split into passes)", n_sums,
+                kMaxSums);
+  TMC_CHECK_ARG(t >= 1 && h >= 2 && w >= 2 && lh >= 1 && lw >= 1, "warp_lattice_sums: bad shape t=%d h=%d w=%d lattice=%dx%d",
+                t, h, w, lh, lw);
+  TMC_CHECK_ARG(pixel_spacing > 0.f, "warp_lattice_sums: pixel_spacing must be > 0");
+  TMC_CHECK_ARG((long)(lh + kRxPad) * w < (1l << 31), "warp_lattice_sums: lattice rows x width overflows int");
+  return warp_lattice_launch(image, t, h, w, lattice, lh, lw, pixel_spacing, nullptr, nullptr, nullptr, 0, frame_weights,
+                             n_sums, out_sums, workspace, stream);
 }
 
 TMC_API int tmc_pixel_shifts(const float* lattice, int lh, int lw, int h, int w, float pixel_spacing, float* out,

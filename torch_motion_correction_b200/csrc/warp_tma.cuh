@@ -15,8 +15,11 @@
 //     through its "empty" mbarrier.  No block-wide barrier in the frame loop; frame sums live in registers.
 //   Pixels whose taps leave the box (shift varying by more than the 4-px margin inside one tile) or touch the image
 //   border (border-clamped taps / zero outside) take the generic global-memory path.
+// The WEIGHTED instantiation forms n_sums frame-weighted sums at once (tmc_warp_lattice_sums): the accumulators of a
+// thread's 4 pixels are one float4 per sum in thread-private shared memory, in front of the (then shallower) ring.
 #pragma once
 #include <cuda.h>
+#include <type_traits>
 
 namespace tma {
 
@@ -170,10 +173,20 @@ struct Params {
   float2 nden, rcp, half_scale;  // .x = y axis, .y = x axis
   float inv_px;
 };
+// the weighted instantiation's parameters (a separate type: growing Params changes the register allocation of the others)
+struct SumsParams : Params {
+  const float* weights;  // (n_sums, T) frame weights
+  int n_sums;
+  float* out_sums;  // (n_sums, H, W)
+  int acc_bytes;    // shared-memory accumulators in front of the ring: n_sums * kConsumers float4s
+};
+template <bool WEIGHTED>
+using KernelParams = typename std::conditional<WEIGHTED, SumsParams, Params>::type;
 
-template <bool WRITE_STACK, bool WRITE_SUM, bool NORMALISE>
+template <bool WRITE_STACK, bool WRITE_SUM, bool NORMALISE, bool WEIGHTED = false>
 __global__ void __launch_bounds__(kThreads, 1)
-warp_tma_kernel(const __grid_constant__ CUtensorMap img_map, const __grid_constant__ CUtensorMap rx_map, const Params p) {
+warp_tma_kernel(const __grid_constant__ CUtensorMap img_map, const __grid_constant__ CUtensorMap rx_map,
+                const KernelParams<WEIGHTED> p) {
   extern __shared__ unsigned char smem_raw[];
   __shared__ __align__(8) uint64_t full_bar[kMaxStages];
   __shared__ __align__(8) uint64_t empty_bar[kMaxStages];
@@ -182,6 +195,12 @@ warp_tma_kernel(const __grid_constant__ CUtensorMap img_map, const __grid_consta
   // box AND inside the image (the zero-filled part of a box that hangs over the frame edge is never used)
   __shared__ __align__(16) int stage_hdr[kMaxStages][8];
   unsigned char* stages = smem_raw + ((128u - (smem_u32(smem_raw) & 127u)) & 127u);
+  static_assert(!WEIGHTED || (kRows == 4 && !WRITE_STACK && !WRITE_SUM && !NORMALISE), "weighted sums: 4 rows, no other output");
+  float4* sums_acc = nullptr;
+  if constexpr (WEIGHTED) {
+    sums_acc = reinterpret_cast<float4*>(stages);
+    stages += p.acc_bytes;
+  }
   const int tid = threadIdx.x;
   const int T = p.T, H = p.H, W = p.W, lh = p.lh;
   const int lhp = lh + 3;
@@ -319,6 +338,7 @@ warp_tma_kernel(const __grid_constant__ CUtensorMap img_map, const __grid_consta
     float acc[kRows];
 #pragma unroll
     for (int r = 0; r < kRows; ++r) acc[r] = 0.f;
+    if constexpr (WEIGHTED) zero_sums(sums_acc + tid, kConsumers, p.n_sums);
 
     // the frame loop, specialised on whether the thread's 4 rows read the same lattice rows (warp-uniform, true for all
     // but the few row groups that straddle a lattice cell boundary): no branch inside the coordinate arithmetic, so
@@ -452,6 +472,7 @@ warp_tma_kernel(const __grid_constant__ CUtensorMap img_map, const __grid_consta
           if (WRITE_STACK && y_base + r < H) p.out_stack[((size_t)f * H + y_base + r) * W + x] = o;
           if (WRITE_SUM) acc[r] += o;
         }
+        if constexpr (WEIGHTED) accumulate_sums(sums_acc + tid, kConsumers, p.weights, T, f, p.n_sums, v);
       }
       __syncwarp();
       if (lane == 0) mbar_arrive_addr(empty0 + 8u * stage);
@@ -471,6 +492,7 @@ warp_tma_kernel(const __grid_constant__ CUtensorMap img_map, const __grid_consta
         }
       }
     }
+    if constexpr (WEIGHTED) if (active) store_sums(sums_acc + tid, kConsumers, p.n_sums, p.out_sums, H, W, x, y_base, H);
   }
 }
 

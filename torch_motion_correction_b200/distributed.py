@@ -139,6 +139,41 @@ def correct_motion_sum_frame_split(local_frames, deformation_grid, pixel_spacing
     return total
 
 
+def correct_motion_sums_frame_split(local_frames, deformation_grid, pixel_spacing, frame_offset, total_frames,
+                                    grid_type="catmull_rom", *, dose_per_frame=None, pre_exposure=0.0, voltage=300.0,
+                                    half_sets=False, group=None, device=None) -> dict:
+    """``correct_motion_sums`` of a movie whose frames [frame_offset, frame_offset + t_local) live on this rank: every
+    rank forms its frames' sums with the exposure filter of the WHOLE movie (factorised on the first rank of ``group``
+    and broadcast, so that all ranks use the same tables) and the (h, w) outputs are all-reduced.  Every output is linear
+    in the frames, so the partial sums add up to the single-process result."""
+    from .correct_motion import _field, _movie, check_sums_arguments, warp_sums
+    from .dose_weight import exposure_filter_lowrank
+
+    dev = resolve_device(local_frames, device)
+    check_sums_arguments(local_frames.shape, None, dose_per_frame)
+    if not (0 <= frame_offset and frame_offset + local_frames.shape[0] <= total_frames):
+        raise ValueError(f"frames [{frame_offset}, {frame_offset + local_frames.shape[0]}) outside a movie of {total_frames}")
+    movie = _movie(local_frames, dev)
+    field = _field(deformation_grid, dev)
+    rank, world = _world(group)
+    lowrank = None
+    if dose_per_frame is not None:
+        if rank == 0:
+            h, w = movie.shape[-2:]
+            lowrank = exposure_filter_lowrank(h, w, pixel_spacing, range(total_frames), dose_per_frame, pre_exposure,
+                                              voltage, half_sets)
+        if world > 1:
+            box = [lowrank]
+            dist.broadcast_object_list(box, src=dist.get_global_rank(group, 0) if group is not None else 0, group=group)
+            lowrank = box[0]
+    out = warp_sums(movie, field, pixel_spacing, grid_kind(grid_type), frame_offset, total_frames, half_sets, lowrank,
+                    pixel_spacing, voltage)
+    if world > 1:
+        for name in sorted(out):
+            dist.all_reduce(out[name], op=dist.ReduceOp.SUM, group=group)
+    return out
+
+
 def estimate_global_motion_frame_split(local_frames, pixel_spacing, frame_offset, total_frames, mean_std,
                                        reference_frame=None, b_factor=500, frequency_range=(300, 10), group=None):
     """``estimate_global_motion`` for a frame-split movie: the owner of the reference frame
