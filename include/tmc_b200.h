@@ -71,6 +71,10 @@ int tmc_remove_hot_pixels(float* stack, int t, int h, int w, double* moments, fl
                           int* hot_count, tmc_stream_t stream);
 /* every frame minus its own mean (moments[f][0] / n), in place */
 int tmc_subtract_frame_means(float* stack, int t, long n, const double* moments, tmc_stream_t stream);
+/* frame grouping (MotionCor2 -Group, RELION "group frames"): movie (t, h, w) -> groups (t / frame_group, h, w), the sums
+ * of frame_group consecutive frames; the last group also takes the t % frame_group leftover frames.  At least 2 groups.
+ * Each sum is movie[first] + movie[first + 1] + ... added left to right in fp32 (one rounding per add, no reordering). */
+int tmc_group_frames(const float* movie, int t, int h, int w, int frame_group, float* groups, tmc_stream_t stream);
 
 /* ---- cubic spline grids: torch_cubic_spline_grids.Cubic{CatmullRom,BSpline}Grid3d as used at
  *      deformation_field_utils.py:9-93, estimate_motion_optimizer.py:487-490, correct_motion.py:288-305 */
@@ -88,6 +92,11 @@ int tmc_spline_eval_backward(int c, int n0, int n1, int n2, int kind, const floa
 int tmc_spline_lattice(const float* coeffs, int c, int n0, int n1, int n2, int kind, const float* coeffs2, int m0, int m1,
                        int m2, int kind2, int n_frames, int frame_offset, int total_frames, int lh, int lw, float* lattice,
                        float* workspace, tmc_stream_t stream);
+/* tmc_spline_lattice at t = times[f] (device, n_frames floats): a field estimated on frame-group sums evaluated at the
+ * raw frames.  Times outside [0, 1] extend the end interval's cubic (the interval index is clamped, t is not). */
+int tmc_spline_lattice_times(const float* coeffs, int c, int n0, int n1, int n2, int kind, const float* coeffs2, int m0,
+                             int m1, int m2, int kind2, int n_frames, const float* times, int lh, int lw, float* lattice,
+                             float* workspace, tmc_stream_t stream);
 
 /* ---- warp: correct_motion.py:81-185 (_correct_frame, get_pixel_shifts) + sample_image_2d -------- */
 long tmc_warp_workspace_floats(int t, int w, int lh); /* t * 2 * (lh + 3) * w: x-interpolated lattice, reflection-padded rows */

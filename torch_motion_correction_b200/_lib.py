@@ -41,10 +41,12 @@ _SIGNATURES = {
     "tmc_hot_pixel_workspace_bytes": (L, [I]),
     "tmc_remove_hot_pixels": (I, [P, I, I, I, P, F, I, P, P, P]),
     "tmc_subtract_frame_means": (I, [P, I, L, P, P]),
+    "tmc_group_frames": (I, [P, I, I, I, I, P, P]),
     "tmc_spline_workspace_floats": (L, [I, I, I, I]),
     "tmc_spline_eval": (I, [P, I, I, I, I, I, P, L, P, P, P]),
     "tmc_spline_eval_backward": (I, [I, I, I, I, I, P, L, P, F, P, P, P]),
     "tmc_spline_lattice": (I, [P, I, I, I, I, I, P, I, I, I, I, I, I, I, I, I, P, P, P]),
+    "tmc_spline_lattice_times": (I, [P, I, I, I, I, I, P, I, I, I, I, I, P, I, I, P, P, P]),
     "tmc_warp_workspace_floats": (L, [I, I, I]),
     "tmc_warp_lattice": (I, [P, I, I, I, P, I, I, F, P, P, P, I, P, P]),
     "tmc_warp_lattice_sums": (I, [P, I, I, I, P, I, I, F, P, I, P, P, P]),

@@ -73,8 +73,9 @@ def spline_eval_backward(shape, kind: int, tyx: torch.Tensor, grad_out: torch.Te
     return grad
 
 
-def spline_lattice(coeffs, kind, n_frames, lh, lw, coeffs2=None, kind2=0, frame_offset=0, total_frames=None):
-    """(n_frames, c, lh, lw) lattice of the field at t = linspace(0,1,total)[offset + f]."""
+def spline_lattice(coeffs, kind, n_frames, lh, lw, coeffs2=None, kind2=0, frame_offset=0, total_frames=None, times=None):
+    """(n_frames, c, lh, lw) lattice of the field at t = linspace(0,1,total)[offset + f], or at t = times[f] when
+    ``times`` (device float32 (n_frames,)) is given."""
     c, n0, n1, n2 = coeffs.shape
     total = n_frames if total_frames is None else total_frames
     n_ws = query("tmc_spline_workspace_floats", c, n0, n1, n2)
@@ -85,9 +86,25 @@ def spline_lattice(coeffs, kind, n_frames, lh, lw, coeffs2=None, kind2=0, frame_
     ws = _f32((n_ws,), coeffs)
     lattice = _f32((n_frames, c, lh, lw), coeffs)
     with torch.cuda.device(coeffs.device):
-        call("tmc_spline_lattice", ptr(coeffs), c, n0, n1, n2, kind, ptr(coeffs2), m0, m1, m2, kind2, n_frames,
-             frame_offset, total, lh, lw, ptr(lattice), ptr(ws), stream_ptr(coeffs.device))
+        if times is None:
+            call("tmc_spline_lattice", ptr(coeffs), c, n0, n1, n2, kind, ptr(coeffs2), m0, m1, m2, kind2, n_frames,
+                 frame_offset, total, lh, lw, ptr(lattice), ptr(ws), stream_ptr(coeffs.device))
+        else:
+            if times.shape != (n_frames,) or times.dtype != torch.float32 or times.device != coeffs.device or \
+                    not times.is_contiguous():
+                raise ValueError(f"times must be a contiguous float32 ({n_frames},) tensor on {coeffs.device}")
+            call("tmc_spline_lattice_times", ptr(coeffs), c, n0, n1, n2, kind, ptr(coeffs2), m0, m1, m2, kind2, n_frames,
+                 ptr(times), lh, lw, ptr(lattice), ptr(ws), stream_ptr(coeffs.device))
     return lattice
+
+
+def group_frames(movie, frame_group):
+    """(n_groups, h, w) sums of frame_group consecutive frames of a contiguous fp32 device movie (tmc_group_frames)."""
+    t, h, w = movie.shape
+    out = _f32((t // frame_group, h, w), movie)
+    with torch.cuda.device(movie.device):
+        call("tmc_group_frames", ptr(movie), t, h, w, int(frame_group), ptr(out), stream_ptr(movie.device))
+    return out
 
 
 def warp_lattice(image, lattice, pixel_spacing, mean_std=None, out_stack=None, out_sum=None, accumulate_sum=False):

@@ -11,6 +11,7 @@ import torch
 
 from . import _ops
 from ._common import as_f32, grid_kind, resolve_device
+from .frame_groups import frame_groups
 
 
 def _movie(image: torch.Tensor, dev: torch.device) -> torch.Tensor:
@@ -25,6 +26,28 @@ def _field(deformation_grid: torch.Tensor, dev: torch.device) -> torch.Tensor:
     return as_f32(deformation_grid, dev)
 
 
+def _frame_times(frame_group, total, first, stop, dev):
+    """Device float32 time of each of the frames first .. stop - 1 of a ``total``-frame movie on the time axis of a field
+    estimated with ``estimate_motion(..., frame_group=...)`` (``frame_groups``); None without grouping (None or 1)."""
+    if frame_group is None:
+        return None
+    groups = frame_groups(total, frame_group)
+    if groups.group_size == 1:
+        return None
+    if not 0 <= first < stop <= total:
+        raise ValueError(f"frames [{first}, {stop}) outside a movie of {total}")
+    return torch.from_numpy(groups.times[first:stop]).to(dev)
+
+
+def _lattice(field, kind, n_frames, frame_offset=0, total_frames=None, frame_group=None):
+    """The warp's (n_frames, 2, 10 gh, 10 gw) lattice for frames frame_offset .. of a total_frames movie."""
+    gh, gw = field.shape[-2:]
+    total = n_frames if total_frames is None else total_frames
+    times = _frame_times(frame_group, total, frame_offset, frame_offset + n_frames, field.device)
+    return _ops.spline_lattice(field, kind, n_frames, 10 * gh, 10 * gw, frame_offset=frame_offset, total_frames=total,
+                               times=times)
+
+
 def correct_motion(
     image: torch.Tensor,
     deformation_grid: torch.Tensor,
@@ -33,19 +56,22 @@ def correct_motion(
     grid_type: str = "catmull_rom",
     device: torch.device = None,
     _mean_std: torch.Tensor | None = None,
+    *,
+    frame_group: int | None = None,
 ) -> torch.Tensor:
     """(t, h, w) movie warped by a (yx, nt, nh, nw) Angstrom field -> (t, h, w).
 
     Reference: correct_motion.py:18-78 (spline -> 10x lattice -> bicubic lattice lookup ->
     bicubic frame gather; quirk Q17).  ``grad`` is accepted for signature compatibility; like
     the reference the result is detached.
+
+    ``frame_group=G``: the field was estimated with ``estimate_motion(..., frame_group=G)`` on this movie, so its time
+    axis runs over the group sums; every raw frame is corrected at its place on that axis (``frame_groups``).
     """
     dev = resolve_device(image, device)
     movie = _movie(image, dev)
     field = _field(deformation_grid, dev)
-    t = movie.shape[0]
-    gh, gw = field.shape[-2:]
-    lattice = _ops.spline_lattice(field, grid_kind(grid_type), t, 10 * gh, 10 * gw)
+    lattice = _lattice(field, grid_kind(grid_type), movie.shape[0], frame_group=frame_group)
     out = torch.empty_like(movie)
     # _mean_std (internal): warp the normalised movie (image - mean) / std without materialising it
     _ops.warp_lattice(movie, lattice, pixel_spacing, mean_std=_mean_std, out_stack=out)
@@ -101,20 +127,20 @@ def correct_motion_sum(
     accumulate: bool = False,
     frame_offset: int = 0,
     total_frames: int | None = None,
+    *,
+    frame_group: int | None = None,
 ) -> torch.Tensor:
     """Fused ``correct_motion(...).sum(dim=0)`` that never materialises the warped stack.
 
     New (additive) entry point: the reference leaves the frame sum to the caller
     (``examples/ttMotion.py:398``).  ``frame_offset``/``total_frames`` let one rank warp a
-    contiguous block of frames of a larger movie (frame-split multi-GPU)."""
+    contiguous block of frames of a larger movie (frame-split multi-GPU).  ``frame_group``: as for
+    ``correct_motion``; the groups are those of the whole ``total_frames`` movie."""
     dev = resolve_device(image, device)
     movie = _movie(image, dev)
     field = _field(deformation_grid, dev)
     t, h, w = movie.shape
-    gh, gw = field.shape[-2:]
-    lattice = _ops.spline_lattice(
-        field, grid_kind(grid_type), t, 10 * gh, 10 * gw, frame_offset=frame_offset, total_frames=total_frames
-    )
+    lattice = _lattice(field, grid_kind(grid_type), t, frame_offset, total_frames, frame_group)
     if out is None:
         out = torch.empty((h, w), dtype=torch.float32, device=dev)
         accumulate = False
@@ -148,10 +174,11 @@ def check_sums_arguments(shape, frame_range, dose_per_frame) -> tuple[int, int]:
 
 
 def warp_sums(movie, field, pixel_spacing, kind, frame_offset, total_frames, half_sets, lowrank, pixel_size=None,
-              voltage=300.0) -> dict:
+              voltage=300.0, times=None) -> dict:
     """Frame sums of ``movie`` (frames frame_offset .. of a movie of total_frames) in one pass of the weighted-sum warp
     (two or more beyond 19 sums), plus the low-rank dose-weighted sums of ``lowrank`` (exposure_filter_lowrank).  Every
-    output is linear in the frames, so sums over blocks of one movie add up to the sums over the movie."""
+    output is linear in the frames, so sums over blocks of one movie add up to the sums over the movie.  ``times``
+    (device float32 (t,), optional): the field's time at each frame, instead of its place in linspace(0, 1, total)."""
     from . import _fourier
     from ._lib import call, ptr, query, stream_ptr
 
@@ -179,7 +206,8 @@ def warp_sums(movie, field, pixel_spacing, kind, frame_offset, total_frames, hal
     weights = torch.from_numpy(np.stack(rows).astype(np.float32)).to(dev)
     n_sums = weights.shape[0]
     gh, gw = field.shape[-2:]
-    lattice = _ops.spline_lattice(field, kind, t, 10 * gh, 10 * gw, frame_offset=frame_offset, total_frames=total_frames)
+    lattice = _ops.spline_lattice(field, kind, t, 10 * gh, 10 * gw, frame_offset=frame_offset, total_frames=total_frames,
+                                  times=times)
     lh, lw = lattice.shape[-2:]
     ws = torch.empty((query("tmc_warp_workspace_floats", t, w, lh),), dtype=torch.float32, device=dev)
     sums = torch.empty((n_sums, h, w), dtype=torch.float32, device=dev)
@@ -222,6 +250,7 @@ def correct_motion_sums(
     voltage: float = 300.0,
     half_sets: bool = False,
     frame_range: tuple[int, int] | None = None,
+    frame_group: int | None = None,
 ) -> dict[str, torch.Tensor]:
     """Frame sums of the motion-corrected movie, never materialising the corrected stack: {name: (h, w) fp32}.
 
@@ -239,11 +268,16 @@ def correct_motion_sums(
 
     ``frame_range=(first, stop)`` restricts every sum to frames first .. stop - 1: only those frames are read, the field
     is evaluated at their place in the whole movie, exposure still counts all earlier frames and the dose
-    normalisation runs over the included frames."""
+    normalisation runs over the included frames.
+
+    ``frame_group=G``: the field was estimated with ``estimate_motion(..., frame_group=G)`` on this movie; every raw frame
+    is warped at its time on the group axis (``frame_groups``), while half sets and exposures stay those of the raw
+    frames."""
     first, stop = check_sums_arguments(image.shape, frame_range, dose_per_frame)
     kind = grid_kind(grid_type)
     dev = resolve_device(image, device)
     total = image.shape[0]
+    times = _frame_times(frame_group, total, first, stop, dev)
     movie = _movie(image[first:stop], dev)
     field = _field(deformation_grid, dev)
     lowrank = None
@@ -253,7 +287,7 @@ def correct_motion_sums(
         h, w = movie.shape[-2:]
         lowrank = exposure_filter_lowrank(h, w, pixel_spacing, range(first, stop), dose_per_frame, pre_exposure,
                                           voltage, half_sets)
-    return warp_sums(movie, field, pixel_spacing, kind, first, total, half_sets, lowrank, pixel_spacing, voltage)
+    return warp_sums(movie, field, pixel_spacing, kind, first, total, half_sets, lowrank, pixel_spacing, voltage, times)
 
 
 def get_pixel_shifts(

@@ -166,6 +166,39 @@ subtract_frame_means_kernel(float* __restrict__ stack, long n, const double* __r
   }
 }
 
+// frames whose loads one thread keeps in flight before it adds them (16 B each on the vector path)
+constexpr int kGroupUnroll = 4;
+
+__device__ __forceinline__ float4 add_rn(float4 a, float4 b) {
+  return make_float4(__fadd_rn(a.x, b.x), __fadd_rn(a.y, b.y), __fadd_rn(a.z, b.z), __fadd_rn(a.w, b.w));
+}
+__device__ __forceinline__ float add_rn(float a, float b) { return __fadd_rn(a, b); }
+
+// dst[g][i] = src[first_g][i] + src[first_g + 1][i] + ... (left to right, one rounding per add): group g holds frames
+// g * group_size .. and the last group also takes the t % group_size leftovers.  One thread owns one element (a float4
+// on the vector path) of one group; it issues kGroupUnroll frames' loads before adding them in ascending order.
+template <typename V>
+__global__ void __launch_bounds__(kPrepThreads)
+group_frames_kernel(const V* __restrict__ src, long n, int t, int group_size, int n_groups, V* __restrict__ dst) {
+  const int g = blockIdx.y;
+  const long i = (long)blockIdx.x * kPrepThreads + threadIdx.x;
+  if (i >= n) return;
+  const int first = g * group_size;
+  const int count = (g == n_groups - 1) ? t - first : group_size;
+  const V* p = src + (long)first * n + i;
+  V acc = __ldg(p);
+  int f = 1;
+  for (; f + kGroupUnroll <= count; f += kGroupUnroll) {
+    V v[kGroupUnroll];
+#pragma unroll
+    for (int k = 0; k < kGroupUnroll; ++k) v[k] = __ldg(p + (long)(f + k) * n);
+#pragma unroll
+    for (int k = 0; k < kGroupUnroll; ++k) acc = add_rn(acc, v[k]);
+  }
+  for (; f < count; ++f) acc = add_rn(acc, __ldg(p + (long)f * n));
+  dst[(long)g * n + i] = acc;
+}
+
 int blocks_per_frame(int t) {
   int b = (148 * 8 + t - 1) / t;
   return b < 1 ? 1 : b;
@@ -222,5 +255,30 @@ TMC_API int tmc_subtract_frame_means(float* stack, int t, long n, const double* 
   dim3 grid(blocks_per_frame(t), t);
   TMC_TIMED("subtract_frame_means_kernel", stream, subtract_frame_means_kernel<<<grid, kPrepThreads, 0, stream>>>(stack, n, moments));
   TMC_CHECK_LAUNCH("tmc_subtract_frame_means");
+  return TMC_OK;
+}
+
+// frame grouping: movie (t, h, w) -> groups (t / frame_group, h, w), sums of frame_group consecutive frames, the last
+// group also taking the t % frame_group leftover frames.  Each sum is x[first], then x[f] added in ascending order with
+// one fp32 rounding per add.  float4 loads when both pointers are 16-byte aligned and h * w % 4 == 0, scalar otherwise.
+TMC_API int tmc_group_frames(const float* movie, int t, int h, int w, int frame_group, float* groups, cudaStream_t stream) {
+  TMC_CHECK_ARG(movie && groups, "group_frames: null pointer");
+  TMC_CHECK_ARG(t >= 1 && h >= 1 && w >= 1, "group_frames: bad movie shape (%d, %d, %d)", t, h, w);
+  TMC_CHECK_ARG(frame_group >= 1, "group_frames: frame_group must be >= 1, got %d", frame_group);
+  const int n_groups = t / frame_group;
+  TMC_CHECK_ARG(n_groups >= 2 && n_groups <= 65535,
+                "group_frames: %d frames in groups of %d give %d groups, need 2 .. 65535", t, frame_group, n_groups);
+  const long n = (long)h * w;
+  const bool vec = n % 4 == 0 && ((reinterpret_cast<uintptr_t>(movie) | reinterpret_cast<uintptr_t>(groups)) & 15) == 0;
+  if (vec) {
+    dim3 grid(tmc_div_up(n / 4, kPrepThreads), n_groups);
+    TMC_TIMED("group_frames_kernel", stream, group_frames_kernel<float4><<<grid, kPrepThreads, 0, stream>>>(
+        reinterpret_cast<const float4*>(movie), n / 4, t, frame_group, n_groups, reinterpret_cast<float4*>(groups)));
+  } else {
+    dim3 grid(tmc_div_up(n, kPrepThreads), n_groups);
+    TMC_TIMED("group_frames_kernel", stream, group_frames_kernel<float><<<grid, kPrepThreads, 0, stream>>>(
+        movie, n, t, frame_group, n_groups, groups));
+  }
+  TMC_CHECK_LAUNCH("tmc_group_frames");
   return TMC_OK;
 }

@@ -229,8 +229,20 @@ __global__ void spline_eval_backward_kernel(int c, int p0, int p1, int p2, int k
   }
 }
 
-// lattice[f][ch][iy][ix] = G1(t_f, y_iy, x_ix) (+ G2(...)); t_f = linspace(0,1,total_frames)[frame_offset + f]
-__global__ void spline_lattice_kernel(PaddedGrid g1, int kind1, PaddedGrid g2, int kind2, int has2, int T, int frame_offset, int total_frames, int lh,
+// where the lattice's normalised frame times come from: t_f = linspace(0,1,total_frames)[frame_offset + f] ...
+struct LinspaceTimes {
+  int frame_offset, total_frames;
+  __device__ __forceinline__ float operator()(int f) const { return linspace01(f + frame_offset, total_frames); }
+};
+// ... or a per-frame table (frame grouping: times of the raw frames on the group time axis, may leave [0, 1])
+struct TableTimes {
+  const float* times;
+  __device__ __forceinline__ float operator()(int f) const { return __ldg(times + f); }
+};
+
+// lattice[f][ch][iy][ix] = G1(t_f, y_iy, x_ix) (+ G2(...))
+template <class Times>
+__global__ void spline_lattice_kernel(PaddedGrid g1, int kind1, PaddedGrid g2, int kind2, int has2, int T, Times times, int lh,
                                       int lw, float* __restrict__ lattice) {
   long i = (long)blockIdx.x * blockDim.x + threadIdx.x;
   long total = (long)T * lh * lw;
@@ -239,7 +251,7 @@ __global__ void spline_lattice_kernel(PaddedGrid g1, int kind1, PaddedGrid g2, i
   long r = i / lw;
   int iy = r % lh;
   int f = r / lh;
-  float ut = linspace01(f + frame_offset, total_frames), uy = linspace01(iy, lh), ux = linspace01(ix, lw);
+  float ut = times(f), uy = linspace01(iy, lh), ux = linspace01(ix, lw);
   float* out = lattice + ((long)f * g1.c * lh + iy) * lw + ix;
   SplineMatrix M = spline_matrix(kind1);
   spline_eval_point(g1, M, ut, uy, ux, out, lh * lw, false);
@@ -301,6 +313,32 @@ TMC_API int tmc_spline_eval_backward(int c, int n0, int n1, int n2, int kind, co
   return TMC_OK;
 }
 
+// padding of the grid(s) + spline_lattice_kernel: the common body of tmc_spline_lattice and tmc_spline_lattice_times
+template <class Times>
+static int spline_lattice_launch(const char* name, const float* coeffs, int c, int n0, int n1, int n2, int kind,
+                                 const float* coeffs2, int m0, int m1, int m2, int kind2, int n_frames, Times times, int lh,
+                                 int lw, float* lattice, float* workspace, cudaStream_t stream) {
+  if (coeffs2)
+    if (int e = check_grid(coeffs2, c, m0, m1, m2, kind2)) return e;
+  PaddedGrid g1, g2;
+  g1.data = workspace;
+  g1.c = c;
+  padded_dims(n0, n1, n2, g1.p0, g1.p1, g1.p2);
+  spline_pad_kernel<<<1, 256, 0, stream>>>(coeffs, c, n0, n1, n2, workspace); tmc_count_launch();
+  g2 = g1;
+  if (coeffs2) {
+    float* ws2 = workspace + tmc_spline_workspace_floats(c, n0, n1, n2);
+    g2.data = ws2;
+    padded_dims(m0, m1, m2, g2.p0, g2.p1, g2.p2);
+    spline_pad_kernel<<<1, 256, 0, stream>>>(coeffs2, c, m0, m1, m2, ws2); tmc_count_launch();
+  }
+  long total = (long)n_frames * lh * lw;
+  spline_lattice_kernel<Times><<<tmc_div_up(total, 128), 128, 0, stream>>>(g1, kind, g2, kind2, coeffs2 != nullptr, n_frames,
+                                                                          times, lh, lw, lattice); tmc_count_launch();
+  TMC_CHECK_LAUNCH(name);
+  return TMC_OK;
+}
+
 // deformation_field_utils.py:42-93 for all frames at once: lattice (T, c, lh, lw).
 // coeffs2 (optional, may be null) is added (correct_motion.py:297-305).
 TMC_API int tmc_spline_lattice(const float* coeffs, int c, int n0, int n1, int n2, int kind, const float* coeffs2, int m0,
@@ -309,22 +347,18 @@ TMC_API int tmc_spline_lattice(const float* coeffs, int c, int n0, int n1, int n
   if (int e = check_grid(coeffs, c, n0, n1, n2, kind)) return e;
   TMC_CHECK_ARG(lattice && workspace && n_frames >= 1 && lh >= 1 && lw >= 1, "spline_lattice: bad arguments");
   TMC_CHECK_ARG(frame_offset >= 0 && frame_offset + n_frames <= total_frames, "spline_lattice: frame range outside the movie");
-  PaddedGrid g1, g2;
-  g1.data = workspace;
-  g1.c = c;
-  padded_dims(n0, n1, n2, g1.p0, g1.p1, g1.p2);
-  spline_pad_kernel<<<1, 256, 0, stream>>>(coeffs, c, n0, n1, n2, workspace); tmc_count_launch();
-  g2 = g1;
-  if (coeffs2) {
-    if (int e = check_grid(coeffs2, c, m0, m1, m2, kind2)) return e;
-    float* ws2 = workspace + tmc_spline_workspace_floats(c, n0, n1, n2);
-    g2.data = ws2;
-    padded_dims(m0, m1, m2, g2.p0, g2.p1, g2.p2);
-    spline_pad_kernel<<<1, 256, 0, stream>>>(coeffs2, c, m0, m1, m2, ws2); tmc_count_launch();
-  }
-  long total = (long)n_frames * lh * lw;
-  spline_lattice_kernel<<<tmc_div_up(total, 128), 128, 0, stream>>>(g1, kind, g2, kind2, coeffs2 != nullptr, n_frames,
-                                                                   frame_offset, total_frames, lh, lw, lattice); tmc_count_launch();
-  TMC_CHECK_LAUNCH("tmc_spline_lattice");
-  return TMC_OK;
+  return spline_lattice_launch("tmc_spline_lattice", coeffs, c, n0, n1, n2, kind, coeffs2, m0, m1, m2, kind2, n_frames,
+                               LinspaceTimes{frame_offset, total_frames}, lh, lw, lattice, workspace, stream);
+}
+
+// tmc_spline_lattice at the normalised times times[f] (device, n_frames floats) instead of linspace(0,1,total)[offset + f]
+TMC_API int tmc_spline_lattice_times(const float* coeffs, int c, int n0, int n1, int n2, int kind, const float* coeffs2,
+                                     int m0, int m1, int m2, int kind2, int n_frames, const float* times, int lh, int lw,
+                                     float* lattice, float* workspace, cudaStream_t stream) {
+  if (int e = check_grid(coeffs, c, n0, n1, n2, kind)) return e;
+  TMC_CHECK_ARG(times && lattice && workspace, "spline_lattice_times: null pointer");
+  TMC_CHECK_ARG(n_frames >= 1 && lh >= 1 && lw >= 1, "spline_lattice_times: bad sizes (%d frames, %d x %d lattice)",
+                n_frames, lh, lw);
+  return spline_lattice_launch("tmc_spline_lattice_times", coeffs, c, n0, n1, n2, kind, coeffs2, m0, m1, m2, kind2,
+                               n_frames, TableTimes{times}, lh, lw, lattice, workspace, stream);
 }

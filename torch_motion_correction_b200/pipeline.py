@@ -61,8 +61,18 @@ def estimate_motion(
     n_refinements: int = 0,
     refinement_tolerance: float = 1e-3,
     return_history: bool = False,
+    frame_group: int | None = None,
 ):
     """Returns ``(field (2, nt, nh, nw) Angstrom, patch_centres)`` (and the refinement history with ``return_history``).
+
+    ``frame_group=G`` (int >= 2; None or 1: off) estimates on the sums of G consecutive frames (``group_frames``: the
+    last group also takes the t % G leftover frames) instead of on single frames -- MotionCor2's ``-Group``, for finely
+    fractionated movies whose single frames hold too few electrons for a usable cross-correlation peak.  Everything
+    below runs unchanged on the t // G group sums, so the returned field's time axis runs over the GROUPS: correct
+    the raw frames with ``correct_motion*(..., frame_group=G)``, which evaluate it at each frame's place between the
+    group centres (``frame_groups``).  The patch-XC exposure pre-filter treats a group as one frame of G *
+    ``dose_per_frame``, so group g is filtered at the exposure at the end of its last frame; for a last group with
+    leftover frames that under-counts its exposure by t % G frames.
 
     ``dose_per_frame`` switches on the exposure pre-filter of the patch cross-correlation.
 
@@ -79,6 +89,15 @@ def estimate_motion(
     from . import _ops
     from ._common import as_f32, resolve_device
 
+    if frame_group is not None:
+        from .frame_groups import frame_groups
+        from .prepare import group_frames
+
+        group_size = frame_groups(image.shape[0], frame_group).group_size
+        if group_size > 1:
+            image = group_frames(image, group_size, device=device)  # freed when this call returns
+            if dose_per_frame is not None:
+                dose_per_frame = dose_per_frame * group_size
     stats = _ops.stack_stats(as_f32(image, resolve_device(image, device)))
     global_field = estimate_global_motion(
         image, pixel_spacing, b_factor=b_factor, frequency_range=frequency_range, device=device, _stats=stats
@@ -119,16 +138,26 @@ def estimate_motion(
 
 
 def motion_correct(image: torch.Tensor, pixel_spacing: float, grid_type: str = "bspline", device=None,
-                   dose_per_frame: float | None = None, pre_exposure: float = 0.0, voltage: float = 300.0, **estimate_kwargs):
+                   dose_per_frame: float | None = None, pre_exposure: float = 0.0, voltage: float = 300.0,
+                   frame_group: int | None = None, **estimate_kwargs):
     """Estimate + correct: returns ``(aligned frame sum (h, w), field)``.
 
     With ``dose_per_frame`` (e-/A^2 per frame) the patch cross-correlation is exposure pre-filtered and the sum is dose
     weighted (``examples/ttMotion.py:331-351,383-398``: correct -> per-frame exposure filter -> sum), which needs the
-    corrected stack instead of the fused sum."""
+    corrected stack instead of the fused sum.
+
+    ``frame_group=G``: estimate on the sums of G consecutive frames (``estimate_motion``), then correct every raw frame
+    with that field.  The dose-weighted sum is then formed without materialising the corrected stack
+    (``correct_motion_sums``), since grouping is meant for movies of hundreds of frames."""
     field, _ = estimate_motion(image, pixel_spacing, grid_type=grid_type, device=device, dose_per_frame=dose_per_frame,
-                               pre_exposure=pre_exposure, voltage=voltage, **estimate_kwargs)
+                               pre_exposure=pre_exposure, voltage=voltage, frame_group=frame_group, **estimate_kwargs)
     if dose_per_frame is None:
-        total = correct_motion_sum(image, field, pixel_spacing, grid_type=grid_type, device=device)
+        total = correct_motion_sum(image, field, pixel_spacing, grid_type=grid_type, device=device, frame_group=frame_group)
+    elif frame_group is not None and frame_group != 1:
+        from .correct_motion import correct_motion_sums
+
+        total = correct_motion_sums(image, field, pixel_spacing, grid_type, device, dose_per_frame=dose_per_frame,
+                                    pre_exposure=pre_exposure, voltage=voltage, frame_group=frame_group)["dose_weighted"]
     else:
         from .correct_motion import correct_motion
         from .dose_weight import dose_weight

@@ -68,3 +68,22 @@ def prepare_movie(movie: torch.Tensor, gain: torch.Tensor | None = None, hot_pix
     if return_hot_pixel_count:
         return out, count
     return out
+
+
+def group_frames(movie: torch.Tensor, frame_group: int, device=None) -> torch.Tensor:
+    """(t, h, w) movie -> (t // frame_group, h, w) fp32 sums of ``frame_group`` consecutive frames, the last group also
+    taking the ``t % frame_group`` leftover frames (``frame_groups.frame_groups`` has the rule).  Each sum adds the frames
+    in ascending order, one fp32 rounding per add.  ``frame_group == 1`` returns ``movie`` itself.
+
+    These are the frames ``estimate_motion(..., frame_group=...)`` estimates on: summing a few low-dose frames gives the
+    cross-correlation peaks a usable signal."""
+    from ._common import as_f32
+    from ._ops import group_frames as _group_frames
+    from .frame_groups import frame_groups
+
+    if movie.ndim != 3:
+        raise ValueError(f"movie must be (t, h, w), got {tuple(movie.shape)}")
+    groups = frame_groups(movie.shape[0], frame_group)
+    if groups.group_size == 1:
+        return movie
+    return _group_frames(as_f32(movie, resolve_device(movie, device)), groups.group_size)
