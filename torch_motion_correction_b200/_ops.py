@@ -43,6 +43,34 @@ def moments_to_mean_std(moments: torch.Tensor) -> torch.Tensor:
     return out
 
 
+def xc_postprocess(shifts, field, pixel_spacing, skip_frame, outlier_rejection, outlier_threshold, temporal_smoothing,
+                   smoothing_window_size) -> None:
+    """In place on ``field`` (2, t, gh, gw) Angstrom: outlier rejection of the (t, gh gw, 2) px ``shifts``, accumulation
+    onto the field, Savitzky-Golay smoothing and one joint mean removed (``skip_frame`` -1: none skipped)."""
+    _, t, gh, gw = field.shape
+    scratch = torch.empty_like(field)
+    with torch.cuda.device(field.device):
+        call("tmc_xc_postprocess", ptr(shifts), t, gh * gw, float(pixel_spacing), int(skip_frame), int(bool(outlier_rejection)),
+             float(outlier_threshold), int(bool(temporal_smoothing)), int(smoothing_window_size), 1, ptr(field), ptr(scratch),
+             stream_ptr(field.device))
+
+
+def global_shifts_to_field(shifts: torch.Tensor, pixel_spacing, reference_frame: int) -> torch.Tensor:
+    """(t, 2) px shifts -> (2, t, 1, 1) Angstrom field, zero at ``reference_frame``."""
+    t = shifts.shape[0]
+    field = _f32((2, t, 1, 1), shifts)
+    with torch.cuda.device(shifts.device):
+        call("tmc_global_shifts_to_field", ptr(shifts), t, float(pixel_spacing), int(reference_frame), ptr(field),
+             stream_ptr(shifts.device))
+    return field
+
+
+def subtract_mean(data: torch.Tensor) -> None:
+    """In place: ``data`` (contiguous float32) -= its mean, one joint scalar."""
+    with torch.cuda.device(data.device):
+        call("tmc_subtract_mean", ptr(data), data.numel(), stream_ptr(data.device))
+
+
 def spline_eval(coeffs: torch.Tensor, kind: int, tyx: torch.Tensor, out=None, ws=None) -> torch.Tensor:
     """``out`` (n, c) / ``ws`` (tmc_spline_workspace_floats) may be preallocated (allocation-free replays)."""
     c, n0, n1, n2 = coeffs.shape

@@ -24,9 +24,7 @@ from . import _fourier, _ops
 from ._common import as_f32, cached_device_tensor, grid_kind, resolve_device
 from ._lib import call, ptr, stream_ptr
 from .correct_motion import correct_motion_fast
-from .deformation_field_utils import resample_deformation_field
-from .estimate_motion_xc import _aliasing_schedule
-from .patch_grid import patch_grid_centers
+from .estimate_motion_xc import global_spectra, leave_one_out_shifts, mean_except_current_spectra, patch_xc_geometry
 
 
 def frame_range(total_frames: int, rank: int, world: int) -> tuple[int, int]:
@@ -42,25 +40,24 @@ def _world(group):
     return 0, 1
 
 
-def all_gather_frames(local: torch.Tensor, total_frames: int, group=None) -> torch.Tensor:
-    """Concatenate per-rank blocks ``local (t_local, ...)`` (rank order == frame order) into
-    ``(total_frames, ...)`` on every rank.  Blocks may differ by one frame: pad, gather, trim."""
-    rank, world = _world(group)
+def all_gather_frames(local: torch.Tensor, total_frames: int, group=None, dim: int = 0) -> torch.Tensor:
+    """Concatenate per-rank blocks ``local`` along ``dim`` (rank order == index order; rank r holds the entries
+    ``frame_range(total_frames, r, world)``) into ``total_frames`` entries on every rank.  Blocks may differ by one
+    entry: pad, gather, trim."""
+    _, world = _world(group)
     if world == 1:
         return local
-    t_max = -(-total_frames // world)
-    padded = local
-    if local.shape[0] < t_max:
-        pad = torch.zeros((t_max - local.shape[0], *local.shape[1:]), dtype=local.dtype, device=local.device)
-        padded = torch.cat([local, pad], dim=0)
-    padded = padded.contiguous()
+    shape = list(local.shape)
+    shape[dim] = -(-total_frames // world)
+    padded = torch.zeros(shape, dtype=local.dtype, device=local.device)
+    padded.narrow(dim, 0, local.shape[dim]).copy_(local)
     parts = [torch.empty_like(padded) for _ in range(world)]
     dist.all_gather(parts, padded, group=group)
     out = []
     for r in range(world):
         f0, f1 = frame_range(total_frames, r, world)
-        out.append(parts[r][: f1 - f0])
-    return torch.cat(out, dim=0)
+        out.append(parts[r].narrow(dim, 0, f1 - f0))
+    return torch.cat(out, dim=dim)
 
 
 def _reshard_frames_to_patches(spec, spec_sub, t, g, words, rank, world, group, frame_major=False):
@@ -98,22 +95,6 @@ def _reshard_frames_to_patches(spec, spec_sub, t, g, words, rank, world, group, 
         full = all_gather_frames(spec, t, group)  # (T, G, words) on every rank
         if g1 > g0:
             put(0, t, full[:, g0:g1])
-
-
-def _all_gather_patches(local, g, rank, world, group):
-    """(t, G_r, c) blocks of consecutive patch ranges (frame_range(g, r, world)) -> (t, G, c) on every rank."""
-    if world == 1:
-        return local
-    g_max = -(-g // world)
-    padded = torch.zeros((local.shape[0], g_max, local.shape[2]), dtype=local.dtype, device=local.device)
-    padded[:, : local.shape[1]] = local
-    parts = [torch.empty_like(padded) for _ in range(world)]
-    dist.all_gather(parts, padded, group=group)
-    out = []
-    for r in range(world):
-        a, b = frame_range(g, r, world)
-        out.append(parts[r][:, : b - a])
-    return torch.cat(out, dim=1)
 
 
 def stack_stats_frame_split(local_frames: torch.Tensor, group=None) -> torch.Tensor:
@@ -180,12 +161,10 @@ def estimate_global_motion_frame_split(local_frames, pixel_spacing, frame_offset
     broadcasts its band-limited spectrum (a few MB); shifts are all-gathered."""
     rank, world = _world(group)
     dev = local_frames.device
-    t_local, h, w = local_frames.shape
+    t_local = local_frames.shape[0]
     if reference_frame is None:
         reference_frame = total_frames // 2
-    plan = _fourier.BandPlan(h, w, dev, pixel_spacing, b_factor, frequency_range)
-    mask, ylo, yhi = _fourier.soft_disc_mask((h, w), min(h, w) / 4, min(h, w) / 8, dev)
-    spec = plan.forward(local_frames, mean_std, mask, ylo, yhi, _fourier.frame_pair_jobs(t_local, dev), job_mode=2)
+    plan, spec = global_spectra(local_frames, mean_std, pixel_spacing, b_factor, frequency_range)
     ref_spec = torch.empty((1, plan.ky, plan.kx, 2), dtype=torch.float32, device=dev)
     owner = next(r for r in range(world) if frame_range(total_frames, r, world)[0] <= reference_frame < frame_range(total_frames, r, world)[1])
     if rank == owner:
@@ -198,11 +177,7 @@ def estimate_global_motion_frame_split(local_frames, pixel_spacing, frame_offset
     prod = _fourier.pair_products(both, ref, cur, plan.plane_elems)
     shifts = plan.peaks(prod.view(t_local, plan.ky, plan.kx, 2), sub_pixel=False)
     shifts = all_gather_frames(shifts, total_frames, group)
-    field = torch.empty((2, total_frames, 1, 1), dtype=torch.float32, device=dev)
-    with torch.cuda.device(dev):
-        call("tmc_global_shifts_to_field", ptr(shifts), total_frames, float(pixel_spacing), int(reference_frame), ptr(field),
-             stream_ptr(dev))
-    return field
+    return _ops.global_shifts_to_field(shifts, pixel_spacing, reference_frame)
 
 
 def estimate_patch_motion_frame_split(local_frames, pixel_spacing, frame_offset, total_frames, mean_std,
@@ -236,85 +211,25 @@ def estimate_patch_motion_frame_split(local_frames, pixel_spacing, frame_offset,
             source_stats = None
         deformation_field = deformation_field * -1  # the reference negates the caller's field in place (Q2)
     p = int(patch_sidelength)
-    centers = patch_grid_centers((t, h, w), (1, p, p), (1, p // 2, p // 2), distribute_patches=True)
-    gh, gw = centers.shape[1:3]
-    g = gh * gw
-    origins = (centers[0, :, :, 1:] - p // 2).reshape(-1, 2).tolist()
-    plan = _fourier.BandPlan(p, p, dev, pixel_spacing, b_factor, frequency_range)
-    mask, ylo, yhi = _fourier.soft_disc_mask((p, p), p / 4, p / 8, dev)
-    if deformation_field is None:
-        field = torch.zeros((2, t, gh, gw), dtype=torch.float32, device=dev)
-    else:
-        field = resample_deformation_field(deformation_field, (t, gh, gw))
-    # planning tensors are pure functions of the geometry: built once per device (no host-blocking copies per call)
-    jobs = cached_device_tensor(
-        ("split_xc_jobs", (t_local, h, w, p)),
-        lambda: torch.tensor([[k, 1, k, 2, y0, x0] for k in range(t_local) for (y0, x0) in origins], dtype=torch.int32), dev)
+    centres, origins, plan, mask, field = patch_xc_geometry((t, h, w), p, pixel_spacing, b_factor, frequency_range,
+                                                            deformation_field, dev)
+    g = len(origins)
     words = 2 * plan.plane_elems * 2  # both mask powers of one (frame, patch), float32 words
-    spec_local = plan.forward(source, source_stats, mask, ylo, yhi, jobs, job_mode=1, frame_shifts=frame_shifts).view(t_local, g, words)
+    _, spec_local = mean_except_current_spectra(source, source_stats, plan, mask, p, origins, frame_shifts)
     # frames for the transforms, patches for the cross-correlation: every rank receives ALL frames of ITS share of the
     # patches (all-to-all, 1/world of an all-gather), forms their leave-one-out references and peaks, and the shifts
     # (KBs) are gathered
     g0, g1 = frame_range(g, rank, world)
     g_sub = g1 - g0
-    spec_sub = torch.zeros((t, max(g_sub, 1), words), dtype=torch.float32, device=dev)
-    _reshard_frames_to_patches(spec_local, spec_sub, t, g, words, rank, world, group, frame_major=True)
-    del spec_local
-
-    def schedule(part):
-        offsets, deltas = _aliasing_schedule(t, "mean_except_current", t // 2)
-        return torch.tensor(offsets if part == 0 else (deltas if deltas else [0]), dtype=torch.int32)
-
-    d_off = cached_device_tensor(("xc_delta_offsets", t), lambda: schedule(0), dev)  # same keys as estimate_motion_xc
-    d_val = cached_device_tensor(("xc_deltas", t), lambda: schedule(1), dev)
     gs = max(g_sub, 1)
-    prod = _fourier.leave_one_out_products(spec_sub, t, gs, plan.plane_elems, d_off, d_val)
-    shifts = plan.peaks(prod.view(t * gs, plan.ky, plan.kx, 2), sub_pixel=bool(sub_pixel_refinement))
-    shifts = _all_gather_patches(shifts.view(t, gs, 2)[:, :g_sub], g, rank, world, group).contiguous()
-    scratch = torch.empty_like(field)
-    with torch.cuda.device(dev):
-        call("tmc_xc_postprocess", ptr(shifts), t, g, float(pixel_spacing), -1, int(bool(outlier_rejection)),
-             float(outlier_threshold), int(bool(temporal_smoothing)), int(smoothing_window_size), 1, ptr(field), ptr(scratch),
-             stream_ptr(dev))
-    return field, cached_device_tensor(("patch_centres", (t, h, w, p)), lambda: centers, dev).clone()
-
-
-def _make_patch_shard_problem(spec_sub, centres_norm_sub, base, kind, loss_code, px, t, ph, pw, resolution, plan, dev):
-    """A ``LocalMotionProblem`` (estimate_motion_optimizer.py) for a subset of the patches with ALL frames, built from
-    spectra ``spec_sub`` (G_r, tp, KY, KX) that are already on the device."""
-    from .estimate_motion_optimizer import LocalMotionProblem, fused_steps_apply
-    from ._lib import query
-
-    prob = LocalMotionProblem.__new__(LocalMotionProblem)
-    g = spec_sub.shape[0]
-    prob.kind, prob.loss_type, prob.dev, prob.px = kind, loss_code, dev, px
-    prob.t, prob.ph, prob.pw = t, ph, pw
-    prob.resolution = resolution
-    prob.g = g
-    prob.base = base
-    prob.plan = plan
-    prob.tp = spec_sub.shape[1]
-    prob.fused = fused_steps_apply(loss_code, g, t, resolution, plan)
-    prob.frame_major = False  # (G, tp, KY, KX): patch-major
-    prob.spec = spec_sub
-    prob.norms = torch.empty((g, t, 2), dtype=torch.float64, device=dev)
-    with torch.cuda.device(dev):
-        call("tmc_local_spectra_norms", ptr(spec_sub), g, t, prob.tp, ph, pw, plan.ky, plan.kx, plan.ky_start, 0, ptr(prob.norms),
-             stream_ptr(dev))
-    prob.centres_norm = centres_norm_sub  # (T, g, 3)
-    prob.eval_base = _ops.spline_eval(base, kind, centres_norm_sub)
-    ws_bytes = query("tmc_local_loss_workspace_bytes", g, t, plan.ky, plan.kx)
-    prob.workspace = torch.empty(((ws_bytes + 7) // 8,), dtype=torch.float64, device=dev)
-    prob.loss = torch.zeros((1,), dtype=torch.float64, device=dev)
-    prob.grad_eval = torch.empty((t, g, 2), dtype=torch.float32, device=dev)
-    prob.eval_new = torch.empty((t, g, 2), dtype=torch.float32, device=dev)
-    prob.grad = torch.empty((2, *resolution), dtype=torch.float32, device=dev)
-    n_ws = query("tmc_spline_workspace_floats", 2, *resolution)
-    prob.ws_eval = torch.empty((n_ws,), dtype=torch.float32, device=dev)
-    prob.ws_back = torch.empty((n_ws,), dtype=torch.float32, device=dev)
-    if prob.fused:
-        prob._setup_fused_steps()
-    return prob
+    spec_sub = torch.zeros((t, gs, words), dtype=torch.float32, device=dev)
+    _reshard_frames_to_patches(spec_local.view(t_local, g, words), spec_sub, t, g, words, rank, world, group, frame_major=True)
+    del spec_local
+    shifts = leave_one_out_shifts(spec_sub, t, gs, plan, sub_pixel_refinement)
+    shifts = all_gather_frames(shifts.view(t, gs, 2)[:, :g_sub], g, group, dim=1).contiguous()
+    _ops.xc_postprocess(shifts, field, pixel_spacing, -1, outlier_rejection, outlier_threshold, temporal_smoothing,
+                        smoothing_window_size)
+    return field, centres.clone()
 
 
 def estimate_local_motion_frame_split(local_frames, pixel_spacing, patch_shape, deformation_field_resolution,
@@ -330,7 +245,8 @@ def estimate_local_motion_frame_split(local_frames, pixel_spacing, patch_shape, 
     coefficient gradient (2 nt nh nw floats) is all-reduced, and the Adam update is replicated.  The shuffled mini-batch
     weighting (quirks Q10 / Q11) is drawn on rank 0 and broadcast, so the result equals the single-GPU run with the same
     ``random`` state up to the order of the fp32 sums.  Returns the (2, nt, nh, nw) field (identical on all ranks)."""
-    from .estimate_motion_optimizer import LOSS_TYPES, _shuffled_batches
+    from .estimate_motion_optimizer import (LOSS_TYPES, LocalMotionProblem, _shuffled_batches, base_grid, fused_adam_state,
+                                            local_patches, local_spectra, normalised_centres, patch_scales)
 
     rank, world = _world(group)
     dev = local_frames.device
@@ -343,36 +259,18 @@ def estimate_local_motion_frame_split(local_frames, pixel_spacing, patch_shape, 
     lt = LOSS_TYPES[loss_type]
     kind = grid_kind(grid_type)
     resolution = tuple(int(r) for r in deformation_field_resolution)
-    px = float(pixel_spacing)
     kw = dict(optimizer_kwargs) if optimizer_kwargs is not None else {}
 
-    centers = patch_grid_centers((t, h, w), (1, ph, pw), (1, ph // 2, pw // 2), distribute_patches=True)
-    gh, gw = centers.shape[1:3]
-    g = gh * gw
-    flat = centers[0].reshape(-1, 3)
-    y0 = (flat[:, 1] - ph // 2).tolist()
-    x0 = (flat[:, 2] - pw // 2).tolist()
-    if min(y0) < 0 or min(x0) < 0 or max(y0) + ph > h or max(x0) + pw > w:
-        raise AssertionError(f"Patch size {tuple(patch_shape)} too large for control points in image of shape {(t, h, w)}")
-
-    if initial_deformation_field is None:
-        base = torch.zeros((2, *resolution), dtype=torch.float32, device=dev)
-    else:
-        base = resample_deformation_field(as_f32(initial_deformation_field, dev), resolution)
-        with torch.cuda.device(dev):
-            call("tmc_subtract_mean", ptr(base), base.numel(), stream_ptr(dev))
+    centers, origins = local_patches((t, h, w), patch_shape)
+    g = len(origins[0])
+    base = base_grid(initial_deformation_field, resolution, dev)
 
     # spectra of the local frames: one plane per (frame, patch), frame-major (t_local, G, KY, KX)
-    plan = _fourier.BandPlan(ph, pw, dev, px, b_factor, frequency_range)
-    mask, ylo, yhi = _fourier.soft_disc_mask((ph, pw), pw / 4, pw / 4, dev)  # quirk Q18
+    plan = _fourier.BandPlan(ph, pw, dev, float(pixel_spacing), b_factor, frequency_range)
     words = plan.plane_elems * 2
     if t_local > 0:
-        jobs = cached_device_tensor(
-            ("split_local_jobs", (t_local, h, w, ph, pw)),
-            lambda: torch.tensor([[i, 1, i + 1 if i + 1 < t_local else -1, 1, y0[gi], x0[gi]] for i in range(0, t_local, 2)
-                                  for gi in range(g)], dtype=torch.int32), dev)
         pairs = (t_local + 1) // 2
-        spec = plan.forward(frames, mean_std, mask, ylo, yhi, jobs, job_mode=2)  # planes [pair][patch][frame of the pair]
+        spec = local_spectra(frames, mean_std, plan, patch_shape, origins, True)  # planes [pair][patch][frame of the pair]
         spec = spec.view(pairs, g, 2, words).permute(0, 2, 1, 3).reshape(2 * pairs, g, words)[:t_local].contiguous()
     else:
         spec = torch.zeros((0, g, words), dtype=torch.float32, device=dev)
@@ -384,30 +282,16 @@ def estimate_local_motion_frame_split(local_frames, pixel_spacing, patch_shape, 
     _reshard_frames_to_patches(spec, spec_sub, t, g, words, rank, world, group)
     del spec
 
-    # normalised (t, y, x) centres of this rank's patches, time-major (T, G_r, 3)
-    norm = centers.clone().float()
-    norm[..., 0] /= float(t - 1) if t > 1 else float("nan")
-    norm[..., 1] /= float(h - 1)
-    norm[..., 2] /= float(w - 1)
     centres_sub = cached_device_tensor(("split_centres", (t, h, w, ph, pw), g0, g1),
-                                       lambda: norm.reshape(t, g, 3)[:, g0:max(g1, g0 + 1)].contiguous(), dev)
-    problem = _make_patch_shard_problem(spec_sub, centres_sub, base, kind, lt, px, t, ph, pw, resolution, plan, dev)
+                                       lambda: normalised_centres(centers, (t, h, w))[:, g0:max(g1, g0 + 1)].contiguous(), dev)
+    problem = LocalMotionProblem.from_spectra(spec_sub, False, centres_sub, base, plan, patch_shape, kind, lt, pixel_spacing)
 
     # the mini-batch weighting of every iteration: drawn once (rank 0) and broadcast; each rank uses its patches' columns
-    def patch_scales(batches):
-        scale = [0.0] * g
-        for batch in batches:
-            b = len(batch)
-            sc = 1.0 / (b * t * ph * (pw // 2 + 1)) / (ph * pw) if lt == 0 else 1.0 / (b * t)
-            for gi in batch:
-                scale[gi] = sc
-        return scale
-
     n_iterations = int(n_iterations)
     scales = torch.zeros((max(n_iterations, 1), g), dtype=torch.float32)
     if rank == 0:
         for i in range(n_iterations):
-            scales[i] = torch.tensor(patch_scales(_shuffled_batches(g, 8)), dtype=torch.float32)
+            scales[i] = torch.tensor(patch_scales(_shuffled_batches(g, 8), g, t, ph, pw, lt), dtype=torch.float32)
     scales = scales.to(dev)
     if world > 1:
         dist.broadcast(scales, src=dist.get_global_rank(group, 0) if group is not None else 0, group=group)
@@ -416,9 +300,8 @@ def estimate_local_motion_frame_split(local_frames, pixel_spacing, patch_shape, 
         scales_sub.zero_()  # a rank without patches contributes nothing
 
     new = torch.zeros((2, *resolution), dtype=torch.float32, device=dev)
-    exp_avg, exp_avg_sq = torch.zeros_like(new), torch.zeros_like(new)
-    lr, (b1, b2) = float(kw.get("lr", 0.01)), kw.get("betas", (0.9, 0.999))
-    eps, wd = float(kw.get("eps", 1e-08)), float(kw.get("weight_decay", 0))
+    adam = fused_adam_state(new, kw)
+    exp_avg, exp_avg_sq, lr, b1, b2, eps, wd = adam
     steps = torch.arange(max(n_iterations, 1), dtype=torch.int32, device=dev)  # Adam's step number - 1 of every iteration
     losses = []
     def reduce_gradient(loss, grad):
@@ -435,7 +318,6 @@ def estimate_local_motion_frame_split(local_frames, pixel_spacing, patch_shape, 
         if problem.fused:
             # three launches and one all-reduce per iteration: [Adam on the reduced gradient + next shifts] -> loss /
             # gradient kernel -> backward to the coefficient gradient (tmc_local_steps modes 1, 2, 3)
-            adam = (exp_avg, exp_avg_sq, lr, float(b1), float(b2), eps, wd)
             for i in range(n_iterations):
                 problem.fused_steps(new, scales_sub, i, 1, 1 if i == 0 else 2, problem.loss, adam=adam)
                 reduce_gradient(problem.loss, problem.grad)
@@ -445,11 +327,10 @@ def estimate_local_motion_frame_split(local_frames, pixel_spacing, patch_shape, 
             for i in range(n_iterations):
                 loss, grad = problem.loss_and_grad(new, scales_sub[i])
                 reduce_gradient(loss, grad)
-                call("tmc_adam_step", ptr(new), ptr(grad), ptr(exp_avg), ptr(exp_avg_sq), new.numel(), lr, float(b1), float(b2), eps,
-                     wd, steps.data_ptr() + 4 * i, stream)
+                call("tmc_adam_step", ptr(new), ptr(grad), ptr(exp_avg), ptr(exp_avg_sq), new.numel(), lr, b1, b2, eps, wd,
+                     steps.data_ptr() + 4 * i, stream)
     final = (new + base).contiguous()
-    with torch.cuda.device(dev):
-        call("tmc_subtract_mean", ptr(final), final.numel(), stream_ptr(dev))
+    _ops.subtract_mean(final)
     if return_losses:
         return final, [float(l) for l in losses]
     return final

@@ -70,6 +70,83 @@ def _setup_optimizer(optimizer_type: str, parameters, **kwargs: Any) -> torch.op
     raise ValueError(f"Unsupported optimizer: {optimizer_type}. Choose 'adam', 'sgd', 'rmsprop', or 'lbfgs'.")
 
 
+def local_patches(shape, patch_shape):
+    """Patch grid of the optimiser on a (t, h, w) movie: (centres (t, gh, gw, 3), window origins (y0 list, x0 list)).
+    Patch window = floor(centre) - p // 2, no clipping (patch_utils.py:117-120,173-183; quirk Q20)."""
+    t, h, w = shape
+    ph, pw = patch_shape
+    centers = patch_grid_centers((t, h, w), (1, ph, pw), (1, ph // 2, pw // 2), distribute_patches=True)
+    flat = centers[0].reshape(-1, 3)
+    y0 = (flat[:, 1] - ph // 2).tolist()
+    x0 = (flat[:, 2] - pw // 2).tolist()
+    if min(y0) < 0 or min(x0) < 0 or max(y0) + ph > h or max(x0) + pw > w:
+        raise AssertionError(f"Patch size {tuple(patch_shape)} too large for control points in image of shape {(t, h, w)}")
+    return centers, (y0, x0)
+
+
+def normalised_centres(centers: torch.Tensor, shape) -> torch.Tensor:
+    """Normalised (t, y, x) patch centres, (T, G, 3) time-major (patch_utils.py:88-93,157-172; quirk Q10)."""
+    t, h, w = shape
+    norm = centers.clone().float()
+    norm[..., 0] /= float(t - 1) if t > 1 else float("nan")
+    norm[..., 1] /= float(h - 1)
+    norm[..., 2] /= float(w - 1)
+    return norm.reshape(t, -1, 3).contiguous()
+
+
+def base_grid(initial_field, resolution, dev) -> torch.Tensor:
+    """Frozen base grid (estimate_motion_optimizer.py:135-158): zeros, or the initial field resampled onto the spline
+    grid with its mean removed."""
+    if initial_field is None:
+        return torch.zeros((2, *resolution), dtype=torch.float32, device=dev)
+    base = resample_deformation_field(as_f32(initial_field, dev), resolution)
+    _ops.subtract_mean(base)
+    return base
+
+
+def local_spectra(movie, stats, plan, patch_shape, origins, frame_major: bool) -> torch.Tensor:
+    """Spectra FW[g][t] = rfft2(mask * patch) * band * envelope on the pass-band box of every patch and frame of
+    ``movie``, frames packed in pairs: (g * tp, KY, KX, 2) planes, patch by patch or, ``frame_major``, frame pair by
+    frame pair (the two layouts the optimiser kernels read)."""
+    t, h, w = movie.shape
+    ph, pw = patch_shape
+    y0, x0 = origins
+    g = len(y0)
+    mask, ylo, yhi = _fourier.soft_disc_mask((ph, pw), pw / 4, pw / 4, movie.device)  # quirk Q18: smoothing pw/4
+
+    def build_jobs():
+        pairs = [(i, i + 1 if i + 1 < t else -1) for i in range(0, t, 2)]
+        order = [(pair, gi) for pair in pairs for gi in range(g)] if frame_major else \
+            [(pair, gi) for gi in range(g) for pair in pairs]
+        return torch.tensor([[a, 1, b, 1, y0[gi], x0[gi]] for (a, b), gi in order], dtype=torch.int32)
+
+    jobs = cached_device_tensor(("local_jobs", (t, h, w, ph, pw), frame_major), build_jobs, movie.device)
+    return plan.forward(movie, stats, mask, ylo, yhi, jobs, job_mode=2)
+
+
+def patch_scales(batches, g: int, t: int, ph: int, pw: int, loss_type: int) -> list:
+    """Per-patch weight reproducing the reference's per-mini-batch ``mean`` (quirk Q11): the gradient is the SUM over
+    mini-batches of each batch's mean-reduced loss."""
+    scale = [0.0] * g
+    for batch in batches:
+        b = len(batch)
+        if loss_type == 0:
+            s = 1.0 / (b * t * ph * (pw // 2 + 1)) / (ph * pw)
+        else:
+            s = 1.0 / (b * t)
+        for gi in batch:
+            scale[gi] = s
+    return scale
+
+
+def fused_adam_state(coef: torch.Tensor, optimizer_kwargs: dict) -> tuple:
+    """State and hyper-parameters of the fused Adam update of ``coef``: (exp_avg, exp_avg_sq, lr, b1, b2, eps,
+    weight_decay), torch.optim.Adam's defaults unless ``optimizer_kwargs`` sets them."""
+    b1, b2 = optimizer_kwargs.get("betas", (0.9, 0.999))
+    return (torch.zeros_like(coef), torch.zeros_like(coef), float(optimizer_kwargs.get("lr", 0.01)), float(b1), float(b2),
+            float(optimizer_kwargs.get("eps", 1e-08)), float(optimizer_kwargs.get("weight_decay", 0)))
+
+
 class LocalMotionProblem:
     """Device-resident state of one ``estimate_local_motion`` call: band-limited patch spectra,
     their norms, normalised patch centres and the frozen base grid's values at the centres."""
@@ -78,91 +155,69 @@ class LocalMotionProblem:
                  grid_type, loss_type, stats=None):
         if loss_type not in LOSS_TYPES:
             raise ValueError(f"Invalid loss type: {loss_type}. Must be 'mse', 'cc' or 'ncc'.")
-        self.kind = grid_kind(grid_type)
-        self.loss_type = LOSS_TYPES[loss_type]
-        self.dev = dev
-        self.px = float(pixel_spacing)
+        kind = grid_kind(grid_type)
         movie = as_f32(image, dev)
         t, h, w = movie.shape
         ph, pw = patch_shape
-        self.t, self.ph, self.pw = t, ph, pw
-        self.geometry = (t, h, w, ph, pw)
-        self.resolution = tuple(int(r) for r in resolution)
+        resolution = tuple(int(r) for r in resolution)
         if stats is None:
             stats = _ops.stack_stats(movie)
-        centers = patch_grid_centers((t, h, w), (1, ph, pw), (1, ph // 2, pw // 2), distribute_patches=True)
-        self.centers = centers
-        gh, gw = centers.shape[1:3]
-        self.g = gh * gw
-        flat = centers[0].reshape(-1, 3)
-        # patch window = floor(centre) - p // 2, no clipping (patch_utils.py:117-120,173-183; quirk Q20)
-        y0 = (flat[:, 1] - ph // 2).tolist()
-        x0 = (flat[:, 2] - pw // 2).tolist()
-        if min(y0) < 0 or min(x0) < 0 or max(y0) + ph > h or max(x0) + pw > w:
-            raise AssertionError(f"Patch size {tuple(patch_shape)} too large for control points in image of shape {(t, h, w)}")
+        centers, origins = local_patches((t, h, w), patch_shape)
+        base = base_grid(initial_field, resolution, dev)
+        plan = _fourier.BandPlan(ph, pw, dev, pixel_spacing, b_factor, frequency_range)
+        # for the tiled path the jobs are listed frame pair by frame pair, so the 50 %-overlapping patches of a pair run
+        # back to back and every frame comes from HBM once (patch-major order re-read it 2.3x: ncu); _init_state takes
+        # the same decision
+        frame_major = fused_steps_apply(LOSS_TYPES[loss_type], len(origins[0]), t, resolution, plan)
+        spec = local_spectra(movie, stats, plan, patch_shape, origins, frame_major)
+        geometry = (t, h, w, ph, pw)
+        centres_norm = cached_device_tensor(("local_centres", geometry), lambda: normalised_centres(centers, (t, h, w)), dev)
+        self._init_state(spec, frame_major, centres_norm, base, plan, patch_shape, kind, LOSS_TYPES[loss_type],
+                         pixel_spacing, geometry)
 
-        # frozen base grid (estimate_motion_optimizer.py:135-158)
-        if initial_field is None:
-            base = torch.zeros((2, *self.resolution), dtype=torch.float32, device=dev)
-        else:
-            base = resample_deformation_field(as_f32(initial_field, dev), self.resolution)
-            with torch.cuda.device(dev):
-                call("tmc_subtract_mean", ptr(base), base.numel(), stream_ptr(dev))
-        self.base = base
+    @classmethod
+    def from_spectra(cls, spec, frame_major, centres_norm, base, plan, patch_shape, kind, loss_type, pixel_spacing):
+        """A problem over spectra that are already on the device (the frame-split optimiser's share of the patches, with
+        ALL frames): spec / centres_norm laid out as ``local_spectra`` / ``normalised_centres`` make them.  Not entered
+        in the separable-weights cache, since its centres are no function of a movie geometry."""
+        problem = cls.__new__(cls)
+        problem._init_state(spec, frame_major, centres_norm, base, plan, patch_shape, kind, loss_type, pixel_spacing, None)
+        return problem
 
-        # spectra FW[g][t] = rfft2(mask * patch) * band * envelope on the pass-band box
-        self.plan = _fourier.BandPlan(ph, pw, dev, pixel_spacing, b_factor, frequency_range)
-        mask, ylo, yhi = _fourier.soft_disc_mask((ph, pw), pw / 4, pw / 4, dev)  # quirk Q18: smoothing pw/4
+    def _init_state(self, spec, frame_major, centres_norm, base, plan, patch_shape, kind, loss_type, pixel_spacing,
+                    geometry):
+        """Everything an iteration reads or writes, from the spectra (g * tp planes in ``frame_major`` order), the
+        (T, G, 3) normalised centres and the (2, nt, nh, nw) base grid.  ``geometry`` (t, h, w, ph, pw), which the
+        centres are a function of, keys the cache of the separable spline weights; None: not cached."""
+        self.spec, self.frame_major, self.centres_norm, self.base, self.plan = spec, frame_major, centres_norm, base, plan
+        self.kind, self.loss_type, self.px = kind, loss_type, float(pixel_spacing)
+        dev = spec.device
+        t, g = centres_norm.shape[:2]
+        self.dev, self.t, self.g = dev, t, g
+        self.ph, self.pw = patch_shape
         self.tp = 2 * ((t + 1) // 2)
-        self.fused = fused_steps_apply(self.loss_type, self.g, t, self.resolution, self.plan)
-        # frame-pair jobs; for the tiled path they are listed frame pair by frame pair, so the 50 %-overlapping patches of
-        # a pair run back to back and every frame comes from HBM once (patch-major order re-read it 2.3x: ncu)
-        self.frame_major = self.fused
-
-        def build_jobs():
-            jobs = []
-            if self.frame_major:
-                for i in range(0, t, 2):
-                    for gi in range(self.g):
-                        jobs.append([i, 1, i + 1 if i + 1 < t else -1, 1, y0[gi], x0[gi]])
-            else:
-                for gi in range(self.g):
-                    for i in range(0, t, 2):
-                        jobs.append([i, 1, i + 1 if i + 1 < t else -1, 1, y0[gi], x0[gi]])
-            return torch.tensor(jobs, dtype=torch.int32)
-
-        jobs = cached_device_tensor(("local_jobs", (t, h, w, ph, pw), self.frame_major), build_jobs, dev)
-        self.spec = self.plan.forward(movie, stats, mask, ylo, yhi, jobs, job_mode=2)  # (g * tp, KY, KX, 2), order see above
-        self.norms = torch.empty((self.g, t, 2), dtype=torch.float64, device=dev)
-        p = self.plan
+        self.resolution = tuple(base.shape[1:])
+        self.fused = fused_steps_apply(loss_type, g, t, self.resolution, plan)
+        self.norms = torch.empty((g, t, 2), dtype=torch.float64, device=dev)
+        p = plan
         with torch.cuda.device(dev):
-            call("tmc_local_spectra_norms", ptr(self.spec), self.g, t, self.tp, ph, pw, p.ky, p.kx, p.ky_start,
-                 int(self.frame_major), ptr(self.norms), stream_ptr(dev))
-
-        # normalised (t, y, x) centres, (T, G, 3) time-major (patch_utils.py:88-93,157-172; quirk Q10)
-        def build_centres():
-            norm = centers.clone().float()
-            norm[..., 0] /= float(t - 1) if t > 1 else float("nan")
-            norm[..., 1] /= float(h - 1)
-            norm[..., 2] /= float(w - 1)
-            return norm.reshape(t, self.g, 3).contiguous()
-
-        self.centres_norm = cached_device_tensor(("local_centres", (t, h, w, ph, pw)), build_centres, dev)
-        self.eval_base = _ops.spline_eval(base, self.kind, self.centres_norm)  # (T, G, 2)
-        ws_bytes = query("tmc_local_loss_workspace_bytes", self.g, t, p.ky, p.kx)
+            call("tmc_local_spectra_norms", ptr(spec), g, t, self.tp, self.ph, self.pw, p.ky, p.kx, p.ky_start,
+                 int(frame_major), ptr(self.norms), stream_ptr(dev))
+        self.eval_base = _ops.spline_eval(base, kind, centres_norm)  # (T, G, 2)
+        ws_bytes = query("tmc_local_loss_workspace_bytes", g, t, p.ky, p.kx)
         self.workspace = torch.empty(((ws_bytes + 7) // 8,), dtype=torch.float64, device=dev)
         self.loss = torch.zeros((1,), dtype=torch.float64, device=dev)
-        self.grad_eval = torch.empty((t, self.g, 2), dtype=torch.float32, device=dev)
+        self.grad_eval = torch.empty((t, g, 2), dtype=torch.float32, device=dev)
         # everything an iteration touches is allocated once: a captured step allocates nothing
-        self.eval_new = torch.empty((t, self.g, 2), dtype=torch.float32, device=dev)
+        self.eval_new = torch.empty((t, g, 2), dtype=torch.float32, device=dev)
         self.grad = torch.empty((2, *self.resolution), dtype=torch.float32, device=dev)
         n_ws = query("tmc_spline_workspace_floats", 2, *self.resolution)
         self.ws_eval = torch.empty((n_ws,), dtype=torch.float32, device=dev)
         self.ws_back = torch.empty((n_ws,), dtype=torch.float32, device=dev)
         if self.fused:
-            self._setup_fused_steps()
+            self._setup_fused_steps(geometry)
 
-    def _setup_fused_steps(self):
+    def _setup_fused_steps(self, geometry):
         """State of the one-kernel iteration (csrc/optimizer_tiled.cu): tiled spectra, the separable dense spline
         weights of the patch centres, accumulators.  The (g * tp, KY, KX) spectra are released."""
         dev, t, p = self.dev, self.t, self.plan
@@ -179,7 +234,6 @@ class LocalMotionProblem:
         # (T, nt) time matrix and a dense (G, nh nw) spatial matrix, phantom nodes folded in (spline of unit grids)
         # keyed by the geometry the centres are a function of (never by a device pointer); problems built from ad-hoc
         # centres (frame-split patch shards) carry no geometry key and are not cached
-        geometry = getattr(self, "geometry", None)
         key = ("local_weights", (dev.type, dev.index), self.kind, self.resolution, geometry) if geometry is not None else None
         hit = _separable_weights.get(key) if key is not None else None
         if hit is None:
@@ -213,19 +267,8 @@ class LocalMotionProblem:
                  float(b2), float(eps), float(wd), int(first_row), int(mode), int(n_steps), ptr(loss_out), ptr(self.grad),
                  ptr(self.step_ws), stream_ptr(self.dev))
 
-    def patch_scales(self, batches) -> torch.Tensor:
-        """Per-patch weight reproducing the reference's per-mini-batch ``mean`` (quirk Q11): the
-        gradient is the SUM over mini-batches of each batch's mean-reduced loss."""
-        scale = [0.0] * self.g
-        for batch in batches:
-            b = len(batch)
-            if self.loss_type == 0:
-                s = 1.0 / (b * self.t * self.ph * (self.pw // 2 + 1)) / (self.ph * self.pw)
-            else:
-                s = 1.0 / (b * self.t)
-            for gi in batch:
-                scale[gi] = s
-        return scale
+    def patch_scales(self, batches) -> list:
+        return patch_scales(batches, self.g, self.t, self.ph, self.pw, self.loss_type)
 
     def loss_and_grad(self, new_data: torch.Tensor, scale: torch.Tensor, iteration: torch.Tensor | None = None, row: int = 0):
         """Sum over mini-batches of the batch losses (device float64 (1,)) and d/d new_data.
@@ -383,9 +426,8 @@ def estimate_local_motion(
         # (torch.optim.Adam's foreach path costs ~15 launches for these <= few hundred parameters)
         fused_adam = optimizer_type.lower() == "adam" and not kwargs.get("amsgrad", False)
         if fused_adam:
-            exp_avg, exp_avg_sq = torch.zeros_like(new.data), torch.zeros_like(new.data)
-            lr, (b1, b2) = float(kwargs.get("lr", 0.01)), kwargs.get("betas", (0.9, 0.999))
-            eps, wd = float(kwargs.get("eps", 1e-08)), float(kwargs.get("weight_decay", 0))
+            adam = fused_adam_state(new.data, kwargs)
+            exp_avg, exp_avg_sq, lr, b1, b2, eps, wd = adam
 
         def one_step(i: int):
             if problem.fused:
@@ -396,8 +438,8 @@ def estimate_local_motion(
                 loss, grad = problem.loss_and_grad(new.data, scales[i])
             if fused_adam:
                 with torch.cuda.device(dev):
-                    call("tmc_adam_step", ptr(new.data), ptr(grad), ptr(exp_avg), ptr(exp_avg_sq), new.numel(), lr, float(b1),
-                         float(b2), eps, wd, ptr(counter), stream_ptr(dev))
+                    call("tmc_adam_step", ptr(new.data), ptr(grad), ptr(exp_avg), ptr(exp_avg_sq), new.numel(), lr, b1, b2,
+                         eps, wd, ptr(counter), stream_ptr(dev))
             else:
                 new.grad = grad
                 optimizer.step()
@@ -408,7 +450,7 @@ def estimate_local_motion(
         done = 0
         if problem.fused and fused_adam and not return_trajectory:
             losses = torch.empty((n_iterations,), dtype=torch.float64, device=dev)
-            problem.fused_steps(new.data, scales, 0, n_iterations, 0, losses, (exp_avg, exp_avg_sq, lr, b1, b2, eps, wd))
+            problem.fused_steps(new.data, scales, 0, n_iterations, 0, losses, adam)
             done = n_iterations
         elif fused and not problem.fused and not return_trajectory and n_iterations >= 4 and (fused_adam or _graph_capable(optimizer)):
             done = _run_captured(one_step, n_iterations, dev)
@@ -420,8 +462,7 @@ def estimate_local_motion(
                 )
 
     final = (new.data + problem.base).contiguous()
-    with torch.cuda.device(dev):
-        call("tmc_subtract_mean", ptr(final), final.numel(), stream_ptr(dev))
+    _ops.subtract_mean(final)
     if return_trajectory:
         return final, trajectory
     return final

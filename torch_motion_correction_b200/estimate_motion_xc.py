@@ -10,7 +10,6 @@ import torch
 
 from . import _fourier, _ops
 from ._common import as_f32, cached_device_tensor, resolve_device
-from ._lib import call, ptr, stream_ptr
 from .correct_motion import correct_motion, correct_motion_fast
 from .deformation_field_utils import resample_deformation_field
 from .patch_grid import patch_grid_centers
@@ -34,18 +33,22 @@ def estimate_global_motion(
     if reference_frame is None:
         reference_frame = t // 2
     stats = _stats if _stats is not None else _ops.stack_stats(movie)  # _stats: the pipeline computes them once per movie
-    plan = _fourier.BandPlan(h, w, dev, pixel_spacing, b_factor, frequency_range)
-    mask, ylo, yhi = _fourier.soft_disc_mask((h, w), min(h, w) / 4, min(h, w) / 8, dev)
-    spec = plan.forward(movie, stats, mask, ylo, yhi, _fourier.frame_pair_jobs(t, dev), job_mode=2)
+    plan, spec = global_spectra(movie, stats, pixel_spacing, b_factor, frequency_range)
     cur = torch.arange(t, dtype=torch.int32, device=dev)
     ref = torch.full((t,), int(reference_frame), dtype=torch.int32, device=dev)
     prod = _fourier.pair_products(spec, ref, cur, plan.plane_elems)
     shifts = plan.peaks(prod.view(t, plan.ky, plan.kx, 2), sub_pixel=False)
-    field = torch.empty((2, t, 1, 1), dtype=torch.float32, device=dev)
-    with torch.cuda.device(dev):
-        call("tmc_global_shifts_to_field", ptr(shifts), t, float(pixel_spacing), int(reference_frame), ptr(field),
-             stream_ptr(dev))
-    return field
+    return _ops.global_shifts_to_field(shifts, pixel_spacing, reference_frame)
+
+
+def global_spectra(frames: torch.Tensor, stats, pixel_spacing, b_factor, frequency_range):
+    """(plan, band-limited whole-frame spectra of ``frames`` (plane k = frame k)) under the soft disc of the whole-frame
+    cross-correlation."""
+    t, h, w = frames.shape
+    dev = frames.device
+    plan = _fourier.BandPlan(h, w, dev, pixel_spacing, b_factor, frequency_range)
+    mask, ylo, yhi = _fourier.soft_disc_mask((h, w), min(h, w) / 4, min(h, w) / 8, dev)
+    return plan, plan.forward(frames, stats, mask, ylo, yhi, _fourier.frame_pair_jobs(t, dev), job_mode=2)
 
 
 class _CacheModel:
@@ -106,6 +109,50 @@ def _aliasing_schedule(t: int, strategy: str, reference_frame: int):
         offsets.append(len(deltas))
         prev = row
     return offsets, deltas
+
+
+def patch_xc_geometry(shape, p: int, pixel_spacing, b_factor, frequency_range, base_field, dev):
+    """Patch grid of the cross-correlation of a (t, h, w) movie with p x p patches at 50 % overlap: (device centres
+    (t, gh, gw, 3), window origins [y0, x0] of every patch, plan, (mask, ylo, yhi), initial (2, t, gh, gw) field: zeros,
+    or ``base_field`` resampled onto the grid)."""
+    t, h, w = shape
+    centers = patch_grid_centers((t, h, w), (1, p, p), (1, p // 2, p // 2), distribute_patches=True)
+    gh, gw = centers.shape[1:3]
+    origins = (centers[0, :, :, 1:] - p // 2).reshape(-1, 2).tolist()
+    plan = _fourier.BandPlan(p, p, dev, pixel_spacing, b_factor, frequency_range)
+    mask = _fourier.soft_disc_mask((p, p), p / 4, p / 8, dev)
+    if base_field is None:
+        field = torch.zeros((2, t, gh, gw), dtype=torch.float32, device=dev)
+    else:
+        field = resample_deformation_field(base_field, (t, gh, gw))
+    return cached_device_tensor(("patch_centres", (t, h, w, p)), lambda: centers, dev), origins, plan, mask, field
+
+
+def mean_except_current_spectra(source, source_stats, plan, mask, p: int, origins, frame_shifts):
+    """(jobs, spectra) of every (frame, patch) of ``source`` under mask powers 1 and 2 (quirk Q1), frame-major: planes
+    (frame, patch, power)."""
+    t, h, w = source.shape
+    jobs = cached_device_tensor(
+        ("xc_jobs_mean", (t, h, w, p)),
+        lambda: torch.tensor([[k, 1, k, 2, y0, x0] for k in range(t) for (y0, x0) in origins], dtype=torch.int32),
+        source.device)
+    return jobs, plan.forward(source, source_stats, *mask, jobs, job_mode=1, frame_shifts=frame_shifts)
+
+
+def leave_one_out_shifts(spec: torch.Tensor, t: int, g: int, plan, sub_pixel) -> torch.Tensor:
+    """(t * g, 2) px peak shifts of every (frame, patch) against the sum of the other frames, from the frame-major
+    spectra of both mask powers of ALL t frames (``mean_except_current``; the mask powers of the leave-one-out
+    references follow the reference's patch cache, quirk Q1)."""
+    dev = spec.device
+
+    def schedule(part):
+        offsets, deltas = _aliasing_schedule(t, "mean_except_current", t // 2)
+        return torch.tensor(offsets if part == 0 else (deltas if deltas else [0]), dtype=torch.int32)
+
+    d_off = cached_device_tensor(("xc_delta_offsets", t), lambda: schedule(0), dev)
+    d_val = cached_device_tensor(("xc_deltas", t), lambda: schedule(1), dev)
+    prod = _fourier.leave_one_out_products(spec, t, g, plan.plane_elems, d_off, d_val)
+    return plan.peaks(prod.view(t * g, plan.ky, plan.kx, 2), sub_pixel=bool(sub_pixel))
 
 
 def estimate_motion_cross_correlation_patches(
@@ -186,36 +233,16 @@ def estimate_motion_cross_correlation_patches(
             source_stats = None
 
     p = int(patch_sidelength)
-    centers = patch_grid_centers((t, h, w), (1, p, p), (1, p // 2, p // 2), distribute_patches=True)
-    gh, gw = centers.shape[1:3]
-    n_patches = gh * gw
-    origins = (centers[0, :, :, 1:] - p // 2).reshape(-1, 2).tolist()
-
-    plan = _fourier.BandPlan(p, p, dev, pixel_spacing, b_factor, frequency_range)
-    mask, ylo, yhi = _fourier.soft_disc_mask((p, p), p / 4, p / 8, dev)
-
-    if deformation_field is None:
-        field = torch.zeros((2, t, gh, gw), dtype=torch.float32, device=dev)
-    else:
-        field = resample_deformation_field(deformation_field, (t, gh, gw))
+    centres, origins, plan, mask, field = patch_xc_geometry((t, h, w), p, pixel_spacing, b_factor, frequency_range,
+                                                            deformation_field, dev)
+    n_patches = len(origins)
 
     skip = -1
     if reference_strategy == "mean_except_current":
-        geometry = (t, h, w, p)
-        jobs = cached_device_tensor(
-            ("xc_jobs_mean", geometry),
-            lambda: torch.tensor([[k, 1, k, 2, y0, x0] for k in range(t) for (y0, x0) in origins], dtype=torch.int32), dev)
-        spec = plan.forward(source, source_stats, mask, ylo, yhi, jobs, job_mode=1, frame_shifts=frame_shifts)
+        jobs, spec = mean_except_current_spectra(source, source_stats, plan, mask, p, origins, frame_shifts)
         if dose_per_frame is not None:
             plan.dose_filter(spec, jobs, t, pixel_spacing, pre_exposure, dose_per_frame, voltage)
-
-        def schedule(part):
-            offsets, deltas = _aliasing_schedule(t, reference_strategy, reference_frame)
-            return torch.tensor(offsets if part == 0 else (deltas if deltas else [0]), dtype=torch.int32)
-
-        d_off = cached_device_tensor(("xc_delta_offsets", t), lambda: schedule(0), dev)
-        d_val = cached_device_tensor(("xc_deltas", t), lambda: schedule(1), dev)
-        prod = _fourier.leave_one_out_products(spec, t, n_patches, plan.plane_elems, d_off, d_val)
+        shifts = leave_one_out_shifts(spec, t, n_patches, plan, sub_pixel_refinement)
     else:
         skip = int(reference_frame)
 
@@ -226,16 +253,13 @@ def estimate_motion_cross_correlation_patches(
             )
 
         jobs = cached_device_tensor(("xc_jobs_middle", (t, h, w, p), int(reference_frame)), middle_jobs, dev)
-        spec = plan.forward(source, source_stats, mask, ylo, yhi, jobs, frame_shifts=frame_shifts)
+        spec = plan.forward(source, source_stats, *mask, jobs, frame_shifts=frame_shifts)
         if dose_per_frame is not None:
             plan.dose_filter(spec, jobs, t, pixel_spacing, pre_exposure, dose_per_frame, voltage)
         items = torch.arange(t * n_patches, dtype=torch.int32, device=dev)
         prod = _fourier.pair_products(spec, 2 * items + 1, 2 * items, plan.plane_elems)
-    shifts = plan.peaks(prod.view(t * n_patches, plan.ky, plan.kx, 2), sub_pixel=bool(sub_pixel_refinement))
+        shifts = plan.peaks(prod.view(t * n_patches, plan.ky, plan.kx, 2), sub_pixel=bool(sub_pixel_refinement))
 
-    scratch = torch.empty_like(field)
-    with torch.cuda.device(dev):
-        call("tmc_xc_postprocess", ptr(shifts), t, n_patches, float(pixel_spacing), skip, int(bool(outlier_rejection)),
-             float(outlier_threshold), int(bool(temporal_smoothing)), int(smoothing_window_size), 1, ptr(field), ptr(scratch),
-             stream_ptr(dev))
-    return field, cached_device_tensor(("patch_centres", (t, h, w, p)), lambda: centers, dev).clone()
+    _ops.xc_postprocess(shifts, field, pixel_spacing, skip, outlier_rejection, outlier_threshold, temporal_smoothing,
+                        smoothing_window_size)
+    return field, centres.clone()

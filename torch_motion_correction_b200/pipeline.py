@@ -26,7 +26,7 @@ def cumulative_patch_field(global_field: torch.Tensor, pixel_spacing: float, pat
     global track, quirk Q5, in the result.)
     ``patch_estimator(pre)`` must return ``(field (2, t, gh, gw), centres)`` computed with ``temporal_smoothing=False``
     and may negate ``pre`` in place or not."""
-    from ._lib import call, ptr, stream_ptr
+    from . import _ops
     from .deformation_field_utils import resample_deformation_field
 
     pre = global_field / float(pixel_spacing)
@@ -36,11 +36,8 @@ def cumulative_patch_field(global_field: torch.Tensor, pixel_spacing: float, pat
     used_base = resample_deformation_field(-handed, (t, gh, gw))  # what the estimator accumulated the patch shifts on
     field = (xc_field - used_base + resample_deformation_field(global_field, (t, gh, gw))).contiguous()
     zero_shifts = torch.zeros((t, gh * gw, 2), dtype=torch.float32, device=field.device)
-    scratch = torch.empty_like(field)
-    with torch.cuda.device(field.device):
-        # smoothing + one joint mean (quirk Q4) of the composed field: the estimator's own tail with nothing to add
-        call("tmc_xc_postprocess", ptr(zero_shifts), t, gh * gw, float(pixel_spacing), -1, 0, 0.0, 1, int(smoothing_window_size),
-             1, ptr(field), ptr(scratch), stream_ptr(field.device))
+    # smoothing + one joint mean (quirk Q4) of the composed field: the estimator's own tail with nothing to add
+    _ops.xc_postprocess(zero_shifts, field, pixel_spacing, -1, False, 0.0, True, smoothing_window_size)
     return field, centres
 
 
