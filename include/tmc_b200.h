@@ -223,6 +223,20 @@ int tmc_fourier_shift(void* spec, int t, int ny, int nx, const float* field, flo
 int tmc_irfft2_full(const void* spec, int nitems, int ny, int nx, const void* plan_x, const void* plan_y, void* tmp,
                     float* out, tmc_stream_t stream);
 
+/* ---- Fourier crop ("binning", MotionCor2 -FtBin) of whole frames ---------------------------------------------------- */
+/* image (t, h, w) -> out (t, out_h, out_w): rfft2, keep ky in [-out_h/2, out_h/2) and kx in [0, out_w/2], irfft2 at
+ * (out_h, out_w), times out_h out_w / (h w) so the mean pixel value is kept (the self-paired columns kx = 0 and
+ * kx = out_w/2 enter through their Hermitian part, as in numpy's irfft2).  All four sides even, out sides <= in sides,
+ * all four full-spectrum lengths (tmc_fft_supported_length == 1).  jobs: frame-pair jobs as for tmc_rfft2_band
+ * (job_mode 2) covering the t frames in order; plan_x / plan_y / plan_x_out / plan_y_out: plans of w, h, out_w, out_h;
+ * workspace: tmc_fourier_crop_workspace_bytes(t, h, w, out_h, out_w) bytes (-1: bad arguments).  Power-of-two heights
+ * cropped by 2 or 4 to >= 256 rows run the column passes as one kernel that keeps the cropped spectrum on chip
+ * (environment TMC_FFT_CROP_FUSED=0, read per call: two passes through HBM instead; the result is the same). */
+long tmc_fourier_crop_workspace_bytes(int t, int h, int w, int out_h, int out_w);
+int tmc_fourier_crop(const float* image, int t, int h, int w, int out_h, int out_w, const int* jobs, int njobs,
+                     const void* plan_x, const void* plan_y, const void* plan_x_out, const void* plan_y_out, void* workspace,
+                     float* out, tmc_stream_t stream);
+
 /* fused correct_motion_fast (power-of-two frame sides >= 256): rows r2c -> columns (FFT, phase, inverse FFT in one
  * kernel) -> rows c2r.  jobs: frame-pair jobs as for tmc_rfft2_band (job_mode 2) covering the t frames in order;
  * tmp: 2*njobs*ny*(nx/2+1) complex64; phase: t*ny complex64; out (t, ny, nx). */

@@ -29,7 +29,7 @@ from .optimization_state import OptimizationState, OptimizationTracker
 from .patch_grid import patch_grid_centers
 from .spline_grids import CubicBSplineGrid3d, CubicCatmullRomGrid3d
 from .pipeline import estimate_motion, motion_correct, motion_correct_many
-from .prepare import group_frames, prepare_movie
+from .prepare import fourier_crop, group_frames, prepare_movie
 from .movie_io import mrc_movies, read_mrc, read_mrc_header, write_mrc
 from .utils import normalize_image
 
@@ -55,6 +55,7 @@ __all__ = [
     "dose_weight",
     "prepare_movie",
     "group_frames",
+    "fourier_crop",
     "read_mrc",
     "read_mrc_header",
     "write_mrc",

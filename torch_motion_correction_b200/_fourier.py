@@ -226,6 +226,35 @@ class BandPlan:
         return out
 
 
+class CropPlan:
+    """Tables of one Fourier crop (h, w) -> (out_h, out_w) of whole frames (tmc_fourier_crop); the sizes have passed
+    ``prepare.fourier_crop_shape``."""
+
+    def __init__(self, h: int, w: int, out_h: int, out_w: int, device: torch.device):
+        self.h, self.w, self.out_h, self.out_w, self.device = h, w, out_h, out_w, device
+        self.tw = [twiddles(n, device) for n in (w, h, out_w, out_h)]
+
+    def crop(self, image: torch.Tensor) -> torch.Tensor:
+        """(t, h, w) contiguous fp32 on the plan's device -> (t, out_h, out_w).  Frames go through in chunks whose
+        row -> column intermediate stays near CHUNK_BYTES."""
+        t = image.shape[0]
+        dev = self.device
+        out = torch.empty((t, self.out_h, self.out_w), dtype=torch.float32, device=dev)
+        geometry = (self.h, self.w, self.out_h, self.out_w)
+        per_job = query("tmc_fourier_crop_workspace_bytes", 2, *geometry)
+        chunk = 2 * max(1, min((t + 1) // 2, CHUNK_BYTES // per_job))  # frames per call
+        ws = torch.empty((query("tmc_fourier_crop_workspace_bytes", min(chunk, t), *geometry),), dtype=torch.uint8, device=dev)
+        in_frame, out_frame = self.h * self.w * 4, self.out_h * self.out_w * 4
+        with torch.cuda.device(dev):
+            stream = stream_ptr(dev)
+            for f0 in range(0, t, chunk):
+                n = min(chunk, t - f0)
+                jobs = frame_pair_jobs(n, dev)
+                call("tmc_fourier_crop", image.data_ptr() + f0 * in_frame, n, *geometry, ptr(jobs), jobs.shape[0],
+                     *(ptr(tw) for tw in self.tw), ptr(ws), out.data_ptr() + f0 * out_frame, stream)
+        return out
+
+
 _tiles: dict = {}
 _self_paired: dict = {}
 

@@ -66,6 +66,8 @@ _SIGNATURES = {
     "tmc_xc_peak_partials": (I, [I, I]),
     "tmc_xc_peaks": (I, [P, I, I, I, I, I, I, I, P, P, P, P, P, P]),
     "tmc_irfft2_full": (I, [P, I, I, I, P, P, P, P, P]),
+    "tmc_fourier_crop_workspace_bytes": (L, [I, I, I, I, I]),
+    "tmc_fourier_crop": (I, [P, I, I, I, I, I, P, I, P, P, P, P, P, P, P]),
     "tmc_fourier_shift": (I, [P, I, I, I, P, F, P]),
     "tmc_fourier_shift_frames_supported": (I, [I, I]),
     "tmc_fourier_shift_frames": (I, [P, I, I, I, P, P, I, P, F, P, P, P, P, P, P]),

@@ -802,6 +802,93 @@ inline bool decimated_full_fits(int n) {
          fft_smem_runtime(m) + 1ull * b * n * sizeof(float2) <= kMaxSmem;
 }
 
+// row pass of tmc_rfft2_band: tmp[2 job + {0, 1}][y][kx] = row DFTs of the jobs' windows, kx < kx_count
+int rfft2_rows(const float* image, int h, int w, const float* mean_std, const float* mask, int ny, int nx, const int* jobs,
+               int njobs, int job_mode, const int* frame_shifts, int x_margin, int ylo, int yhi, int kx_count,
+               const AxisPlan& px, void* tmp, cudaStream_t stream) {
+  return dispatch_fft(nx, "rfft2_band", [&](auto M, auto BLU) {
+    constexpr int MM = decltype(M)::value;
+    constexpr bool BB = decltype(BLU)::value;
+    if constexpr (MM == 1024 && !BB) {
+      // polyphase path: four 256-point warp-level FFTs per row, only the band is ever formed
+      if (yhi > ylo && kx_count <= 128 && job_mode != 0 && use_poly() && px.R == 1) {
+        int rows_per_cta = 32;  // measured on C2: 64 .. 256 rows per CTA change the row kernels by less than 2 %
+        while (rows_per_cta > 8 && (long)tmc_div_up(yhi - ylo, rows_per_cta) * njobs < 148 * 6) rows_per_cta -= 8;
+        dim3 grid(tmc_div_up(yhi - ylo, rows_per_cta), njobs);
+        if (job_mode == 1) {
+          if (int e = enable_smem(poly::rows_forward_poly<1>, poly::smem_bytes)) return e;
+          TMC_TIMED("rows_forward_poly<1>", stream,
+                    poly::rows_forward_poly<1><<<grid, poly::kThreads, poly::smem_bytes, stream>>>(
+                        image, h, w, mean_std, mask, jobs, frame_shifts, x_margin, ylo, yhi, ny, kx_count, px.tw, (float2*)tmp,
+                        rows_per_cta));
+        } else {
+          if (int e = enable_smem(poly::rows_forward_poly<2>, poly::smem_bytes)) return e;
+          TMC_TIMED("rows_forward_poly<2>", stream,
+                    poly::rows_forward_poly<2><<<grid, poly::kThreads, poly::smem_bytes, stream>>>(
+                        image, h, w, mean_std, mask, jobs, frame_shifts, x_margin, ylo, yhi, ny, kx_count, px.tw, (float2*)tmp,
+                        rows_per_cta));
+        }
+        return TMC_OK;
+      }
+    }
+    if constexpr ((MM == 8192 || MM == 4096) && !BB) {
+      // rows of two frames as two half-length complex transforms of pixel pairs instead of one full-length transform
+      // of a packed pair (the 8192-point kernel is confined to one 8-warp CTA per SM)
+      if (yhi > ylo && job_mode == 2 && px.R == 1 && kx_count <= MM / 2 && use_real2n(MM)) {
+        constexpr int NH = MM / 2;
+        constexpr int B = fft2::Cfg<NH>::B;
+        int rows_per_cta = B * 4;
+        while (rows_per_cta > B && (long)tmc_div_up(yhi - ylo, rows_per_cta) * njobs < 148 * 8) rows_per_cta -= B;
+        dim3 grid(tmc_div_up(yhi - ylo, rows_per_cta), njobs);
+        constexpr size_t smem = rows_forward_real2n_smem_bytes<NH>();
+        if (int e = enable_smem(rows_forward_real2n<NH>, smem)) return e;
+        TMC_TIMED(MM == 8192 ? "rows_forward_real2n<4096>" : "rows_forward_real2n<2048>", stream,
+                  rows_forward_real2n<NH><<<grid, fft2::kThreads, smem, stream>>>(image, h, w, mean_std, mask, jobs, frame_shifts, x_margin,
+                                                                                   ylo, yhi, ny, kx_count, px.tw, (float2*)tmp,
+                                                                                   rows_per_cta));
+        return TMC_OK;
+      }
+    }
+    if constexpr (use_fast_path<MM, BB>()) if (px.R == 1) {
+      if (yhi > ylo) {
+        constexpr int B = fft2::Cfg<MM>::B;
+        // enough CTAs to fill the chip a few times over, each amortising its twiddle-table load
+        int rows_per_cta = B * 4;
+        while (rows_per_cta > B && (long)tmc_div_up(yhi - ylo, rows_per_cta) * njobs < 148 * 8) rows_per_cta -= B;
+        dim3 grid(tmc_div_up(yhi - ylo, rows_per_cta), njobs);
+        constexpr size_t smem = rows_forward_smem_bytes<MM>();
+#define TMC_ROWS_FWD(MODE)                                                                                      \
+  {                                                                                                             \
+    if (int e = enable_smem(rows_forward_p2<MM, MODE>, smem)) return e;                                         \
+    tmc_timing_begin(stream);                                                                                   \
+    rows_forward_p2<MM, MODE><<<grid, fft2::kThreads, smem, stream>>>(image, h, w, mean_std, mask, jobs, frame_shifts, \
+                                                                     x_margin, ylo, yhi, ny, kx_count, px.tw,          \
+                                                                     (float2*)tmp, rows_per_cta);                      \
+    tmc_timing_end(MM == 4096 ? "rows_forward_p2<4096>" : "rows_forward_p2", stream);                            \
+  }
+        if (job_mode == 1) TMC_ROWS_FWD(1) else if (job_mode == 2) TMC_ROWS_FWD(2) else TMC_ROWS_FWD(0)
+#undef TMC_ROWS_FWD
+        tmc_count_launch();
+      }
+      return TMC_OK;
+    }
+    // generic kernel (Bluestein lengths, small transforms, decimated long axes); the accumulators of a decimated axis
+    // follow the two transform buffers
+    const size_t smem = fft_smem_bytes<MM>() + (px.R > 1 ? 2ull * batch_for(MM) * kx_count * sizeof(float2) : 0);
+    if (smem > kMaxSmem) {
+      tmc_set_error("rfft2_band: band of %d bins too wide for the decimated row transform of length %d", kx_count, nx);
+      return TMC_ERR_UNSUPPORTED;
+    }
+    if (int e = enable_smem(rows_forward_kernel<MM, BB>, smem)) return e;
+    dim3 grid(tmc_div_up(yhi - ylo, batch_for(MM)), njobs);
+    if (yhi > ylo) {
+      TMC_TIMED("rows_forward_kernel", stream, rows_forward_kernel<MM, BB><<<grid, kThreads, smem, stream>>>(
+          image, h, w, mean_std, mask, jobs, frame_shifts, x_margin, ylo, yhi, ny, kx_count, px, (float2*)tmp));
+    }
+    return TMC_OK;
+  });
+}
+
 }  // namespace
 
 // ---- C ABI ---------------------------------------------------------------------------------------
@@ -903,87 +990,8 @@ TMC_API int tmc_rfft2_band(const float* image, int t, int h, int w, const float*
   TMC_CHECK_ARG(kx_count >= 1 && kx_count <= nx / 2 + 1 && ky_count >= 1 && ky_count <= ny, "rfft2_band: bad band box");
   if (njobs == 0) return TMC_OK;
   const AxisPlan px = make_axis_plan(plan_x, nx), py = make_axis_plan(plan_y, ny);
-  int rc = dispatch_fft(nx, "rfft2_band", [&](auto M, auto BLU) {
-    constexpr int MM = decltype(M)::value;
-    constexpr bool BB = decltype(BLU)::value;
-    if constexpr (MM == 1024 && !BB) {
-      // polyphase path: four 256-point warp-level FFTs per row, only the band is ever formed
-      if (yhi > ylo && kx_count <= 128 && job_mode != 0 && use_poly() && px.R == 1) {
-        int rows_per_cta = 32;  // measured on C2: 64 .. 256 rows per CTA change the row kernels by less than 2 %
-        while (rows_per_cta > 8 && (long)tmc_div_up(yhi - ylo, rows_per_cta) * njobs < 148 * 6) rows_per_cta -= 8;
-        dim3 grid(tmc_div_up(yhi - ylo, rows_per_cta), njobs);
-        if (job_mode == 1) {
-          if (int e = enable_smem(poly::rows_forward_poly<1>, poly::smem_bytes)) return e;
-          TMC_TIMED("rows_forward_poly<1>", stream,
-                    poly::rows_forward_poly<1><<<grid, poly::kThreads, poly::smem_bytes, stream>>>(
-                        image, h, w, mean_std, mask, jobs, frame_shifts, x_margin, ylo, yhi, ny, kx_count, px.tw, (float2*)tmp,
-                        rows_per_cta));
-        } else {
-          if (int e = enable_smem(poly::rows_forward_poly<2>, poly::smem_bytes)) return e;
-          TMC_TIMED("rows_forward_poly<2>", stream,
-                    poly::rows_forward_poly<2><<<grid, poly::kThreads, poly::smem_bytes, stream>>>(
-                        image, h, w, mean_std, mask, jobs, frame_shifts, x_margin, ylo, yhi, ny, kx_count, px.tw, (float2*)tmp,
-                        rows_per_cta));
-        }
-        return TMC_OK;
-      }
-    }
-    if constexpr ((MM == 8192 || MM == 4096) && !BB) {
-      // rows of two frames as two half-length complex transforms of pixel pairs instead of one full-length transform
-      // of a packed pair (the 8192-point kernel is confined to one 8-warp CTA per SM)
-      if (yhi > ylo && job_mode == 2 && px.R == 1 && kx_count <= MM / 2 && use_real2n(MM)) {
-        constexpr int NH = MM / 2;
-        constexpr int B = fft2::Cfg<NH>::B;
-        int rows_per_cta = B * 4;
-        while (rows_per_cta > B && (long)tmc_div_up(yhi - ylo, rows_per_cta) * njobs < 148 * 8) rows_per_cta -= B;
-        dim3 grid(tmc_div_up(yhi - ylo, rows_per_cta), njobs);
-        constexpr size_t smem = rows_forward_real2n_smem_bytes<NH>();
-        if (int e = enable_smem(rows_forward_real2n<NH>, smem)) return e;
-        TMC_TIMED(MM == 8192 ? "rows_forward_real2n<4096>" : "rows_forward_real2n<2048>", stream,
-                  rows_forward_real2n<NH><<<grid, fft2::kThreads, smem, stream>>>(image, h, w, mean_std, mask, jobs, frame_shifts, x_margin,
-                                                                                   ylo, yhi, ny, kx_count, px.tw, (float2*)tmp,
-                                                                                   rows_per_cta));
-        return TMC_OK;
-      }
-    }
-    if constexpr (use_fast_path<MM, BB>()) if (px.R == 1) {
-      if (yhi > ylo) {
-        constexpr int B = fft2::Cfg<MM>::B;
-        // enough CTAs to fill the chip a few times over, each amortising its twiddle-table load
-        int rows_per_cta = B * 4;
-        while (rows_per_cta > B && (long)tmc_div_up(yhi - ylo, rows_per_cta) * njobs < 148 * 8) rows_per_cta -= B;
-        dim3 grid(tmc_div_up(yhi - ylo, rows_per_cta), njobs);
-        constexpr size_t smem = rows_forward_smem_bytes<MM>();
-#define TMC_ROWS_FWD(MODE)                                                                                      \
-  {                                                                                                             \
-    if (int e = enable_smem(rows_forward_p2<MM, MODE>, smem)) return e;                                         \
-    tmc_timing_begin(stream);                                                                                   \
-    rows_forward_p2<MM, MODE><<<grid, fft2::kThreads, smem, stream>>>(image, h, w, mean_std, mask, jobs, frame_shifts, \
-                                                                     x_margin, ylo, yhi, ny, kx_count, px.tw,          \
-                                                                     (float2*)tmp, rows_per_cta);                      \
-    tmc_timing_end(MM == 4096 ? "rows_forward_p2<4096>" : "rows_forward_p2", stream);                            \
-  }
-        if (job_mode == 1) TMC_ROWS_FWD(1) else if (job_mode == 2) TMC_ROWS_FWD(2) else TMC_ROWS_FWD(0)
-#undef TMC_ROWS_FWD
-        tmc_count_launch();
-      }
-      return TMC_OK;
-    }
-    // generic kernel (Bluestein lengths, small transforms, decimated long axes); the accumulators of a decimated axis
-    // follow the two transform buffers
-    const size_t smem = fft_smem_bytes<MM>() + (px.R > 1 ? 2ull * batch_for(MM) * kx_count * sizeof(float2) : 0);
-    if (smem > kMaxSmem) {
-      tmc_set_error("rfft2_band: band of %d bins too wide for the decimated row transform of length %d", kx_count, nx);
-      return TMC_ERR_UNSUPPORTED;
-    }
-    if (int e = enable_smem(rows_forward_kernel<MM, BB>, smem)) return e;
-    dim3 grid(tmc_div_up(yhi - ylo, batch_for(MM)), njobs);
-    if (yhi > ylo) {
-      TMC_TIMED("rows_forward_kernel", stream, rows_forward_kernel<MM, BB><<<grid, kThreads, smem, stream>>>(
-          image, h, w, mean_std, mask, jobs, frame_shifts, x_margin, ylo, yhi, ny, kx_count, px, (float2*)tmp));
-    }
-    return TMC_OK;
-  });
+  int rc = rfft2_rows(image, h, w, mean_std, mask, ny, nx, jobs, njobs, job_mode, frame_shifts, x_margin, ylo, yhi, kx_count,
+                      px, tmp, stream);
   if (rc) return rc;
   TMC_CHECK_LAUNCH("tmc_rfft2_band(rows)");
   rc = dispatch_fft(ny, "rfft2_band", [&](auto M, auto BLU) {
@@ -1153,47 +1161,153 @@ TMC_API int tmc_xc_peaks(const void* prod, int nitems, int ny, int nx, int kx_co
   return TMC_OK;
 }
 
-// Full inverse: spec (nitems, ny, nx/2+1) complex64 -> out (nitems, ny, nx) f32 (irfftn, backward norm)
-TMC_API int tmc_irfft2_full(const void* spec, int nitems, int ny, int nx, const void* plan_x, const void* plan_y, void* tmp,
-                            float* out, cudaStream_t stream) {
-  TMC_CHECK_ARG(spec && plan_x && plan_y && tmp && out, "irfft2_full: null pointer");
-  if (nitems == 0) return TMC_OK;
-  const int kx = nx / 2 + 1;
-  const AxisPlan px = make_axis_plan(plan_x, nx), py = make_axis_plan(plan_y, ny);
-  int rc = dispatch_fft(ny, "irfft2_full", [&](auto M, auto BLU) {
+namespace {
+
+// inverse column pass of a (nitems, KY, KX) box (ky = ky_start + kyb, the box spans every ky of length ny) -> tmp
+// (nitems, ny, KX); entries beyond the box are zero
+int irfft2_cols(const void* spec, int nitems, int ny, int KX, int KY, int ky_start, const AxisPlan& py, void* tmp,
+                cudaStream_t stream, const char* who) {
+  return dispatch_fft(ny, who, [&](auto M, auto BLU) {
     constexpr int MM = decltype(M)::value;
     constexpr bool BB = decltype(BLU)::value;
     if constexpr (use_fast_path<MM, BB>()) if (py.R == 1) {
       if (int e = enable_smem(cols_inverse_p2<MM>, fft2::Cfg<MM>::smem_bytes)) return e;
-      dim3 grid(tmc_div_up(kx, fft2::Cfg<MM>::B), nitems);
-      TMC_TIMED(sized_label<MM>("cols_inverse_p2<4096>", "cols_inverse_p2<1024>", "cols_inverse_p2"), stream, cols_inverse_p2<MM><<<grid, fft2::kThreads, fft2::Cfg<MM>::smem_bytes, stream>>>((const float2*)spec, kx, ny, 0, py.tw,
+      dim3 grid(tmc_div_up(KX, fft2::Cfg<MM>::B), nitems);
+      TMC_TIMED(sized_label<MM>("cols_inverse_p2<4096>", "cols_inverse_p2<1024>", "cols_inverse_p2"), stream, cols_inverse_p2<MM><<<grid, fft2::kThreads, fft2::Cfg<MM>::smem_bytes, stream>>>((const float2*)spec, KX, KY, ky_start, py.tw,
                                                                                       (float2*)tmp));
       return TMC_OK;
     }
     if (int e = enable_smem(cols_inverse_kernel<MM, BB>, fft_smem_bytes<MM>())) return e;
-    dim3 grid(tmc_div_up(kx, batch_for(MM)), nitems);
-    TMC_TIMED("cols_inverse_kernel", stream, cols_inverse_kernel<MM, BB><<<grid, kThreads, fft_smem_bytes<MM>(), stream>>>((const float2*)spec, kx, ny, 0, py, (float2*)tmp));
+    dim3 grid(tmc_div_up(KX, batch_for(MM)), nitems);
+    TMC_TIMED("cols_inverse_kernel", stream, cols_inverse_kernel<MM, BB><<<grid, kThreads, fft_smem_bytes<MM>(), stream>>>((const float2*)spec, KX, KY, ky_start, py, (float2*)tmp));
     return TMC_OK;
   });
-  if (rc) return rc;
-  rc = dispatch_fft(nx, "irfft2_full", [&](auto M, auto BLU) {
+}
+
+// c2r row pass: tmp (nitems, ny, KX) -> out (nitems, ny, nx) f32 times `scale`.  Keeps only the real part of the
+// kx = 0 and kx = nx/2 entries, as c2r does.
+int irfft2_rows(const void* tmp, int nitems, int ny, int nx, int KX, const AxisPlan& px, float scale, float* out,
+                cudaStream_t stream, const char* who) {
+  return dispatch_fft(nx, who, [&](auto M, auto BLU) {
     constexpr int MM = decltype(M)::value;
     constexpr bool BB = decltype(BLU)::value;
     if constexpr (use_fast_path<MM, BB>()) if (px.R == 1) {
       if (int e = enable_smem(rows_inverse_store_p2<MM>, rows_inverse_smem_bytes<MM>())) return e;
       dim3 grid(tmc_div_up(ny, rows_per_cta_inverse<MM>()), nitems);
       TMC_TIMED(sized_label<MM>("rows_inverse_store_p2<4096>", "rows_inverse_store_p2<1024>", "rows_inverse_store_p2"), stream, rows_inverse_store_p2<MM><<<grid, fft2::kThreads, rows_inverse_smem_bytes<MM>(), stream>>>(
-          (const float2*)tmp, ny, kx, px.tw, 1.0f / ((float)nx * (float)ny), out));
+          (const float2*)tmp, ny, KX, px.tw, scale, out));
       return TMC_OK;
     }
     if (int e = enable_smem(rows_inverse_store_kernel<MM, BB>, fft_smem_bytes<MM>())) return e;
     dim3 grid(tmc_div_up(ny, 2 * batch_for(MM)), nitems);
-    TMC_TIMED("rows_inverse_store_kernel", stream, rows_inverse_store_kernel<MM, BB><<<grid, kThreads, fft_smem_bytes<MM>(), stream>>>((const float2*)tmp, ny, kx, px,
-                                                                                       1.0f / ((float)nx * (float)ny), out));
+    TMC_TIMED("rows_inverse_store_kernel", stream, rows_inverse_store_kernel<MM, BB><<<grid, kThreads, fft_smem_bytes<MM>(), stream>>>((const float2*)tmp, ny, KX, px,
+                                                                                       scale, out));
     return TMC_OK;
   });
-  if (rc) return rc;
+}
+
+}  // namespace
+
+// Full inverse: spec (nitems, ny, nx/2+1) complex64 -> out (nitems, ny, nx) f32 (irfftn, backward norm)
+TMC_API int tmc_irfft2_full(const void* spec, int nitems, int ny, int nx, const void* plan_x, const void* plan_y, void* tmp,
+                            float* out, cudaStream_t stream) {
+  TMC_CHECK_ARG(spec && plan_x && plan_y && tmp && out, "irfft2_full: null pointer");
+  if (nitems == 0) return TMC_OK;
+  const AxisPlan px = make_axis_plan(plan_x, nx), py = make_axis_plan(plan_y, ny);
+  if (int rc = irfft2_cols(spec, nitems, ny, nx / 2 + 1, ny, 0, py, tmp, stream, "irfft2_full")) return rc;
+  if (int rc = irfft2_rows(tmp, nitems, ny, nx, nx / 2 + 1, px, 1.0f / ((float)nx * (float)ny), out, stream, "irfft2_full"))
+    return rc;
   TMC_CHECK_LAUNCH("tmc_irfft2_full");
+  return TMC_OK;
+}
+
+// Fourier crop ("binning") of whole frames: bytes of the workspace tmc_fourier_crop needs for t frames
+TMC_API long tmc_fourier_crop_workspace_bytes(int t, int h, int w, int out_h, int out_w) {
+  if (t < 1 || h < 1 || w < 1 || out_h < 1 || out_w < 2) return -1;
+  const long planes = 2l * ((t + 1) / 2);
+  return planes * ((long)h + out_h) * (out_w / 2 + 1) * (long)sizeof(float2);
+}
+
+namespace {
+
+// TMC_FFT_CROP_FUSED=0 selects the composed column passes of tmc_fourier_crop where the fused kernel would run (A/B
+// testing; read per call: tests toggle it)
+inline bool use_crop_fused() {
+  const char* e = getenv("TMC_FFT_CROP_FUSED");
+  return !(e && e[0] == '0');
+}
+
+// calls f(IntC<N>{}, IntC<M>{}) when cols_crop_p2<N, M> serves a crop of h rows to out_h rows (powers of two, out_h h/2
+// or h/4 and >= 256); returns -1 without calling f otherwise
+template <typename F>
+int dispatch_crop_cols(int h, int out_h, F&& f) {
+#define TMC_CROP_CASE(NN, MM) \
+  if (h == NN && out_h == MM) return f(IntC<NN>{}, IntC<MM>{});
+  TMC_CROP_CASE(512, 256) TMC_CROP_CASE(1024, 512) TMC_CROP_CASE(1024, 256) TMC_CROP_CASE(2048, 1024)
+  TMC_CROP_CASE(2048, 512) TMC_CROP_CASE(4096, 2048) TMC_CROP_CASE(4096, 1024) TMC_CROP_CASE(8192, 4096)
+  TMC_CROP_CASE(8192, 2048)
+#undef TMC_CROP_CASE
+  return -1;
+}
+
+}  // namespace
+
+// image (t, h, w) f32 -> out (t, out_h, out_w) f32: rfft2, keep ky in [-out_h/2, out_h/2) and kx in [0, out_w/2], irfft2 at
+// (out_h, out_w), times out_h out_w / (h w) (the mean pixel value is kept).  Passes: rows r2c keeping kx <= out_w/2
+// (tmc_rfft2_band's row pass); the columns, fused (cols_crop_p2: forward at h, keep the ky box, inverse at out_h, in one
+// kernel) for the power-of-two crops dispatch_crop_cols lists, otherwise forward at h into the ky box and inverse at
+// out_h as two passes; rows c2r at out_w.
+// The box is not Hermitian on its self-paired columns kx = 0 and kx = out_w/2 (and ky = -out_h/2 has no partner); the
+// c2r row pass keeps only the real part of those columns' inverse, which is the inverse of their Hermitian part, as
+// numpy's and torch's irfft2 do.
+// jobs: frame-pair jobs (tmc_rfft2_band format, job_mode 2) covering the t frames in order (plane index == frame index
+// relative to out); workspace: tmc_fourier_crop_workspace_bytes(t, ...); plan_*: tmc_fft_plan_init buffers for w, h,
+// out_w, out_h.
+TMC_API int tmc_fourier_crop(const float* image, int t, int h, int w, int out_h, int out_w, const int* jobs, int njobs,
+                             const void* plan_x, const void* plan_y, const void* plan_x_out, const void* plan_y_out,
+                             void* workspace, float* out, cudaStream_t stream) {
+  TMC_CHECK_ARG(image && jobs && plan_x && plan_y && plan_x_out && plan_y_out && workspace && out,
+                "fourier_crop: null pointer");
+  TMC_CHECK_ARG(t >= 1 && 2 * njobs >= t && njobs <= (t + 1) / 2, "fourier_crop: jobs do not cover the frames");
+  TMC_CHECK_ARG(h >= 2 && w >= 2 && h % 2 == 0 && w % 2 == 0 && out_h >= 2 && out_w >= 2 && out_h % 2 == 0 &&
+                    out_w % 2 == 0,
+                "fourier_crop: sides must be even, got (%d, %d) -> (%d, %d)", h, w, out_h, out_w);
+  TMC_CHECK_ARG(out_h <= h && out_w <= w, "fourier_crop: output (%d, %d) larger than the input (%d, %d)", out_h, out_w, h, w);
+  for (int n : {h, w, out_h, out_w})
+    if (tmc_fft_supported_length(n) != 1) {
+      tmc_set_error("fourier_crop: transform length %d is not supported for full-spectrum transforms", n);
+      return TMC_ERR_UNSUPPORTED;
+    }
+  const int KX = out_w / 2 + 1;
+  float2* rows = (float2*)workspace;                       // (2 njobs, h, KX), then (t, out_h, KX)
+  float2* box = rows + 2l * njobs * h * KX;                // (2 njobs, out_h, KX)
+  const AxisPlan px_in = make_axis_plan(plan_x, w), py_in = make_axis_plan(plan_y, h);
+  const AxisPlan px = make_axis_plan(plan_x_out, out_w), py = make_axis_plan(plan_y_out, out_h);
+  const float scale = 1.0f / ((float)h * (float)w);
+  int rc = use_crop_fused() ? dispatch_crop_cols(h, out_h, [&](auto N, auto M) { return 0; }) : -1;
+  if (rc == 0) {
+    if ((rc = rfft2_rows(image, h, w, nullptr, nullptr, h, w, jobs, njobs, 2, nullptr, 0, 0, h, KX, px_in, rows, stream)))
+      return rc;
+    rc = dispatch_crop_cols(h, out_h, [&](auto N, auto M) {
+      constexpr int NN = decltype(N)::value, MM = decltype(M)::value;
+      constexpr size_t smem = cols_crop_smem_bytes<NN, MM>();
+      if (int e = enable_smem(cols_crop_p2<NN, MM>, smem)) return e;
+      dim3 grid(tmc_div_up(KX, fft2::Cfg<MM>::B), t);
+      TMC_TIMED("cols_crop_p2", stream, cols_crop_p2<NN, MM><<<grid, fft2::kThreads, smem, stream>>>(
+          (const float2*)rows, KX, py_in.tw, py.tw, box));
+      return TMC_OK;
+    });
+    if (rc) return rc;
+    rc = irfft2_rows(box, t, out_h, out_w, KX, px, scale, out, stream, "fourier_crop");
+  } else {
+    if ((rc = tmc_rfft2_band(image, t, h, w, nullptr, nullptr, h, w, jobs, njobs, 2, nullptr, 0, 0, h, KX, out_h,
+                             -(out_h / 2), nullptr, plan_x, plan_y, rows, box, stream)))
+      return rc;
+    if ((rc = irfft2_cols(box, t, out_h, KX, out_h, -(out_h / 2), py, rows, stream, "fourier_crop"))) return rc;
+    rc = irfft2_rows(rows, t, out_h, out_w, KX, px, scale, out, stream, "fourier_crop");
+  }
+  if (rc) return rc;
+  TMC_CHECK_LAUNCH("tmc_fourier_crop");
   return TMC_OK;
 }
 

@@ -703,6 +703,90 @@ cols_shift_p2(float2* __restrict__ tmp, int KX, int NX, const float2* __restrict
     }
 }
 
+// ---- Fourier crop, column pass: FFT along y at N, keep ky in [-M/2, M/2), inverse FFT at M ----------------------
+// tmp[plane][y][kx] (N rows) -> out[plane][y'][kx] (M rows, unnormalised): the forward and inverse column passes of
+// tmc_fourier_crop in one kernel, so the cropped spectrum never goes through HBM.  A CTA takes Cfg<M>::B columns; their
+// N-point transforms run in groups of Cfg<N>::B, each group leaving its M kept bins (re/im swapped: the next forward FFT
+// is the inverse) in the M-point buffers.  The M-point transform reads its inputs in the order cols_inverse_p2 reads
+// them from HBM, so both crop paths compute the same values.
+template <int N, int M>
+constexpr size_t cols_crop_smem_bytes() {
+  using CN = fft2::Cfg<N>;
+  using CM = fft2::Cfg<M>;
+  return (size_t)(CN::B * CN::STRIDE + CM::B * CM::STRIDE + 64 + CN::TW_HI + 64 + CM::TW_HI) * sizeof(float2);
+}
+
+template <int N, int M>
+__global__ void __launch_bounds__(fft2::kThreads)
+cols_crop_p2(const float2* __restrict__ tmp, int KX, const float2* __restrict__ tw_n, const float2* __restrict__ tw_m,
+             float2* __restrict__ out) {
+  using CN = fft2::Cfg<N>;
+  using CM = fft2::Cfg<M>;
+  using PN = fft2::Plan<N>;
+  using PM = fft2::Plan<M>;
+  static_assert(M < N && CM::B % CN::B == 0, "a CTA's M-point columns split into whole groups of N-point columns");
+  extern __shared__ float2 smem[];
+  float2* data_m = smem + CN::B * CN::STRIDE;
+  float2* tables = data_m + CM::B * CM::STRIDE;
+  fft2::Smem<N> sn(smem);
+  sn.tw_lo = tables;
+  sn.tw_hi = tables + 64;
+  fft2::Smem<M> sm(data_m);
+  sm.tw_lo = tables + 64 + CN::TW_HI;
+  sm.tw_hi = sm.tw_lo + 64;
+  fft2::load_twiddles<N>(sn, tw_n);
+  fft2::load_twiddles<M>(sm, tw_m);
+  const long plane = blockIdx.y;
+  const int kx0 = blockIdx.x * CM::B;
+  const float2* src = tmp + plane * N * KX;
+  {
+    const int seq = threadIdx.x % CN::B, j = threadIdx.x / CN::B;
+    float2* myseq = smem + seq * CN::STRIDE;
+#pragma unroll 1
+    for (int grp = 0; grp < CM::B / CN::B; ++grp) {
+      const int slot = grp * CN::B + seq;
+      const bool active = kx0 + slot < KX;
+      float2 v[CN::VPT];
+#pragma unroll
+      for (int g = 0; g < PN::First::G; ++g)
+#pragma unroll
+        for (int r = 0; r < PN::First::R; ++r)
+          v[g * PN::First::R + r] = active ? src[(long)PN::First::in_index(j, g, r) * KX + kx0 + slot] : make_float2(0.f, 0.f);
+      __syncthreads();  // tables loaded; the previous group has taken its last-pass inputs out of the N-point buffers
+      fft2::fft_regs_to_regs<N>(sn, myseq, j, v);
+      float2* mseq = data_m + slot * CM::STRIDE;
+#pragma unroll
+      for (int g = 0; g < PN::Last::G; ++g)
+#pragma unroll
+        for (int r = 0; r < PN::Last::R; ++r) {
+          const int ky = PN::Last::out_index(j, g, r);
+          const int pos = ky < M / 2 ? ky : (ky >= N - M / 2 ? ky - (N - M) : -1);
+          if (pos >= 0) {
+            const float2 val = PN::Last::result(v, g, r);
+            mseq[fft2::pad_idx(pos)] = make_float2(val.y, val.x);
+          }
+        }
+    }
+  }
+  __syncthreads();
+  const int seq = threadIdx.x % CM::B, j = threadIdx.x / CM::B;
+  float2* mseq = data_m + seq * CM::STRIDE;
+  float2 u[CM::VPT];
+  PM::First::load(mseq, j, u);
+  __syncthreads();
+  fft2::fft_regs_to_regs<M>(sm, mseq, j, u);
+  const int kx = kx0 + seq;
+  if (kx >= KX) return;
+  float2* dst = out + plane * M * KX + kx;
+#pragma unroll
+  for (int g = 0; g < PM::Last::G; ++g)
+#pragma unroll
+    for (int r = 0; r < PM::Last::R; ++r) {
+      const float2 val = PM::Last::result(u, g, r);
+      dst[(long)PM::Last::out_index(j, g, r) * KX] = make_float2(val.y, val.x);
+    }
+}
+
 // Four adjacent columns per CTA for the lengths whose FFT occupies a whole 256-thread group (Cfg<N>::B == 1, N = 4096):
 // with one column per CTA every 8-byte element of the (ny, nx/2+1) spectrum costs its own 32-byte sector on the way in
 // and on the way out (ncu r01g: 6.5x the algorithmic L2 traffic, the kernel's limiter).  Here a 512-thread CTA stages a

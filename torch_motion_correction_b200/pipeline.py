@@ -136,7 +136,7 @@ def estimate_motion(
 
 def motion_correct(image: torch.Tensor, pixel_spacing: float, grid_type: str = "bspline", device=None,
                    dose_per_frame: float | None = None, pre_exposure: float = 0.0, voltage: float = 300.0,
-                   frame_group: int | None = None, **estimate_kwargs):
+                   frame_group: int | None = None, fourier_bin: float | None = None, **estimate_kwargs):
     """Estimate + correct: returns ``(aligned frame sum (h, w), field)``.
 
     With ``dose_per_frame`` (e-/A^2 per frame) the patch cross-correlation is exposure pre-filtered and the sum is dose
@@ -145,7 +145,20 @@ def motion_correct(image: torch.Tensor, pixel_spacing: float, grid_type: str = "
 
     ``frame_group=G``: estimate on the sums of G consecutive frames (``estimate_motion``), then correct every raw frame
     with that field.  The dose-weighted sum is then formed without materialising the corrected stack
-    (``correct_motion_sums``), since grouping is meant for movies of hundreds of frames."""
+    (``correct_motion_sums``), since grouping is meant for movies of hundreds of frames.
+
+    ``fourier_bin=b`` (real >= 1; None or 1: off) Fourier-crops the movie by b first (``fourier_crop``: MotionCor2's
+    ``-FtBin``, for super-resolution movies) and runs everything on the cropped movie at ``b * pixel_spacing``:
+    estimation, frame grouping, the exposure pre-filter and the (dose-weighted) sum.  The sum is returned binned,
+    (h / b, w / b), and the field in Angstrom as always; ``patch_sidelength`` and the other keywords given in pixels are
+    then binned pixels.  To estimate binned but correct at full resolution, pass the field with the original movie and
+    pixel spacing to ``correct_motion_sums`` and crop the result (see ``fourier_crop``)."""
+    if fourier_bin is not None:
+        from .prepare import fourier_crop
+
+        binned = fourier_crop(image, fourier_bin, device=device)  # checks fourier_bin; factor 1 returns image itself
+        if binned is not image:
+            image, pixel_spacing = binned, fourier_bin * pixel_spacing  # the binned movie is freed when this call returns
     field, _ = estimate_motion(image, pixel_spacing, grid_type=grid_type, device=device, dose_per_frame=dose_per_frame,
                                pre_exposure=pre_exposure, voltage=voltage, frame_group=frame_group, **estimate_kwargs)
     if dose_per_frame is None:

@@ -87,3 +87,67 @@ def group_frames(movie: torch.Tensor, frame_group: int, device=None) -> torch.Te
     if groups.group_size == 1:
         return movie
     return _group_frames(as_f32(movie, resolve_device(movie, device)), groups.group_size)
+
+
+def fourier_crop_shape(shape, factor) -> tuple[int, int]:
+    """(h, w) -> (h', w') = (h / factor, w / factor), the frame size ``fourier_crop`` returns; the one place its argument
+    rules live.  Raised before any CUDA call:
+
+    * ``ValueError`` unless ``factor`` is a real number >= 1; for ``factor == 1`` the result is (h, w) and nothing else is
+      checked;
+    * ``ValueError`` unless h and w are even and h / factor, w / factor are whole numbers (to 1e-6 relative) that are even
+      too: factor 2 takes 11520 x 8184 to 5760 x 4092, factor 1.5 takes 5760 x 4092 to 3840 x 2728;
+    * ``NotImplementedError`` unless all four sides are lengths of the full-spectrum transforms
+      (``_fourier.unsupported_lengths``)."""
+    import math
+    import numbers
+
+    from ._fourier import unsupported_lengths
+
+    h, w = (int(n) for n in shape)
+    if isinstance(factor, bool) or not isinstance(factor, numbers.Real) or not math.isfinite(factor) or factor < 1:
+        raise ValueError(f"factor must be a real number >= 1, got {factor!r}")
+    if factor == 1:
+        return h, w
+    if h % 2 or w % 2:
+        raise ValueError(f"Fourier cropping needs even frame sides, got ({h}, {w})")
+    out = []
+    for n in (h, w):
+        exact = n / float(factor)
+        m = round(exact)
+        if m < 2 or m % 2 or abs(exact - m) > 1e-6 * exact:
+            raise ValueError(f"factor {factor} takes side {n} to {exact:g}, which is not an even whole number")
+        out.append(m)
+    for ny, nx in ((h, w), tuple(out)):
+        msg = unsupported_lengths(ny, nx, full=True)
+        if msg:
+            raise NotImplementedError(msg)
+    return out[0], out[1]
+
+
+def fourier_crop(image: torch.Tensor, factor, device=None) -> torch.Tensor:
+    """Fourier crop ("binning", MotionCor2 ``-FtBin``): (h, w) or (t, h, w) -> (h', w') or (t, h', w') fp32 with
+    (h', w') = ``fourier_crop_shape((h, w), factor)``.  ``factor == 1`` returns ``image`` itself.
+
+    Per frame: rfft2, keep the box ky in [-h'/2, h'/2), kx in [0, w'/2], irfft2 at (h', w'), times h' w' / (h w) so the
+    mean pixel value is kept.  The box's columns kx = 0 and kx = w'/2 enter through their Hermitian part, as in
+    numpy's and torch's irfft2.  Output pixel (i, j) is the band-limited image sampled at input position
+    (factor i, factor j): the field of view is unchanged and the pixel spacing becomes ``factor`` times the input's.
+
+    Deformation fields are in Angstrom on normalised coordinates, so a field estimated on the cropped movie also
+    describes the original one.  Normalised y maps to input row y factor (h' - 1) instead of y (h - 1), which is at most
+    factor - 1 input pixels apart at the far edge (the same for x).  To estimate on the binned movie but correct at full
+    resolution and crop afterwards, compose: ``fourier_crop(correct_motion_sums(movie, field, px)["sum"], 2)``."""
+    from ._common import as_f32
+    from ._fourier import CropPlan
+
+    if image.ndim not in (2, 3) or (image.ndim == 3 and image.shape[0] == 0):
+        raise ValueError(f"image must be (h, w) or (t, h, w) with t >= 1, got {tuple(image.shape)}")
+    h, w = image.shape[-2:]
+    out_h, out_w = fourier_crop_shape((h, w), factor)
+    if factor == 1:
+        return image
+    dev = resolve_device(image, device)
+    stack = as_f32(image, dev)
+    out = CropPlan(h, w, out_h, out_w, dev).crop(stack if image.ndim == 3 else stack[None])
+    return out if image.ndim == 3 else out[0]
