@@ -75,6 +75,17 @@ int tmc_subtract_frame_means(float* stack, int t, long n, const double* moments,
  * of frame_group consecutive frames; the last group also takes the t % frame_group leftover frames.  At least 2 groups.
  * Each sum is movie[first] + movie[first + 1] + ... added left to right in fp32 (one rounding per add, no reordering). */
 int tmc_group_frames(const float* movie, int t, int h, int w, int frame_group, float* groups, tmc_stream_t stream);
+/* EER electron-event frames (Falcon 4 / 4i) -> counts (n_frames / frames_per_fraction, h, w) of uint8 (count_bytes 1,
+ * frames_per_fraction <= 255) or uint16 (2, <= 65535): fraction k holds the electrons of frames [k F, (k + 1) F).
+ * payload (device, 4-byte aligned, payload_bytes long): the frames' bit streams; frame f is bytes
+ * [frame_offsets[f], frame_offsets[f + 1] - 8) followed by 8 zero bytes; frame_offsets (device int64, n_frames + 1).
+ * Codes are rle_bits (1..16) run lengths, escape 2^rle_bits - 1, each electron followed by sub_bits sub-pixel bits that
+ * are skipped (rle_bits + sub_bits <= 32).  counts (device, 4-byte aligned) must have room for the byte count rounded up
+ * to a multiple of 4; every element is written.  status (device int32, n_frames): 0 decoded, 1 malformed stream (runs out
+ * or moves past h * w before landing on it; contributes nothing), 2 offsets outside the payload.  No workspace. */
+int tmc_eer_render(const void* payload, long payload_bytes, const long long* frame_offsets, int n_frames, int h, int w,
+                   int rle_bits, int sub_bits, int frames_per_fraction, int count_bytes, void* counts, int* status,
+                   tmc_stream_t stream);
 
 /* ---- cubic spline grids: torch_cubic_spline_grids.Cubic{CatmullRom,BSpline}Grid3d as used at
  *      deformation_field_utils.py:9-93, estimate_motion_optimizer.py:487-490, correct_motion.py:288-305 */

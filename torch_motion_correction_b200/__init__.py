@@ -29,8 +29,8 @@ from .optimization_state import OptimizationState, OptimizationTracker
 from .patch_grid import patch_grid_centers
 from .spline_grids import CubicBSplineGrid3d, CubicCatmullRomGrid3d
 from .pipeline import estimate_motion, motion_correct, motion_correct_many
-from .prepare import fourier_crop, group_frames, prepare_movie
-from .movie_io import mrc_movies, read_mrc, read_mrc_header, write_mrc
+from .prepare import fourier_crop, group_frames, prepare_movie, render_eer
+from .movie_io import EerMovie, eer_movies, mrc_movies, read_eer, read_mrc, read_mrc_header, read_tiff, write_mrc
 from .utils import normalize_image
 
 __version__ = "0.1.0"
@@ -60,4 +60,9 @@ __all__ = [
     "read_mrc_header",
     "write_mrc",
     "mrc_movies",
+    "render_eer",
+    "read_eer",
+    "eer_movies",
+    "read_tiff",
+    "EerMovie",
 ]

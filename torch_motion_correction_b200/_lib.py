@@ -42,6 +42,7 @@ _SIGNATURES = {
     "tmc_remove_hot_pixels": (I, [P, I, I, I, P, F, I, P, P, P]),
     "tmc_subtract_frame_means": (I, [P, I, L, P, P]),
     "tmc_group_frames": (I, [P, I, I, I, I, P, P]),
+    "tmc_eer_render": (I, [P, L, P, I, I, I, I, I, I, I, P, P, P]),
     "tmc_spline_workspace_floats": (L, [I, I, I, I]),
     "tmc_spline_eval": (I, [P, I, I, I, I, I, P, L, P, P, P]),
     "tmc_spline_eval_backward": (I, [I, I, I, I, I, P, L, P, F, P, P, P]),

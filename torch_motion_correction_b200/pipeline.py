@@ -178,7 +178,7 @@ def motion_correct(image: torch.Tensor, pixel_spacing: float, grid_type: str = "
 
 
 def motion_correct_many(host_movies, pixel_spacing: float, device=None, out_host=None, gain=None, hot_pixel_threshold=None,
-                        zero_frame_means=False, **kwargs):
+                        zero_frame_means=False, eer_frames_per_fraction: int | None = None, **kwargs):
     """Align a sequence of movies held in (ideally pinned) HOST memory; yields ``(sum_host, field)``.
 
     Movies may arrive in their detector-native type (uint8 / int8 / uint16 / int16 / float16, or float32): they cross PCIe as
@@ -192,7 +192,15 @@ def motion_correct_many(host_movies, pixel_spacing: float, device=None, out_host
     The result of movie i is yielded only after movie i+1 has been enqueued and after the device-to-host copy of its sum
     has completed (a CUDA event is waited for), so ``sum_host`` is always safe to read; the overlap is kept because the
     GPU is already busy with movie i+1 while the host waits.  With ``out_host`` the same buffer is reused for every
-    movie: consume it before advancing the generator."""
+    movie: consume it before advancing the generator.
+
+    Items may also be EER movies (``read_eer`` / ``eer_movies``), which need ``eer_frames_per_fraction=F``: only their
+    compressed payload and frame table cross PCIe, into staging buffers that grow to the largest payload seen; they are
+    rendered on the device into a reused counts buffer (``render_eer``: n_frames // F fractions, the trailing frames
+    dropped) and go on as uint8 / uint16 movies.  ``dose_per_frame`` is then the dose of one fraction.  A movie with
+    malformed frames raises ``ValueError`` when its result would be handed out."""
+    from .movie_io import EerMovie
+
     dev = torch.device(device) if device is not None else torch.device("cuda", torch.cuda.current_device())
     movies = iter(host_movies)
     copy_stream = torch.cuda.Stream(device=dev)
@@ -204,7 +212,40 @@ def motion_correct_many(host_movies, pixel_spacing: float, device=None, out_host
     prepared = [None]  # one fp32 buffer: movie i is prepared into it while movie i + 1 is still in flight over PCIe
     gain_dev = gain.to(device=dev, dtype=torch.float32).contiguous() if gain is not None else None
 
+    eer_items = [None, None]  # the EerMovie staged in each slot (None: a tensor in buffers[slot])
+    eer_stage = [[None, None], [None, None]]  # per slot: device payload and frame-table buffers, grown, never shrunk
+    counts = [None]  # rendered EER counts of the current movie
+
+    def start_eer_copy(slot, eer):
+        from .prepare import eer_fractions
+
+        if eer_frames_per_fraction is None:
+            raise ValueError("motion_correct_many: EER movies need eer_frames_per_fraction=")
+        n, _ = eer_fractions(eer, eer_frames_per_fraction)
+        used = n * eer_frames_per_fraction
+        nbytes = int(eer.frame_offsets[used])
+        stage = eer_stage[slot]
+        grown = False
+        if stage[0] is None or stage[0].numel() < nbytes:
+            stage[0] = torch.empty((nbytes,), dtype=torch.uint8, device=dev)
+            grown = True
+        if stage[1] is None or stage[1].numel() < used + 1:
+            stage[1] = torch.empty((used + 1,), dtype=torch.int64, device=dev)
+            grown = True
+        eer_items[slot] = eer
+        with torch.cuda.stream(copy_stream):
+            copy_stream.wait_event(consumed[slot])
+            if grown:  # fresh memory from the main stream's pool: its earlier users must be done with it
+                copy_stream.wait_stream(main)
+            stage[0][:nbytes].copy_(eer.payload[:nbytes], non_blocking=True)
+            stage[1][:used + 1].copy_(eer.frame_offsets[:used + 1], non_blocking=True)
+            ready[slot].record(copy_stream)
+
     def start_copy(slot, host):
+        if isinstance(host, EerMovie):
+            start_eer_copy(slot, host)
+            return
+        eer_items[slot] = None
         if buffers[slot] is None or buffers[slot].shape != host.shape or buffers[slot].dtype != host.dtype:
             buffers[slot] = torch.empty(host.shape, dtype=host.dtype, device=dev)
         with torch.cuda.stream(copy_stream):
@@ -230,7 +271,23 @@ def motion_correct_many(host_movies, pixel_spacing: float, device=None, out_host
         if upcoming is not None:
             start_copy(1 - slot, upcoming)
         main.wait_event(ready[slot])
-        movie = buffers[slot]
+        status = None
+        if eer_items[slot] is not None:
+            from .prepare import eer_counts_buffer, eer_fractions, render_eer_into
+
+            eer = eer_items[slot]
+            n, dtype = eer_fractions(eer, eer_frames_per_fraction)
+            if counts[0] is None or counts[0].shape != (n, eer.h, eer.w) or counts[0].dtype != dtype:
+                counts[0] = eer_counts_buffer((n, eer.h, eer.w), dtype, dev)
+            used = n * eer_frames_per_fraction
+            status = torch.empty((used,), dtype=torch.int32, device=dev)
+            with torch.cuda.device(dev):
+                render_eer_into(eer_stage[slot][0][:int(eer.frame_offsets[used])], eer_stage[slot][1][:used + 1], eer,
+                                eer_frames_per_fraction, counts[0], status)
+            consumed[slot].record(main)  # the staging buffers are free as soon as the movie has been rendered
+            movie = counts[0]
+        else:
+            movie = buffers[slot]
         if movie.dtype != torch.float32 or gain_dev is not None or hot_pixel_threshold is not None or zero_frame_means:
             from .prepare import prepare_movie
 
@@ -244,21 +301,34 @@ def motion_correct_many(host_movies, pixel_spacing: float, device=None, out_host
             total, field = motion_correct(movie, pixel_spacing, device=dev, **kwargs)
             consumed[slot].record(main)
         if pending is not None and out_host is not None:
-            pending[2].synchronize()  # one shared host buffer: hand the previous result out before overwriting it
-            yield pending[0], pending[1]
+            yield _hand_out(pending)  # one shared host buffer: hand the previous result out before overwriting it
             pending = None
         host_sum = out_host if out_host is not None else torch.empty(total.shape, dtype=torch.float32, pin_memory=True)
+        host_status = torch.empty(status.shape, dtype=torch.int32, pin_memory=True) if status is not None else None
         done = torch.cuda.Event()
         d2h_stream.wait_stream(main)
         with torch.cuda.stream(d2h_stream):
             host_sum.copy_(total, non_blocking=True)
+            if status is not None:
+                host_status.copy_(status, non_blocking=True)
             done.record(d2h_stream)
         total.record_stream(d2h_stream)
+        if status is not None:
+            status.record_stream(d2h_stream)
         if pending is not None:
-            pending[2].synchronize()
-            yield pending[0], pending[1]
-        pending = (host_sum, field, done)
+            yield _hand_out(pending)
+        pending = (host_sum, field, done, host_status)
         nxt, slot = upcoming, 1 - slot
     if pending is not None:
-        pending[2].synchronize()
-        yield pending[0], pending[1]
+        yield _hand_out(pending)
+
+
+def _hand_out(pending):
+    """Wait for a result's device-to-host copy; raise if its EER render reported malformed frames."""
+    host_sum, field, done, host_status = pending
+    done.synchronize()
+    if host_status is not None:
+        from .prepare import check_eer_status
+
+        check_eer_status(host_status)
+    return host_sum, field

@@ -70,6 +70,78 @@ def prepare_movie(movie: torch.Tensor, gain: torch.Tensor | None = None, hot_pix
     return out
 
 
+def eer_fractions(eer, frames_per_fraction) -> tuple[int, torch.dtype]:
+    """``(n_fractions, counts dtype)`` of rendering ``eer`` in fractions of ``frames_per_fraction`` hardware frames:
+    ``n_frames // F`` fractions of uint8 counts for F <= 255, uint16 for F <= 65535 (a frame holds at most one electron
+    per pixel, so a fraction's count never exceeds F).  ``ValueError`` for fewer than 2 fractions or a bad F."""
+    import numbers
+
+    if isinstance(frames_per_fraction, bool) or not isinstance(frames_per_fraction, numbers.Integral) or not (
+            1 <= frames_per_fraction <= 65535):
+        raise ValueError(f"frames_per_fraction must be an integer in 1 .. 65535, got {frames_per_fraction!r}")
+    n = eer.n_frames // int(frames_per_fraction)
+    if n < 2:
+        raise ValueError(f"{eer.n_frames} EER frames in fractions of {frames_per_fraction} give {n} fraction(s), need >= 2")
+    return n, torch.uint8 if frames_per_fraction <= 255 else torch.uint16
+
+
+def eer_counts_buffer(shape, dtype, device) -> torch.Tensor:
+    """A counts tensor of ``shape`` whose storage is padded to a whole number of 4-byte words, as the render kernel's
+    word-wide increments need."""
+    n = shape[0] * shape[1] * shape[2]
+    words = (n * (1 if dtype == torch.uint8 else 2) + 3) // 4
+    return torch.empty((words,), dtype=torch.int32, device=device).view(dtype)[:n].view(shape)
+
+
+def render_eer_into(payload, frame_offsets, eer, frames_per_fraction, counts, status) -> None:
+    """Enqueue the render of the first ``counts.shape[0] * F`` frames (device ``payload`` / ``frame_offsets`` laid out as
+    ``eer``'s) into ``counts`` on the current stream; ``status`` (int32, one per rendered frame) gets 0 for a decoded
+    frame, 1 for a malformed one.  No synchronisation."""
+    n_frames = counts.shape[0] * frames_per_fraction
+    call("tmc_eer_render", ptr(payload), int(payload.numel()), ptr(frame_offsets), n_frames, eer.h, eer.w, eer.rle_bits,
+         eer.sub_bits, frames_per_fraction, counts.element_size(), ptr(counts), ptr(status), stream_ptr(counts.device))
+
+
+def check_eer_status(status_host: torch.Tensor, first_frame: int = 0) -> None:
+    """Raise ``ValueError`` naming the frames a render reported as malformed."""
+    bad = torch.nonzero(status_host).flatten().tolist()
+    if bad:
+        shown = ", ".join(str(first_frame + i) for i in bad[:20]) + (", ..." if len(bad) > 20 else "")
+        raise ValueError(f"malformed EER frame(s) {shown}: the bit stream runs out or moves past the frame's last pixel")
+
+
+def render_eer(eer, frames_per_fraction: int, device=None, out: torch.Tensor | None = None) -> torch.Tensor:
+    """EER movie (``read_eer``) -> electron counts (n_frames // F, h, w) on the device, F = ``frames_per_fraction``:
+    fraction k holds the electrons of hardware frames [k F, (k + 1) F).  uint8 for F <= 255, uint16 otherwise.
+
+    The trailing n_frames % F frames are DROPPED, as RELION's EER grouping does (``group_frames`` instead folds leftovers
+    into its last group): the fractions are the movie's frames for everything downstream, the exposure filter included,
+    so they must all carry the same dose.  Raises ``ValueError`` for fewer than 2 fractions.
+
+    Only the compressed payload crosses PCIe; the events are decoded on the device (``tmc_eer_render``).  A malformed
+    frame (its stream runs out, or moves past the last pixel, before it ends) contributes nothing and makes this raise
+    ``ValueError`` naming it: that check reads the per-frame status back, one host synchronisation per call.  The counts
+    go on through ``prepare_movie`` (gain, hot pixels, frame means -> fp32) like any other integer movie.
+    ``out``: a contiguous tensor of that shape and dtype whose size is a multiple of 4 bytes, reused instead of a new one."""
+    n, dtype = eer_fractions(eer, frames_per_fraction)
+    dev = resolve_device(eer.payload, device if device is not None else "cuda")  # the payload is a host tensor
+    shape = (n, eer.h, eer.w)
+    if out is None:
+        out = eer_counts_buffer(shape, dtype, dev)
+    elif tuple(out.shape) != shape or out.dtype != dtype or not out.is_contiguous() or out.device != dev or (
+            out.numel() * out.element_size()) % 4:
+        raise ValueError(f"out must be a contiguous {dtype} tensor of shape {shape} on {dev} with a size that is a "
+                         "multiple of 4 bytes")
+    used = n * frames_per_fraction
+    with torch.cuda.device(dev):
+        payload = eer.payload[:int(eer.frame_offsets[used])].to(dev, non_blocking=True)
+        offsets = eer.frame_offsets[:used + 1].to(dev, non_blocking=True)
+        status = torch.empty((used,), dtype=torch.int32, device=dev)
+        render_eer_into(payload, offsets, eer, frames_per_fraction, out, status)
+        check_eer_status(status.cpu())
+    return out
+
+
 def group_frames(movie: torch.Tensor, frame_group: int, device=None) -> torch.Tensor:
     """(t, h, w) movie -> (t // frame_group, h, w) fp32 sums of ``frame_group`` consecutive frames, the last group also
     taking the ``t % frame_group`` leftover frames (``frame_groups.frame_groups`` has the rule).  Each sum adds the frames
