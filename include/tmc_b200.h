@@ -17,6 +17,15 @@
  *     tmc_last_error() holds a thread-local message for the last non-zero status;
  *   - thread-safe for concurrent use from different host threads on different streams/devices;
  *   - images are float32, spectra complex64 (interleaved re,im), indices int32;
+ *   - counts of any size: tmc_rfft2_band (njobs), tmc_xc_pair_products and tmc_xc_peaks (nitems) and
+ *     tmc_irfft2_full (nitems) split longer calls into launches of at most 65535 planes / items themselves;
+ *     counts limited to 65535 per call (status 1 beyond, split the call): frames t of tmc_convert_stack,
+ *     tmc_remove_hot_pixels, tmc_subtract_frame_means, tmc_warp_dense_shifts, tmc_pixel_tyx, tmc_fourier_shift,
+ *     tmc_fourier_shift_frames and tmc_fourier_crop; frame groups of tmc_group_frames; patches g of
+ *     tmc_xc_leave_one_out_products, tmc_local_spectra_norms, tmc_local_loss_grad, tmc_local_steps and
+ *     tmc_local_tile_spectra (which limits t too); 2 njobs of tmc_dose_filter_spectra; rows (h, ny, ky_count) of tmc_pixel_shifts,
+ *     tmc_warp_dense_shifts, tmc_pixel_tyx, tmc_warp_lattice_backward, tmc_fourier_shift, tmc_dose_weighted_sum,
+ *     tmc_dose_lowrank_combine, tmc_soft_disc_mask and tmc_band_weights;
  *   - deformation fields are (2 [y,x], nt, nh, nw) float32 in Angstrom, spline `kind` 0 = Catmull-Rom,
  *     1 = cubic B-spline on [0,1]^3 (t, y, x).
  */

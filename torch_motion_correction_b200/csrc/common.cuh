@@ -11,6 +11,10 @@
 
 #define TMC_API extern "C" __attribute__((visibility("default")))
 
+// CUDA caps gridDim.y and gridDim.z at 65535.  Entry points that put a caller's job / item / plane count there either
+// split longer calls into slices of at most this many or reject them (include/tmc_b200.h says which).
+constexpr int kMaxGridYZ = 65535;
+
 // thread-local message for tmc_last_error()
 void tmc_set_error(const char* fmt, ...);
 // bookkeeping for bench.py: every kernel launch of this library is counted

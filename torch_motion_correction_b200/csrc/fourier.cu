@@ -989,6 +989,17 @@ TMC_API int tmc_rfft2_band(const float* image, int t, int h, int w, const float*
   TMC_CHECK_ARG(x_margin >= 0 && 2 * x_margin <= nx, "rfft2_band: bad x_margin %d", x_margin);
   TMC_CHECK_ARG(kx_count >= 1 && kx_count <= nx / 2 + 1 && ky_count >= 1 && ky_count <= ny, "rfft2_band: bad band box");
   if (njobs == 0) return TMC_OK;
+  constexpr int kMaxJobs = kMaxGridYZ / 2;  // the column pass puts 2 njobs planes on grid y
+  if (njobs > kMaxJobs) {  // slices in stream order: each reuses tmp from the start
+    for (int j0 = 0; j0 < njobs; j0 += kMaxJobs) {
+      const int n = njobs - j0 < kMaxJobs ? njobs - j0 : kMaxJobs;
+      if (int rc = tmc_rfft2_band(image, t, h, w, mean_std, mask, ny, nx, jobs + 6l * j0, n, job_mode, frame_shifts, x_margin,
+                                  ylo, yhi, kx_count, ky_count, ky_start, weight, plan_x, plan_y, tmp,
+                                  (float2*)out + 2l * j0 * ky_count * kx_count, stream))
+        return rc;
+    }
+    return TMC_OK;
+  }
   const AxisPlan px = make_axis_plan(plan_x, nx), py = make_axis_plan(plan_y, ny);
   int rc = rfft2_rows(image, h, w, mean_std, mask, ny, nx, jobs, njobs, job_mode, frame_shifts, x_margin, ylo, yhi, kx_count,
                       px, tmp, stream);
@@ -1049,6 +1060,15 @@ TMC_API int tmc_xc_pair_products(const void* spec, const int* ref_plane, const i
                                  void* out, cudaStream_t stream) {
   TMC_CHECK_ARG(spec && ref_plane && cur_plane && out && nitems >= 0 && plane_elems >= 1, "xc_pair_products: bad arguments");
   if (nitems == 0) return TMC_OK;
+  if (nitems > kMaxGridYZ) {
+    for (int i0 = 0; i0 < nitems; i0 += kMaxGridYZ) {
+      const int n = nitems - i0 < kMaxGridYZ ? nitems - i0 : kMaxGridYZ;
+      if (int rc = tmc_xc_pair_products(spec, ref_plane + i0, cur_plane + i0, n, plane_elems, (float2*)out + i0 * plane_elems,
+                                        stream))
+        return rc;
+    }
+    return TMC_OK;
+  }
   dim3 grid((unsigned)(tmc_div_up(plane_elems, 256) < 64 ? tmc_div_up(plane_elems, 256) : 64), nitems);
   TMC_TIMED("xc_pair_product_kernel", stream, xc_pair_product_kernel<<<grid, 256, 0, stream>>>((const float2*)spec, ref_plane, cur_plane, plane_elems, (float2*)out));
   TMC_CHECK_LAUNCH("tmc_xc_pair_products");
@@ -1062,6 +1082,7 @@ TMC_API int tmc_xc_leave_one_out_products(const void* spec, int t, int g, long p
   TMC_CHECK_ARG(spec && delta_offsets && deltas && out && t >= 2 && g >= 1 && plane_elems >= 1,
                 "xc_leave_one_out_products: bad arguments (need t >= 2)");
   TMC_CHECK_ARG(k_begin >= 0 && k_count >= 0 && k_begin + k_count <= t, "xc_leave_one_out_products: bad frame range");
+  TMC_CHECK_ARG(g <= kMaxGridYZ, "xc_leave_one_out_products: at most %d patches per frame, got %d", kMaxGridYZ, g);
   if (k_count == 0) return TMC_OK;
   dim3 grid(tmc_div_up(plane_elems, 128), g);
   TMC_TIMED("xc_leave_one_out_kernel", stream, xc_leave_one_out_kernel<<<grid, 128, 0, stream>>>((const float2*)spec, t, g, plane_elems, delta_offsets, deltas,
@@ -1094,6 +1115,15 @@ TMC_API int tmc_xc_peaks(const void* prod, int nitems, int ny, int nx, int kx_co
   TMC_CHECK_ARG(prod && plan_x && plan_y && tmp && partial && shifts, "xc_peaks: null pointer");
   TMC_CHECK_ARG(kx_count >= 1 && kx_count <= nx / 2 + 1 && ky_count >= 1 && ky_count <= ny, "xc_peaks: bad band box");
   if (nitems == 0) return TMC_OK;
+  if (nitems > kMaxGridYZ) {  // slices in stream order: each reuses tmp and partial from the start
+    for (int i0 = 0; i0 < nitems; i0 += kMaxGridYZ) {
+      const int n = nitems - i0 < kMaxGridYZ ? nitems - i0 : kMaxGridYZ;
+      if (int rc = tmc_xc_peaks((const float2*)prod + (long)i0 * ky_count * kx_count, n, ny, nx, kx_count, ky_count, ky_start,
+                                sub_pixel, plan_x, plan_y, tmp, partial, shifts + 2l * i0, stream))
+        return rc;
+    }
+    return TMC_OK;
+  }
   const AxisPlan px = make_axis_plan(plan_x, nx), py = make_axis_plan(plan_y, ny);
   int rc = dispatch_fft(ny, "xc_peaks", [&](auto M, auto BLU) {
     constexpr int MM = decltype(M)::value;
@@ -1129,7 +1159,8 @@ TMC_API int tmc_xc_peaks(const void* prod, int nitems, int ny, int nx, int kx_co
                       (const float2*)tmp, ny, kx_count, px.tw, (PeakCandidate*)partial));
         return TMC_OK;
       }
-      nparts = tmc_div_up(ny, rows_per_cta_inverse<MM>());
+      // the full-length p2 kernel below; a decimated axis (R > 1) runs the generic kernel, two rows per CTA
+      if (px.R == 1) nparts = tmc_div_up(ny, rows_per_cta_inverse<MM>());
     }
     if constexpr (MM == 1024 && !BB) {
       if (kx_count <= 128 && use_poly() && px.R == 1) {
@@ -1213,6 +1244,15 @@ TMC_API int tmc_irfft2_full(const void* spec, int nitems, int ny, int nx, const 
                             float* out, cudaStream_t stream) {
   TMC_CHECK_ARG(spec && plan_x && plan_y && tmp && out, "irfft2_full: null pointer");
   if (nitems == 0) return TMC_OK;
+  if (nitems > kMaxGridYZ) {  // slices in stream order: each reuses tmp from the start
+    for (int i0 = 0; i0 < nitems; i0 += kMaxGridYZ) {
+      const int n = nitems - i0 < kMaxGridYZ ? nitems - i0 : kMaxGridYZ;
+      if (int rc = tmc_irfft2_full((const float2*)spec + (long)i0 * ny * (nx / 2 + 1), n, ny, nx, plan_x, plan_y, tmp,
+                                   out + (long)i0 * ny * nx, stream))
+        return rc;
+    }
+    return TMC_OK;
+  }
   const AxisPlan px = make_axis_plan(plan_x, nx), py = make_axis_plan(plan_y, ny);
   if (int rc = irfft2_cols(spec, nitems, ny, nx / 2 + 1, ny, 0, py, tmp, stream, "irfft2_full")) return rc;
   if (int rc = irfft2_rows(tmp, nitems, ny, nx, nx / 2 + 1, px, 1.0f / ((float)nx * (float)ny), out, stream, "irfft2_full"))
@@ -1273,6 +1313,7 @@ TMC_API int tmc_fourier_crop(const float* image, int t, int h, int w, int out_h,
                     out_w % 2 == 0,
                 "fourier_crop: sides must be even, got (%d, %d) -> (%d, %d)", h, w, out_h, out_w);
   TMC_CHECK_ARG(out_h <= h && out_w <= w, "fourier_crop: output (%d, %d) larger than the input (%d, %d)", out_h, out_w, h, w);
+  TMC_CHECK_ARG(t <= kMaxGridYZ, "fourier_crop: at most %d frames per call, got %d", kMaxGridYZ, t);
   for (int n : {h, w, out_h, out_w})
     if (tmc_fft_supported_length(n) != 1) {
       tmc_set_error("fourier_crop: transform length %d is not supported for full-spectrum transforms", n);
@@ -1314,6 +1355,7 @@ TMC_API int tmc_fourier_crop(const float* image, int t, int h, int w, int out_h,
 // spec (t, ny, nx/2+1) *= exp(-2 pi i (fy sy + fx sx)); (sy, sx) = sign * field (2, t) (device)
 TMC_API int tmc_fourier_shift(void* spec, int t, int ny, int nx, const float* field, float sign, cudaStream_t stream) {
   TMC_CHECK_ARG(spec && field && t >= 1 && ny >= 1 && nx >= 2, "fourier_shift: bad arguments");
+  TMC_CHECK_ARG(t <= kMaxGridYZ && ny <= kMaxGridYZ, "fourier_shift: at most %d frames and rows, got (%d, %d)", kMaxGridYZ, t, ny);
   const int kx = nx / 2 + 1;
   dim3 grid(tmc_div_up(kx, 128), ny, t);
   TMC_TIMED("fourier_shift_kernel", stream, fourier_shift_kernel<<<grid, 128, 0, stream>>>((float2*)spec, t, ny, nx, kx, field, sign));
@@ -1335,6 +1377,7 @@ TMC_API int tmc_fourier_shift_frames(const float* image, int t, int ny, int nx, 
                                      void* tmp, void* phase, float* out, cudaStream_t stream) {
   TMC_CHECK_ARG(image && jobs && field && plan_x && plan_y && tmp && phase && out, "fourier_shift_frames: null pointer");
   TMC_CHECK_ARG(t >= 1 && 2 * njobs >= t, "fourier_shift_frames: jobs do not cover the frames");
+  TMC_CHECK_ARG(t <= kMaxGridYZ && njobs <= kMaxGridYZ, "fourier_shift_frames: at most %d frames per call, got %d", kMaxGridYZ, t);
   if (!tmc_fourier_shift_frames_supported(ny, nx)) {
     tmc_set_error("fourier_shift_frames: fused path needs power-of-two frame sides >= 256, got (%d, %d)", ny, nx);
     return TMC_ERR_UNSUPPORTED;

@@ -500,6 +500,7 @@ __global__ void shifts_grad_to_eval_kernel(const float* __restrict__ grad_shifts
 TMC_API int tmc_local_spectra_norms(const void* spec, int g, int t, int tp, int ny, int nx, int ky_count, int kx_count,
                                     int ky_start, int frame_major, double* norms, cudaStream_t stream) {
   TMC_CHECK_ARG(spec && norms && g >= 1 && t >= 1 && tp >= t, "local_spectra_norms: bad arguments");
+  TMC_CHECK_ARG(g <= kMaxGridYZ, "local_spectra_norms: at most %d patches, got %d", kMaxGridYZ, g);
   BandGeom geom{ny, nx, ky_count, kx_count, ky_start};
   TMC_CUDA(cudaMemsetAsync(norms, 0, sizeof(double) * (size_t)g * t * 2, stream));
   dim3 grid(tmc_div_up((long)ky_count * kx_count, kOptThreads), g);
@@ -532,6 +533,7 @@ TMC_API int tmc_local_loss_grad(const void* spec, const double* norms, const flo
                 "local_loss_grad: null pointer");
   TMC_CHECK_ARG(g >= 1 && t >= 1 && tp >= t && loss_type >= 0 && loss_type <= 2 && pixel_spacing > 0.f,
                 "local_loss_grad: bad arguments");
+  TMC_CHECK_ARG(g <= kMaxGridYZ, "local_loss_grad: at most %d patches, got %d", kMaxGridYZ, g);
   BandGeom geom{ny, nx, ky_count, kx_count, ky_start};
   const long bins = (long)ky_count * kx_count;
   float* wf = (float*)workspace;

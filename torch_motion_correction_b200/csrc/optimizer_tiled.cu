@@ -504,6 +504,7 @@ TMC_API int tmc_local_steps(const void* tiled, const int* tiles, int n_tiles, in
                             void* workspace, cudaStream_t stream) {
   TMC_CHECK_ARG(tiled && tiles && sum_norms && eval_base && w_t && w_sp && patch_scale && coef && loss_out && grad_out && workspace,
                 "local_steps: null pointer");
+  TMC_CHECK_ARG(g >= 1 && g <= kMaxGridYZ, "local_steps: at most %d patches, got %d", kMaxGridYZ, g);
   TMC_CHECK_ARG(mode >= 0 && mode <= 3, "local_steps: mode must be 0 .. 3");
   TMC_CHECK_ARG(mode == 1 || (exp_avg && exp_avg_sq), "local_steps: Adam state missing");
   TMC_CHECK_ARG(mode == 0 || n_steps == 1, "local_steps: modes 1 .. 3 take one step");

@@ -164,7 +164,10 @@ TMC_API int tmc_xc_postprocess(const float* shifts, int t, int g, float pixel_sp
       savgol_linear_kernel<<<tmc_div_up(2 * g, 64), 64, 0, stream>>>(scratch, t, g, window, field); tmc_count_launch();
     }
   }
-  if (subtract_mean) subtract_mean_kernel<<<1, 256, 0, stream>>>(field, 2l * t * g); tmc_count_launch();
+  if (subtract_mean) {
+    subtract_mean_kernel<<<1, 256, 0, stream>>>(field, 2l * t * g);
+    tmc_count_launch();
+  }
   TMC_CHECK_LAUNCH("tmc_xc_postprocess");
   return TMC_OK;
 }

@@ -211,6 +211,7 @@ int blocks_per_frame(int t) {
 TMC_API int tmc_convert_stack(const void* src, int dtype, int t, long n, const float* gain, float* dst, double* moments,
                               cudaStream_t stream) {
   TMC_CHECK_ARG(src && dst && t >= 1 && n >= 1, "convert_stack: bad arguments");
+  TMC_CHECK_ARG(t <= kMaxGridYZ, "convert_stack: at most %d frames per call, got %d", kMaxGridYZ, t);
   TMC_CHECK_ARG(dtype >= 0 && dtype <= 5,
                 "convert_stack: dtype must be 0 (uint8), 1 (uint16), 2 (int16), 3 (float16), 4 (float32) or 5 (int8)");
   if (moments) TMC_CUDA(cudaMemsetAsync(moments, 0, sizeof(double) * 2 * (size_t)t, stream));
@@ -238,6 +239,7 @@ TMC_API int tmc_remove_hot_pixels(float* stack, int t, int h, int w, double* mom
                                   void* workspace, int* hot_count, cudaStream_t stream) {
   TMC_CHECK_ARG(stack && moments && workspace && t >= 1 && h >= 1 && w >= 1 && capacity >= 1 && threshold > 0.f,
                 "remove_hot_pixels: bad arguments");
+  TMC_CHECK_ARG(t <= kMaxGridYZ, "remove_hot_pixels: at most %d frames per call, got %d", kMaxGridYZ, t);
   int* count = reinterpret_cast<int*>(workspace);
   HotPixel* list = reinterpret_cast<HotPixel*>(reinterpret_cast<char*>(workspace) + 16);
   TMC_CUDA(cudaMemsetAsync(count, 0, sizeof(int), stream));
@@ -252,6 +254,7 @@ TMC_API int tmc_remove_hot_pixels(float* stack, int t, int h, int w, double* mom
 // set_frames_mean_zero (examples/ttMotion.py:180-202): every frame minus its own mean (moments[f].sum / n), in place
 TMC_API int tmc_subtract_frame_means(float* stack, int t, long n, const double* moments, cudaStream_t stream) {
   TMC_CHECK_ARG(stack && moments && t >= 1 && n >= 1, "subtract_frame_means: bad arguments");
+  TMC_CHECK_ARG(t <= kMaxGridYZ, "subtract_frame_means: at most %d frames per call, got %d", kMaxGridYZ, t);
   dim3 grid(blocks_per_frame(t), t);
   TMC_TIMED("subtract_frame_means_kernel", stream, subtract_frame_means_kernel<<<grid, kPrepThreads, 0, stream>>>(stack, n, moments));
   TMC_CHECK_LAUNCH("tmc_subtract_frame_means");

@@ -224,7 +224,7 @@ TMC_API int tmc_dose_filter_spectra(void* spec, const int* jobs, int njobs, int 
                                                 dose_per_frame, voltage_kv >= 300.f ? 1.0f : 0.8f, tables, tables + bins);
     tmc_count_launch();
   }
-  TMC_CHECK_ARG(2l * njobs <= 65535, "dose_filter_spectra: too many planes for one launch (chunk the jobs)");
+  TMC_CHECK_ARG(2l * njobs <= kMaxGridYZ, "dose_filter_spectra: too many planes for one launch (chunk the jobs)");
   dim3 grid(tmc_div_up(bins, 256), 2 * njobs);
   dose_filter_spectra_kernel<<<grid, 256, 0, stream>>>((float2*)spec, jobs, bins, tables, tables + bins, pre_exposure,
                                                       dose_per_frame); tmc_count_launch();
@@ -240,6 +240,7 @@ TMC_API int tmc_dose_weighted_sum(const void* spec, int t, int ny, int nx, float
                                   int finalize, cudaStream_t stream) {
   TMC_CHECK_ARG(spec && out && t >= 1 && ny >= 1 && nx >= 2 && pixel_size > 0.f && frame_offset >= 0,
                 "dose_weighted_sum: bad arguments");
+  TMC_CHECK_ARG(ny <= kMaxGridYZ, "dose_weighted_sum: at most %d rows, got %d", kMaxGridYZ, ny);
   dim3 grid(tmc_div_up(nx / 2 + 1, 128), ny);
   dose_weighted_sum_kernel<<<grid, 128, 0, stream>>>((const float2*)spec, t, ny, nx, pixel_size, pre_exposure, dose_per_frame,
                                                     voltage_kv >= 300.f ? 1.0f : 0.8f, frame_offset, (float2*)out, den2,
@@ -253,6 +254,7 @@ TMC_API int tmc_soft_disc_mask(int h, int w, float radius, float smoothing_radiu
                                cudaStream_t stream) {
   TMC_CHECK_ARG(mask && workspace && h >= 1 && w >= 1 && radius >= 0.f && smoothing_radius >= 0.f,
                 "soft_disc_mask: bad arguments");
+  TMC_CHECK_ARG(h <= kMaxGridYZ, "soft_disc_mask: at most %d rows, got %d", kMaxGridYZ, h);
   const int cy = h / 2, cx = w / 2;  // torch_grid_utils: centre = shape // 2
   disc_rows_kernel<<<tmc_div_up(h, 128), 128, 0, stream>>>(h, w, cy, cx, radius, workspace); tmc_count_launch();
   dim3 grid(tmc_div_up(w, 128), h);
@@ -265,6 +267,7 @@ TMC_API int tmc_band_weights(int ny, int nx, int ky_count, int kx_count, int ky_
                              float b_factor, float pixel_size, int use_envelope, float* weight, cudaStream_t stream) {
   TMC_CHECK_ARG(weight && ny >= 1 && nx >= 1 && ky_count >= 1 && kx_count >= 1 && kx_count <= nx / 2 + 1 && pixel_size > 0.f,
                 "band_weights: bad arguments");
+  TMC_CHECK_ARG(ky_count <= kMaxGridYZ, "band_weights: at most %d rows, got %d", kMaxGridYZ, ky_count);
   dim3 grid(tmc_div_up(kx_count, 128), ky_count);
   band_weight_kernel<<<grid, 128, 0, stream>>>(ny, nx, ky_count, kx_count, ky_start, low, high, use_band, b_factor,
                                               pixel_size, use_envelope, weight); tmc_count_launch();
@@ -281,6 +284,7 @@ TMC_API int tmc_dose_lowrank_combine(const void* spec, int n_spec, int ny, int n
   TMC_CHECK_ARG(spec && table && plane_outputs && out, "dose_lowrank_combine: null pointer");
   TMC_CHECK_ARG(n_spec >= 1 && ny >= 1 && nx >= 2 && n_table >= 2, "dose_lowrank_combine: bad shape n_spec=%d ny=%d nx=%d "
                 "n_table=%d", n_spec, ny, nx, n_table);
+  TMC_CHECK_ARG(ny <= kMaxGridYZ, "dose_lowrank_combine: at most %d rows, got %d", kMaxGridYZ, ny);
   TMC_CHECK_ARG(n_out >= 1 && n_out <= kMaxLowRankOutputs, "dose_lowrank_combine: n_out=%d outside [1, %d]", n_out,
                 kMaxLowRankOutputs);
   TMC_CHECK_ARG(pixel_size > 0.f && x_max > 0.f, "dose_lowrank_combine: pixel_size and x_max must be > 0");

@@ -814,6 +814,7 @@ TMC_API int tmc_warp_lattice_sums(const float* image, int t, int h, int w, const
 TMC_API int tmc_pixel_shifts(const float* lattice, int lh, int lw, int h, int w, float pixel_spacing, float* out,
                              cudaStream_t stream) {
   TMC_CHECK_ARG(lattice && out && lh >= 1 && lw >= 1 && h >= 2 && w >= 2 && pixel_spacing > 0.f, "pixel_shifts: bad arguments");
+  TMC_CHECK_ARG(h <= kMaxGridYZ, "pixel_shifts: at most %d rows, got %d", kMaxGridYZ, h);
   dim3 grid(tmc_div_up(w, 128), h);
   TMC_TIMED("pixel_shifts_kernel", stream, pixel_shifts_kernel<<<grid, 128, 0, stream>>>(lattice, lh, lw, h, w, pixel_spacing, out));
   TMC_CHECK_LAUNCH("tmc_pixel_shifts");
@@ -823,6 +824,7 @@ TMC_API int tmc_pixel_shifts(const float* lattice, int lh, int lw, int h, int w,
 TMC_API int tmc_warp_dense_shifts(const float* image, int t, int h, int w, const float* shifts, float* out_stack,
                                   cudaStream_t stream) {
   TMC_CHECK_ARG(image && shifts && out_stack && t >= 1 && h >= 2 && w >= 2, "warp_dense_shifts: bad arguments");
+  TMC_CHECK_ARG(t <= kMaxGridYZ && h <= kMaxGridYZ, "warp_dense_shifts: at most %d frames and rows, got (%d, %d)", kMaxGridYZ, t, h);
   dim3 grid(tmc_div_up(w, 128), h, t);
   TMC_TIMED("warp_dense_shifts_kernel", stream, warp_dense_shifts_kernel<<<grid, 128, 0, stream>>>(image, t, h, w, shifts, out_stack));
   TMC_CHECK_LAUNCH("tmc_warp_dense_shifts");
@@ -831,6 +833,7 @@ TMC_API int tmc_warp_dense_shifts(const float* image, int t, int h, int w, const
 
 TMC_API int tmc_pixel_tyx(int h, int w, int t, int frame_offset, int total_frames, float* tyx, cudaStream_t stream) {
   TMC_CHECK_ARG(tyx && t >= 1 && h >= 2 && w >= 2 && total_frames >= t + frame_offset, "pixel_tyx: bad arguments");
+  TMC_CHECK_ARG(t <= kMaxGridYZ && h <= kMaxGridYZ, "pixel_tyx: at most %d frames and rows, got (%d, %d)", kMaxGridYZ, t, h);
   dim3 grid(tmc_div_up(w, 128), h, t);
   TMC_TIMED("pixel_tyx_kernel", stream, pixel_tyx_kernel<<<grid, 128, 0, stream>>>(h, w, t, frame_offset, total_frames, tyx));
   TMC_CHECK_LAUNCH("tmc_pixel_tyx");
@@ -844,6 +847,7 @@ TMC_API int tmc_warp_lattice_backward(const float* image, int t, int h, int w, c
                                       cudaStream_t stream) {
   TMC_CHECK_ARG(image && lattice && grad_out && grad_lattice && workspace, "warp_lattice_backward: null pointer");
   TMC_CHECK_ARG(t >= 1 && h >= 2 && w >= 2 && lh >= 1 && lw >= 1 && pixel_spacing > 0.f, "warp_lattice_backward: bad arguments");
+  TMC_CHECK_ARG(h <= kMaxGridYZ, "warp_lattice_backward: at most %d rows, got %d", kMaxGridYZ, h);
   const long rows = (long)t * 2 * lh;
   float* rx = workspace;
   float* grad_rx = workspace + rows * w;
