@@ -250,8 +250,8 @@ int tmc_irfft2_full(const void* spec, int nitems, int ny, int nx, const void* pl
  * all four full-spectrum lengths (tmc_fft_supported_length == 1).  jobs: frame-pair jobs as for tmc_rfft2_band
  * (job_mode 2) covering the t frames in order; plan_x / plan_y / plan_x_out / plan_y_out: plans of w, h, out_w, out_h;
  * workspace: tmc_fourier_crop_workspace_bytes(t, h, w, out_h, out_w) bytes (-1: bad arguments).  Power-of-two heights
- * cropped by 2 or 4 to >= 256 rows run the column passes as one kernel that keeps the cropped spectrum on chip
- * (environment TMC_FFT_CROP_FUSED=0, read per call: two passes through HBM instead; the result is the same). */
+ * cropped by 2 or 4 to >= 256 rows run the column passes as one kernel that keeps the cropped spectrum on chip; other
+ * heights run them as two passes through HBM (forward into the ky box, inverse at out_h). */
 long tmc_fourier_crop_workspace_bytes(int t, int h, int w, int out_h, int out_w);
 int tmc_fourier_crop(const float* image, int t, int h, int w, int out_h, int out_w, const int* jobs, int njobs,
                      const void* plan_x, const void* plan_y, const void* plan_x_out, const void* plan_y_out, void* workspace,

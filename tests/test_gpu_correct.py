@@ -7,7 +7,8 @@ import torch
 import torch_motion_correction_b200 as tmc
 from oracle import deps
 from oracle import reference_path as rp
-from torch_motion_correction_b200 import _ops
+from torch_motion_correction_b200 import _lib, _ops
+from warp_kernels import at_offset, warp_kernels_ran
 
 pytestmark = pytest.mark.gpu
 
@@ -138,32 +139,34 @@ def test_correct_motion_ragged_sizes_and_big_shifts(dev, shape):
     assert float((want == 0).float().mean()) > 0.01  # the case really exercises the zero fill
 
 
-@pytest.mark.parametrize("tma", ["0", "1"])
+@pytest.mark.parametrize("layout", ["aligned", "offset"])
 @pytest.mark.parametrize("amplitude", [2.0, 40.0])
 @pytest.mark.parametrize("shape,grid", [((5, 300, 388), (3, 4, 5)), ((3, 331, 260), (3, 2, 2)), ((41, 64, 128), (41, 1, 1))])
-def test_correct_motion_tma_tiles(dev, shape, grid, amplitude, tma, monkeypatch):
-    """Images with 16-byte aligned rows run on the TMA-staged tile kernel (TMC_WARP_TMA=0: the global-memory kernel):
+def test_correct_motion_tma_tiles(dev, shape, grid, amplitude, layout):
+    """Images with 16-byte aligned rows run on the TMA-staged tile kernel (one float off: the global-memory kernel):
     smooth fields (taps inside the staged boxes), a wild field (boxes hang over the frame edge, taps leave the boxes:
     per-pixel fall-backs, zero fill outside the frame), ragged tile edges, more frames than pipeline stages, stack
     output and fused sum, accumulation into an existing sum."""
-    monkeypatch.setenv("TMC_WARP_TMA", tma)
     g = torch.Generator().manual_seed(21)
     img = torch.randn(shape, generator=g)
     field = torch.randn((2, *grid), generator=g) * amplitude
     want = rp.correct_motion(img, field, 1.1, "bspline")
-    got = tmc.correct_motion(img.to(dev), field.to(dev), 1.1, grid_type="bspline")
+    m = img.to(dev) if layout == "aligned" else at_offset(img.to(dev))
+    _lib.kernel_timing(True)
+    got = tmc.correct_motion(m, field.to(dev), 1.1, grid_type="bspline")
     assert rel_l2(got, want) <= REL_L2
-    total = tmc.correct_motion_sum(img.to(dev), field.to(dev), 1.1, grid_type="bspline")
+    total = tmc.correct_motion_sum(m, field.to(dev), 1.1, grid_type="bspline")
     assert rel_l2(total, want.sum(dim=0)) <= REL_L2
     # accumulate into an existing sum (frame blocks of one movie)
     again = total.clone()
-    tmc.correct_motion_sum(img.to(dev), field.to(dev), 1.1, grid_type="bspline", out=again, accumulate=True)
+    tmc.correct_motion_sum(m, field.to(dev), 1.1, grid_type="bspline", out=again, accumulate=True)
     assert rel_l2(again, 2 * want.sum(dim=0)) <= REL_L2
+    assert warp_kernels_ran() == {"warp_tma_kernel" if layout == "aligned" else "warp_lattice_kernel"}
 
 
-def test_tma_and_global_memory_kernels_agree(dev, monkeypatch):
+def test_tma_and_global_memory_kernels_agree(dev):
     """Same arithmetic up to the evaluation order of the Keys weights: 2048^2, shifts of a few pixels plus one corner
-    pushed far outside, normalised output."""
+    pushed far outside, normalised output.  The frames one float off their allocation run on the global-memory kernel."""
     g = torch.Generator().manual_seed(5)
     img = torch.randn((7, 2048, 2048), generator=g).to(dev)
     field = torch.randn((2, 3, 5, 5), generator=g) * 4.0
@@ -175,10 +178,11 @@ def test_tma_and_global_memory_kernels_agree(dev, monkeypatch):
     stats = _ops.stack_stats(img)
     lattice = _ops.spline_lattice(field, grid_kind("bspline"), 7, 50, 50)
     outs = {}
-    for tma in ("0", "1"):
-        monkeypatch.setenv("TMC_WARP_TMA", tma)
+    for tma, frames, kernel in (("1", img, "warp_tma_kernel"), ("0", at_offset(img), "warp_lattice_kernel")):
         stack, total = torch.empty_like(img), torch.empty_like(img[0])
-        _ops.warp_lattice(img, lattice, 0.83, mean_std=stats, out_stack=stack, out_sum=total)
+        _lib.kernel_timing(True)
+        _ops.warp_lattice(frames, lattice, 0.83, mean_std=stats, out_stack=stack, out_sum=total)
+        assert warp_kernels_ran() == {kernel}
         outs[tma] = (stack, total)
     # the kernels evaluate the Keys weights in different (equivalent) orders: ~1e-7 per weight, 16 taps
     assert rel_l2(outs["1"][0], outs["0"][0]) <= 5e-6

@@ -8,6 +8,7 @@ import pytest
 import torch
 import torch.distributed as dist
 import torch.multiprocessing as mp
+from warp_kernels import at_offset, warp_kernels_ran
 
 pytestmark = pytest.mark.gpu
 
@@ -42,13 +43,19 @@ def _exact_dose_weighted(stack, frames, px, dose, pre, kv, total_rows):
     return torch.fft.irfft2(acc / torch.sqrt(den2), s=(h, w))
 
 
-@pytest.mark.parametrize("tma", ["1", "0"])
-@pytest.mark.parametrize("shape", [(6, 96, 128), (7, 64, 90), (3, 600, 5000), (25, 256, 384)])
-def test_sum_is_correct_motion_sum(shape, tma, monkeypatch):
+# tma: whether aligned frames of this shape run on the TMA kernel.  It needs rows of a multiple of 4 floats and lattice
+# cells of more than 5.4 rows (the 30 lattice rows of _case's field over 96 or 128 rows are too short).
+@pytest.mark.parametrize("layout", ["aligned", "offset"])
+@pytest.mark.parametrize("shape,tma", [((6, 96, 128), False), ((7, 64, 90), False), ((3, 600, 5000), True),
+                                       ((25, 256, 384), True)])
+def test_sum_is_correct_motion_sum(shape, tma, layout):
     import torch_motion_correction_b200 as tmc
+    from torch_motion_correction_b200 import _lib
 
-    monkeypatch.setenv("TMC_WARP_TMA", tma)
     movie, field = _case(*shape, seed=1)
+    if layout == "offset":
+        movie = at_offset(movie)
+    _lib.kernel_timing(True)
     got = tmc.correct_motion_sums(movie, field, 0.83, half_sets=True)
     want = tmc.correct_motion_sum(movie, field, 0.83)
     assert float((got["sum"] - want).abs().max()) <= 1e-6 * float(want.abs().max())
@@ -57,6 +64,7 @@ def test_sum_is_correct_motion_sum(shape, tma, monkeypatch):
     stack = tmc.correct_motion(movie, field, 0.83)
     assert _rel(got["sum_even"], stack[0::2].sum(0)) <= 1e-6
     assert _rel(got["sum_odd"], stack[1::2].sum(0)) <= 1e-6
+    assert warp_kernels_ran() == {"warp_tma_kernel" if tma and layout == "aligned" else "warp_lattice_kernel"}
 
 
 @pytest.mark.parametrize(
@@ -94,12 +102,16 @@ def test_dose_weighted_matches_the_oracle_dose_weight():
     assert _rel(got["dose_weighted"].cpu(), want) <= 1e-4
 
 
-@pytest.mark.parametrize("tma", ["1", "0"])
-def test_frame_range(tma, monkeypatch):
+@pytest.mark.parametrize("layout", ["aligned", "offset"])
+@pytest.mark.parametrize("shape,tma", [((12, 128, 128), False), ((12, 256, 256), True)])
+def test_frame_range(shape, tma, layout):
     import torch_motion_correction_b200 as tmc
+    from torch_motion_correction_b200 import _lib
 
-    monkeypatch.setenv("TMC_WARP_TMA", tma)
-    movie, field = _case(12, 128, 128, seed=4)
+    movie, field = _case(*shape, seed=4)
+    if layout == "offset":
+        movie = at_offset(movie)
+    _lib.kernel_timing(True)
     a, b = 3, 10
     got = tmc.correct_motion_sums(movie, field, 0.9, dose_per_frame=1.2, pre_exposure=0.7, half_sets=True, frame_range=(a, b))
     want = tmc.correct_motion_sum(movie[a:b], field, 0.9, frame_offset=a, total_frames=12)
@@ -110,6 +122,7 @@ def test_frame_range(tma, monkeypatch):
     assert _rel(got["dose_weighted"], _exact_dose_weighted(stack, rows, 0.9, 1.2, 0.7, 300.0, rows)) <= 1e-5
     want_odd = _exact_dose_weighted(stack[0::2], rows[0::2], 0.9, 1.2, 0.7, 300.0, rows)
     assert _rel(got["dose_weighted_odd"], want_odd) <= 1e-5
+    assert warp_kernels_ran() == {"warp_tma_kernel" if tma and layout == "aligned" else "warp_lattice_kernel"}
 
 
 def test_peak_memory_stays_below_one_stack():

@@ -7,7 +7,7 @@ import torch
 import torch_motion_correction_b200 as tmc
 from oracle import deps
 from oracle import reference_path as rp
-from torch_motion_correction_b200 import _fourier, _ops
+from torch_motion_correction_b200 import _fourier, _lib, _ops
 
 pytestmark = pytest.mark.gpu
 
@@ -246,28 +246,35 @@ def test_global_motion_k3_frame_size(dev):
     assert float((got.cpu() - want).abs().max()) <= 1e-5
 
 
-def test_half_length_row_transforms_agree_with_the_full_length_kernels(dev, monkeypatch):
-    """4096-point rows of frame pairs: two 2048-point transforms of pixel pairs (rows_forward_real2n, the default) against
-    one 4096-point transform of the packed pair (TMC_FFT_REAL2N=0) and against torch.fft; odd window origins take the
-    4-byte load path, an odd frame count the single-frame job."""
+def test_half_length_row_transforms_agree_with_the_full_length_kernels(dev):
+    """4096-point rows of frame pairs: two 2048-point transforms of pixel pairs (rows_forward_real2n, taken by a band of
+    kx_count <= n/2) and one 4096-point transform of the packed pair (rows_forward_p2<4096>, taken by the full spectrum,
+    kx_count = n/2 + 1), both against torch.fft in float64 and against each other on the band's bins; odd window origins
+    take the 4-byte load path, an odd frame count the single-frame job."""
     n = 4096
     g = torch.Generator().manual_seed(23)
     movie = (torch.randn((3, 700, n + 8), generator=g) * 2.0 + 1.0).to(dev)
-    plan = _fourier.BandPlan(512, n, dev, 0.83, 500, (300, 10))
+    band = _fourier.BandPlan(512, n, dev, 0.83, 500, (300, 10))
+    full = _fourier.BandPlan(512, n, dev, full=True)
     mask, ylo, yhi = _fourier.soft_disc_mask((512, n), 128.0, 64.0, dev)
     jobs = torch.tensor([[0, 1, 1, 1, 100, 4], [2, 1, -1, 1, 37, 5]], dtype=torch.int32).to(dev)
     out = {}
-    for flag in ("1", "0"):
-        monkeypatch.setenv("TMC_FFT_REAL2N", flag)
-        out[flag] = as_complex(plan.forward(movie, None, mask, ylo, yhi, jobs, job_mode=2)).clone()
-    scale = float(out["0"][:3].abs().max())  # plane 3 (no second frame in the last job) is never written
-    assert float((out["1"][:3] - out["0"][:3]).abs().max()) <= 5e-6 * scale
-    ky = (torch.arange(plan.ky, device=dev) + plan.ky_start) % 512
+    for name, plan, kernel in (("band", band, "rows_forward_real2n<2048>"), ("full", full, "rows_forward_p2<4096>")):
+        _lib.kernel_timing(True)
+        out[name] = as_complex(plan.forward(movie, None, mask, ylo, yhi, jobs, job_mode=2)).clone()
+        torch.cuda.synchronize()
+        ran = set(_lib.kernel_timing_report())
+        _lib.kernel_timing(False)
+        assert kernel in ran, (name, ran)
+    ky = (torch.arange(band.ky, device=dev) + band.ky_start) % 512
+    # plane 3 (no second frame in the last job) is never written
+    shared = out["full"][:3][:, ky][:, :, : band.kx] * band.weight
+    assert float((out["band"][:3] - shared).abs().max()) <= 5e-6 * float(shared.abs().max())
     for plane, (f, y0, x0) in ((0, (0, 100, 4)), (1, (1, 100, 4)), (2, (2, 37, 5))):
-        want = torch.fft.rfftn((movie[f, y0 : y0 + 512, x0 : x0 + n] * mask).double(), dim=(-2, -1))[ky][:, : plan.kx]
-        want = want * plan.weight.double()
-        err = (out["1"][plane].to(torch.complex128) - want).abs().max() / want.abs().max()
-        assert float(err) < 5e-6, (plane, float(err))
+        spectrum = torch.fft.rfftn((movie[f, y0 : y0 + 512, x0 : x0 + n] * mask).double(), dim=(-2, -1))
+        for name, want in (("band", spectrum[ky][:, : band.kx] * band.weight.double()), ("full", spectrum)):
+            err = (out[name][plane].to(torch.complex128) - want).abs().max() / want.abs().max()
+            assert float(err) < 5e-6, (name, plane, float(err))
 
 
 def test_global_motion_non_power_of_two_frames(dev):

@@ -118,12 +118,43 @@ def test_self_paired_columns_enter_through_their_hermitian_part(shape, factor):
     assert rel <= 1e-5, rel
 
 
+def _composed_crop(image, h2, w2):
+    """The crop through the library's composed column passes, built from public entry points: tmc_rfft2_band at full
+    height into the box ky in [-h2/2, h2/2), kx in [0, w2/2]; the box rolled into FFT order; tmc_irfft2_full at (h2, w2),
+    whose 1 / (h2 w2) times h2 w2 / (h w) is the crop's 1 / (h w) exactly when that ratio is a power of two."""
+    from torch_motion_correction_b200 import _fourier, _lib
+
+    t, h, w = image.shape
+    kx = w2 // 2 + 1
+    jobs = _fourier.frame_pair_jobs(t, DEV)
+    njobs = jobs.shape[0]
+    tw_w, tw_h, tw_w2, tw_h2 = (_fourier.twiddles(n, DEV) for n in (w, h, w2, h2))
+    rows = torch.empty((2 * njobs, h, kx, 2), dtype=torch.float32, device=DEV)
+    box = torch.empty((2 * njobs, h2, kx, 2), dtype=torch.float32, device=DEV)
+    out = torch.empty((t, h2, w2), dtype=torch.float32, device=DEV)
+    stream = _lib.stream_ptr(DEV)
+    _lib.call("tmc_rfft2_band", image.data_ptr(), t, h, w, None, None, h, w, jobs.data_ptr(), njobs, 2, None, 0, 0, h, kx,
+              h2, -(h2 // 2), None, tw_w.data_ptr(), tw_h.data_ptr(), rows.data_ptr(), box.data_ptr(), stream)
+    spec = torch.roll(box[:t], h2 // 2, dims=1).contiguous()
+    _lib.call("tmc_irfft2_full", spec.data_ptr(), t, h2, w2, tw_w2.data_ptr(), tw_h2.data_ptr(), rows.data_ptr(),
+              out.data_ptr(), stream)
+    ratio = h2 * w2 / (h * w)
+    assert ratio == 2.0 ** round(np.log2(ratio))
+    return out * ratio
+
+
 @pytest.mark.parametrize("shape,factor", [((3, 8192, 8192), 2), ((3, 1024, 1024), 4), ((5, 2048, 768), 2)])
-def test_fused_and_composed_column_passes_agree(shape, factor, monkeypatch):
+def test_fused_and_composed_column_passes_agree(shape, factor):
+    """Power-of-two heights halved or quartered run the fused column kernel (cols_crop_p2)."""
+    from torch_motion_correction_b200 import _lib
+
     image = _noise(shape, seed=shape[1] + 7)
+    _lib.kernel_timing(True)
     fused = tmc.fourier_crop(image, factor)
-    monkeypatch.setenv("TMC_FFT_CROP_FUSED", "0")
-    composed = tmc.fourier_crop(image, factor)
+    torch.cuda.synchronize()
+    assert "cols_crop_p2" in _lib.kernel_timing_report()
+    _lib.kernel_timing(False)
+    composed = _composed_crop(image, *fused.shape[1:])
     rel = _worst_rel(fused, composed.double())
     print(f"[fourier_crop] fused vs composed {shape} / {factor}: worst per-frame rel L2 {rel:.2e}, "
           f"bitwise {torch.equal(fused, composed)}")

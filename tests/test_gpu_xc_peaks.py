@@ -53,10 +53,10 @@ def _pow2(n):
     return 16 <= n <= 8192 and n & (n - 1) == 0
 
 
-def row_kernel(nx, kx, real2n=True):
+def row_kernel(nx, kx):
     """Name of the row kernel tmc_xc_peaks runs for rows of nx points with kx_count = kx."""
     if _pow2(nx) and nx >= 256:
-        if nx in (4096, 8192) and kx <= nx // 4 and real2n:
+        if nx in (4096, 8192) and kx <= nx // 4:
             return f"rows_inverse_argmax_real2n<{nx // 2}>"
         if nx == 1024 and kx <= 128:
             return POLY
@@ -188,12 +188,12 @@ def sweep_positions(ny, nx):
     return np.array(ys), np.array(xs)
 
 
-def check_sweep(case, real2n=True, monkeypatch=None):
+def check_sweep(case):
     ny, nx = case.ny, case.nx
     ys, xs = sweep_positions(ny, nx)
     prod = case.ramp(ys, xs)
     got, ran = case.peaks(prod, sub_pixel=False)
-    assert row_kernel(nx, case.plan.kx, real2n) in ran, ran
+    assert row_kernel(nx, case.plan.kx) in ran, ran
     assert col_kernel(ny) in ran, ran
     # integer peak: the surface of item i is S0 rolled to (ys[i], xs[i])
     gy, gx = got[:, 0].astype(np.int64) % ny, got[:, 1].astype(np.int64) % nx
@@ -214,7 +214,7 @@ def check_sweep(case, real2n=True, monkeypatch=None):
         worst = max(worst, circular_err(sub[i, 0], wy, ny), circular_err(sub[i, 1], wx, nx))
         if not (1 <= gy[i] < ny - 1 and 1 <= gx[i] < nx - 1):  # border: no refinement, same value as without
             assert sub[i, 0] == got[i, 0] and sub[i, 1] == got[i, 1]
-    print(f"[subpx] {row_kernel(nx, case.plan.kx, real2n)} {ny}x{nx} kx={case.plan.kx}: sweep {worst:.2e} px")
+    print(f"[subpx] {row_kernel(nx, case.plan.kx)} {ny}x{nx} kx={case.plan.kx}: sweep {worst:.2e} px")
     assert worst <= SUBPX_BOUND, worst
     return got
 
@@ -224,13 +224,6 @@ def test_peak_sweep_every_row_block(dev, c):
     """One batch of items whose peaks sweep the rows and columns, so every CTA's share of the surface holds a peak in
     some item; the wrap (<= n // 2) and border (no refinement) positions; exact against the float64 surface."""
     check_sweep(Case(dev, *c))
-
-
-@pytest.mark.parametrize("c", [(32, 4096, 1000, 21), (16, 8192, 2000, 13)], ids=case_id)
-def test_peak_sweep_without_half_length_rows(dev, c, monkeypatch):
-    """TMC_FFT_REAL2N=0 (read per call) takes the full-length p2 row kernels where real2n would run."""
-    monkeypatch.setenv("TMC_FFT_REAL2N", "0")
-    check_sweep(Case(dev, *c), real2n=False)
 
 
 FRACTIONAL_CASES = [c for c in ROW_CASES + COL_CASES if c[0] * c[1] <= 1 << 20]
@@ -303,7 +296,7 @@ def test_chunked_peaks_are_bitwise_equal(dev, monkeypatch):
 
 
 def test_cases_cover_every_row_kernel():
-    names = {row_kernel(nx, kx) for _, nx, kx, _ in ROW_CASES + FULL_CASES} | {row_kernel(4096, 1000, False)}
+    names = {row_kernel(nx, kx) for _, nx, kx, _ in ROW_CASES + FULL_CASES}
     assert names == {GEN, POLY, P2, P2_1024, P2_4096, R2N_2048, R2N_4096}
 
 

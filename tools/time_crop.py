@@ -1,7 +1,6 @@
 """Time of Fourier cropping by 2 of 40-frame movies: fourier_crop at 8192^2, K3 super-resolution 11520 x 8184 and K3
-5760 x 4092 with the bytes it moves and per-kernel times of one call; at 8192^2 the fused column kernel against the
-composed column passes (TMC_FFT_CROP_FUSED=0) and two chunk sizes, alternating in rounds; motion_correct(fourier_bin=2)
-against motion_correct at 8192^2 end to end with peak extra device memory.
+5760 x 4092 with the bytes it moves and per-kernel times of one call; at 8192^2 two chunk sizes, alternating in rounds;
+motion_correct(fourier_bin=2) against motion_correct at 8192^2 end to end with peak extra device memory.
 
 CUDA events around each call after warm-up; every movie (5.3 to 15 GB) is far larger than the 126 MB L2.  Prints the
 card and its power limit, then one JSON line per measurement.  Usage: python tools/time_crop.py [--reps N] [--frames T]"""
@@ -85,23 +84,19 @@ def main():
                           "kernel_ms_one_call": kernels}), flush=True)
         if h == 8192:
             ab = {}
-            for _ in range(3):  # rounds: every variant runs between the others
-                for fused in ("1", "0"):
-                    for chunk in (1 << 30, 8 << 30):
-                        os.environ["TMC_FFT_CROP_FUSED"] = fused
-                        _fourier.CHUNK_BYTES = chunk
-                        ab.setdefault((fused, chunk), []).append(timed(lambda: tmc.fourier_crop(movie, 2), args.reps)["median_ms"])
-            for (fused, chunk), meds in ab.items():
-                os.environ["TMC_FFT_CROP_FUSED"] = fused
+            for _ in range(3):  # rounds: every chunk size runs between the others
+                for chunk in (1 << 30, 8 << 30):
+                    _fourier.CHUNK_BYTES = chunk
+                    ab.setdefault(chunk, []).append(timed(lambda: tmc.fourier_crop(movie, 2), args.reps)["median_ms"])
+            for chunk, meds in ab.items():
                 _fourier.CHUNK_BYTES = chunk
                 _lib.kernel_timing(True)
                 tmc.fourier_crop(movie, 2)
                 torch.cuda.synchronize()
                 kernels = {k: round(ms, 3) for k, (_, ms) in _lib.kernel_timing_report().items()}
                 _lib.kernel_timing(False)
-                print(json.dumps({"shape": [t, h, w], "what": "fourier_crop A/B", "fused_columns": fused == "1",
-                                  "chunk_bytes": chunk, "round_medians_ms": meds, "kernel_ms_one_call": kernels}), flush=True)
-            os.environ.pop("TMC_FFT_CROP_FUSED")
+                print(json.dumps({"shape": [t, h, w], "what": "fourier_crop chunk sizes", "chunk_bytes": chunk,
+                                  "round_medians_ms": meds, "kernel_ms_one_call": kernels}), flush=True)
             _fourier.CHUNK_BYTES = default_chunk
         del movie
         torch.cuda.empty_cache()

@@ -22,8 +22,6 @@ NVCC_FLAGS = [
     "-DTMC_B200=1",
     "-shared",
 ]
-# experiment hook: extra -D flags (e.g. TMC_EXTRA_NVCC_FLAGS="-DTMC_POLY_MINB=3") rebuild the library with them
-NVCC_FLAGS[-1:-1] = os.environ.get("TMC_EXTRA_NVCC_FLAGS", "").split()
 
 
 def _sources():

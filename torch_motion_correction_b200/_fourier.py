@@ -4,7 +4,6 @@ weights), band-box geometry, workspace chunking.  No arithmetic on image data ha
 from __future__ import annotations
 
 import ctypes
-import os
 
 import numpy as np
 import torch
@@ -16,7 +15,7 @@ _C64 = 8  # bytes per complex64
 #: row -> column intermediates of one launch are capped at this many bytes.  Measured on B200 (C2 step): 48 MB 29.8 ms,
 #: 96 MB (L2-sized, the first design) 28.5 ms, 192 MB 28.0 ms, 768 MB 27.4 ms, 4 GB 27.3 ms -- fewer, larger launches
 #: (less tail, fewer twiddle-table loads) beat L2 residency of the intermediate
-CHUNK_BYTES = int(os.environ.get("TMC_FFT_CHUNK_BYTES", str(1 << 30)))
+CHUNK_BYTES = 1 << 30
 
 _twiddles: dict = {}
 _masks: dict = {}

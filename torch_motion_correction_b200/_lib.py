@@ -13,8 +13,7 @@ from ctypes import c_char_p, c_double, c_float, c_int, c_long, c_void_p
 import torch
 
 _PKG_DIR = os.path.dirname(os.path.abspath(__file__))
-# TMC_B200_LIB: an alternative build of the same library (A/B experiments: tools/build_variant.sh)
-LIB_PATH = os.environ.get("TMC_B200_LIB") or os.path.join(_PKG_DIR, "libtmc_b200.so")
+LIB_PATH = os.path.join(_PKG_DIR, "libtmc_b200.so")
 
 _lib = None
 

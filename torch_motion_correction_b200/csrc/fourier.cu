@@ -621,29 +621,6 @@ rows_inverse_store_kernel(const float2* __restrict__ tmp, int NY, int KX, AxisPl
 #include "fourier_p2.cuh"
 #include "fourier_poly.cuh"
 
-// TMC_FFT_POLY=0 selects the 1024-point block-level row kernels instead of the polyphase ones (A/B testing)
-inline bool use_poly() {
-  static const bool on = [] {
-    const char* e = getenv("TMC_FFT_POLY");
-    return !(e && e[0] == '0');
-  }();
-  return on;
-}
-
-// rows of two frames as half-length transforms of pixel pairs (rows_forward_real2n) for 8192- and 4096-point rows;
-// TMC_FFT_REAL2N=0 selects the full-length kernels (A/B testing; read per call: tests toggle it).  Measured, 40 frames:
-// 8192^2 12.4 -> 4.7 ms, 4096^2 1.28 -> 1.20 ms.
-inline bool use_real2n(int) {
-  const char* e = getenv("TMC_FFT_REAL2N");
-  return !(e && e[0] == '0');
-}
-
-// TMC_FFT_COL_QUADS=0 selects the one-column-per-CTA kernel for 4096-point whole-frame columns (A/B testing)
-inline bool use_col_quads() {
-  const char* e = getenv("TMC_FFT_COL_QUADS");
-  return !(e && e[0] == '0');
-}
-
 template <int M, bool BLU>
 constexpr bool use_fast_path() {
   return !BLU && M >= 256;
@@ -811,7 +788,7 @@ int rfft2_rows(const float* image, int h, int w, const float* mean_std, const fl
     constexpr bool BB = decltype(BLU)::value;
     if constexpr (MM == 1024 && !BB) {
       // polyphase path: four 256-point warp-level FFTs per row, only the band is ever formed
-      if (yhi > ylo && kx_count <= 128 && job_mode != 0 && use_poly() && px.R == 1) {
+      if (yhi > ylo && kx_count <= 128 && job_mode != 0 && px.R == 1) {
         int rows_per_cta = 32;  // measured on C2: 64 .. 256 rows per CTA change the row kernels by less than 2 %
         while (rows_per_cta > 8 && (long)tmc_div_up(yhi - ylo, rows_per_cta) * njobs < 148 * 6) rows_per_cta -= 8;
         dim3 grid(tmc_div_up(yhi - ylo, rows_per_cta), njobs);
@@ -833,8 +810,9 @@ int rfft2_rows(const float* image, int h, int w, const float* mean_std, const fl
     }
     if constexpr ((MM == 8192 || MM == 4096) && !BB) {
       // rows of two frames as two half-length complex transforms of pixel pairs instead of one full-length transform
-      // of a packed pair (the 8192-point kernel is confined to one 8-warp CTA per SM)
-      if (yhi > ylo && job_mode == 2 && px.R == 1 && kx_count <= MM / 2 && use_real2n(MM)) {
+      // of a packed pair (the 8192-point kernel is confined to one 8-warp CTA per SM).  Measured, 40 frames: 8192^2
+      // 12.4 -> 4.7 ms, 4096^2 1.28 -> 1.20 ms.
+      if (yhi > ylo && job_mode == 2 && px.R == 1 && kx_count <= MM / 2) {
         constexpr int NH = MM / 2;
         constexpr int B = fft2::Cfg<NH>::B;
         int rows_per_cta = B * 4;
@@ -1149,7 +1127,7 @@ TMC_API int tmc_xc_peaks(const void* prod, int nitems, int ny, int nx, int kx_co
     constexpr bool BB = decltype(BLU)::value;
     if constexpr ((MM == 8192 || MM == 4096) && !BB) {
       // one row per half-length transform instead of two rows per full-length transform (see rows_forward_real2n)
-      if (px.R == 1 && kx_count <= MM / 4 && use_real2n(MM)) {
+      if (px.R == 1 && kx_count <= MM / 4) {
         constexpr int NH = MM / 2;
         if (int e = enable_smem(rows_inverse_argmax_real2n<NH>, rows_inverse_real2n_smem_bytes<NH>())) return e;
         nparts = tmc_div_up(ny, rows_per_cta_inverse_real2n<NH>());
@@ -1163,7 +1141,7 @@ TMC_API int tmc_xc_peaks(const void* prod, int nitems, int ny, int nx, int kx_co
       if (px.R == 1) nparts = tmc_div_up(ny, rows_per_cta_inverse<MM>());
     }
     if constexpr (MM == 1024 && !BB) {
-      if (kx_count <= 128 && use_poly() && px.R == 1) {
+      if (kx_count <= 128 && px.R == 1) {
         if (int e = enable_smem(poly::rows_inverse_argmax_poly, poly::smem_bytes)) return e;
         dim3 grid(nparts, nitems);
         TMC_TIMED("rows_inverse_argmax_poly", stream, poly::rows_inverse_argmax_poly<<<grid, poly::kThreads, poly::smem_bytes, stream>>>((const float2*)tmp, ny, kx_count, px.tw,
@@ -1270,13 +1248,6 @@ TMC_API long tmc_fourier_crop_workspace_bytes(int t, int h, int w, int out_h, in
 
 namespace {
 
-// TMC_FFT_CROP_FUSED=0 selects the composed column passes of tmc_fourier_crop where the fused kernel would run (A/B
-// testing; read per call: tests toggle it)
-inline bool use_crop_fused() {
-  const char* e = getenv("TMC_FFT_CROP_FUSED");
-  return !(e && e[0] == '0');
-}
-
 // calls f(IntC<N>{}, IntC<M>{}) when cols_crop_p2<N, M> serves a crop of h rows to out_h rows (powers of two, out_h h/2
 // or h/4 and >= 256); returns -1 without calling f otherwise
 template <typename F>
@@ -1325,7 +1296,7 @@ TMC_API int tmc_fourier_crop(const float* image, int t, int h, int w, int out_h,
   const AxisPlan px_in = make_axis_plan(plan_x, w), py_in = make_axis_plan(plan_y, h);
   const AxisPlan px = make_axis_plan(plan_x_out, out_w), py = make_axis_plan(plan_y_out, out_h);
   const float scale = 1.0f / ((float)h * (float)w);
-  int rc = use_crop_fused() ? dispatch_crop_cols(h, out_h, [&](auto N, auto M) { return 0; }) : -1;
+  int rc = dispatch_crop_cols(h, out_h, [&](auto N, auto M) { return 0; });
   if (rc == 0) {
     if ((rc = rfft2_rows(image, h, w, nullptr, nullptr, h, w, jobs, njobs, 2, nullptr, 0, 0, h, KX, px_in, rows, stream)))
       return rc;
@@ -1406,19 +1377,15 @@ TMC_API int tmc_fourier_shift_frames(const float* image, int t, int ny, int nx, 
   rc = dispatch_fft(ny, "fourier_shift_frames", [&](auto M, auto BLU) {
     constexpr int MM = decltype(M)::value;
     if constexpr (MM == 4096 && !decltype(BLU)::value) {
-      if (use_col_quads()) {
-        constexpr size_t smem = (size_t)(4 * fft2::Cfg<MM>::STRIDE + 64 + fft2::Cfg<MM>::TW_HI) * sizeof(float2);
-        if (int e = enable_smem(cols_shift_quad_p2<MM>, smem)) return e;
-        dim3 grid(tmc_div_up(kx, 4), t);
-        TMC_TIMED("cols_shift_quad_p2", stream,
-                  cols_shift_quad_p2<MM><<<grid, 512, smem, stream>>>((float2*)tmp, kx, nx, (const float2*)phase, field, t, sign, py.tw));
-        return TMC_OK;
-      }
-    }
-    if constexpr (use_fast_path<MM, decltype(BLU)::value>()) {
+      constexpr size_t smem = (size_t)(4 * fft2::Cfg<MM>::STRIDE + 64 + fft2::Cfg<MM>::TW_HI) * sizeof(float2);
+      if (int e = enable_smem(cols_shift_quad_p2<MM>, smem)) return e;
+      dim3 grid(tmc_div_up(kx, 4), t);
+      TMC_TIMED("cols_shift_quad_p2", stream,
+                cols_shift_quad_p2<MM><<<grid, 512, smem, stream>>>((float2*)tmp, kx, nx, (const float2*)phase, field, t, sign, py.tw));
+    } else if constexpr (use_fast_path<MM, decltype(BLU)::value>()) {
       if (int e = enable_smem(cols_shift_p2<MM>, fft2::Cfg<MM>::smem_bytes)) return e;
       dim3 grid(tmc_div_up(kx, fft2::Cfg<MM>::B), t);
-      TMC_TIMED(sized_label<MM>("cols_shift_p2<4096>", "cols_shift_p2<1024>", "cols_shift_p2"), stream, cols_shift_p2<MM><<<grid, fft2::kThreads, fft2::Cfg<MM>::smem_bytes, stream>>>((float2*)tmp, kx, nx, (const float2*)phase,
+      TMC_TIMED(MM == 1024 ? "cols_shift_p2<1024>" : "cols_shift_p2", stream, cols_shift_p2<MM><<<grid, fft2::kThreads, fft2::Cfg<MM>::smem_bytes, stream>>>((float2*)tmp, kx, nx, (const float2*)phase,
                                                                                     field, t, sign, py.tw));
     }
     return TMC_OK;

@@ -25,10 +25,7 @@
 namespace {
 
 constexpr int kTileKy = 8, kTileKx = 16, kTileBins = kTileKy * kTileKx;
-#ifndef TMC_CHUNK_FRAMES
-#define TMC_CHUNK_FRAMES 8
-#endif
-constexpr int kChunkFrames = TMC_CHUNK_FRAMES;
+constexpr int kChunkFrames = 8;  // frames per bulk copy
 constexpr int kMaxChunks = 256 / kChunkFrames;  // T <= 256
 constexpr int kTileThreads = 256;
 constexpr int kCoefThreads = 1024;

@@ -134,12 +134,10 @@ __device__ __forceinline__ float gather_bicubic(const float* __restrict__ frame,
   return acc;
 }
 
-constexpr int kTileX = 128;    // threads along x
-#ifndef TMC_WARP_ROWS
-#define TMC_WARP_ROWS 4
-#endif
+constexpr int kTileX = 128;      // threads along x
 constexpr int kTileYGroups = 2;  // thread rows per CTA
-constexpr int kRows = TMC_WARP_ROWS;         // vertically adjacent output pixels per thread
+constexpr int kRows = 4;         // vertically adjacent output pixels per thread
+constexpr int kMinBlocks = 2;    // CTAs per SM that warp_lattice_kernel's register budget must allow
 
 // Stage 1: interpolate every lattice row along x once per (frame, channel, lattice row, image
 // column): RX[f][ch][a][x] = sum_b wx_b(x) * L[f][ch][a][jx_b(x)].  Same x-then-y order as ATen.
@@ -285,12 +283,9 @@ __device__ __noinline__ void warp_pixel_generic_sums(const float* __restrict__ i
 // measured alternatives on B200 (C2, fused sum): 4 rows per thread at 128 registers (2 CTAs per SM) 4.3 ms (4.1 ms with
 // the shared tap rows); capped at 80 registers (3 CTAs per SM) 5.4 ms (4.9 ms with shared tap rows); 2 rows per thread 4.6-4.8 ms; uncapped registers (1 CTA per SM) 6.2 ms;
 // prefetch.global.L2 of the next frame's rows +2 %
-template <bool WRITE_STACK, bool WRITE_SUM, bool NORMALISE, bool WEIGHTED = false>
-#ifndef TMC_WARP_MINB
-#define TMC_WARP_MINB 2
-#endif
 // (the weighted sums keep no sum in registers but load the weights: at 2 CTAs per SM they would spill, so 1)
-__global__ void __launch_bounds__(kTileX* kTileYGroups, WEIGHTED ? 1 : TMC_WARP_MINB)
+template <bool WRITE_STACK, bool WRITE_SUM, bool NORMALISE, bool WEIGHTED = false>
+__global__ void __launch_bounds__(kTileX* kTileYGroups, WEIGHTED ? 1 : kMinBlocks)
 warp_lattice_kernel(const float* __restrict__ image, int T, int H, int W, const float* __restrict__ rx, int lh,
                     float pixel_spacing, const float* __restrict__ mean_std, float* __restrict__ out_stack,
                     float* __restrict__ out_sum, int accumulate_sum, int x_begin, int x_end, int y_begin, int y_end,
@@ -674,10 +669,7 @@ static int warp_lattice_launch(const float* image, int t, int h, int w, const fl
     TMC_TIMED("lattice_xinterp_kernel", stream, lattice_xinterp_kernel<<<g1, 128, 0, stream>>>(lattice, t, lh, lw, w, workspace, 1));
   }
   const bool s = out_stack != nullptr, a = out_sum != nullptr, n = mean_std != nullptr;
-  // TMC_WARP_TMA=0 keeps everything on the global-memory kernel (A/B testing; read per call: tests toggle it)
-  const char* tma_env = getenv("TMC_WARP_TMA");
-  const bool tma_on = !(tma_env && tma_env[0] == '0');
-  if (tma_on && tma::supported(image, workspace, t, h, w, lh)) {
+  if (tma::supported(image, workspace, t, h, w, lh)) {
     // frame tiles staged by TMA, one persistent CTA per SM
     CUtensorMap img_map, rx_map;
     const bool ok = tma::make_map_3d(&img_map, image, (uint64_t)w, (uint64_t)h, (uint64_t)t, tma::kBoxW, tma::kBoxH, 1) &&
@@ -703,10 +695,6 @@ static int warp_lattice_launch(const float* image, int t, int h, int w, const fl
         const int n = (tma::kMaxSmemBytes - 128 - prm.acc_bytes) / prm.stage_bytes;
         if (n < prm.n_stages) prm.n_stages = n;
       }
-      if (const char* e = getenv("TMC_WARP_TMA_STAGES")) {  // experiment: shallower ring
-        const int v = atoi(e);
-        if (v >= 2 && v < prm.n_stages) prm.n_stages = v;
-      }
       const size_t smem_bytes = (size_t)prm.acc_bytes + (size_t)prm.n_stages * prm.stage_bytes + 128;  // + alignment slack
       prm.pixel_spacing = pixel_spacing;
       prm.mean_std = mean_std;
@@ -715,10 +703,6 @@ static int warp_lattice_launch(const float* image, int t, int h, int w, const fl
       prm.accumulate_sum = accumulate_sum;
       prm.tiles_x = tmc_div_up(w, tma::kTX);
       prm.n_tiles = prm.tiles_x * tmc_div_up(h, tma::kTY);
-      {
-        const char* dbg = getenv("TMC_WARP_TMA_DEBUG");
-        prm.debug = dbg ? atoi(dbg) : 0;
-      }
       tma::fill_constants(prm);
       int dev_id = 0, sms = 148;
       TMC_CUDA(cudaGetDevice(&dev_id));

@@ -23,13 +23,9 @@
 
 namespace tma {
 
-#ifndef TMC_TMA_TX
-#define TMC_TMA_TX 32
-#define TMC_TMA_TY 60
-#endif
 // output tile: one consumer warp per 4 image rows.  32 x 60 = 15 consumer warps + the producer warp = 16 warps of 128
 // registers, 4 per scheduler (with 14 warps two schedulers would idle a quarter of the time)
-constexpr int kTX = TMC_TMA_TX, kTY = TMC_TMA_TY;
+constexpr int kTX = 32, kTY = 60;
 constexpr int kMargin = 4;              // how far a pixel's shift may differ from the tile-centre shift
 constexpr int kBoxW = kTX + 2 * kMargin + 8;   // 48: + 3 tap columns + up to 3 columns of alignment slack (see below), 16-byte rows
 constexpr int kBoxH = kTY + 2 * kMargin + 3;   // 71
@@ -114,16 +110,10 @@ __device__ __forceinline__ void tma_load_3d(void* dst, const CUtensorMap* map, i
       : "memory");
 }
 
-// packed fp32x2 arithmetic (FFMA2 / FMUL2 / FADD2) or, with -DTMC_TMA_SCALAR, the same as pairs of scalar instructions
-#ifdef TMC_TMA_SCALAR
-__device__ __forceinline__ float2 pk_fma(float2 a, float2 b, float2 c) { return make_float2(__fmaf_rn(a.x, b.x, c.x), __fmaf_rn(a.y, b.y, c.y)); }
-__device__ __forceinline__ float2 pk_mul(float2 a, float2 b) { return make_float2(__fmul_rn(a.x, b.x), __fmul_rn(a.y, b.y)); }
-__device__ __forceinline__ float2 pk_add(float2 a, float2 b) { return make_float2(__fadd_rn(a.x, b.x), __fadd_rn(a.y, b.y)); }
-#else
+// packed fp32x2 arithmetic (FFMA2 / FMUL2 / FADD2)
 __device__ __forceinline__ float2 pk_fma(float2 a, float2 b, float2 c) { return __ffma2_rn(a, b, c); }
 __device__ __forceinline__ float2 pk_mul(float2 a, float2 b) { return __fmul2_rn(a, b); }
 __device__ __forceinline__ float2 pk_add(float2 a, float2 b) { return __fadd2_rn(a, b); }
-#endif
 
 // Keys cubic-convolution weights (A = -0.75, ATen's bicubic) of two fractions at once (.x = y axis, .y = x axis) in
 // factored form: w0 = A t (1 - t)^2, w3 = A t^2 (1 - t), w1 = ((A + 2) t - (A + 3)) t^2 + 1, w2 = w1(1 - t).  Same
@@ -167,7 +157,6 @@ struct Params {
   float* out_sum;
   int accumulate_sum;
   int tiles_x, n_tiles;
-  int debug;  // TMC_WARP_TMA_DEBUG: 4 = the consumers skip the arithmetic (times the memory pipeline alone)
   // constants of the coordinate chain, formed on the host so that they reach the arithmetic as constant-bank operands
   // (the kernel is bound by register-file reads: a register operand less per instruction is what counts)
   float2 nden, rcp, half_scale;  // .x = y axis, .y = x axis
@@ -347,7 +336,7 @@ warp_tma_kernel(const __grid_constant__ CUtensorMap img_map, const __grid_consta
     constexpr bool SAME = decltype(same_tag)::value;
     for (int f = 0; f < T; ++f) {
       mbar_wait_addr(full0 + 8u * stage, phase);
-      if (active && !(p.debug & 4)) {
+      if (active) {
         const float* simg = reinterpret_cast<const float*>(stages + (size_t)stage * p.stage_bytes);
         const float* srx = simg + kImgBytesPadded / 4;
         const int4 org = lds_int4(hdr0 + 32u * stage);       // oy + 1, ox + 1, by_lo, by_n

@@ -9,7 +9,6 @@ drives the coefficient update exactly as in the reference (same defaults)."""
 
 from __future__ import annotations
 
-import os
 import random
 from typing import Any, cast
 
@@ -25,7 +24,7 @@ from .patch_grid import patch_grid_centers
 LOSS_TYPES = {"mse": 0, "cc": 1, "ncc": 2}
 
 #: use the one-kernel iteration (csrc/optimizer_tiled.cu) for the "mse" / "cc" losses when the frame count fits
-FUSED_STEPS = os.environ.get("TMC_FUSED_STEPS", "1") != "0"
+FUSED_STEPS = True
 
 
 def fused_steps_apply(loss_type: int, g: int, t: int, resolution, plan) -> bool:
@@ -324,11 +323,8 @@ def _run_captured(one_step, n_iterations: int, dev: torch.device) -> int:
                 graph.capture_end()
             kernels_per_step = query("tmc_launch_count") - launches_before
         except Exception as exc:  # pragma: no cover - capture refused: finish eagerly
-            import os
             import warnings
 
-            if os.environ.get("TMC_DEBUG"):
-                raise
             warnings.warn(f"CUDA-graph capture of the optimiser step failed ({exc}); running eagerly", stacklevel=2)
             main.wait_stream(side)
             return 1
