@@ -230,6 +230,8 @@ int tmc_xc_leave_one_out_products(const void* spec, int t, int g, long plane_ele
                                   const int* deltas, int k_begin, int k_count, void* out, tmc_stream_t stream);
 
 /* ---- inverse transform + peak: irfftn, argmax, parabola, wrap at estimate_motion_xc.py:113-121,350-369,414-483 */
+/* partial results per item of tmc_xc_peaks for (ny, nx): the most CTAs its inverse row pass launches for any
+ * kx_count (-1: unsupported nx) */
 int tmc_xc_peak_partials(int ny, int nx);
 /* prod (nitems, ky_count, kx_count) -> shifts (nitems, 2) = (dy, dx) px.  tmp: nitems*ny*kx_count complex64;
  * partial: nitems * tmc_xc_peak_partials(ny, nx) * 8 bytes. */

@@ -504,23 +504,19 @@ struct PeakCandidate {
 
 __device__ __forceinline__ bool better(float v, int i, float bv, int bi) { return v > bv || (v == bv && i < bi); }
 
-// tmp[item][NY][KX] -> per-CTA maximum of the real correlation surface: partial[item][blockIdx.x]
-template <int MX, bool BLU>
-__global__ void __launch_bounds__(kThreads)
-rows_inverse_argmax_kernel(const float2* __restrict__ tmp, int NY, int KX, AxisPlan plan,
-                           PeakCandidate* __restrict__ partial) {
+// Shared body of the generic inverse row kernels: c2r transforms of this CTA's 2 B rows, two rows per transform and, on a
+// decimated axis, one sub-sequence r at a time.  Calls consume(ya, x, v) for every output sample x of the row pair
+// (ya, ya + 1): v.y is row ya, v.x row ya + 1 (when ya + 1 < NY).
+template <int MX, bool BLU, typename Consume>
+__device__ __forceinline__ void rows_inverse_generic(const float2* __restrict__ src, int NY, int KX, const AxisPlan& plan,
+                                                     float2* smem, Consume&& consume) {
   constexpr int B = batch_for(MX);
   constexpr int STRIDE = padded_len(MX);
   const int NS = BLU ? plan.n : MX;
   const int R = plan.R, NX = plan.n_total;
-  extern __shared__ float2 smem[];
   float2* a = smem;
   float2* b = smem + B * STRIDE;
-  const long item = blockIdx.y;
   const int row0 = blockIdx.x * 2 * B;
-  const float2* src = tmp + item * NY * KX;
-  float best = -INFINITY;
-  int best_idx = 0x7fffffff;
   const bool gather = R > 1 && 2 * KX - 1 > NS;  // the band aliases onto itself: full spectrum of a decimated axis
   for (int r = 0; r < R; ++r) {
     for (int idx = threadIdx.x; idx < B * STRIDE; idx += kThreads) a[idx] = make_float2(0.f, 0.f);
@@ -536,19 +532,33 @@ rows_inverse_argmax_kernel(const float2* __restrict__ tmp, int NY, int KX, AxisP
       const int s = idx / NS, m_ = idx % NS;
       const int ya = row0 + 2 * s;
       if (ya >= NY) continue;
-      const float2 v = res[s * STRIDE + pad_idx(m_)];  // swapped: v.y = row ya, v.x = row ya+1
-      const int ia = ya * NX + R * m_ + r;
-      if (better(v.y, ia, best, best_idx)) {
-        best = v.y;
-        best_idx = ia;
-      }
-      if (ya + 1 < NY && better(v.x, ia + NX, best, best_idx)) {
-        best = v.x;
-        best_idx = ia + NX;
-      }
+      consume(ya, R * m_ + r, res[s * STRIDE + pad_idx(m_)]);
     }
     __syncthreads();
   }
+}
+
+// tmp[item][NY][KX] -> per-CTA maximum of the real correlation surface: partial[item][blockIdx.x]
+template <int MX, bool BLU>
+__global__ void __launch_bounds__(kThreads)
+rows_inverse_argmax_kernel(const float2* __restrict__ tmp, int NY, int KX, AxisPlan plan,
+                           PeakCandidate* __restrict__ partial) {
+  extern __shared__ float2 smem[];
+  const long item = blockIdx.y;
+  const int NX = plan.n_total;
+  float best = -INFINITY;
+  int best_idx = 0x7fffffff;
+  rows_inverse_generic<MX, BLU>(tmp + item * NY * KX, NY, KX, plan, smem, [&](int ya, int x, float2 v) {
+    const int ia = ya * NX + x;
+    if (better(v.y, ia, best, best_idx)) {
+      best = v.y;
+      best_idx = ia;
+    }
+    if (ya + 1 < NY && better(v.x, ia + NX, best, best_idx)) {
+      best = v.x;
+      best_idx = ia + NX;
+    }
+  });
 #pragma unroll
   for (int o = 16; o > 0; o >>= 1) {
     const float ov = __shfl_xor_sync(0xffffffffu, best, o);
@@ -583,39 +593,14 @@ template <int MX, bool BLU>
 __global__ void __launch_bounds__(kThreads)
 rows_inverse_store_kernel(const float2* __restrict__ tmp, int NY, int KX, AxisPlan plan, float scale,
                           float* __restrict__ out) {
-  constexpr int B = batch_for(MX);
-  constexpr int STRIDE = padded_len(MX);
-  const int NS = BLU ? plan.n : MX;
-  const int R = plan.R, NX = plan.n_total;
   extern __shared__ float2 smem[];
-  float2* a = smem;
-  float2* b = smem + B * STRIDE;
   const long item = blockIdx.y;
-  const int row0 = blockIdx.x * 2 * B;
-  const float2* src = tmp + item * NY * KX;
+  const int NX = plan.n_total;
   float* dst = out + item * NY * NX;
-  const bool gather = R > 1 && 2 * KX - 1 > NS;  // the band aliases onto itself: full spectrum of a decimated axis
-  for (int r = 0; r < R; ++r) {
-    for (int idx = threadIdx.x; idx < B * STRIDE; idx += kThreads) a[idx] = make_float2(0.f, 0.f);
-    __syncthreads();
-    for (int s = 0; s < B; ++s) {
-      const int ya = row0 + 2 * s, yb = ya + 1;
-      if (ya < NY)
-        load_c2r_pair(src + (long)ya * KX, yb < NY ? src + (long)yb * KX : nullptr, KX, NX, NS, R, r, gather, a + s * STRIDE);
-    }
-    __syncthreads();
-    const float2* res = dft_smem<MX, BLU>(a, b, plan);
-    for (int idx = threadIdx.x; idx < B * NS; idx += kThreads) {
-      const int s = idx / NS, m_ = idx % NS;
-      const int ya = row0 + 2 * s;
-      if (ya >= NY) continue;
-      const float2 v = res[s * STRIDE + pad_idx(m_)];
-      const int x = R * m_ + r;
-      dst[(long)ya * NX + x] = v.y * scale;
-      if (ya + 1 < NY) dst[(long)(ya + 1) * NX + x] = v.x * scale;
-    }
-    __syncthreads();
-  }
+  rows_inverse_generic<MX, BLU>(tmp + item * NY * KX, NY, KX, plan, smem, [&](int ya, int x, float2 v) {
+    dst[(long)ya * NX + x] = v.y * scale;
+    if (ya + 1 < NY) dst[(long)(ya + 1) * NX + x] = v.x * scale;
+  });
 }
 
 #include "fourier_p2.cuh"
@@ -716,12 +701,6 @@ __global__ void fourier_shift_kernel(float2* __restrict__ spec, int T, int NY, i
 
 #define TMC_FOR_EACH_M(X) X(16) X(32) X(64) X(128) X(256) X(512) X(1024) X(2048) X(4096) X(8192)
 
-// timing label of a size-templated kernel (the two sizes of the benchmark get their own rows)
-template <int MM>
-constexpr const char* sized_label(const char* l4096, const char* l1024, const char* other) {
-  return MM == 4096 ? l4096 : (MM == 1024 ? l1024 : other);
-}
-
 template <int V>
 struct IntC {
   static constexpr int value = V;
@@ -779,91 +758,206 @@ inline bool decimated_full_fits(int n) {
          fft_smem_runtime(m) + 1ull * b * n * sizeof(float2) <= kMaxSmem;
 }
 
-// row pass of tmc_rfft2_band: tmp[2 job + {0, 1}][y][kx] = row DFTs of the jobs' windows, kx < kx_count
-int rfft2_rows(const float* image, int h, int w, const float* mean_std, const float* mask, int ny, int nx, const int* jobs,
-               int njobs, int job_mode, const int* frame_shifts, int x_margin, int ylo, int yhi, int kx_count,
-               const AxisPlan& px, void* tmp, cudaStream_t stream) {
-  return dispatch_fft(nx, "rfft2_band", [&](auto M, auto BLU) {
+// Timing label of a templated kernel: "name<S>" at the template values S listed (the sizes the benchmark reports on rows
+// of their own, or the kernel's job modes), the plain name at the others.  Spelled by the preprocessor, so every label
+// is a string literal.
+#define TMC_LABEL1(name, N, S1) ((N) == S1 ? name "<" #S1 ">" : name)
+#define TMC_LABEL2(name, N, S1, S2) ((N) == S2 ? name "<" #S2 ">" : TMC_LABEL1(name, N, S1))
+
+// enables `smem` bytes of dynamic shared memory for `kernel`, then launches, times and counts it
+template <typename... P, typename... A>
+int launch(const char* label, void (*kernel)(P...), dim3 grid, int threads, size_t smem, cudaStream_t stream, A... args) {
+  if (int e = enable_smem(kernel, smem)) return e;
+  TMC_TIMED(label, stream, kernel<<<grid, threads, smem, stream>>>(args...));
+  return TMC_OK;
+}
+
+// Rows per CTA of a forward row pass over `rows` rows of njobs jobs: `most`, lowered in steps of `step` (to no fewer than
+// `step`) until the grid covers the 148 SMs `waves` times over; each CTA amortises its twiddle-table load over its rows.
+inline int rows_per_cta_to_fill(int rows, int njobs, int most, int step, int waves) {
+  int rows_per_cta = most;
+  while (rows_per_cta > step && (long)tmc_div_up(rows, rows_per_cta) * njobs < 148 * waves) rows_per_cta -= step;
+  return rows_per_cta;
+}
+
+// Calls f(first, count) for slices of at most `limit` of n items, in stream order: entry points that put a caller's
+// count on grid y (at most kMaxGridYZ).  Every slice reuses the caller's workspace from its start.
+template <typename F>
+int for_each_slice(int n, int limit, F&& f) {
+  for (int i0 = 0; i0 < n; i0 += limit)
+    if (int rc = f(i0, n - i0 < limit ? n - i0 : limit)) return rc;
+  return TMC_OK;
+}
+
+// ---- the passes of a 2-D transform ------------------------------------------------------------------
+// Each pass chooses its kernel from the transform length, the axis plan's decimation, the band and the job mode, and
+// sizes its grid; the entry points chain passes.
+
+// forward row pass (tmc_rfft2_band's arguments): tmp[2 job + {0, 1}][y][kx] = row DFTs of the jobs' windows, kx < kx_count
+int rows_forward(const float* image, int h, int w, const float* mean_std, const float* mask, int ny, int nx, const int* jobs,
+                 int njobs, int job_mode, const int* frame_shifts, int x_margin, int ylo, int yhi, int kx_count,
+                 const AxisPlan& px, void* tmp, cudaStream_t stream, const char* who) {
+  return dispatch_fft(nx, who, [&](auto M, auto BLU) {
     constexpr int MM = decltype(M)::value;
     constexpr bool BB = decltype(BLU)::value;
+    const int rows = yhi - ylo;
     if constexpr (MM == 1024 && !BB) {
       // polyphase path: four 256-point warp-level FFTs per row, only the band is ever formed
-      if (yhi > ylo && kx_count <= 128 && job_mode != 0 && px.R == 1) {
-        int rows_per_cta = 32;  // measured on C2: 64 .. 256 rows per CTA change the row kernels by less than 2 %
-        while (rows_per_cta > 8 && (long)tmc_div_up(yhi - ylo, rows_per_cta) * njobs < 148 * 6) rows_per_cta -= 8;
-        dim3 grid(tmc_div_up(yhi - ylo, rows_per_cta), njobs);
-        if (job_mode == 1) {
-          if (int e = enable_smem(poly::rows_forward_poly<1>, poly::smem_bytes)) return e;
-          TMC_TIMED("rows_forward_poly<1>", stream,
-                    poly::rows_forward_poly<1><<<grid, poly::kThreads, poly::smem_bytes, stream>>>(
-                        image, h, w, mean_std, mask, jobs, frame_shifts, x_margin, ylo, yhi, ny, kx_count, px.tw, (float2*)tmp,
-                        rows_per_cta));
-        } else {
-          if (int e = enable_smem(poly::rows_forward_poly<2>, poly::smem_bytes)) return e;
-          TMC_TIMED("rows_forward_poly<2>", stream,
-                    poly::rows_forward_poly<2><<<grid, poly::kThreads, poly::smem_bytes, stream>>>(
-                        image, h, w, mean_std, mask, jobs, frame_shifts, x_margin, ylo, yhi, ny, kx_count, px.tw, (float2*)tmp,
-                        rows_per_cta));
-        }
-        return TMC_OK;
+      if (rows > 0 && kx_count <= 128 && job_mode != 0 && px.R == 1) {
+        // measured on C2: 64 .. 256 rows per CTA change the row kernels by less than 2 %
+        const int rows_per_cta = rows_per_cta_to_fill(rows, njobs, 32, 8, 6);
+        return launch(TMC_LABEL2("rows_forward_poly", job_mode, 1, 2),
+                      job_mode == 1 ? poly::rows_forward_poly<1> : poly::rows_forward_poly<2>,
+                      dim3(tmc_div_up(rows, rows_per_cta), njobs), poly::kThreads, poly::smem_bytes, stream, image, h, w,
+                      mean_std, mask, jobs, frame_shifts, x_margin, ylo, yhi, ny, kx_count, px.tw, (float2*)tmp, rows_per_cta);
       }
     }
     if constexpr ((MM == 8192 || MM == 4096) && !BB) {
       // rows of two frames as two half-length complex transforms of pixel pairs instead of one full-length transform
       // of a packed pair (the 8192-point kernel is confined to one 8-warp CTA per SM).  Measured, 40 frames: 8192^2
       // 12.4 -> 4.7 ms, 4096^2 1.28 -> 1.20 ms.
-      if (yhi > ylo && job_mode == 2 && px.R == 1 && kx_count <= MM / 2) {
+      if (rows > 0 && job_mode == 2 && px.R == 1 && kx_count <= MM / 2) {
         constexpr int NH = MM / 2;
         constexpr int B = fft2::Cfg<NH>::B;
-        int rows_per_cta = B * 4;
-        while (rows_per_cta > B && (long)tmc_div_up(yhi - ylo, rows_per_cta) * njobs < 148 * 8) rows_per_cta -= B;
-        dim3 grid(tmc_div_up(yhi - ylo, rows_per_cta), njobs);
-        constexpr size_t smem = rows_forward_real2n_smem_bytes<NH>();
-        if (int e = enable_smem(rows_forward_real2n<NH>, smem)) return e;
-        TMC_TIMED(MM == 8192 ? "rows_forward_real2n<4096>" : "rows_forward_real2n<2048>", stream,
-                  rows_forward_real2n<NH><<<grid, fft2::kThreads, smem, stream>>>(image, h, w, mean_std, mask, jobs, frame_shifts, x_margin,
-                                                                                   ylo, yhi, ny, kx_count, px.tw, (float2*)tmp,
-                                                                                   rows_per_cta));
-        return TMC_OK;
+        const int rows_per_cta = rows_per_cta_to_fill(rows, njobs, B * 4, B, 8);
+        return launch(TMC_LABEL2("rows_forward_real2n", NH, 2048, 4096), rows_forward_real2n<NH>,
+                      dim3(tmc_div_up(rows, rows_per_cta), njobs), fft2::kThreads, rows_forward_real2n_smem_bytes<NH>(),
+                      stream, image, h, w, mean_std, mask, jobs, frame_shifts, x_margin, ylo, yhi, ny, kx_count, px.tw,
+                      (float2*)tmp, rows_per_cta);
       }
     }
     if constexpr (use_fast_path<MM, BB>()) if (px.R == 1) {
-      if (yhi > ylo) {
-        constexpr int B = fft2::Cfg<MM>::B;
-        // enough CTAs to fill the chip a few times over, each amortising its twiddle-table load
-        int rows_per_cta = B * 4;
-        while (rows_per_cta > B && (long)tmc_div_up(yhi - ylo, rows_per_cta) * njobs < 148 * 8) rows_per_cta -= B;
-        dim3 grid(tmc_div_up(yhi - ylo, rows_per_cta), njobs);
-        constexpr size_t smem = rows_forward_smem_bytes<MM>();
-#define TMC_ROWS_FWD(MODE)                                                                                      \
-  {                                                                                                             \
-    if (int e = enable_smem(rows_forward_p2<MM, MODE>, smem)) return e;                                         \
-    tmc_timing_begin(stream);                                                                                   \
-    rows_forward_p2<MM, MODE><<<grid, fft2::kThreads, smem, stream>>>(image, h, w, mean_std, mask, jobs, frame_shifts, \
-                                                                     x_margin, ylo, yhi, ny, kx_count, px.tw,          \
-                                                                     (float2*)tmp, rows_per_cta);                      \
-    tmc_timing_end(MM == 4096 ? "rows_forward_p2<4096>" : "rows_forward_p2", stream);                            \
-  }
-        if (job_mode == 1) TMC_ROWS_FWD(1) else if (job_mode == 2) TMC_ROWS_FWD(2) else TMC_ROWS_FWD(0)
-#undef TMC_ROWS_FWD
-        tmc_count_launch();
-      }
-      return TMC_OK;
+      if (rows <= 0) return TMC_OK;
+      constexpr int B = fft2::Cfg<MM>::B;
+      const int rows_per_cta = rows_per_cta_to_fill(rows, njobs, B * 4, B, 8);
+      return launch(TMC_LABEL1("rows_forward_p2", MM, 4096),
+                    job_mode == 1 ? rows_forward_p2<MM, 1> : job_mode == 2 ? rows_forward_p2<MM, 2> : rows_forward_p2<MM, 0>,
+                    dim3(tmc_div_up(rows, rows_per_cta), njobs), fft2::kThreads, rows_forward_smem_bytes<MM>(), stream, image,
+                    h, w, mean_std, mask, jobs, frame_shifts, x_margin, ylo, yhi, ny, kx_count, px.tw, (float2*)tmp,
+                    rows_per_cta);
     }
     // generic kernel (Bluestein lengths, small transforms, decimated long axes); the accumulators of a decimated axis
     // follow the two transform buffers
     const size_t smem = fft_smem_bytes<MM>() + (px.R > 1 ? 2ull * batch_for(MM) * kx_count * sizeof(float2) : 0);
     if (smem > kMaxSmem) {
-      tmc_set_error("rfft2_band: band of %d bins too wide for the decimated row transform of length %d", kx_count, nx);
+      tmc_set_error("%s: band of %d bins too wide for the decimated row transform of length %d", who, kx_count, nx);
       return TMC_ERR_UNSUPPORTED;
     }
-    if (int e = enable_smem(rows_forward_kernel<MM, BB>, smem)) return e;
-    dim3 grid(tmc_div_up(yhi - ylo, batch_for(MM)), njobs);
-    if (yhi > ylo) {
-      TMC_TIMED("rows_forward_kernel", stream, rows_forward_kernel<MM, BB><<<grid, kThreads, smem, stream>>>(
-          image, h, w, mean_std, mask, jobs, frame_shifts, x_margin, ylo, yhi, ny, kx_count, px, (float2*)tmp));
+    if (rows <= 0) return TMC_OK;
+    return launch("rows_forward_kernel", rows_forward_kernel<MM, BB>, dim3(tmc_div_up(rows, batch_for(MM)), njobs), kThreads,
+                  smem, stream, image, h, w, mean_std, mask, jobs, frame_shifts, x_margin, ylo, yhi, ny, kx_count, px,
+                  (float2*)tmp);
+  });
+}
+
+// forward column pass: plane p of tmp (nplanes, ny, KX), rows [ylo, yhi) non-zero -> out (nplanes, KY, KX),
+// ky = ky_start + kyb, times weight (KY, KX, nullable)
+int cols_forward(const void* tmp, int nplanes, int ny, int ylo, int yhi, int KX, int KY, int ky_start, const float* weight,
+                 const AxisPlan& py, void* out, cudaStream_t stream, const char* who) {
+  return dispatch_fft(ny, who, [&](auto M, auto BLU) {
+    constexpr int MM = decltype(M)::value;
+    constexpr bool BB = decltype(BLU)::value;
+    if constexpr (use_fast_path<MM, BB>()) if (py.R == 1) {
+      return launch(TMC_LABEL2("cols_forward_p2", MM, 1024, 4096), cols_forward_p2<MM>,
+                    dim3(tmc_div_up(KX, fft2::Cfg<MM>::B), nplanes), fft2::kThreads, fft2::Cfg<MM>::smem_bytes, stream,
+                    (const float2*)tmp, ylo, yhi, KX, KY, ky_start, weight, py.tw, (float2*)out);
     }
-    return TMC_OK;
+    const size_t smem = fft_smem_bytes<MM>() + (py.R > 1 ? 1ull * batch_for(MM) * KY * sizeof(float2) : 0);
+    if (smem > kMaxSmem) {
+      tmc_set_error("%s: band of %d bins too wide for the decimated column transform of length %d", who, KY, ny);
+      return TMC_ERR_UNSUPPORTED;
+    }
+    return launch("cols_forward_kernel", cols_forward_kernel<MM, BB>, dim3(tmc_div_up(KX, batch_for(MM)), nplanes), kThreads,
+                  smem, stream, (const float2*)tmp, ylo, yhi, KX, KY, ky_start, weight, py, (float2*)out);
+  });
+}
+
+// inverse column pass of a (nitems, KY, KX) box (ky = ky_start + kyb, the box spans every ky of length ny) -> tmp
+// (nitems, ny, KX); entries beyond the box are zero
+int cols_inverse(const void* spec, int nitems, int ny, int KX, int KY, int ky_start, const AxisPlan& py, void* tmp,
+                 cudaStream_t stream, const char* who) {
+  return dispatch_fft(ny, who, [&](auto M, auto BLU) {
+    constexpr int MM = decltype(M)::value;
+    constexpr bool BB = decltype(BLU)::value;
+    if constexpr (use_fast_path<MM, BB>()) if (py.R == 1) {
+      return launch(TMC_LABEL2("cols_inverse_p2", MM, 1024, 4096), cols_inverse_p2<MM>,
+                    dim3(tmc_div_up(KX, fft2::Cfg<MM>::B), nitems), fft2::kThreads, fft2::Cfg<MM>::smem_bytes, stream,
+                    (const float2*)spec, KX, KY, ky_start, py.tw, (float2*)tmp);
+    }
+    return launch("cols_inverse_kernel", cols_inverse_kernel<MM, BB>, dim3(tmc_div_up(KX, batch_for(MM)), nitems), kThreads,
+                  fft_smem_bytes<MM>(), stream, (const float2*)spec, KX, KY, ky_start, py, (float2*)tmp);
+  });
+}
+
+// The inverse row pass's kernel for rows of length R * n served by FFT size MM (BB: Bluestein) with a band of KX bins.
+// The peak search (argmax) also has the half-length and polyphase kernels for narrow bands; the store has not.
+enum class RowsInverseKernel { real2n, poly, p2, generic };
+struct RowsInverseChoice {
+  RowsInverseKernel kernel;
+  int rows_per_cta;
+};
+
+template <int MM, bool BB>
+RowsInverseChoice choose_rows_inverse(int R, int KX, bool argmax) {
+  if constexpr ((MM == 8192 || MM == 4096) && !BB) {
+    // one row per half-length transform instead of two rows per full-length transform (see rows_forward_real2n)
+    if (argmax && R == 1 && KX <= MM / 4) return {RowsInverseKernel::real2n, rows_per_cta_inverse_real2n<MM / 2>()};
+  }
+  if constexpr (MM == 1024 && !BB) {
+    if (argmax && R == 1 && KX <= 128) return {RowsInverseKernel::poly, poly::kRowsPerCta};
+  }
+  if constexpr (use_fast_path<MM, BB>()) {
+    if (R == 1) return {RowsInverseKernel::p2, rows_per_cta_inverse<MM>()};
+  }
+  return {RowsInverseKernel::generic, 2 * batch_for(MM)};  // decimated axes run here too
+}
+
+// CTAs per item of the inverse row pass: the peak search's partial results per item (-1: unsupported length)
+int rows_inverse_ctas(int ny, int nx, int KX, bool argmax) {
+  const int R = decimation_for(nx);
+  if (R == 0) return -1;
+  return dispatch_fft(nx, "rows_inverse", [&](auto M, auto BLU) {
+    return tmc_div_up(ny, choose_rows_inverse<decltype(M)::value, decltype(BLU)::value>(R, KX, argmax).rows_per_cta);
+  });
+}
+
+// c2r row pass: tmp (nitems, ny, KX) -> partial != nullptr: the maximum of each CTA's rows into partial[item][cta]
+// (rows_inverse_ctas of them per item); otherwise out (nitems, ny, nx) f32 times `scale`.  Keeps only the real part of
+// the kx = 0 and kx = nx/2 entries, as c2r does.
+int rows_inverse(const void* tmp, int nitems, int ny, int nx, int KX, const AxisPlan& px, PeakCandidate* partial,
+                 float scale, float* out, cudaStream_t stream, const char* who) {
+  return dispatch_fft(nx, who, [&](auto M, auto BLU) {
+    constexpr int MM = decltype(M)::value;
+    constexpr bool BB = decltype(BLU)::value;
+    const RowsInverseChoice c = choose_rows_inverse<MM, BB>(px.R, KX, partial != nullptr);
+    const dim3 grid(tmc_div_up(ny, c.rows_per_cta), nitems);
+    const float2* src = (const float2*)tmp;
+    if (partial != nullptr) {
+      if constexpr ((MM == 8192 || MM == 4096) && !BB) {
+        if (c.kernel == RowsInverseKernel::real2n)
+          return launch(TMC_LABEL2("rows_inverse_argmax_real2n", MM / 2, 2048, 4096), rows_inverse_argmax_real2n<MM / 2>,
+                        grid, fft2::kThreads, rows_inverse_real2n_smem_bytes<MM / 2>(), stream, src, ny, KX, px.tw, partial);
+      }
+      if constexpr (MM == 1024 && !BB) {
+        if (c.kernel == RowsInverseKernel::poly)
+          return launch("rows_inverse_argmax_poly", poly::rows_inverse_argmax_poly, grid, poly::kThreads, poly::smem_bytes,
+                        stream, src, ny, KX, px.tw, partial);
+      }
+      if constexpr (use_fast_path<MM, BB>()) {
+        if (c.kernel == RowsInverseKernel::p2)
+          return launch(TMC_LABEL2("rows_inverse_argmax_p2", MM, 1024, 4096), rows_inverse_argmax_p2<MM>, grid,
+                        fft2::kThreads, rows_inverse_smem_bytes<MM>(), stream, src, ny, KX, px.tw, partial);
+      }
+      return launch("rows_inverse_argmax_kernel", rows_inverse_argmax_kernel<MM, BB>, grid, kThreads, fft_smem_bytes<MM>(),
+                    stream, src, ny, KX, px, partial);
+    }
+    if constexpr (use_fast_path<MM, BB>()) {
+      if (c.kernel == RowsInverseKernel::p2)
+        return launch(TMC_LABEL2("rows_inverse_store_p2", MM, 1024, 4096), rows_inverse_store_p2<MM>, grid, fft2::kThreads,
+                      rows_inverse_smem_bytes<MM>(), stream, src, ny, KX, px.tw, scale, out);
+    }
+    return launch("rows_inverse_store_kernel", rows_inverse_store_kernel<MM, BB>, grid, kThreads, fft_smem_bytes<MM>(),
+                  stream, src, ny, KX, px, scale, out);
   });
 }
 
@@ -917,9 +1011,8 @@ TMC_API int tmc_fft_plan_init(int n_total, void* plan, cudaStream_t stream) {
     p.n_total = m;
     int rc = dispatch_fft(m, "fft_plan_init", [&](auto M, auto) {
       constexpr int MM = decltype(M)::value;
-      if (int e = enable_smem(c2c_rows_kernel<MM, false>, fft_smem_bytes<MM>())) return e;
-      TMC_TIMED("c2c_rows_kernel", stream, c2c_rows_kernel<MM, false><<<1, kThreads, fft_smem_bytes<MM>(), stream>>>(bhat, 1, p, bhat));
-      return TMC_OK;
+      return launch("c2c_rows_kernel", c2c_rows_kernel<MM, false>, dim3(1), kThreads, fft_smem_bytes<MM>(), stream, bhat, 1, p,
+                    bhat);
     });
     if (rc) return rc;
   }
@@ -935,10 +1028,8 @@ TMC_API int tmc_fft_c2c_rows(const void* in, int rows, int n, const void* plan, 
   int rc = dispatch_fft(n, "fft_c2c_rows", [&](auto M, auto BLU) {
     constexpr int MM = decltype(M)::value;
     constexpr bool BB = decltype(BLU)::value;
-    if (int e = enable_smem(c2c_rows_kernel<MM, BB>, fft_smem_bytes<MM>())) return e;
-    TMC_TIMED("c2c_rows_kernel", stream, c2c_rows_kernel<MM, BB><<<tmc_div_up(rows, batch_for(MM)), kThreads, fft_smem_bytes<MM>(), stream>>>(
-        (const float2*)in, rows, p, (float2*)out));
-    return TMC_OK;
+    return launch("c2c_rows_kernel", c2c_rows_kernel<MM, BB>, dim3(tmc_div_up(rows, batch_for(MM))), kThreads,
+                  fft_smem_bytes<MM>(), stream, (const float2*)in, rows, p, (float2*)out);
   });
   if (rc) return rc;
   TMC_CHECK_LAUNCH("tmc_fft_c2c_rows");
@@ -966,47 +1057,19 @@ TMC_API int tmc_rfft2_band(const float* image, int t, int h, int w, const float*
   TMC_CHECK_ARG(0 <= ylo && ylo <= yhi && yhi <= ny, "rfft2_band: bad row support [%d,%d)", ylo, yhi);
   TMC_CHECK_ARG(x_margin >= 0 && 2 * x_margin <= nx, "rfft2_band: bad x_margin %d", x_margin);
   TMC_CHECK_ARG(kx_count >= 1 && kx_count <= nx / 2 + 1 && ky_count >= 1 && ky_count <= ny, "rfft2_band: bad band box");
-  if (njobs == 0) return TMC_OK;
-  constexpr int kMaxJobs = kMaxGridYZ / 2;  // the column pass puts 2 njobs planes on grid y
-  if (njobs > kMaxJobs) {  // slices in stream order: each reuses tmp from the start
-    for (int j0 = 0; j0 < njobs; j0 += kMaxJobs) {
-      const int n = njobs - j0 < kMaxJobs ? njobs - j0 : kMaxJobs;
-      if (int rc = tmc_rfft2_band(image, t, h, w, mean_std, mask, ny, nx, jobs + 6l * j0, n, job_mode, frame_shifts, x_margin,
-                                  ylo, yhi, kx_count, ky_count, ky_start, weight, plan_x, plan_y, tmp,
-                                  (float2*)out + 2l * j0 * ky_count * kx_count, stream))
-        return rc;
-    }
-    return TMC_OK;
-  }
   const AxisPlan px = make_axis_plan(plan_x, nx), py = make_axis_plan(plan_y, ny);
-  int rc = rfft2_rows(image, h, w, mean_std, mask, ny, nx, jobs, njobs, job_mode, frame_shifts, x_margin, ylo, yhi, kx_count,
-                      px, tmp, stream);
-  if (rc) return rc;
-  TMC_CHECK_LAUNCH("tmc_rfft2_band(rows)");
-  rc = dispatch_fft(ny, "rfft2_band", [&](auto M, auto BLU) {
-    constexpr int MM = decltype(M)::value;
-    constexpr bool BB = decltype(BLU)::value;
-    if constexpr (use_fast_path<MM, BB>()) if (py.R == 1) {
-      if (int e = enable_smem(cols_forward_p2<MM>, fft2::Cfg<MM>::smem_bytes)) return e;
-      dim3 grid(tmc_div_up(kx_count, fft2::Cfg<MM>::B), 2 * njobs);
-      TMC_TIMED(sized_label<MM>("cols_forward_p2<4096>", "cols_forward_p2<1024>", "cols_forward_p2"), stream, cols_forward_p2<MM><<<grid, fft2::kThreads, fft2::Cfg<MM>::smem_bytes, stream>>>(
-          (const float2*)tmp, ylo, yhi, kx_count, ky_count, ky_start, weight, py.tw, (float2*)out));
-      return TMC_OK;
-    }
-    const size_t smem = fft_smem_bytes<MM>() + (py.R > 1 ? 1ull * batch_for(MM) * ky_count * sizeof(float2) : 0);
-    if (smem > kMaxSmem) {
-      tmc_set_error("rfft2_band: band of %d bins too wide for the decimated column transform of length %d", ky_count, ny);
-      return TMC_ERR_UNSUPPORTED;
-    }
-    if (int e = enable_smem(cols_forward_kernel<MM, BB>, smem)) return e;
-    dim3 grid(tmc_div_up(kx_count, batch_for(MM)), 2 * njobs);
-    TMC_TIMED("cols_forward_kernel", stream, cols_forward_kernel<MM, BB><<<grid, kThreads, smem, stream>>>(
-                  (const float2*)tmp, ylo, yhi, kx_count, ky_count, ky_start, weight, py, (float2*)out));
+  // the column pass puts 2 njobs planes on grid y
+  return for_each_slice(njobs, kMaxGridYZ / 2, [&](int j0, int n) {
+    if (int rc = rows_forward(image, h, w, mean_std, mask, ny, nx, jobs + 6l * j0, n, job_mode, frame_shifts, x_margin, ylo,
+                              yhi, kx_count, px, tmp, stream, "rfft2_band"))
+      return rc;
+    TMC_CHECK_LAUNCH("tmc_rfft2_band(rows)");
+    if (int rc = cols_forward(tmp, 2 * n, ny, ylo, yhi, kx_count, ky_count, ky_start, weight, py,
+                              (float2*)out + 2l * j0 * ky_count * kx_count, stream, "rfft2_band"))
+      return rc;
+    TMC_CHECK_LAUNCH("tmc_rfft2_band(cols)");
     return TMC_OK;
   });
-  if (rc) return rc;
-  TMC_CHECK_LAUNCH("tmc_rfft2_band(cols)");
-  return TMC_OK;
 }
 
 // shifts[f] = (rint(scale * field[0][f]), rint(scale * field[1][f])) for a (2, t) field; *not_integer is set to 1 when
@@ -1037,20 +1100,13 @@ TMC_API int tmc_integer_shifts(const float* field, int t, float scale, int* shif
 TMC_API int tmc_xc_pair_products(const void* spec, const int* ref_plane, const int* cur_plane, int nitems, long plane_elems,
                                  void* out, cudaStream_t stream) {
   TMC_CHECK_ARG(spec && ref_plane && cur_plane && out && nitems >= 0 && plane_elems >= 1, "xc_pair_products: bad arguments");
-  if (nitems == 0) return TMC_OK;
-  if (nitems > kMaxGridYZ) {
-    for (int i0 = 0; i0 < nitems; i0 += kMaxGridYZ) {
-      const int n = nitems - i0 < kMaxGridYZ ? nitems - i0 : kMaxGridYZ;
-      if (int rc = tmc_xc_pair_products(spec, ref_plane + i0, cur_plane + i0, n, plane_elems, (float2*)out + i0 * plane_elems,
-                                        stream))
-        return rc;
-    }
+  return for_each_slice(nitems, kMaxGridYZ, [&](int i0, int n) {
+    dim3 grid((unsigned)(tmc_div_up(plane_elems, 256) < 64 ? tmc_div_up(plane_elems, 256) : 64), n);
+    TMC_TIMED("xc_pair_product_kernel", stream, xc_pair_product_kernel<<<grid, 256, 0, stream>>>(
+        (const float2*)spec, ref_plane + i0, cur_plane + i0, plane_elems, (float2*)out + i0 * plane_elems));
+    TMC_CHECK_LAUNCH("tmc_xc_pair_products");
     return TMC_OK;
-  }
-  dim3 grid((unsigned)(tmc_div_up(plane_elems, 256) < 64 ? tmc_div_up(plane_elems, 256) : 64), nitems);
-  TMC_TIMED("xc_pair_product_kernel", stream, xc_pair_product_kernel<<<grid, 256, 0, stream>>>((const float2*)spec, ref_plane, cur_plane, plane_elems, (float2*)out));
-  TMC_CHECK_LAUNCH("tmc_xc_pair_products");
-  return TMC_OK;
+  });
 }
 
 // spec planes [T][G][2]; out items [k_count][G] for frames k_begin .. k_begin + k_count - 1;
@@ -1069,19 +1125,12 @@ TMC_API int tmc_xc_leave_one_out_products(const void* spec, int t, int g, long p
   return TMC_OK;
 }
 
+// Partial results per item of tmc_xc_peaks: the most CTAs its inverse row pass launches for any band width.  A length
+// switches kernels at one band width at most (the half-length and polyphase kernels take the narrow bands), so the
+// narrowest and the widest band cover every kernel it can run.
 TMC_API int tmc_xc_peak_partials(int ny, int nx) {
-  const int R = decimation_for(nx);
-  if (R == 0) return -1;
-  const int m = fft_size_for(nx / R);
-  if (R == 1 && m == nx && m >= 256) {  // power-of-two fast path: several row-pair batches per CTA
-    const int b = 256 / (m / 16) > 0 ? 256 / (m / 16) : 1;
-    if (m == 8192 || m == 4096) {  // may run as half-length transforms, one row each (rows_inverse_argmax_real2n): more CTAs
-      const int bh = 256 / (m / 32) > 0 ? 256 / (m / 32) : 1;
-      return tmc_div_up(ny, bh * kRowIters);
-    }
-    return tmc_div_up(ny, 2 * b * kRowIters);
-  }
-  return tmc_div_up(ny, 2 * batch_for(m));
+  const int narrow = rows_inverse_ctas(ny, nx, 1, true), wide = rows_inverse_ctas(ny, nx, nx / 2 + 1, true);
+  return narrow > wide ? narrow : wide;
 }
 
 // Inverse 2-D transform of band-limited products + argmax (+ parabola) + wrap.
@@ -1092,151 +1141,38 @@ TMC_API int tmc_xc_peaks(const void* prod, int nitems, int ny, int nx, int kx_co
                          cudaStream_t stream) {
   TMC_CHECK_ARG(prod && plan_x && plan_y && tmp && partial && shifts, "xc_peaks: null pointer");
   TMC_CHECK_ARG(kx_count >= 1 && kx_count <= nx / 2 + 1 && ky_count >= 1 && ky_count <= ny, "xc_peaks: bad band box");
-  if (nitems == 0) return TMC_OK;
-  if (nitems > kMaxGridYZ) {  // slices in stream order: each reuses tmp and partial from the start
-    for (int i0 = 0; i0 < nitems; i0 += kMaxGridYZ) {
-      const int n = nitems - i0 < kMaxGridYZ ? nitems - i0 : kMaxGridYZ;
-      if (int rc = tmc_xc_peaks((const float2*)prod + (long)i0 * ky_count * kx_count, n, ny, nx, kx_count, ky_count, ky_start,
-                                sub_pixel, plan_x, plan_y, tmp, partial, shifts + 2l * i0, stream))
-        return rc;
-    }
-    return TMC_OK;
-  }
   const AxisPlan px = make_axis_plan(plan_x, nx), py = make_axis_plan(plan_y, ny);
-  int rc = dispatch_fft(ny, "xc_peaks", [&](auto M, auto BLU) {
-    constexpr int MM = decltype(M)::value;
-    constexpr bool BB = decltype(BLU)::value;
-    if constexpr (use_fast_path<MM, BB>()) if (py.R == 1) {
-      if (int e = enable_smem(cols_inverse_p2<MM>, fft2::Cfg<MM>::smem_bytes)) return e;
-      dim3 grid(tmc_div_up(kx_count, fft2::Cfg<MM>::B), nitems);
-      TMC_TIMED(sized_label<MM>("cols_inverse_p2<4096>", "cols_inverse_p2<1024>", "cols_inverse_p2"), stream, cols_inverse_p2<MM><<<grid, fft2::kThreads, fft2::Cfg<MM>::smem_bytes, stream>>>(
-          (const float2*)prod, kx_count, ky_count, ky_start, py.tw, (float2*)tmp));
-      return TMC_OK;
-    }
-    if (int e = enable_smem(cols_inverse_kernel<MM, BB>, fft_smem_bytes<MM>())) return e;
-    dim3 grid(tmc_div_up(kx_count, batch_for(MM)), nitems);
-    TMC_TIMED("cols_inverse_kernel", stream, cols_inverse_kernel<MM, BB><<<grid, kThreads, fft_smem_bytes<MM>(), stream>>>((const float2*)prod, kx_count, ky_count, ky_start,
-                                                                                 py, (float2*)tmp));
-    return TMC_OK;
-  });
-  if (rc) return rc;
-  TMC_CHECK_LAUNCH("tmc_xc_peaks(cols)");
-  int nparts = tmc_xc_peak_partials(ny, nx);  // size of the caller's buffer per item; the kernel chosen may use fewer
-  rc = dispatch_fft(nx, "xc_peaks", [&](auto M, auto BLU) {
-    constexpr int MM = decltype(M)::value;
-    constexpr bool BB = decltype(BLU)::value;
-    if constexpr ((MM == 8192 || MM == 4096) && !BB) {
-      // one row per half-length transform instead of two rows per full-length transform (see rows_forward_real2n)
-      if (px.R == 1 && kx_count <= MM / 4) {
-        constexpr int NH = MM / 2;
-        if (int e = enable_smem(rows_inverse_argmax_real2n<NH>, rows_inverse_real2n_smem_bytes<NH>())) return e;
-        nparts = tmc_div_up(ny, rows_per_cta_inverse_real2n<NH>());
-        dim3 grid(nparts, nitems);
-        TMC_TIMED(MM == 8192 ? "rows_inverse_argmax_real2n<4096>" : "rows_inverse_argmax_real2n<2048>", stream,
-                  rows_inverse_argmax_real2n<NH><<<grid, fft2::kThreads, rows_inverse_real2n_smem_bytes<NH>(), stream>>>(
-                      (const float2*)tmp, ny, kx_count, px.tw, (PeakCandidate*)partial));
-        return TMC_OK;
-      }
-      // the full-length p2 kernel below; a decimated axis (R > 1) runs the generic kernel, two rows per CTA
-      if (px.R == 1) nparts = tmc_div_up(ny, rows_per_cta_inverse<MM>());
-    }
-    if constexpr (MM == 1024 && !BB) {
-      if (kx_count <= 128 && px.R == 1) {
-        if (int e = enable_smem(poly::rows_inverse_argmax_poly, poly::smem_bytes)) return e;
-        dim3 grid(nparts, nitems);
-        TMC_TIMED("rows_inverse_argmax_poly", stream, poly::rows_inverse_argmax_poly<<<grid, poly::kThreads, poly::smem_bytes, stream>>>((const float2*)tmp, ny, kx_count, px.tw,
-                                                                                         (PeakCandidate*)partial));
-        return TMC_OK;
-      }
-    }
-    if constexpr (use_fast_path<MM, BB>()) if (px.R == 1) {
-      if (int e = enable_smem(rows_inverse_argmax_p2<MM>, rows_inverse_smem_bytes<MM>())) return e;
-      dim3 grid(nparts, nitems);
-      TMC_TIMED(sized_label<MM>("rows_inverse_argmax_p2<4096>", "rows_inverse_argmax_p2<1024>", "rows_inverse_argmax_p2"), stream, rows_inverse_argmax_p2<MM><<<grid, fft2::kThreads, rows_inverse_smem_bytes<MM>(), stream>>>(
-          (const float2*)tmp, ny, kx_count, px.tw, (PeakCandidate*)partial));
-      return TMC_OK;
-    }
-    if (int e = enable_smem(rows_inverse_argmax_kernel<MM, BB>, fft_smem_bytes<MM>())) return e;
-    dim3 grid(nparts, nitems);
-    TMC_TIMED("rows_inverse_argmax_kernel", stream, rows_inverse_argmax_kernel<MM, BB><<<grid, kThreads, fft_smem_bytes<MM>(), stream>>>((const float2*)tmp, ny, kx_count, px,
-                                                                                        (PeakCandidate*)partial));
-    return TMC_OK;
-  });
-  if (rc) return rc;
-  TMC_CHECK_LAUNCH("tmc_xc_peaks(rows)");
-  TMC_TIMED("peak_finalize_kernel", stream, peak_finalize_kernel<<<nitems, 128, 0, stream>>>((const float2*)tmp, (const PeakCandidate*)partial, nparts, ny, nx,
-                                                   kx_count, sub_pixel, shifts));
-  TMC_CHECK_LAUNCH("tmc_xc_peaks(finalize)");
-  return TMC_OK;
-}
-
-namespace {
-
-// inverse column pass of a (nitems, KY, KX) box (ky = ky_start + kyb, the box spans every ky of length ny) -> tmp
-// (nitems, ny, KX); entries beyond the box are zero
-int irfft2_cols(const void* spec, int nitems, int ny, int KX, int KY, int ky_start, const AxisPlan& py, void* tmp,
-                cudaStream_t stream, const char* who) {
-  return dispatch_fft(ny, who, [&](auto M, auto BLU) {
-    constexpr int MM = decltype(M)::value;
-    constexpr bool BB = decltype(BLU)::value;
-    if constexpr (use_fast_path<MM, BB>()) if (py.R == 1) {
-      if (int e = enable_smem(cols_inverse_p2<MM>, fft2::Cfg<MM>::smem_bytes)) return e;
-      dim3 grid(tmc_div_up(KX, fft2::Cfg<MM>::B), nitems);
-      TMC_TIMED(sized_label<MM>("cols_inverse_p2<4096>", "cols_inverse_p2<1024>", "cols_inverse_p2"), stream, cols_inverse_p2<MM><<<grid, fft2::kThreads, fft2::Cfg<MM>::smem_bytes, stream>>>((const float2*)spec, KX, KY, ky_start, py.tw,
-                                                                                      (float2*)tmp));
-      return TMC_OK;
-    }
-    if (int e = enable_smem(cols_inverse_kernel<MM, BB>, fft_smem_bytes<MM>())) return e;
-    dim3 grid(tmc_div_up(KX, batch_for(MM)), nitems);
-    TMC_TIMED("cols_inverse_kernel", stream, cols_inverse_kernel<MM, BB><<<grid, kThreads, fft_smem_bytes<MM>(), stream>>>((const float2*)spec, KX, KY, ky_start, py, (float2*)tmp));
+  return for_each_slice(nitems, kMaxGridYZ, [&](int i0, int n) {
+    if (int rc = cols_inverse((const float2*)prod + (long)i0 * ky_count * kx_count, n, ny, kx_count, ky_count, ky_start, py,
+                              tmp, stream, "xc_peaks"))
+      return rc;
+    TMC_CHECK_LAUNCH("tmc_xc_peaks(cols)");
+    if (int rc = rows_inverse(tmp, n, ny, nx, kx_count, px, (PeakCandidate*)partial, 0.f, nullptr, stream, "xc_peaks"))
+      return rc;
+    TMC_CHECK_LAUNCH("tmc_xc_peaks(rows)");
+    const int nparts = rows_inverse_ctas(ny, nx, kx_count, true);
+    TMC_TIMED("peak_finalize_kernel", stream, peak_finalize_kernel<<<n, 128, 0, stream>>>(
+        (const float2*)tmp, (const PeakCandidate*)partial, nparts, ny, nx, kx_count, sub_pixel, shifts + 2l * i0));
+    TMC_CHECK_LAUNCH("tmc_xc_peaks(finalize)");
     return TMC_OK;
   });
 }
-
-// c2r row pass: tmp (nitems, ny, KX) -> out (nitems, ny, nx) f32 times `scale`.  Keeps only the real part of the
-// kx = 0 and kx = nx/2 entries, as c2r does.
-int irfft2_rows(const void* tmp, int nitems, int ny, int nx, int KX, const AxisPlan& px, float scale, float* out,
-                cudaStream_t stream, const char* who) {
-  return dispatch_fft(nx, who, [&](auto M, auto BLU) {
-    constexpr int MM = decltype(M)::value;
-    constexpr bool BB = decltype(BLU)::value;
-    if constexpr (use_fast_path<MM, BB>()) if (px.R == 1) {
-      if (int e = enable_smem(rows_inverse_store_p2<MM>, rows_inverse_smem_bytes<MM>())) return e;
-      dim3 grid(tmc_div_up(ny, rows_per_cta_inverse<MM>()), nitems);
-      TMC_TIMED(sized_label<MM>("rows_inverse_store_p2<4096>", "rows_inverse_store_p2<1024>", "rows_inverse_store_p2"), stream, rows_inverse_store_p2<MM><<<grid, fft2::kThreads, rows_inverse_smem_bytes<MM>(), stream>>>(
-          (const float2*)tmp, ny, KX, px.tw, scale, out));
-      return TMC_OK;
-    }
-    if (int e = enable_smem(rows_inverse_store_kernel<MM, BB>, fft_smem_bytes<MM>())) return e;
-    dim3 grid(tmc_div_up(ny, 2 * batch_for(MM)), nitems);
-    TMC_TIMED("rows_inverse_store_kernel", stream, rows_inverse_store_kernel<MM, BB><<<grid, kThreads, fft_smem_bytes<MM>(), stream>>>((const float2*)tmp, ny, KX, px,
-                                                                                       scale, out));
-    return TMC_OK;
-  });
-}
-
-}  // namespace
 
 // Full inverse: spec (nitems, ny, nx/2+1) complex64 -> out (nitems, ny, nx) f32 (irfftn, backward norm)
 TMC_API int tmc_irfft2_full(const void* spec, int nitems, int ny, int nx, const void* plan_x, const void* plan_y, void* tmp,
                             float* out, cudaStream_t stream) {
   TMC_CHECK_ARG(spec && plan_x && plan_y && tmp && out, "irfft2_full: null pointer");
-  if (nitems == 0) return TMC_OK;
-  if (nitems > kMaxGridYZ) {  // slices in stream order: each reuses tmp from the start
-    for (int i0 = 0; i0 < nitems; i0 += kMaxGridYZ) {
-      const int n = nitems - i0 < kMaxGridYZ ? nitems - i0 : kMaxGridYZ;
-      if (int rc = tmc_irfft2_full((const float2*)spec + (long)i0 * ny * (nx / 2 + 1), n, ny, nx, plan_x, plan_y, tmp,
-                                   out + (long)i0 * ny * nx, stream))
-        return rc;
-    }
-    return TMC_OK;
-  }
   const AxisPlan px = make_axis_plan(plan_x, nx), py = make_axis_plan(plan_y, ny);
-  if (int rc = irfft2_cols(spec, nitems, ny, nx / 2 + 1, ny, 0, py, tmp, stream, "irfft2_full")) return rc;
-  if (int rc = irfft2_rows(tmp, nitems, ny, nx, nx / 2 + 1, px, 1.0f / ((float)nx * (float)ny), out, stream, "irfft2_full"))
-    return rc;
-  TMC_CHECK_LAUNCH("tmc_irfft2_full");
-  return TMC_OK;
+  return for_each_slice(nitems, kMaxGridYZ, [&](int i0, int n) {
+    if (int rc = cols_inverse((const float2*)spec + (long)i0 * ny * (nx / 2 + 1), n, ny, nx / 2 + 1, ny, 0, py, tmp, stream,
+                              "irfft2_full"))
+      return rc;
+    if (int rc = rows_inverse(tmp, n, ny, nx, nx / 2 + 1, px, nullptr, 1.0f / ((float)nx * (float)ny),
+                              out + (long)i0 * ny * nx, stream, "irfft2_full"))
+      return rc;
+    TMC_CHECK_LAUNCH("tmc_irfft2_full");
+    return TMC_OK;
+  });
 }
 
 // Fourier crop ("binning") of whole frames: bytes of the workspace tmc_fourier_crop needs for t frames
@@ -1298,25 +1234,22 @@ TMC_API int tmc_fourier_crop(const float* image, int t, int h, int w, int out_h,
   const float scale = 1.0f / ((float)h * (float)w);
   int rc = dispatch_crop_cols(h, out_h, [&](auto N, auto M) { return 0; });
   if (rc == 0) {
-    if ((rc = rfft2_rows(image, h, w, nullptr, nullptr, h, w, jobs, njobs, 2, nullptr, 0, 0, h, KX, px_in, rows, stream)))
+    if ((rc = rows_forward(image, h, w, nullptr, nullptr, h, w, jobs, njobs, 2, nullptr, 0, 0, h, KX, px_in, rows, stream,
+                           "fourier_crop")))
       return rc;
     rc = dispatch_crop_cols(h, out_h, [&](auto N, auto M) {
       constexpr int NN = decltype(N)::value, MM = decltype(M)::value;
-      constexpr size_t smem = cols_crop_smem_bytes<NN, MM>();
-      if (int e = enable_smem(cols_crop_p2<NN, MM>, smem)) return e;
-      dim3 grid(tmc_div_up(KX, fft2::Cfg<MM>::B), t);
-      TMC_TIMED("cols_crop_p2", stream, cols_crop_p2<NN, MM><<<grid, fft2::kThreads, smem, stream>>>(
-          (const float2*)rows, KX, py_in.tw, py.tw, box));
-      return TMC_OK;
+      return launch("cols_crop_p2", cols_crop_p2<NN, MM>, dim3(tmc_div_up(KX, fft2::Cfg<MM>::B), t), fft2::kThreads,
+                    cols_crop_smem_bytes<NN, MM>(), stream, (const float2*)rows, KX, py_in.tw, py.tw, box);
     });
     if (rc) return rc;
-    rc = irfft2_rows(box, t, out_h, out_w, KX, px, scale, out, stream, "fourier_crop");
+    rc = rows_inverse(box, t, out_h, out_w, KX, px, nullptr, scale, out, stream, "fourier_crop");
   } else {
     if ((rc = tmc_rfft2_band(image, t, h, w, nullptr, nullptr, h, w, jobs, njobs, 2, nullptr, 0, 0, h, KX, out_h,
                              -(out_h / 2), nullptr, plan_x, plan_y, rows, box, stream)))
       return rc;
-    if ((rc = irfft2_cols(box, t, out_h, KX, out_h, -(out_h / 2), py, rows, stream, "fourier_crop"))) return rc;
-    rc = irfft2_rows(rows, t, out_h, out_w, KX, px, scale, out, stream, "fourier_crop");
+    if ((rc = cols_inverse(box, t, out_h, KX, out_h, -(out_h / 2), py, rows, stream, "fourier_crop"))) return rc;
+    rc = rows_inverse(rows, t, out_h, out_w, KX, px, nullptr, scale, out, stream, "fourier_crop");
   }
   if (rc) return rc;
   TMC_CHECK_LAUNCH("tmc_fourier_crop");
@@ -1355,20 +1288,8 @@ TMC_API int tmc_fourier_shift_frames(const float* image, int t, int ny, int nx, 
   }
   const int kx = nx / 2 + 1;
   const AxisPlan px = make_axis_plan(plan_x, nx), py = make_axis_plan(plan_y, ny);
-  int rc = dispatch_fft(nx, "fourier_shift_frames", [&](auto M, auto BLU) {
-    constexpr int MM = decltype(M)::value;
-    if constexpr (use_fast_path<MM, decltype(BLU)::value>()) {
-      constexpr int B = fft2::Cfg<MM>::B;
-      int rows_per_cta = B * 4;
-      while (rows_per_cta > B && (long)tmc_div_up(ny, rows_per_cta) * njobs < 148 * 8) rows_per_cta -= B;
-      constexpr size_t smem = rows_forward_smem_bytes<MM>();
-      if (int e = enable_smem(rows_forward_p2<MM, 2>, smem)) return e;
-      dim3 grid(tmc_div_up(ny, rows_per_cta), njobs);
-      TMC_TIMED("rows_forward_p2", stream, rows_forward_p2<MM, 2><<<grid, fft2::kThreads, smem, stream>>>(image, ny, nx, mean_std, nullptr, jobs, nullptr, 0, 0, ny, ny,
-                                                                    kx, px.tw, (float2*)tmp, rows_per_cta));
-    }
-    return TMC_OK;
-  });
+  int rc = rows_forward(image, ny, nx, mean_std, nullptr, ny, nx, jobs, njobs, 2, nullptr, 0, 0, ny, kx, px, tmp, stream,
+                        "fourier_shift_frames");
   if (rc) return rc;
   {
     dim3 grid(tmc_div_up(ny, 128), t);
@@ -1378,29 +1299,17 @@ TMC_API int tmc_fourier_shift_frames(const float* image, int t, int ny, int nx, 
     constexpr int MM = decltype(M)::value;
     if constexpr (MM == 4096 && !decltype(BLU)::value) {
       constexpr size_t smem = (size_t)(4 * fft2::Cfg<MM>::STRIDE + 64 + fft2::Cfg<MM>::TW_HI) * sizeof(float2);
-      if (int e = enable_smem(cols_shift_quad_p2<MM>, smem)) return e;
-      dim3 grid(tmc_div_up(kx, 4), t);
-      TMC_TIMED("cols_shift_quad_p2", stream,
-                cols_shift_quad_p2<MM><<<grid, 512, smem, stream>>>((float2*)tmp, kx, nx, (const float2*)phase, field, t, sign, py.tw));
+      return launch("cols_shift_quad_p2", cols_shift_quad_p2<MM>, dim3(tmc_div_up(kx, 4), t), 512, smem, stream, (float2*)tmp,
+                    kx, nx, (const float2*)phase, field, t, sign, py.tw);
     } else if constexpr (use_fast_path<MM, decltype(BLU)::value>()) {
-      if (int e = enable_smem(cols_shift_p2<MM>, fft2::Cfg<MM>::smem_bytes)) return e;
-      dim3 grid(tmc_div_up(kx, fft2::Cfg<MM>::B), t);
-      TMC_TIMED(MM == 1024 ? "cols_shift_p2<1024>" : "cols_shift_p2", stream, cols_shift_p2<MM><<<grid, fft2::kThreads, fft2::Cfg<MM>::smem_bytes, stream>>>((float2*)tmp, kx, nx, (const float2*)phase,
-                                                                                    field, t, sign, py.tw));
+      return launch(TMC_LABEL1("cols_shift_p2", MM, 1024), cols_shift_p2<MM>, dim3(tmc_div_up(kx, fft2::Cfg<MM>::B), t),
+                    fft2::kThreads, fft2::Cfg<MM>::smem_bytes, stream, (float2*)tmp, kx, nx, (const float2*)phase, field, t,
+                    sign, py.tw);
     }
     return TMC_OK;
   });
   if (rc) return rc;
-  rc = dispatch_fft(nx, "fourier_shift_frames", [&](auto M, auto BLU) {
-    constexpr int MM = decltype(M)::value;
-    if constexpr (use_fast_path<MM, decltype(BLU)::value>()) {
-      if (int e = enable_smem(rows_inverse_store_p2<MM>, rows_inverse_smem_bytes<MM>())) return e;
-      dim3 grid(tmc_div_up(ny, rows_per_cta_inverse<MM>()), t);
-      TMC_TIMED(sized_label<MM>("rows_inverse_store_p2<4096>", "rows_inverse_store_p2<1024>", "rows_inverse_store_p2"), stream, rows_inverse_store_p2<MM><<<grid, fft2::kThreads, rows_inverse_smem_bytes<MM>(), stream>>>(
-          (const float2*)tmp, ny, kx, px.tw, 1.0f / ((float)nx * (float)ny), out));
-    }
-    return TMC_OK;
-  });
+  rc = rows_inverse(tmp, t, ny, nx, kx, px, nullptr, 1.0f / ((float)nx * (float)ny), out, stream, "fourier_shift_frames");
   if (rc) return rc;
   TMC_CHECK_LAUNCH("tmc_fourier_shift_frames");
   return TMC_OK;

@@ -179,7 +179,9 @@ rows_forward_poly(const float* __restrict__ image, int H, int W, const float* __
 }
 
 // ---- inverse rows + argmax: tmp[item][y][kx] -> partial[item][cta] ------------------------------------
-// CTA = 32 rows (16 row pairs, two per warp); same partial layout as rows_inverse_argmax_p2<1024>.
+// CTA = kRowsPerCta rows (row pairs, two per warp); same partial layout as rows_inverse_argmax_p2<1024>.
+constexpr int kRowsPerCta = 32;
+
 __global__ void __launch_bounds__(kThreads, 3)
 rows_inverse_argmax_poly(const float2* __restrict__ tmp, int NY, int KX, const float2* __restrict__ tw,
                          PeakCandidate* __restrict__ partial) {
@@ -197,8 +199,8 @@ rows_inverse_argmax_poly(const float2* __restrict__ tmp, int NY, int KX, const f
   float best = -INFINITY;
   int best_idx = 0x7fffffff;
   __syncthreads();
-  for (int pair = warp; pair < 16; pair += kWarps) {
-    const int ya = blockIdx.x * 32 + 2 * pair;
+  for (int pair = warp; pair < kRowsPerCta / 2; pair += kWarps) {
+    const int ya = blockIdx.x * kRowsPerCta + 2 * pair;
     if (ya >= NY) break;
     const bool has_b = ya + 1 < NY;
     const float2* rowa = src + (long)ya * KX;
