@@ -95,6 +95,19 @@ int tmc_group_frames(const float* movie, int t, int h, int w, int frame_group, f
 int tmc_eer_render(const void* payload, long payload_bytes, const long long* frame_offsets, int n_frames, int h, int w,
                    int rle_bits, int sub_bits, int frames_per_fraction, int count_bytes, void* counts, int* status,
                    tmc_stream_t stream);
+/* TIFF LZW (compression 5) strips -> a (n_rows, w) stack of sample_bytes (1 or 2) byte samples, little-endian.
+ * payload (device, payload_bytes long): strip s is bytes [strip_offsets[s], strip_offsets[s + 1] - 8) followed by 8 zero
+ * bytes; strip_offsets (device int64, n_strips + 1).  Strip s decodes into the stack's bytes [out_offsets[s],
+ * out_offsets[s + 1]) (device int64, n_strips + 1; whole rows).  predictor 2 (horizontal differencing) is undone along
+ * every row of the stack afterwards, modulo 2^(8 sample_bytes); 1 leaves the samples as decoded.  Any number of strips.
+ * workspace (device) of at least tmc_tiff_lzw_workspace_bytes(payload_bytes, n_strips) bytes.  status (device int32,
+ * n_strips): 0 decoded; 1 malformed (a code names an undefined entry, the table passes 4096 entries without a Clear, or
+ * the stream ends before the strip's rows are full: the rows hold what was decoded, then zeros); 2 offsets outside the
+ * payload or the stack (rows not written).  Codes after a strip's rows are full are ignored. */
+long tmc_tiff_lzw_workspace_bytes(long payload_bytes, int n_strips);
+int tmc_tiff_lzw_decode(const void* payload, long payload_bytes, const long long* strip_offsets,
+                        const long long* out_offsets, int n_strips, long n_rows, int w, int sample_bytes, int predictor,
+                        void* out, void* workspace, long workspace_bytes, int* status, tmc_stream_t stream);
 
 /* ---- cubic spline grids: torch_cubic_spline_grids.Cubic{CatmullRom,BSpline}Grid3d as used at
  *      deformation_field_utils.py:9-93, estimate_motion_optimizer.py:487-490, correct_motion.py:288-305 */

@@ -29,8 +29,9 @@ from .optimization_state import OptimizationState, OptimizationTracker
 from .patch_grid import patch_grid_centers
 from .spline_grids import CubicBSplineGrid3d, CubicCatmullRomGrid3d
 from .pipeline import estimate_motion, motion_correct, motion_correct_many
-from .prepare import fourier_crop, group_frames, prepare_movie, render_eer
-from .movie_io import EerMovie, eer_movies, mrc_movies, read_eer, read_mrc, read_mrc_header, read_tiff, write_mrc
+from .prepare import decode_tiff, fourier_crop, group_frames, prepare_movie, render_eer
+from .movie_io import (EerMovie, TiffMovie, eer_movies, mrc_movies, read_eer, read_mrc, read_mrc_header, read_tiff,
+                       read_tiff_movie, tiff_movies, write_mrc)
 from .utils import normalize_image
 
 __version__ = "0.1.0"
@@ -65,4 +66,8 @@ __all__ = [
     "eer_movies",
     "read_tiff",
     "EerMovie",
+    "decode_tiff",
+    "read_tiff_movie",
+    "tiff_movies",
+    "TiffMovie",
 ]

@@ -42,6 +42,8 @@ _SIGNATURES = {
     "tmc_subtract_frame_means": (I, [P, I, L, P, P]),
     "tmc_group_frames": (I, [P, I, I, I, I, P, P]),
     "tmc_eer_render": (I, [P, L, P, I, I, I, I, I, I, I, P, P, P]),
+    "tmc_tiff_lzw_workspace_bytes": (L, [L, I]),
+    "tmc_tiff_lzw_decode": (I, [P, L, P, P, I, L, I, I, I, P, P, L, P, P]),
     "tmc_spline_workspace_floats": (L, [I, I, I, I]),
     "tmc_spline_eval": (I, [P, I, I, I, I, I, P, L, P, P, P]),
     "tmc_spline_eval_backward": (I, [I, I, I, I, I, P, L, P, F, P, P, P]),

@@ -9,9 +9,12 @@ The reference's example script reads movies with third-party readers (``mrcfile`
 * EER (Falcon 4 / 4i electron-event lists in a little-endian TIFF or BigTIFF, one IFD per hardware frame, compression
   65000 / 65001 / 65002): ``read_eer`` only reads the compressed strips into one pinned buffer; the events are rendered
   into count fractions on the device (``prepare.render_eer``, ``csrc/eer.cu``), so only the compressed bytes cross PCIe;
-* uncompressed TIFF images and stacks (``read_tiff``): Falcon gain references.
+* uncompressed TIFF images and stacks (``read_tiff``): Falcon gain references;
+* LZW-compressed TIFF movies (Gatan K3, ``read_tiff_movie``): as for EER only the compressed strips are read into one
+  pinned buffer and they are decoded on the device (``prepare.decode_tiff``, ``csrc/tiff_lzw.cu``).
 
-Compressed TIFF (LZW, deflate), 8K rendering from the EER sub-pixel bits and the EER XML metadata stay out of scope.
+Deflate / zstd / JPEG TIFF, tiled and big-endian TIFF, float TIFF movies, 8K rendering from the EER sub-pixel bits and
+the EER XML metadata stay out of scope.
 
 PARITY UNPINNED against ``mrcfile`` and against a real Falcon EER file (neither is available here): the MRC layout is
 the published one and is pinned by ``tests/test_movie_io.py`` on hand-built headers; the EER container and bit stream
@@ -168,6 +171,7 @@ def mrc_movies(paths: Iterable[Union[str, Path]], pinned: bool = True) -> Iterat
 _TIFF_TYPE_SIZES = {1: 1, 3: 2, 4: 4, 16: 8}  # BYTE, SHORT, LONG, LONG8: the integer types of the tags read here
 _TAG_WIDTH, _TAG_LENGTH, _TAG_BITS, _TAG_COMPRESSION = 256, 257, 258, 259
 _TAG_STRIP_OFFSETS, _TAG_SAMPLES, _TAG_ROWS_PER_STRIP, _TAG_STRIP_COUNTS, _TAG_SAMPLE_FORMAT = 273, 277, 278, 279, 339
+_TAG_FILL_ORDER, _TAG_PREDICTOR, _TAG_TILE_WIDTH = 266, 317, 322
 _TAG_EER_RLE, _TAG_EER_HORZ, _TAG_EER_VERT = 65007, 65008, 65009
 #: EER compression -> (rle_bits, sub_bits) of the fixed codecs; 65002 reads them from tags 65007-65009
 _EER_CODECS = {65000: (8, 4), 65001: (7, 4)}
@@ -363,7 +367,12 @@ def read_tiff(path: Union[str, Path], pinned: bool = True) -> torch.Tensor:
         kinds.add((d.get(_TAG_BITS, (1,))[0], d.get(_TAG_SAMPLE_FORMAT, (1,))[0]))
     if len(kinds) != 1 or next(iter(kinds)) not in _TIFF_SAMPLE_TYPES:
         raise ValueError(f"{path}: sample types {sorted(kinds)} (bits, format); supported: uint8, uint16, int16, float32")
-    dtype = _TIFF_SAMPLE_TYPES[kinds.pop()]
+    out = _read_uncompressed(path, ifds, 0, h, w, _TIFF_SAMPLE_TYPES[kinds.pop()], pinned)
+    return out[0] if len(ifds) == 1 else out
+
+
+def _read_uncompressed(path, ifds, first, h, w, dtype, pinned) -> torch.Tensor:
+    """The uncompressed pages ``ifds`` (page ``first`` of the file first) as an (n, h, w) host tensor."""
     strips = _strips(path, ifds, os.path.getsize(path))
     out = torch.empty((len(ifds), h, w), dtype=dtype, pin_memory=bool(pinned and torch.cuda.is_available()))
     raw = memoryview((out.view(torch.int16) if dtype == torch.uint16 else out).numpy().reshape(-1)).cast("B")
@@ -373,11 +382,125 @@ def read_tiff(path: Union[str, Path], pinned: bool = True) -> torch.Tensor:
             pos = i * plane
             for o, c in page:
                 if pos + c > (i + 1) * plane:
-                    raise ValueError(f"{path}: page {i} holds more than {h} x {w} samples")
+                    raise ValueError(f"{path}: page {first + i} holds more than {h} x {w} samples")
                 f.seek(o)
                 if f.readinto(raw[pos:pos + c]) != c:
-                    raise ValueError(f"{path}: short read in page {i}")
+                    raise ValueError(f"{path}: short read in page {first + i}")
                 pos += c
             if pos != (i + 1) * plane:
-                raise ValueError(f"{path}: page {i} holds {pos - i * plane} bytes, expected {plane}")
-    return out[0] if len(ifds) == 1 else out
+                raise ValueError(f"{path}: page {first + i} holds {pos - i * plane} bytes, expected {plane}")
+    return out
+
+
+_LZW_SAMPLE_TYPES = {(8, 1): torch.uint8, (8, 2): torch.int8, (16, 1): torch.uint16, (16, 2): torch.int16}
+_LZW_PAD = 8  # zero bytes after every strip: the decoder's 3-byte code window may reach 2 bytes past a strip's end
+
+
+class TiffMovie:
+    """An LZW-compressed TIFF movie read by ``read_tiff_movie``: its compressed strips, ready for ``decode_tiff`` /
+    ``motion_correct_many``.
+
+    ``payload`` (uint8 host tensor, pinned by default) holds strip s at bytes ``[strip_offsets[s], strip_offsets[s + 1]
+    - 8)``, followed by 8 zero bytes; ``strip_offsets`` (int64, n_strips + 1).  Strip s decodes into the bytes
+    ``[out_offsets[s], out_offsets[s + 1])`` of the (n_frames, h, w) stack (int64, n_strips + 1; whole rows, frame by
+    frame).  ``dtype``: uint8, int8, uint16 or int16; ``predictor``: 1 (none) or 2 (horizontal differencing)."""
+
+    def __init__(self, payload: torch.Tensor, strip_offsets: torch.Tensor, out_offsets: torch.Tensor, n_frames: int, h: int,
+                 w: int, dtype: torch.dtype, predictor: int):
+        self.payload, self.strip_offsets, self.out_offsets = payload, strip_offsets, out_offsets
+        self.n_frames, self.h, self.w, self.dtype, self.predictor = int(n_frames), int(h), int(w), dtype, int(predictor)
+
+    @property
+    def n_strips(self) -> int:
+        return int(self.strip_offsets.shape[0]) - 1
+
+    @property
+    def shape(self) -> tuple[int, int, int]:
+        return self.n_frames, self.h, self.w
+
+    def __repr__(self):
+        return (f"TiffMovie({self.n_frames} frames of {self.h} x {self.w} {self.dtype}, {self.n_strips} LZW strips, "
+                f"predictor={self.predictor}, {int(self.payload.numel())} payload bytes)")
+
+
+def read_tiff_movie(path: Union[str, Path], pinned: bool = True, frames: slice | None = None):
+    """The pages of a little-endian TIFF / BigTIFF movie (``frames``: a contiguous slice of them, as in ``read_mrc``).
+
+    LZW pages (compression 5) give a ``TiffMovie``: the selected pages' strips, concatenated in order into one page-locked
+    buffer with 8 zero bytes after each, and the two offset tables; nothing is decoded here (``decode_tiff`` does that on
+    the device).  The pages must all be LZW, of one size and one sample type: 8 or 16 bits, unsigned or signed
+    (SampleFormat 1 / 2), one sample per pixel, Predictor 1 or 2, stored in strips with FillOrder 1.  If every page is
+    uncompressed the (n, h, w) host tensor is returned instead, read as ``read_tiff`` reads it, so that a folder of either
+    kind goes through ``tiff_movies``.  Anything else raises ``ValueError`` naming the page: other compressions (deflate,
+    JPEG, zstd, PackBits ...), Predictor 3, tiles, FillOrder 2, mixed pages, and strips in the pre-TIFF-6 LZW variant
+    (libtiff's test: first byte 0 and the low bit of the second byte set)."""
+    wanted = {_TAG_WIDTH, _TAG_LENGTH, _TAG_BITS, _TAG_COMPRESSION, _TAG_STRIP_OFFSETS, _TAG_SAMPLES, _TAG_ROWS_PER_STRIP,
+              _TAG_STRIP_COUNTS, _TAG_SAMPLE_FORMAT, _TAG_FILL_ORDER, _TAG_PREDICTOR, _TAG_TILE_WIDTH}
+    ifds = _tiff_ifds(path, wanted)
+    kinds = set()
+    for i, d in enumerate(ifds):
+        comp = d.get(_TAG_COMPRESSION, (1,))[0]
+        if comp not in (1, 5):
+            raise ValueError(f"{path}: page {i} has compression {comp}; only LZW (5) and uncompressed (1) TIFF are read")
+        if _TAG_TILE_WIDTH in d:
+            raise ValueError(f"{path}: page {i} is tiled; only strips are read")
+        if d.get(_TAG_FILL_ORDER, (1,))[0] != 1:
+            raise ValueError(f"{path}: page {i} has FillOrder {d[_TAG_FILL_ORDER][0]}; only 1 (MSB first) is read")
+        if d.get(_TAG_SAMPLES, (1,))[0] != 1:
+            raise ValueError(f"{path}: page {i} has {d[_TAG_SAMPLES][0]} samples per pixel, expected 1")
+        pred = d.get(_TAG_PREDICTOR, (1,))[0]
+        if comp == 5 and pred not in (1, 2):
+            raise ValueError(f"{path}: page {i} has Predictor {pred}; only 1 (none) and 2 (horizontal) are read")
+        kinds.add((comp, d.get(_TAG_BITS, (1,))[0], d.get(_TAG_SAMPLE_FORMAT, (1,))[0], pred if comp == 5 else 1))
+    if len(kinds) != 1:
+        raise ValueError(f"{path}: mixed pages (compression, bits, sample format, predictor) {sorted(kinds)}")
+    comp, bits, fmt, predictor = kinds.pop()
+    h, w = _frame_size(path, ifds)
+    first, last = _contiguous(frames, len(ifds), "read_tiff_movie")
+    if comp == 1:
+        if (bits, fmt) not in _TIFF_SAMPLE_TYPES:
+            raise ValueError(f"{path}: samples of {bits} bits, format {fmt}; supported: uint8, uint16, int16, float32")
+        return _read_uncompressed(path, ifds[first:last], first, h, w, _TIFF_SAMPLE_TYPES[(bits, fmt)], pinned)
+    if (bits, fmt) not in _LZW_SAMPLE_TYPES:
+        raise ValueError(f"{path}: LZW samples of {bits} bits, format {fmt}; supported: uint8, int8, uint16, int16")
+    dtype = _LZW_SAMPLE_TYPES[(bits, fmt)]
+    row_bytes = w * (bits // 8)
+    pages = ifds[first:last]
+    strips = _strips(path, pages, os.path.getsize(path))
+    lengths, out_starts = [], []
+    for i, (d, page) in enumerate(zip(pages, strips)):
+        rps = min(d.get(_TAG_ROWS_PER_STRIP, (h,))[0], h)
+        if rps < 1 or len(page) != -(-h // rps):
+            raise ValueError(f"{path}: page {first + i} has {len(page)} strips for {h} rows of {rps}")
+        lengths += [c for _, c in page]
+        out_starts += [(i * h + r) * row_bytes for r in range(0, h, rps)]
+    lengths = np.asarray(lengths, dtype=np.int64)
+    offsets = np.zeros(len(lengths) + 1, dtype=np.int64)
+    np.cumsum(lengths + _LZW_PAD, out=offsets[1:])
+    out_offsets = np.asarray(out_starts + [len(pages) * h * row_bytes], dtype=np.int64)
+    pin = bool(pinned and torch.cuda.is_available())
+    payload = torch.empty((int(offsets[-1]),), dtype=torch.uint8, pin_memory=pin)
+    view = payload.numpy()
+    with open(path, "rb") as f:
+        s = 0
+        for i, page in enumerate(strips):
+            for o, c in page:
+                pos = int(offsets[s])
+                f.seek(o)
+                if f.readinto(memoryview(view[pos:pos + c])) != c:
+                    raise ValueError(f"{path}: short read in page {first + i}")
+                view[pos + c:pos + c + _LZW_PAD] = 0
+                if c >= 2 and view[pos] == 0 and view[pos + 1] & 1:
+                    raise ValueError(f"{path}: page {first + i} holds a strip in the pre-TIFF-6 (old-style) LZW variant")
+                s += 1
+    tables = [torch.from_numpy(offsets), torch.from_numpy(out_offsets)]
+    if pin:
+        tables = [t.pin_memory() for t in tables]
+    return TiffMovie(payload, tables[0], tables[1], len(pages), h, w, dtype, predictor)
+
+
+def tiff_movies(paths: Iterable[Union[str, Path]], pinned: bool = True) -> Iterator:
+    """The TIFF movies of ``paths`` one after the other (``read_tiff_movie``: a ``TiffMovie`` for LZW files, an (n, h, w)
+    host tensor for uncompressed ones): the TIFF counterpart of ``mrc_movies`` for ``motion_correct_many``."""
+    for p in paths:
+        yield read_tiff_movie(p, pinned=pinned)

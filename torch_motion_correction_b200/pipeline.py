@@ -198,8 +198,12 @@ def motion_correct_many(host_movies, pixel_spacing: float, device=None, out_host
     compressed payload and frame table cross PCIe, into staging buffers that grow to the largest payload seen; they are
     rendered on the device into a reused counts buffer (``render_eer``: n_frames // F fractions, the trailing frames
     dropped) and go on as uint8 / uint16 movies.  ``dose_per_frame`` is then the dose of one fraction.  A movie with
-    malformed frames raises ``ValueError`` when its result would be handed out."""
-    from .movie_io import EerMovie
+    malformed frames raises ``ValueError`` when its result would be handed out.
+
+    Items may also be LZW TIFF movies (``read_tiff_movie`` / ``tiff_movies``): the same way, only their compressed strips
+    and two offset tables cross PCIe; they are decoded on the device into a reused buffer (``decode_tiff``) and go on in
+    their file's sample type.  A movie with malformed strips raises ``ValueError`` when its result would be handed out."""
+    from .movie_io import EerMovie, TiffMovie
 
     dev = torch.device(device) if device is not None else torch.device("cuda", torch.cuda.current_device())
     movies = iter(host_movies)
@@ -212,40 +216,77 @@ def motion_correct_many(host_movies, pixel_spacing: float, device=None, out_host
     prepared = [None]  # one fp32 buffer: movie i is prepared into it while movie i + 1 is still in flight over PCIe
     gain_dev = gain.to(device=dev, dtype=torch.float32).contiguous() if gain is not None else None
 
-    eer_items = [None, None]  # the EerMovie staged in each slot (None: a tensor in buffers[slot])
-    eer_stage = [[None, None], [None, None]]  # per slot: device payload and frame-table buffers, grown, never shrunk
-    counts = [None]  # rendered EER counts of the current movie
+    coded_items = [None, None]  # the EerMovie / TiffMovie staged in each slot (None: a tensor in buffers[slot])
+    # per slot: device payload buffer and offset-table buffers of the compressed item, grown, never shrunk
+    coded_stage = [[None, None, None], [None, None, None]]
+    decoded = {}  # "eer" / "tiff": the reused device buffer the current movie is rendered / decoded into
+    tiff_workspace = [None]
 
-    def start_eer_copy(slot, eer):
+    def coded_parts(item):
+        """The host payload and offset tables of a compressed item that cross PCIe."""
+        if isinstance(item, TiffMovie):
+            return item.payload, [item.strip_offsets, item.out_offsets]
         from .prepare import eer_fractions
 
         if eer_frames_per_fraction is None:
             raise ValueError("motion_correct_many: EER movies need eer_frames_per_fraction=")
-        n, _ = eer_fractions(eer, eer_frames_per_fraction)
+        n, _ = eer_fractions(item, eer_frames_per_fraction)
         used = n * eer_frames_per_fraction
-        nbytes = int(eer.frame_offsets[used])
-        stage = eer_stage[slot]
+        return item.payload[:int(item.frame_offsets[used])], [item.frame_offsets[:used + 1]]
+
+    def start_coded_copy(slot, item):
+        payload, tables = coded_parts(item)
+        stage = coded_stage[slot]
         grown = False
-        if stage[0] is None or stage[0].numel() < nbytes:
-            stage[0] = torch.empty((nbytes,), dtype=torch.uint8, device=dev)
-            grown = True
-        if stage[1] is None or stage[1].numel() < used + 1:
-            stage[1] = torch.empty((used + 1,), dtype=torch.int64, device=dev)
-            grown = True
-        eer_items[slot] = eer
+        for i, (src, dtype) in enumerate([(payload, torch.uint8)] + [(t, torch.int64) for t in tables]):
+            if stage[i] is None or stage[i].numel() < src.numel():
+                stage[i] = torch.empty((src.numel(),), dtype=dtype, device=dev)
+                grown = True
+        coded_items[slot] = item
         with torch.cuda.stream(copy_stream):
             copy_stream.wait_event(consumed[slot])
             if grown:  # fresh memory from the main stream's pool: its earlier users must be done with it
                 copy_stream.wait_stream(main)
-            stage[0][:nbytes].copy_(eer.payload[:nbytes], non_blocking=True)
-            stage[1][:used + 1].copy_(eer.frame_offsets[:used + 1], non_blocking=True)
+            for i, src in enumerate([payload] + tables):
+                stage[i][:src.numel()].copy_(src, non_blocking=True)
             ready[slot].record(copy_stream)
 
+    def decode_staged(slot):
+        """Render / decode the compressed item of ``slot`` on the main stream: ``(movie, status, check)``, ``check``
+        raising for a malformed item once ``status`` is on the host."""
+        from functools import partial
+
+        from . import prepare
+
+        item, stage = coded_items[slot], coded_stage[slot]
+        if isinstance(item, TiffMovie):
+            buf = decoded.get("tiff")
+            if buf is None or tuple(buf.shape) != item.shape or buf.dtype != item.dtype:
+                buf = decoded["tiff"] = torch.empty(item.shape, dtype=item.dtype, device=dev)
+            need = prepare.tiff_workspace_bytes(item)
+            if tiff_workspace[0] is None or tiff_workspace[0].numel() < need:
+                tiff_workspace[0] = torch.empty((need,), dtype=torch.uint8, device=dev)
+            status = torch.empty((item.n_strips,), dtype=torch.int32, device=dev)
+            with torch.cuda.device(dev):
+                prepare.decode_tiff_into(stage[0][:item.payload.numel()], stage[1][:item.n_strips + 1],
+                                         stage[2][:item.n_strips + 1], item, buf, tiff_workspace[0], status)
+            return buf, status, partial(prepare.check_tiff_status, movie=item)
+        n, dtype = prepare.eer_fractions(item, eer_frames_per_fraction)
+        buf = decoded.get("eer")
+        if buf is None or tuple(buf.shape) != (n, item.h, item.w) or buf.dtype != dtype:
+            buf = decoded["eer"] = prepare.eer_counts_buffer((n, item.h, item.w), dtype, dev)
+        used = n * eer_frames_per_fraction
+        status = torch.empty((used,), dtype=torch.int32, device=dev)
+        with torch.cuda.device(dev):
+            prepare.render_eer_into(stage[0][:int(item.frame_offsets[used])], stage[1][:used + 1], item,
+                                    eer_frames_per_fraction, buf, status)
+        return buf, status, prepare.check_eer_status
+
     def start_copy(slot, host):
-        if isinstance(host, EerMovie):
-            start_eer_copy(slot, host)
+        if isinstance(host, (EerMovie, TiffMovie)):
+            start_coded_copy(slot, host)
             return
-        eer_items[slot] = None
+        coded_items[slot] = None
         if buffers[slot] is None or buffers[slot].shape != host.shape or buffers[slot].dtype != host.dtype:
             buffers[slot] = torch.empty(host.shape, dtype=host.dtype, device=dev)
         with torch.cuda.stream(copy_stream):
@@ -271,21 +312,10 @@ def motion_correct_many(host_movies, pixel_spacing: float, device=None, out_host
         if upcoming is not None:
             start_copy(1 - slot, upcoming)
         main.wait_event(ready[slot])
-        status = None
-        if eer_items[slot] is not None:
-            from .prepare import eer_counts_buffer, eer_fractions, render_eer_into
-
-            eer = eer_items[slot]
-            n, dtype = eer_fractions(eer, eer_frames_per_fraction)
-            if counts[0] is None or counts[0].shape != (n, eer.h, eer.w) or counts[0].dtype != dtype:
-                counts[0] = eer_counts_buffer((n, eer.h, eer.w), dtype, dev)
-            used = n * eer_frames_per_fraction
-            status = torch.empty((used,), dtype=torch.int32, device=dev)
-            with torch.cuda.device(dev):
-                render_eer_into(eer_stage[slot][0][:int(eer.frame_offsets[used])], eer_stage[slot][1][:used + 1], eer,
-                                eer_frames_per_fraction, counts[0], status)
-            consumed[slot].record(main)  # the staging buffers are free as soon as the movie has been rendered
-            movie = counts[0]
+        status = check = None
+        if coded_items[slot] is not None:
+            movie, status, check = decode_staged(slot)
+            consumed[slot].record(main)  # the staging buffers are free as soon as the movie has been decoded
         else:
             movie = buffers[slot]
         if movie.dtype != torch.float32 or gain_dev is not None or hot_pixel_threshold is not None or zero_frame_means:
@@ -317,18 +347,16 @@ def motion_correct_many(host_movies, pixel_spacing: float, device=None, out_host
             status.record_stream(d2h_stream)
         if pending is not None:
             yield _hand_out(pending)
-        pending = (host_sum, field, done, host_status)
+        pending = (host_sum, field, done, host_status, check)
         nxt, slot = upcoming, 1 - slot
     if pending is not None:
         yield _hand_out(pending)
 
 
 def _hand_out(pending):
-    """Wait for a result's device-to-host copy; raise if its EER render reported malformed frames."""
-    host_sum, field, done, host_status = pending
+    """Wait for a result's device-to-host copy; raise if its EER render / TIFF decode reported malformed input."""
+    host_sum, field, done, host_status, check = pending
     done.synchronize()
     if host_status is not None:
-        from .prepare import check_eer_status
-
-        check_eer_status(host_status)
+        check(host_status)
     return host_sum, field

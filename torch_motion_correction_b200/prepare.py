@@ -5,6 +5,7 @@ float32 at ``:357``) as CUDA kernels behind the C ABI (``csrc/prepare.cu``)."""
 
 from __future__ import annotations
 
+import numpy as np
 import torch
 
 from ._common import resolve_device
@@ -139,6 +140,57 @@ def render_eer(eer, frames_per_fraction: int, device=None, out: torch.Tensor | N
         status = torch.empty((used,), dtype=torch.int32, device=dev)
         render_eer_into(payload, offsets, eer, frames_per_fraction, out, status)
         check_eer_status(status.cpu())
+    return out
+
+
+def tiff_workspace_bytes(movie) -> int:
+    """Device workspace of decoding ``movie`` (``read_tiff_movie``)."""
+    return int(query("tmc_tiff_lzw_workspace_bytes", int(movie.payload.numel()), movie.n_strips))
+
+
+def decode_tiff_into(payload, strip_offsets, out_offsets, movie, out, workspace, status) -> None:
+    """Enqueue the decode of ``movie``'s strips (device ``payload`` / tables laid out as ``movie``'s) into ``out`` on the
+    current stream; ``status`` (int32, one per strip) gets 0 for a decoded strip, 1 for a malformed one.  No
+    synchronisation."""
+    call("tmc_tiff_lzw_decode", ptr(payload), int(payload.numel()), ptr(strip_offsets), ptr(out_offsets), movie.n_strips,
+         movie.n_frames * movie.h, movie.w, out.element_size(), movie.predictor, ptr(out), ptr(workspace),
+         int(workspace.numel()), ptr(status), stream_ptr(out.device))
+
+
+def check_tiff_status(status_host: torch.Tensor, movie) -> None:
+    """Raise ``ValueError`` naming the frames and strips (counted within their frame) a decode reported as malformed."""
+    bad = torch.nonzero(status_host).flatten().numpy()
+    if bad.size:
+        frame_bytes = movie.h * movie.w * movie.dtype.itemsize
+        frame_of = movie.out_offsets[:-1].numpy() // frame_bytes
+        first_strip = np.searchsorted(frame_of, frame_of[bad])
+        shown = ", ".join(f"frame {f} strip {s}" for f, s in zip(frame_of[bad][:20], (bad - first_strip)[:20]))
+        raise ValueError(f"malformed LZW strip(s): {shown}{', ...' if bad.size > 20 else ''} (a code names an undefined "
+                         "entry, the code table overflows, or the stream ends before the strip's rows are full)")
+
+
+def decode_tiff(movie, device=None, out: torch.Tensor | None = None) -> torch.Tensor:
+    """LZW TIFF movie (``read_tiff_movie``) -> its (n_frames, h, w) stack on the device, in the file's sample type
+    (uint8, int8, uint16 or int16), Predictor 2 undone.
+
+    Only the compressed payload and its two offset tables cross PCIe; the strips are decoded on the device
+    (``tmc_tiff_lzw_decode``).  A malformed strip makes this raise ``ValueError`` naming its frame and strip: that check
+    reads the per-strip status back, one host synchronisation per call.  The stack goes on through ``prepare_movie``
+    (gain, hot pixels, frame means -> fp32) like any other integer movie.  ``out``: a contiguous tensor of that shape and
+    dtype on the device, reused instead of a new one."""
+    dev = resolve_device(movie.payload, device if device is not None else "cuda")  # the payload is a host tensor
+    if out is None:
+        out = torch.empty(movie.shape, dtype=movie.dtype, device=dev)
+    elif tuple(out.shape) != movie.shape or out.dtype != movie.dtype or not out.is_contiguous() or out.device != dev:
+        raise ValueError(f"out must be a contiguous {movie.dtype} tensor of shape {movie.shape} on {dev}")
+    with torch.cuda.device(dev):
+        payload = movie.payload.to(dev, non_blocking=True)
+        strip_offsets = movie.strip_offsets.to(dev, non_blocking=True)
+        out_offsets = movie.out_offsets.to(dev, non_blocking=True)
+        workspace = torch.empty((tiff_workspace_bytes(movie),), dtype=torch.uint8, device=dev)
+        status = torch.empty((movie.n_strips,), dtype=torch.int32, device=dev)
+        decode_tiff_into(payload, strip_offsets, out_offsets, movie, out, workspace, status)
+        check_tiff_status(status.cpu(), movie)
     return out
 
 
