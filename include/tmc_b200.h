@@ -246,10 +246,16 @@ int tmc_xc_leave_one_out_products(const void* spec, int t, int g, long plane_ele
 /* partial results per item of tmc_xc_peaks for (ny, nx): the most CTAs its inverse row pass launches for any
  * kx_count (-1: unsupported nx) */
 int tmc_xc_peak_partials(int ny, int nx);
+/* bytes of the workspace of tmc_xc_peaks for nitems items (0: the band needs none; workspace may then be NULL).
+ * Bands of 2 kx_count - 1 <= nx / 4 on the half-length and polyphase row kernels bound every row from its samples at
+ * x = 4m and transform only the row blocks that can hold the maximum; the workspace then starts with the int32 count of
+ * those blocks (of the last slice of at most 65535 items). */
+long tmc_xc_peaks_workspace_bytes(int nitems, int ny, int nx, int kx_count);
 /* prod (nitems, ky_count, kx_count) -> shifts (nitems, 2) = (dy, dx) px.  tmp: nitems*ny*kx_count complex64;
- * partial: nitems * tmc_xc_peak_partials(ny, nx) * 8 bytes. */
+ * partial: nitems * tmc_xc_peak_partials(ny, nx) * 8 bytes; workspace: tmc_xc_peaks_workspace_bytes bytes. */
 int tmc_xc_peaks(const void* prod, int nitems, int ny, int nx, int kx_count, int ky_count, int ky_start, int sub_pixel,
-                 const void* plan_x, const void* plan_y, void* tmp, void* partial, float* shifts, tmc_stream_t stream);
+                 const void* plan_x, const void* plan_y, void* tmp, void* partial, void* workspace, float* shifts,
+                 tmc_stream_t stream);
 
 /* ---- whole-frame Fourier shift: correct_motion.py:484-496 + torch_fourier_shift.fourier_shift_dft_2d */
 /* spec (t, ny, nx/2+1) *= exp(-2 pi i (f_y s_y + f_x s_x)), (s_y, s_x)[f] = sign * field[(0|1) * t + f] */

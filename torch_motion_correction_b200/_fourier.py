@@ -168,8 +168,9 @@ class BandPlan:
                      float(dose_per_frame), float(voltage), ptr(tables), stream_ptr(dev))
 
     # -- inverse + peak ---------------------------------------------------------------------------
-    def peaks(self, prod: torch.Tensor, sub_pixel: bool, shifts=None):
-        """prod (nitems, KY, KX, 2) -> (nitems, 2) px shifts (dy, dx)."""
+    def peaks(self, prod: torch.Tensor, sub_pixel: bool, shifts=None, workspace_out: list | None = None):
+        """prod (nitems, KY, KX, 2) -> (nitems, 2) px shifts (dy, dx).  ``workspace_out``: a list that receives the
+        search's workspace (tmc_xc_peaks_workspace_bytes; None when the band needs none)."""
         nitems = prod.shape[0]
         dev = prod.device
         if shifts is None:
@@ -179,6 +180,8 @@ class BandPlan:
         tmp = torch.empty((chunk * per_item // 4,), dtype=torch.float32, device=dev)
         nparts = query("tmc_xc_peak_partials", self.ny, self.nx)
         partial = torch.empty((chunk * nparts * 2,), dtype=torch.float32, device=dev)
+        ws_bytes = query("tmc_xc_peaks_workspace_bytes", chunk, self.ny, self.nx, self.kx)
+        workspace = torch.empty((ws_bytes,), dtype=torch.uint8, device=dev) if ws_bytes else None
         prod_base, shifts_base = prod.data_ptr(), shifts.data_ptr()
         with torch.cuda.device(dev):
             stream = stream_ptr(dev)
@@ -186,7 +189,9 @@ class BandPlan:
                 n = min(chunk, nitems - i0)
                 call("tmc_xc_peaks", prod_base + i0 * self.plane_elems * _C64, n, self.ny, self.nx, self.kx, self.ky,
                      self.ky_start, int(sub_pixel), ptr(self.tw_x), ptr(self.tw_y), ptr(tmp), ptr(partial),
-                     shifts_base + i0 * 2 * 4, stream)
+                     ptr(workspace), shifts_base + i0 * 2 * 4, stream)
+        if workspace_out is not None:
+            workspace_out.append(workspace)
         return shifts
 
     def shift_frames(self, image: torch.Tensor, mean_std, field: torch.Tensor) -> torch.Tensor:

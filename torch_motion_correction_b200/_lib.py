@@ -66,7 +66,8 @@ _SIGNATURES = {
     "tmc_xc_pair_products": (I, [P, P, P, I, L, P, P]),
     "tmc_xc_leave_one_out_products": (I, [P, I, I, L, P, P, I, I, P, P]),
     "tmc_xc_peak_partials": (I, [I, I]),
-    "tmc_xc_peaks": (I, [P, I, I, I, I, I, I, I, P, P, P, P, P, P]),
+    "tmc_xc_peaks_workspace_bytes": (L, [I, I, I, I]),
+    "tmc_xc_peaks": (I, [P, I, I, I, I, I, I, I, P, P, P, P, P, P, P]),
     "tmc_irfft2_full": (I, [P, I, I, I, P, P, P, P, P]),
     "tmc_fourier_crop_workspace_bytes": (L, [I, I, I, I, I]),
     "tmc_fourier_crop": (I, [P, I, I, I, I, I, P, I, P, P, P, P, P, P, P]),

@@ -43,11 +43,12 @@ struct Smem {
   __device__ explicit Smem(float2* base) : data(base), tw_lo(base + Cfg<N>::B * Cfg<N>::STRIDE), tw_hi(tw_lo + 64) {}
 };
 
-// fill the factorised twiddle tables from the global W_N^m table; caller syncs afterwards
+// fill the factorised twiddle tables from the global W_N^m table (or, stride s, from the W_{sN}^m table of a transform
+// s times longer: W_N^m = W_{sN}^{s m}); caller syncs afterwards
 template <int N>
-__device__ __forceinline__ void load_twiddles(const Smem<N>& sm, const float2* __restrict__ tw) {
+__device__ __forceinline__ void load_twiddles(const Smem<N>& sm, const float2* __restrict__ tw, int stride = 1) {
   for (int i = threadIdx.x; i < 64 + Cfg<N>::TW_HI; i += kThreads)
-    sm.tw_lo[i] = i < 64 ? __ldg(tw + i) : __ldg(tw + (i - 64) * 64);
+    sm.tw_lo[i] = i < 64 ? __ldg(tw + stride * i) : __ldg(tw + stride * (i - 64) * 64);
 }
 
 template <int N>

@@ -13,6 +13,7 @@
 //    instead of storing the correlation surface.
 #include "common.cuh"
 #include <stdlib.h>
+#include <cmath>
 #include "fft_core.cuh"
 #include "fft_core2.cuh"
 
@@ -611,6 +612,44 @@ constexpr bool use_fast_path() {
   return !BLU && M >= 256;
 }
 
+// ---- live row blocks of the peak search (after rows_coarse_bound_p2) ---------------------------
+// One CTA per item: T = the largest lo of the item's coarse CTAs.  A fine row block is live if its hi >= T, or if any
+// bound of the item is not finite (every block stays live, as without the bound).  Dead blocks get the partial result
+// (-inf, INT_MAX), which peak_finalize_kernel never picks; live (item, block) pairs are appended to list, *count of them.
+__global__ void __launch_bounds__(256)
+rows_select_live(const float* __restrict__ hi, int nfine, const float* __restrict__ lo, int ncoarse,
+                 PeakCandidate* __restrict__ partial, int2* __restrict__ list, int* __restrict__ count) {
+  __shared__ float s_t[8];
+  const long item = blockIdx.x;
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+  float t = -INFINITY;
+  bool bad = false;
+  for (int i = threadIdx.x; i < ncoarse; i += 256) {
+    const float v = lo[item * ncoarse + i];
+    bad |= !isfinite(v);
+    t = fmaxf(t, v);
+  }
+  for (int i = threadIdx.x; i < nfine; i += 256) bad |= !isfinite(hi[item * nfine + i]);
+#pragma unroll
+  for (int o = 16; o > 0; o >>= 1) t = fmaxf(t, __shfl_xor_sync(0xffffffffu, t, o));
+  if (lane == 0) s_t[warp] = t;
+  bad = __syncthreads_or(bad);
+  for (int i = 0; i < 8; ++i) t = fmaxf(t, s_t[i]);
+  for (int b0 = 0; b0 < nfine; b0 += 256) {
+    const int b = b0 + threadIdx.x;
+    bool live = false;
+    if (b < nfine) {
+      live = bad || hi[item * nfine + b] >= t;
+      if (!live) partial[item * nfine + b] = PeakCandidate{-INFINITY, 0x7fffffff};
+    }
+    const unsigned mask = __ballot_sync(0xffffffffu, live);
+    int at = 0;
+    if (lane == 0 && mask) at = atomicAdd(count, __popc(mask));
+    at = __shfl_sync(0xffffffffu, at, 0);
+    if (live) list[at + __popc(mask & ((1u << lane) - 1))] = make_int2((int)item, b);
+  }
+}
+
 // ---- peak finalisation: argmax over CTAs, 3-point parabola, wrap ---------------------------
 
 // value of the real surface at (y, x) from the column-transformed rows (direct KX-term sum)
@@ -890,21 +929,25 @@ int cols_inverse(const void* spec, int nitems, int ny, int KX, int KY, int ky_st
 }
 
 // The inverse row pass's kernel for rows of length R * n served by FFT size MM (BB: Bluestein) with a band of KX bins.
-// The peak search (argmax) also has the half-length and polyphase kernels for narrow bands; the store has not.
+// The peak search (argmax) also has the half-length and polyphase kernels for narrow bands; the store has not.  Those
+// two run after the coarse bound (rows_coarse_bound_p2) where the band fits a quarter-length transform: only on the
+// row blocks that can hold the maximum.
 enum class RowsInverseKernel { real2n, poly, p2, generic };
 struct RowsInverseChoice {
   RowsInverseKernel kernel;
   int rows_per_cta;
+  bool coarse = false;
 };
 
 template <int MM, bool BB>
 RowsInverseChoice choose_rows_inverse(int R, int KX, bool argmax) {
+  const bool coarse = 2 * KX - 1 <= MM / 4;
   if constexpr ((MM == 8192 || MM == 4096) && !BB) {
     // one row per half-length transform instead of two rows per full-length transform (see rows_forward_real2n)
-    if (argmax && R == 1 && KX <= MM / 4) return {RowsInverseKernel::real2n, rows_per_cta_inverse_real2n<MM / 2>()};
+    if (argmax && R == 1 && KX <= MM / 4) return {RowsInverseKernel::real2n, rows_per_cta_inverse_real2n<MM / 2>(), coarse};
   }
   if constexpr (MM == 1024 && !BB) {
-    if (argmax && R == 1 && KX <= 128) return {RowsInverseKernel::poly, poly::kRowsPerCta};
+    if (argmax && R == 1 && KX <= 128) return {RowsInverseKernel::poly, poly::kRowsPerCta, coarse};
   }
   if constexpr (use_fast_path<MM, BB>()) {
     if (R == 1) return {RowsInverseKernel::p2, rows_per_cta_inverse<MM>()};
@@ -921,27 +964,94 @@ int rows_inverse_ctas(int ny, int nx, int KX, bool argmax) {
   });
 }
 
+// Workspace of the coarse bound for n items (at most kMaxGridYZ: one slice), laid out from `base`:
+//   int count, int2 list[n][fine], float hi[n][fine], float lo[n][coarse]
+// fine = row blocks of the fine kernel, coarse = CTAs of the coarse pass per item.
+struct CoarseWorkspace {
+  int* count;
+  int2* list;
+  float* hi;
+  float* lo;
+};
+
+size_t coarse_workspace_bytes(int n, int fine, int coarse) { return 16 + 12ull * n * fine + 4ull * n * coarse; }
+
+CoarseWorkspace coarse_workspace(void* base, int n, int fine) {
+  char* p = (char*)base;
+  CoarseWorkspace w;
+  w.count = (int*)p;
+  w.list = (int2*)(p + 16);
+  w.hi = (float*)(p + 16 + 8l * n * fine);
+  w.lo = w.hi + (long)n * fine;
+  return w;
+}
+
+// rows of N points: bound every row from its samples at x = 4m, select the live fine row blocks (rows_per_fine rows
+// each) of the n items into the workspace, dead ones into partial
+template <int N>
+int coarse_select(const float2* src, int n, int ny, int KX, const AxisPlan& px, int rows_per_fine, PeakCandidate* partial,
+                  void* workspace, cudaStream_t stream, CoarseWorkspace* ws) {
+  constexpr int ROWS = rows_per_cta_inverse<N / 4>();  // rows per CTA of rows_coarse_bound_p2<N / 4>
+  const int nfine = tmc_div_up(ny, rows_per_fine), ncoarse = tmc_div_up(ny, ROWS);
+  if (ROWS % rows_per_fine != 0) {
+    tmc_set_error("xc_peaks: a coarse CTA of %d rows does not cover whole row blocks of %d", ROWS, rows_per_fine);
+    return TMC_ERR_UNSUPPORTED;
+  }
+  *ws = coarse_workspace(workspace, n, nfine);
+  // eps_y = 32 eps32 (log2 N + 8) * 2 max(L1), curv = 2 (2 pi / N)^2, both rounded up
+  const float eps_rel = (float)(64.0 * 0x1p-23 * (std::log2((double)N) + 8.0) * (1.0 + 1e-6));
+  const float curv = (float)(2.0 * (2.0 * M_PI / N) * (2.0 * M_PI / N) * (1.0 + 1e-6));
+  const float2* tw = (const float2*)px.tw;
+  constexpr int M = N / 4;
+  const int rc = launch(M == 2048 ? "rows_coarse_bound_p2<2048>" : TMC_LABEL2("rows_coarse_bound_p2", M, 256, 1024),
+                        rows_coarse_bound_p2<M>, dim3(ncoarse, n), fft2::kThreads, rows_inverse_smem_bytes<M>(), stream, src,
+                        ny, KX, tw, rows_per_fine, eps_rel, curv, ws->hi, ws->lo);
+  if (rc) return rc;
+  TMC_CUDA(cudaMemsetAsync(ws->count, 0, sizeof(int), stream));
+  TMC_TIMED("rows_select_live", stream, rows_select_live<<<n, 256, 0, stream>>>(ws->hi, nfine, ws->lo, ncoarse, partial,
+                                                                                ws->list, ws->count));
+  return TMC_OK;
+}
+
+// CTAs of a fine row kernel that walks the live list: three per SM (the kernels' residency)
+int live_list_ctas() {
+  int dev = 0, sms = 148;
+  if (cudaGetDevice(&dev) == cudaSuccess) cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
+  return 3 * sms;
+}
+
 // c2r row pass: tmp (nitems, ny, KX) -> partial != nullptr: the maximum of each CTA's rows into partial[item][cta]
-// (rows_inverse_ctas of them per item); otherwise out (nitems, ny, nx) f32 times `scale`.  Keeps only the real part of
-// the kx = 0 and kx = nx/2 entries, as c2r does.
+// (rows_inverse_ctas of them per item; workspace: tmc_xc_peaks_workspace_bytes); otherwise out (nitems, ny, nx) f32
+// times `scale`.  Keeps only the real part of the kx = 0 and kx = nx/2 entries, as c2r does.
 int rows_inverse(const void* tmp, int nitems, int ny, int nx, int KX, const AxisPlan& px, PeakCandidate* partial,
-                 float scale, float* out, cudaStream_t stream, const char* who) {
+                 void* workspace, float scale, float* out, cudaStream_t stream, const char* who) {
   return dispatch_fft(nx, who, [&](auto M, auto BLU) {
     constexpr int MM = decltype(M)::value;
     constexpr bool BB = decltype(BLU)::value;
     const RowsInverseChoice c = choose_rows_inverse<MM, BB>(px.R, KX, partial != nullptr);
-    const dim3 grid(tmc_div_up(ny, c.rows_per_cta), nitems);
+    dim3 grid(tmc_div_up(ny, c.rows_per_cta), nitems);
     const float2* src = (const float2*)tmp;
     if (partial != nullptr) {
+      RowBlocks blocks{nullptr, nullptr, (int)grid.x};
+      if constexpr ((MM == 8192 || MM == 4096 || MM == 1024) && !BB) {
+        if (c.coarse) {
+          CoarseWorkspace ws;
+          if (int rc = coarse_select<MM>(src, nitems, ny, KX, px, c.rows_per_cta, partial, workspace, stream, &ws))
+            return rc;
+          blocks = RowBlocks{ws.list, ws.count, (int)grid.x};
+          grid = dim3(live_list_ctas());
+        }
+      }
       if constexpr ((MM == 8192 || MM == 4096) && !BB) {
         if (c.kernel == RowsInverseKernel::real2n)
           return launch(TMC_LABEL2("rows_inverse_argmax_real2n", MM / 2, 2048, 4096), rows_inverse_argmax_real2n<MM / 2>,
-                        grid, fft2::kThreads, rows_inverse_real2n_smem_bytes<MM / 2>(), stream, src, ny, KX, px.tw, partial);
+                        grid, fft2::kThreads, rows_inverse_real2n_smem_bytes<MM / 2>(), stream, src, ny, KX, px.tw, partial,
+                        blocks);
       }
       if constexpr (MM == 1024 && !BB) {
         if (c.kernel == RowsInverseKernel::poly)
           return launch("rows_inverse_argmax_poly", poly::rows_inverse_argmax_poly, grid, poly::kThreads, poly::smem_bytes,
-                        stream, src, ny, KX, px.tw, partial);
+                        stream, src, ny, KX, px.tw, partial, blocks);
       }
       if constexpr (use_fast_path<MM, BB>()) {
         if (c.kernel == RowsInverseKernel::p2)
@@ -959,6 +1069,23 @@ int rows_inverse(const void* tmp, int nitems, int ny, int nx, int KX, const Axis
     return launch("rows_inverse_store_kernel", rows_inverse_store_kernel<MM, BB>, grid, kThreads, fft_smem_bytes<MM>(),
                   stream, src, ny, KX, px, scale, out);
   });
+}
+
+// bytes of the peak search's workspace for n items (0: the band runs the full search)
+size_t peaks_workspace_bytes(int n, int ny, int nx, int KX) {
+  const int R = decimation_for(nx);
+  if (R == 0) return 0;
+  size_t bytes = 0;
+  dispatch_fft(nx, "xc_peaks", [&](auto M, auto BLU) {
+    constexpr int MM = decltype(M)::value;
+    const RowsInverseChoice c = choose_rows_inverse<MM, decltype(BLU)::value>(R, KX, true);
+    if constexpr (MM == 8192 || MM == 4096 || MM == 1024) {
+      if (c.coarse)
+        bytes = coarse_workspace_bytes(n, tmc_div_up(ny, c.rows_per_cta), tmc_div_up(ny, rows_per_cta_inverse<MM / 4>()));
+    }
+    return TMC_OK;
+  });
+  return bytes;
 }
 
 }  // namespace
@@ -1133,21 +1260,32 @@ TMC_API int tmc_xc_peak_partials(int ny, int nx) {
   return narrow > wide ? narrow : wide;
 }
 
+// Bytes of tmc_xc_peaks's workspace for nitems items (0: this band needs none).  Where the band fits a quarter-length
+// row transform, the search bounds every row from its samples at x = 4m first and runs the full-length row transforms
+// only on the row blocks that can hold the maximum; the workspace then starts with the int32 count of those blocks (of
+// the last slice of at most 65535 items).
+TMC_API long tmc_xc_peaks_workspace_bytes(int nitems, int ny, int nx, int kx_count) {
+  if (nitems < 1 || ny < 1 || kx_count < 1 || kx_count > nx / 2 + 1) return 0;
+  return (long)peaks_workspace_bytes(nitems < kMaxGridYZ ? nitems : kMaxGridYZ, ny, nx, kx_count);
+}
+
 // Inverse 2-D transform of band-limited products + argmax (+ parabola) + wrap.
 //  prod (nitems, KY, KX) complex64; tmp: nitems*ny*KX complex64; partial: nitems*tmc_xc_peak_partials(ny,nx)*8 bytes;
-//  shifts (nitems, 2) f32 = (dy, dx) px.
+//  workspace: tmc_xc_peaks_workspace_bytes(nitems, ny, nx, kx_count) bytes; shifts (nitems, 2) f32 = (dy, dx) px.
 TMC_API int tmc_xc_peaks(const void* prod, int nitems, int ny, int nx, int kx_count, int ky_count, int ky_start,
-                         int sub_pixel, const void* plan_x, const void* plan_y, void* tmp, void* partial, float* shifts,
-                         cudaStream_t stream) {
+                         int sub_pixel, const void* plan_x, const void* plan_y, void* tmp, void* partial, void* workspace,
+                         float* shifts, cudaStream_t stream) {
   TMC_CHECK_ARG(prod && plan_x && plan_y && tmp && partial && shifts, "xc_peaks: null pointer");
   TMC_CHECK_ARG(kx_count >= 1 && kx_count <= nx / 2 + 1 && ky_count >= 1 && ky_count <= ny, "xc_peaks: bad band box");
+  TMC_CHECK_ARG(workspace || tmc_xc_peaks_workspace_bytes(nitems, ny, nx, kx_count) == 0, "xc_peaks: null workspace");
   const AxisPlan px = make_axis_plan(plan_x, nx), py = make_axis_plan(plan_y, ny);
   return for_each_slice(nitems, kMaxGridYZ, [&](int i0, int n) {
     if (int rc = cols_inverse((const float2*)prod + (long)i0 * ky_count * kx_count, n, ny, kx_count, ky_count, ky_start, py,
                               tmp, stream, "xc_peaks"))
       return rc;
     TMC_CHECK_LAUNCH("tmc_xc_peaks(cols)");
-    if (int rc = rows_inverse(tmp, n, ny, nx, kx_count, px, (PeakCandidate*)partial, 0.f, nullptr, stream, "xc_peaks"))
+    if (int rc = rows_inverse(tmp, n, ny, nx, kx_count, px, (PeakCandidate*)partial, workspace, 0.f, nullptr, stream,
+                              "xc_peaks"))
       return rc;
     TMC_CHECK_LAUNCH("tmc_xc_peaks(rows)");
     const int nparts = rows_inverse_ctas(ny, nx, kx_count, true);
@@ -1167,7 +1305,7 @@ TMC_API int tmc_irfft2_full(const void* spec, int nitems, int ny, int nx, const 
     if (int rc = cols_inverse((const float2*)spec + (long)i0 * ny * (nx / 2 + 1), n, ny, nx / 2 + 1, ny, 0, py, tmp, stream,
                               "irfft2_full"))
       return rc;
-    if (int rc = rows_inverse(tmp, n, ny, nx, nx / 2 + 1, px, nullptr, 1.0f / ((float)nx * (float)ny),
+    if (int rc = rows_inverse(tmp, n, ny, nx, nx / 2 + 1, px, nullptr, nullptr, 1.0f / ((float)nx * (float)ny),
                               out + (long)i0 * ny * nx, stream, "irfft2_full"))
       return rc;
     TMC_CHECK_LAUNCH("tmc_irfft2_full");
@@ -1243,13 +1381,13 @@ TMC_API int tmc_fourier_crop(const float* image, int t, int h, int w, int out_h,
                     cols_crop_smem_bytes<NN, MM>(), stream, (const float2*)rows, KX, py_in.tw, py.tw, box);
     });
     if (rc) return rc;
-    rc = rows_inverse(box, t, out_h, out_w, KX, px, nullptr, scale, out, stream, "fourier_crop");
+    rc = rows_inverse(box, t, out_h, out_w, KX, px, nullptr, nullptr, scale, out, stream, "fourier_crop");
   } else {
     if ((rc = tmc_rfft2_band(image, t, h, w, nullptr, nullptr, h, w, jobs, njobs, 2, nullptr, 0, 0, h, KX, out_h,
                              -(out_h / 2), nullptr, plan_x, plan_y, rows, box, stream)))
       return rc;
     if ((rc = cols_inverse(box, t, out_h, KX, out_h, -(out_h / 2), py, rows, stream, "fourier_crop"))) return rc;
-    rc = rows_inverse(rows, t, out_h, out_w, KX, px, nullptr, scale, out, stream, "fourier_crop");
+    rc = rows_inverse(rows, t, out_h, out_w, KX, px, nullptr, nullptr, scale, out, stream, "fourier_crop");
   }
   if (rc) return rc;
   TMC_CHECK_LAUNCH("tmc_fourier_crop");
@@ -1309,7 +1447,7 @@ TMC_API int tmc_fourier_shift_frames(const float* image, int t, int ny, int nx, 
     return TMC_OK;
   });
   if (rc) return rc;
-  rc = rows_inverse(tmp, t, ny, nx, kx, px, nullptr, 1.0f / ((float)nx * (float)ny), out, stream, "fourier_shift_frames");
+  rc = rows_inverse(tmp, t, ny, nx, kx, px, nullptr, nullptr, 1.0f / ((float)nx * (float)ny), out, stream, "fourier_shift_frames");
   if (rc) return rc;
   TMC_CHECK_LAUNCH("tmc_fourier_shift_frames");
   return TMC_OK;

@@ -153,9 +153,7 @@ rows_forward_real2n(const float* __restrict__ image, int H, int W, const float* 
   using P = fft2::Plan<N>;
   extern __shared__ float2 smem[];
   const fft2::Smem<N> sm(smem);
-  // W_N^m = W_2N^{2m}: the factorised tables of the N-point transform from the 2N-point plan
-  for (int i = threadIdx.x; i < 64 + C::TW_HI; i += fft2::kThreads)
-    sm.tw_lo[i] = i < 64 ? __ldg(tw2n + 2 * i) : __ldg(tw2n + 2 * (i - 64) * 64);
+  fft2::load_twiddles<N>(sm, tw2n, 2);  // W_N^m = W_2N^{2m}: the tables of the N-point transform from the 2N-point plan
   const int seq = threadIdx.x / C::TPS, j = threadIdx.x % C::TPS;
   float2* myseq = sm.data + seq * C::STRIDE;
   float2* stage_p = smem + C::B * C::STRIDE + 64 + C::TW_HI;  // pixel pairs, slot e * kThreads + threadIdx.x
@@ -346,7 +344,7 @@ __host__ __device__ constexpr int rows_per_cta_inverse() {
 }
 
 template <int N>
-constexpr size_t rows_inverse_smem_bytes() {
+__host__ __device__ constexpr size_t rows_inverse_smem_bytes() {
   return fft2::Cfg<N>::smem_bytes + 2ull * fft2::Cfg<N>::B * N * sizeof(float2);
 }
 
@@ -367,15 +365,22 @@ __device__ __forceinline__ float2 c2r_pack(float2 ca, float2 cb, int i, int KX) 
   return make_float2(cb.x - ca.y, ca.x + cb.y);                // Z[N-k] = conj(Ca) + i conj(Cb), stored (im, re)
 }
 
-// Shared driver of the two inverse row kernels: calls consume(ya, has_b, v) with the last-pass outputs of
-// every row pair of this CTA (v swapped: .y = row ya, .x = row ya + 1).
-template <int N, typename Consume>
+struct NoCoeff {
+  __device__ void operator()(int, float2, float2) const {}
+};
+
+// Shared driver of the inverse row kernels: calls consume(ya, has_b, v) with the last-pass outputs of
+// every row pair of this CTA (v swapped: .y = row ya, .x = row ya + 1), and before that on_coeff(i, Ca, Cb) with the
+// coefficients of every packed entry i the calling thread builds.  tw: the W_N^m table, or the table of a
+// transform tw_stride times longer.
+template <int N, typename Consume, typename OnCoeff = NoCoeff>
 __device__ __forceinline__ void rows_inverse_driver(const float2* __restrict__ src, int NY, int KX,
-                                                    const float2* __restrict__ tw, float2* smem, Consume&& consume) {
+                                                    const float2* __restrict__ tw, int tw_stride, float2* smem,
+                                                    Consume&& consume, OnCoeff&& on_coeff = OnCoeff{}) {
   using C = fft2::Cfg<N>;
   using P = fft2::Plan<N>;
   const fft2::Smem<N> sm(smem);
-  fft2::load_twiddles<N>(sm, tw);
+  fft2::load_twiddles<N>(sm, tw, tw_stride);
   const int seq = threadIdx.x / C::TPS, j = threadIdx.x % C::TPS;
   float2* myseq = sm.data + seq * C::STRIDE;
   float2* stage_a = smem + C::B * C::STRIDE + 64 + C::TW_HI;
@@ -417,7 +422,9 @@ __device__ __forceinline__ void rows_inverse_driver(const float2* __restrict__ s
         const int i = P::First::in_index(j, e / R, e % R);
         if (c2r_source_index<N>(i, KX) >= 0) {
           const int slot = e * fft2::kThreads + threadIdx.x;
-          z = c2r_pack<N>(stage_a[slot], has_b ? stage_b[slot] : make_float2(0.f, 0.f), i, KX);
+          const float2 ca = stage_a[slot], cb = has_b ? stage_b[slot] : make_float2(0.f, 0.f);
+          on_coeff(i, ca, cb);
+          z = c2r_pack<N>(ca, cb, i, KX);
         }
       }
       v[e] = z;
@@ -439,7 +446,7 @@ rows_inverse_argmax_p2(const float2* __restrict__ tmp, int NY, int KX, const flo
   const long item = blockIdx.y;
   float best = -INFINITY;
   int best_idx = 0x7fffffff;
-  rows_inverse_driver<N>(tmp + item * NY * KX, NY, KX, tw, smem, [&](int ya, bool has_b, int j, const float2* v) {
+  rows_inverse_driver<N>(tmp + item * NY * KX, NY, KX, tw, 1, smem, [&](int ya, bool has_b, int j, const float2* v) {
     // the thread visits its samples in increasing index order (out_index = j + g TPS + r NS with G TPS == NS: r outer,
     // g inner; row ya, then row ya + 1; later calls have larger ya), so "strictly greater" keeps the first of equal
     // maxima: one compare and two selects per sample
@@ -495,6 +502,28 @@ rows_inverse_argmax_p2(const float2* __restrict__ tmp, int NY, int KX, const flo
   }
 }
 
+// The row blocks (CTA-sized groups of rows, one partial result each) an argmax row kernel visits: its whole grid
+// (blockIdx.x = block, blockIdx.y = item) or, after the coarse bound (rows_coarse_bound_p2), only the live (item, block)
+// pairs of `list`, which the CTAs of a one-dimensional grid share round-robin.
+struct RowBlocks {
+  const int2* list;  // nullptr: the whole grid
+  const int* count;  // entries of list
+  int per_item;      // blocks (partial slots) per item
+};
+
+template <typename F>
+__device__ __forceinline__ void for_each_row_block(const RowBlocks& blocks, F&& f) {
+  if (blocks.list == nullptr) {
+    f((long)blockIdx.y, (int)blockIdx.x);
+    return;
+  }
+  const int n = *blocks.count;
+  for (int w = blockIdx.x; w < n; w += gridDim.x) {
+    const int2 u = blocks.list[w];
+    f((long)u.x, u.y);
+  }
+}
+
 // ---- inverse rows of length 2N as N-point complex transforms + argmax ------------------------------------------------
 //
 // x[0 .. 2N) real with spectrum X[k], k < KX <= N / 2:  z[m] = x[2m] + i x[2m+1] = IDFT_N(Z),
@@ -514,110 +543,263 @@ constexpr size_t rows_inverse_real2n_smem_bytes() {
 template <int N>
 __global__ void __launch_bounds__(fft2::kThreads, N >= 2048 ? 3 : 1)
 rows_inverse_argmax_real2n(const float2* __restrict__ tmp, int NY, int KX, const float2* __restrict__ tw2n,
-                           PeakCandidate* __restrict__ partial) {
+                           PeakCandidate* __restrict__ partial, RowBlocks blocks) {
   using C = fft2::Cfg<N>;
   using P = fft2::Plan<N>;
   extern __shared__ float2 smem[];
   const fft2::Smem<N> sm(smem);
-  for (int i = threadIdx.x; i < 64 + C::TW_HI; i += fft2::kThreads)
-    sm.tw_lo[i] = i < 64 ? __ldg(tw2n + 2 * i) : __ldg(tw2n + 2 * (i - 64) * 64);
-  const long item = blockIdx.y;
-  const float2* src = tmp + item * NY * KX;
+  fft2::load_twiddles<N>(sm, tw2n, 2);  // W_N^m = W_2N^{2m}
   const int seq = threadIdx.x / C::TPS, j = threadIdx.x % C::TPS;
   float2* myseq = sm.data + seq * C::STRIDE;
   float2* stage_a = smem + C::B * C::STRIDE + 64 + C::TW_HI;
-  auto row_of = [&](int it) { return (int)blockIdx.x * rows_per_cta_inverse_real2n<N>() + it * C::B + seq; };
-  auto prefetch = [&](int it) {
-    const int y = row_of(it);
-    if (y >= NY) return;
-    const float2* row = src + (long)y * KX;
-#pragma unroll
-    for (int e = 0; e < C::VPT; ++e) {
-      constexpr int R = P::First::R;
-      // whole blocks of entries are zero for a band-limited spectrum: warp-uniform skip
-      const int lo = (e / R) * C::TPS + (e % R) * P::First::NBR;
-      if (lo >= KX && lo + C::TPS <= N - KX + 1) continue;
-      const int k = c2r_source_index<N>(P::First::in_index(j, e / R, e % R), KX);
-      if (k >= 0) cp_async_f32x2(stage_a + e * fft2::kThreads + threadIdx.x, row + k);
-    }
-  };
-  float best = -INFINITY;
-  int best_idx = 0x7fffffff;
-  prefetch(0);
-  __syncthreads();
-  for (int it = 0; it < kRowIters; ++it) {
-    const int y = row_of(it);
-    const bool active = y < NY;
-    cp_async_commit_and_wait();
-    float2 v[C::VPT];
-#pragma unroll
-    for (int e = 0; e < C::VPT; ++e) {
-      constexpr int R = P::First::R;
-      float2 z = make_float2(0.f, 0.f);
-      const int lo = (e / R) * C::TPS + (e % R) * P::First::NBR;
-      if (active && !(lo >= KX && lo + C::TPS <= N - KX + 1)) {
-        const int i = P::First::in_index(j, e / R, e % R);
-        const int k = c2r_source_index<N>(i, KX);
-        if (k >= 0) {
-          const float2 ca = stage_a[e * fft2::kThreads + threadIdx.x];
-          const float2 w = __ldg(tw2n + k);  // W_2N^k; Y[k] = X[k] conj(W_2N^k)
-          const float2 cb = make_float2(ca.x * w.x + ca.y * w.y, ca.y * w.x - ca.x * w.y);
-          z = c2r_pack<N>(ca, cb, i, KX);
-        }
-      }
-      v[e] = z;
-    }
-    if (it + 1 < kRowIters) prefetch(it + 1);
-    fft2::fft_regs_to_regs<N>(sm, myseq, j, v);
-    if (active) {
-      // samples in increasing index order (m = out_index ascends with r outer, g inner; 2m before 2m + 1; later rows
-      // later): a strictly-greater compare keeps the first of equal maxima
-      const int base = y * (2 * N);
-#pragma unroll
-      for (int r = 0; r < P::Last::R; ++r)
-#pragma unroll
-        for (int g = 0; g < P::Last::G; ++g) {
-          const float2 val = P::Last::result(v, g, r);  // swapped: .y = x[2m], .x = x[2m + 1]
-          const int idx = base + 2 * P::Last::out_index(j, g, r);
-          if (val.y > best) {
-            best = val.y;
-            best_idx = idx;
-          }
-          if (val.x > best) {
-            best = val.x;
-            best_idx = idx + 1;
-          }
-        }
-    }
-    __syncthreads();
-  }
-#pragma unroll
-  for (int o = 16; o > 0; o >>= 1) {
-    const float ov = __shfl_xor_sync(0xffffffffu, best, o);
-    const int oi = __shfl_xor_sync(0xffffffffu, best_idx, o);
-    if (better(ov, oi, best, best_idx)) {
-      best = ov;
-      best_idx = oi;
-    }
-  }
   __shared__ float sval[fft2::kThreads / 32];
   __shared__ int sidx[fft2::kThreads / 32];
-  if ((threadIdx.x & 31) == 0) {
-    sval[threadIdx.x >> 5] = best;
-    sidx[threadIdx.x >> 5] = best_idx;
+  for_each_row_block(blocks, [&](long item, int blk) {
+    const float2* src = tmp + item * NY * KX;
+    auto row_of = [&](int it) { return blk * rows_per_cta_inverse_real2n<N>() + it * C::B + seq; };
+    auto prefetch = [&](int it) {
+      const int y = row_of(it);
+      if (y >= NY) return;
+      const float2* row = src + (long)y * KX;
+#pragma unroll
+      for (int e = 0; e < C::VPT; ++e) {
+        constexpr int R = P::First::R;
+        // whole blocks of entries are zero for a band-limited spectrum: warp-uniform skip
+        const int lo = (e / R) * C::TPS + (e % R) * P::First::NBR;
+        if (lo >= KX && lo + C::TPS <= N - KX + 1) continue;
+        const int k = c2r_source_index<N>(P::First::in_index(j, e / R, e % R), KX);
+        if (k >= 0) cp_async_f32x2(stage_a + e * fft2::kThreads + threadIdx.x, row + k);
+      }
+    };
+    float best = -INFINITY;
+    int best_idx = 0x7fffffff;
+    prefetch(0);
+    __syncthreads();
+    for (int it = 0; it < kRowIters; ++it) {
+      const int y = row_of(it);
+      const bool active = y < NY;
+      cp_async_commit_and_wait();
+      float2 v[C::VPT];
+#pragma unroll
+      for (int e = 0; e < C::VPT; ++e) {
+        constexpr int R = P::First::R;
+        float2 z = make_float2(0.f, 0.f);
+        const int lo = (e / R) * C::TPS + (e % R) * P::First::NBR;
+        if (active && !(lo >= KX && lo + C::TPS <= N - KX + 1)) {
+          const int i = P::First::in_index(j, e / R, e % R);
+          const int k = c2r_source_index<N>(i, KX);
+          if (k >= 0) {
+            const float2 ca = stage_a[e * fft2::kThreads + threadIdx.x];
+            const float2 w = __ldg(tw2n + k);  // W_2N^k; Y[k] = X[k] conj(W_2N^k)
+            const float2 cb = make_float2(ca.x * w.x + ca.y * w.y, ca.y * w.x - ca.x * w.y);
+            z = c2r_pack<N>(ca, cb, i, KX);
+          }
+        }
+        v[e] = z;
+      }
+      if (it + 1 < kRowIters) prefetch(it + 1);
+      fft2::fft_regs_to_regs<N>(sm, myseq, j, v);
+      if (active) {
+        // samples in increasing index order (m = out_index ascends with r outer, g inner; 2m before 2m + 1; later rows
+        // later): a strictly-greater compare keeps the first of equal maxima
+        const int base = y * (2 * N);
+#pragma unroll
+        for (int r = 0; r < P::Last::R; ++r)
+#pragma unroll
+          for (int g = 0; g < P::Last::G; ++g) {
+            const float2 val = P::Last::result(v, g, r);  // swapped: .y = x[2m], .x = x[2m + 1]
+            const int idx = base + 2 * P::Last::out_index(j, g, r);
+            if (val.y > best) {
+              best = val.y;
+              best_idx = idx;
+            }
+            if (val.x > best) {
+              best = val.x;
+              best_idx = idx + 1;
+            }
+          }
+      }
+      __syncthreads();
+    }
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) {
+      const float ov = __shfl_xor_sync(0xffffffffu, best, o);
+      const int oi = __shfl_xor_sync(0xffffffffu, best_idx, o);
+      if (better(ov, oi, best, best_idx)) {
+        best = ov;
+        best_idx = oi;
+      }
+    }
+    if ((threadIdx.x & 31) == 0) {
+      sval[threadIdx.x >> 5] = best;
+      sidx[threadIdx.x >> 5] = best_idx;
+    }
+    __syncthreads();
+    if (threadIdx.x == 0) {
+      for (int i = 1; i < fft2::kThreads / 32; ++i)
+        if (better(sval[i], sidx[i], best, best_idx)) {
+          best = sval[i];
+          best_idx = sidx[i];
+        }
+      PeakCandidate c;
+      c.val = best;
+      c.idx = best_idx;
+      partial[item * blocks.per_item + blk] = c;
+    }
+  });
+}
+
+// ---- coarse bound of the peak search: the row blocks that can hold the maximum --------------------------------------
+//
+// After the column pass, row y of a correlation surface of N-point rows is the real trigonometric polynomial
+//   r(x) = Re c_0 + 2 sum_{0 < k < KX} Re(c_k e^{2 pi i k x / N}),   |r''| <= M2_y = 2 sum_k (2 pi k / N)^2 |c_k|.
+// With 2 KX - 1 <= M = N / 4, k -> k mod M is one-to-one on the band, so the M-point c2r transform of the same KX
+// coefficients is r at x = 4m.  On a cell of width 4 between two such samples (the last cell ends at x = N = 0),
+// r <= max(end samples) + (4^2 / 8) M2_y, so no sample of the row exceeds max_m r(4m) + 2 M2_y.
+// eps_y bounds the fp32 error of the coarse and the fine transform of a row together: the elementwise error of a
+// power-of-two FFT is a few eps32 per level of butterflies times the L1 norm of its (packed) input, so with
+//   L1_y = |Re c_0| + 2 sum_{k>0} |c_k|,   eps_y = 32 eps32 (log2 N + 8) 2 max(L1_ya, L1_ya+1) + 1e-35
+// (ya even: the row pair packed in one transform; the half-length kernels pack a row with its twisted copy) each of
+// the two transforms is within half of eps_y.  Every fine value of row y is then at most
+//   hi_y = max_m C_y(m) + 2 M2_y + eps_y,
+// and the fine value at the row's largest coarse sample C_y is at least lo_y = max_m C_y(m) - eps_y.  The sums take
+// |c_k| from above (abs_ru) and round upward, the subtraction downward, so both bounds hold as computed.  A row block whose largest hi_y is below
+// T = max_y lo_y over the surface can neither hold the fine maximum nor tie with it (rows_select_live drops it); the
+// row with the largest lo_y always stays.  Rows whose L1 norm passes 1e36 (or is not finite) get hi = NaN, which
+// keeps every block of their surface live.
+
+// maximum that propagates NaN from either side
+__device__ __forceinline__ float max_nan(float a, float b) { return (a > b || a != a) ? a : b; }
+
+// An upper bound of |c| without a square root (a directed-rounding square root costs more than the coarse transform):
+// sqrt(M^2 + m^2) with M = max(|Re c|, |Im c|), m = min(...) is convex in m, so it lies below its chord
+// M + (sqrt 2 - 1) m, at most 8 % above |c|.  NaN stays NaN.
+__device__ __forceinline__ float abs_ru(float2 c) {
+  const float ax = fabsf(c.x), ay = fabsf(c.y);
+  return (ax != ax || ay != ay) ? NAN : __fmaf_ru(0.41421357f, fminf(ax, ay), fmaxf(ax, ay));  // 0.41421357f >= sqrt 2 - 1
+}
+
+// adds coefficient c_k (k < KX) of a row to its sums L1 and sum k^2 |c_k|, rounded upward
+__device__ __forceinline__ void add_coeff(int k, float2 c, float& l1, float& k2) {
+  const float a = k == 0 ? fabsf(c.x) : abs_ru(c);
+  l1 = __fadd_ru(l1, k == 0 ? a : 2.f * a);
+  k2 = __fadd_ru(k2, __fmul_ru((float)(k * k), a));
+}
+
+// hi_y and lo_y of the rows of a pair (ya, ya + 1) from each row's largest coarse sample, L1 and sum k^2 |c_k|
+__device__ __forceinline__ void pair_bounds(const float (&cmax)[2], const float (&l1)[2], const float (&k2)[2], float eps_rel,
+                                            float curv, float (&hi)[2], float (&lo)[2]) {
+  const bool ok = l1[0] <= 1e36f && l1[1] <= 1e36f;  // false for NaN
+  const float eps = __fadd_ru(__fmul_ru(eps_rel, fmaxf(l1[0], l1[1])), 1e-35f);
+#pragma unroll
+  for (int h = 0; h < 2; ++h) {
+    hi[h] = ok ? __fadd_ru(__fadd_ru(cmax[h], 2.f * __fmul_ru(curv, k2[h])), eps) : NAN;
+    lo[h] = __fsub_rd(cmax[h], eps);
+  }
+}
+
+// Bounds s_hi / s_lo of this CTA's rows [row0, row0 + ROWS) -> hi[item][fine block] (largest hi_y of the block's
+// fine_rows rows; fine_rows divides ROWS) and lo[item][cta] (largest lo_y).  Every thread calls it after a barrier.
+__device__ __forceinline__ void store_block_bounds(const float* s_hi, const float* s_lo, int ROWS, int row0, int NY,
+                                                   int fine_rows, long item, float* __restrict__ hi, float* __restrict__ lo) {
+  const int rows = min(ROWS, NY - row0);
+  const int nfine = (NY + fine_rows - 1) / fine_rows;
+  const int fb0 = row0 / fine_rows;
+  for (int b = threadIdx.x; b < ROWS / fine_rows && fb0 + b < nfine; b += blockDim.x) {
+    float h = -INFINITY;
+    for (int r = b * fine_rows; r < (b + 1) * fine_rows && r < rows; ++r) h = max_nan(h, s_hi[r]);
+    hi[item * nfine + fb0 + b] = h;
+  }
+  if (threadIdx.x < 32) {
+    const int lane = threadIdx.x;
+    float l = -INFINITY;
+    for (int r = lane; r < rows; r += 32) l = max_nan(l, s_lo[r]);
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) l = max_nan(l, __shfl_xor_sync(0xffffffffu, l, o));
+    if (lane == 0) lo[item * gridDim.x + blockIdx.x] = l;
+  }
+}
+
+// tmp[item][y][kx] of N = 4M point rows -> hi[item][fine block] (largest hi_y of the block's fine_rows rows) and
+// lo[item][cta] (largest lo_y of this CTA's rows).  tw: the W_N^m table of the N-point plan.  eps_rel: the factor of
+// max(L1) in eps_y, curv: 2 (2 pi / N)^2, both rounded upward.  Smem: rows_inverse_smem_bytes<M>().
+template <int M>
+__global__ void __launch_bounds__(fft2::kThreads)
+rows_coarse_bound_p2(const float2* __restrict__ tmp, int NY, int KX, const float2* __restrict__ tw, int fine_rows,
+                     float eps_rel, float curv, float* __restrict__ hi, float* __restrict__ lo) {
+  using C = fft2::Cfg<M>;
+  using P = fft2::Plan<M>;
+  constexpr int ROWS = rows_per_cta_inverse<M>();
+  constexpr int W = C::TPS < 32 ? C::TPS : 32;  // lanes of one sequence in a warp
+  constexpr int NW = C::TPS / W;                // warps of one sequence
+  extern __shared__ float2 smem[];
+  // per row and warp of its sequence: largest coarse sample, L1 and sum k^2 |c_k| of the warp's coefficients
+  __shared__ float s_max[ROWS * NW], s_l1[ROWS * NW], s_k2[ROWS * NW];
+  __shared__ float s_hi[ROWS], s_lo[ROWS];
+  const long item = blockIdx.y;
+  const int row0 = blockIdx.x * ROWS;
+  const int lane = threadIdx.x & 31;
+  const unsigned seq_lanes = W == 32 ? 0xffffffffu : ((1u << W) - 1) << (lane & ~(W - 1));
+  float l1a = 0.f, l1b = 0.f, k2a = 0.f, k2b = 0.f;  // this thread's share of the current row pair's sums
+  auto on_coeff = [&](int i, float2 ca, float2 cb) {
+    if (i >= KX) return;  // entries i < KX hold every k = i of the band once
+    add_coeff(i, ca, l1a, k2a);
+    add_coeff(i, cb, l1b, k2b);
+  };
+  rows_inverse_driver<M>(tmp + item * NY * KX, NY, KX, tw, 4, smem, [&](int ya, bool has_b, int j, const float2* v) {
+    float ma = -INFINITY, mb = -INFINITY;
+#pragma unroll
+    for (int r = 0; r < P::Last::R; ++r)
+#pragma unroll
+      for (int g = 0; g < P::Last::G; ++g) {
+        const float2 val = P::Last::result(v, g, r);  // swapped: .y = row ya, .x = row ya + 1
+        ma = max_nan(ma, val.y);
+        mb = max_nan(mb, val.x);
+      }
+#pragma unroll
+    for (int o = W / 2; o > 0; o >>= 1) {
+      ma = max_nan(ma, __shfl_xor_sync(seq_lanes, ma, o));
+      mb = max_nan(mb, __shfl_xor_sync(seq_lanes, mb, o));
+      l1a = __fadd_ru(l1a, __shfl_xor_sync(seq_lanes, l1a, o));
+      l1b = __fadd_ru(l1b, __shfl_xor_sync(seq_lanes, l1b, o));
+      k2a = __fadd_ru(k2a, __shfl_xor_sync(seq_lanes, k2a, o));
+      k2b = __fadd_ru(k2b, __shfl_xor_sync(seq_lanes, k2b, o));
+    }
+    if (j % W == 0) {
+      const int at = (ya - row0) * NW + j / W;
+      s_max[at] = ma;
+      s_l1[at] = l1a;
+      s_k2[at] = k2a;
+      if (has_b) {
+        s_max[at + NW] = mb;
+        s_l1[at + NW] = l1b;
+        s_k2[at + NW] = k2b;
+      }
+    }
+    l1a = l1b = k2a = k2b = 0.f;
+  }, on_coeff);  // ends with a barrier
+  if (threadIdx.x < ROWS / 2 && row0 + 2 * (int)threadIdx.x < NY) {
+    const int r0 = 2 * threadIdx.x;
+    float cmax[2], l1[2] = {0.f, 0.f}, k2[2] = {0.f, 0.f}, bhi[2], blo[2];
+#pragma unroll
+    for (int h = 0; h < 2; ++h) {
+      cmax[h] = -INFINITY;
+      if (row0 + r0 + h < NY)
+        for (int w = 0; w < NW; ++w) {
+          const int at = (r0 + h) * NW + w;
+          cmax[h] = max_nan(cmax[h], s_max[at]);
+          l1[h] = __fadd_ru(l1[h], s_l1[at]);
+          k2[h] = __fadd_ru(k2[h], s_k2[at]);
+        }
+    }
+    pair_bounds(cmax, l1, k2, eps_rel, curv, bhi, blo);
+    for (int h = 0; h < 2 && row0 + r0 + h < NY; ++h) {
+      s_hi[r0 + h] = bhi[h];
+      s_lo[r0 + h] = blo[h];
+    }
   }
   __syncthreads();
-  if (threadIdx.x == 0) {
-    for (int i = 1; i < fft2::kThreads / 32; ++i)
-      if (better(sval[i], sidx[i], best, best_idx)) {
-        best = sval[i];
-        best_idx = sidx[i];
-      }
-    PeakCandidate c;
-    c.val = best;
-    c.idx = best_idx;
-    partial[item * gridDim.x + blockIdx.x] = c;
-  }
+  store_block_bounds(s_hi, s_lo, ROWS, row0, NY, fine_rows, item, hi, lo);
 }
 
 // ---- inverse rows + store: tmp[item][y][kx] -> out[item][y][x] real ------------------------------------
@@ -629,7 +811,7 @@ rows_inverse_store_p2(const float2* __restrict__ tmp, int NY, int KX, const floa
   extern __shared__ float2 smem[];
   const long item = blockIdx.y;
   float* dst = out + item * NY * N;
-  rows_inverse_driver<N>(tmp + item * NY * KX, NY, KX, tw, smem, [&](int ya, bool has_b, int j, const float2* v) {
+  rows_inverse_driver<N>(tmp + item * NY * KX, NY, KX, tw, 1, smem, [&](int ya, bool has_b, int j, const float2* v) {
 #pragma unroll
     for (int g = 0; g < P::Last::G; ++g)
 #pragma unroll

@@ -179,12 +179,12 @@ rows_forward_poly(const float* __restrict__ image, int H, int W, const float* __
 }
 
 // ---- inverse rows + argmax: tmp[item][y][kx] -> partial[item][cta] ------------------------------------
-// CTA = kRowsPerCta rows (row pairs, two per warp); same partial layout as rows_inverse_argmax_p2<1024>.
+// Row block = kRowsPerCta rows (row pairs, two per warp); same partial layout as rows_inverse_argmax_p2<1024>.
 constexpr int kRowsPerCta = 32;
 
 __global__ void __launch_bounds__(kThreads, 3)
 rows_inverse_argmax_poly(const float2* __restrict__ tmp, int NY, int KX, const float2* __restrict__ tw,
-                         PeakCandidate* __restrict__ partial) {
+                         PeakCandidate* __restrict__ partial, RowBlocks blocks) {
   constexpr int N = 1024;
   extern __shared__ float2 smem[];
   float2* tw_step = smem;
@@ -193,98 +193,100 @@ rows_inverse_argmax_poly(const float2* __restrict__ tmp, int NY, int KX, const f
   const int qh = lane >> 4, j = lane & 15;
   float2* buf = smem + kTableWords + warp * kWarpWords + qh * kBuf;
   load_tables(tw_step, tw_comb, tw);
-  const long item = blockIdx.y;
-  const float2* src = tmp + item * NY * KX;
   const int q0 = 2 * qh;
-  float best = -INFINITY;
-  int best_idx = 0x7fffffff;
-  __syncthreads();
-  for (int pair = warp; pair < kRowsPerCta / 2; pair += kWarps) {
-    const int ya = blockIdx.x * kRowsPerCta + 2 * pair;
-    if (ya >= NY) break;
-    const bool has_b = ya + 1 < NY;
-    const float2* rowa = src + (long)ya * KX;
-    float2 va[16], vb[16];
-#pragma unroll
-    for (int r = 0; r < 16; ++r) {
-      float2 z0 = make_float2(0.f, 0.f), z1 = z0;
-      if (16 * r < KX || 16 * r + 15 > 256 - KX) {
-        const int kk = j + 16 * r;
-        const bool pos = kk < KX, neg = kk > 256 - KX;
-        if (pos || neg) {
-          const int ka = pos ? kk : 256 - kk;  // |k|
-          const float2 ca = __ldg(rowa + ka);
-          const float2 cb = has_b ? __ldg(rowa + KX + ka) : make_float2(0.f, 0.f);
-          // packed spectrum entry of (row ya -> real part, row ya + 1 -> imaginary part), stored (im, re): the forward
-          // transforms below then act as the inverse; multiplying the swapped value by W^{+q k} equals swapping
-          // Z[k] W^{-q k}
-          const float2 z = c2r_pack<N>(ca, cb, pos ? kk : N - ka, KX);
-          z0 = qh ? cmul(z, tw_comb[256 + kk]) : z;
-          z1 = cmul(z, tw_comb[q0 * 256 + kk]);
-        }
-      }
-      va[r] = z0;
-      vb[r] = z1;
-    }
-    fft256_halfwarp(va, j, buf, tw_step);
-    fft256_halfwarp(vb, j, buf, tw_step);
-    // the thread visits its samples in increasing index order (row ya left to right, then row ya + 1; pairs ascend), so
-    // "strictly greater" keeps the first of equal maxima: one compare and two selects per sample
-    const int ia0 = ya * N + 4 * j + q0;
-#pragma unroll
-    for (int k1 = 0; k1 < 16; ++k1) {
-      const float2 a = va[tmcfft::bitrev<16>(k1)], b = vb[tmcfft::bitrev<16>(k1)];  // swapped: .y = row ya, .x = row ya + 1
-      if (a.y > best) {
-        best = a.y;
-        best_idx = ia0 + 64 * k1;
-      }
-      if (b.y > best) {
-        best = b.y;
-        best_idx = ia0 + 64 * k1 + 1;
-      }
-    }
-    if (has_b) {
-#pragma unroll
-      for (int k1 = 0; k1 < 16; ++k1) {
-        const float2 a = va[tmcfft::bitrev<16>(k1)], b = vb[tmcfft::bitrev<16>(k1)];
-        if (a.x > best) {
-          best = a.x;
-          best_idx = ia0 + N + 64 * k1;
-        }
-        if (b.x > best) {
-          best = b.x;
-          best_idx = ia0 + N + 64 * k1 + 1;
-        }
-      }
-    }
-  }
-#pragma unroll
-  for (int o = 16; o > 0; o >>= 1) {
-    const float ov = __shfl_xor_sync(0xffffffffu, best, o);
-    const int oi = __shfl_xor_sync(0xffffffffu, best_idx, o);
-    if (better(ov, oi, best, best_idx)) {
-      best = ov;
-      best_idx = oi;
-    }
-  }
   __shared__ float sval[kWarps];
   __shared__ int sidx[kWarps];
-  if (lane == 0) {
-    sval[warp] = best;
-    sidx[warp] = best_idx;
-  }
-  __syncthreads();
-  if (threadIdx.x == 0) {
-    for (int i = 1; i < kWarps; ++i)
-      if (better(sval[i], sidx[i], best, best_idx)) {
-        best = sval[i];
-        best_idx = sidx[i];
+  __syncthreads();  // twiddle tables
+  for_each_row_block(blocks, [&](long item, int blk) {
+    const float2* src = tmp + item * NY * KX;
+    float best = -INFINITY;
+    int best_idx = 0x7fffffff;
+    for (int pair = warp; pair < kRowsPerCta / 2; pair += kWarps) {
+      const int ya = blk * kRowsPerCta + 2 * pair;
+      if (ya >= NY) break;
+      const bool has_b = ya + 1 < NY;
+      const float2* rowa = src + (long)ya * KX;
+      float2 va[16], vb[16];
+#pragma unroll
+      for (int r = 0; r < 16; ++r) {
+        float2 z0 = make_float2(0.f, 0.f), z1 = z0;
+        if (16 * r < KX || 16 * r + 15 > 256 - KX) {
+          const int kk = j + 16 * r;
+          const bool pos = kk < KX, neg = kk > 256 - KX;
+          if (pos || neg) {
+            const int ka = pos ? kk : 256 - kk;  // |k|
+            const float2 ca = __ldg(rowa + ka);
+            const float2 cb = has_b ? __ldg(rowa + KX + ka) : make_float2(0.f, 0.f);
+            // packed spectrum entry of (row ya -> real part, row ya + 1 -> imaginary part), stored (im, re): the forward
+            // transforms below then act as the inverse; multiplying the swapped value by W^{+q k} equals swapping
+            // Z[k] W^{-q k}
+            const float2 z = c2r_pack<N>(ca, cb, pos ? kk : N - ka, KX);
+            z0 = qh ? cmul(z, tw_comb[256 + kk]) : z;
+            z1 = cmul(z, tw_comb[q0 * 256 + kk]);
+          }
+        }
+        va[r] = z0;
+        vb[r] = z1;
       }
-    PeakCandidate c;
-    c.val = best;
-    c.idx = best_idx;
-    partial[item * gridDim.x + blockIdx.x] = c;
-  }
+      fft256_halfwarp(va, j, buf, tw_step);
+      fft256_halfwarp(vb, j, buf, tw_step);
+      // the thread visits its samples in increasing index order (row ya left to right, then row ya + 1; pairs ascend), so
+      // "strictly greater" keeps the first of equal maxima: one compare and two selects per sample
+      const int ia0 = ya * N + 4 * j + q0;
+#pragma unroll
+      for (int k1 = 0; k1 < 16; ++k1) {
+        const float2 a = va[tmcfft::bitrev<16>(k1)], b = vb[tmcfft::bitrev<16>(k1)];  // swapped: .y = row ya, .x = row ya + 1
+        if (a.y > best) {
+          best = a.y;
+          best_idx = ia0 + 64 * k1;
+        }
+        if (b.y > best) {
+          best = b.y;
+          best_idx = ia0 + 64 * k1 + 1;
+        }
+      }
+      if (has_b) {
+#pragma unroll
+        for (int k1 = 0; k1 < 16; ++k1) {
+          const float2 a = va[tmcfft::bitrev<16>(k1)], b = vb[tmcfft::bitrev<16>(k1)];
+          if (a.x > best) {
+            best = a.x;
+            best_idx = ia0 + N + 64 * k1;
+          }
+          if (b.x > best) {
+            best = b.x;
+            best_idx = ia0 + N + 64 * k1 + 1;
+          }
+        }
+      }
+    }
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) {
+      const float ov = __shfl_xor_sync(0xffffffffu, best, o);
+      const int oi = __shfl_xor_sync(0xffffffffu, best_idx, o);
+      if (better(ov, oi, best, best_idx)) {
+        best = ov;
+        best_idx = oi;
+      }
+    }
+    if (lane == 0) {
+      sval[warp] = best;
+      sidx[warp] = best_idx;
+    }
+    __syncthreads();
+    if (threadIdx.x == 0) {
+      for (int i = 1; i < kWarps; ++i)
+        if (better(sval[i], sidx[i], best, best_idx)) {
+          best = sval[i];
+          best_idx = sidx[i];
+        }
+      PeakCandidate c;
+      c.val = best;
+      c.idx = best_idx;
+      partial[item * blocks.per_item + blk] = c;
+    }
+    __syncthreads();  // sval / sidx are free for the next block
+  });
 }
 
 }  // namespace poly
