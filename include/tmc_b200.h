@@ -247,9 +247,10 @@ int tmc_xc_leave_one_out_products(const void* spec, int t, int g, long plane_ele
  * kx_count (-1: unsupported nx) */
 int tmc_xc_peak_partials(int ny, int nx);
 /* bytes of the workspace of tmc_xc_peaks for nitems items (0: the band needs none; workspace may then be NULL).
- * Bands of 2 kx_count - 1 <= nx / 4 on the half-length and polyphase row kernels bound every row from its samples at
- * x = 4m and transform only the row blocks that can hold the maximum; the workspace then starts with the int32 count of
- * those blocks (of the last slice of at most 65535 items). */
+ * Bands of 2 kx_count - 1 <= nx / 4 on the half-length and polyphase row kernels bound every row by its L1 norm and
+ * the rows of one seed group per item from their samples at x = 4m, and transform only the row blocks that can hold
+ * the maximum; the workspace then starts with four int32 (of the last slice of n <= 65535 items): the count of those
+ * row blocks, n (the groups sampled), and two unused words. */
 long tmc_xc_peaks_workspace_bytes(int nitems, int ny, int nx, int kx_count);
 /* prod (nitems, ky_count, kx_count) -> shifts (nitems, 2) = (dy, dx) px.  tmp: nitems*ny*kx_count complex64;
  * partial: nitems * tmc_xc_peak_partials(ny, nx) * 8 bytes; workspace: tmc_xc_peaks_workspace_bytes bytes. */

@@ -3,8 +3,9 @@ python tools/time_peaks.py [frame size, default 4096]
 
 Builds the two searches of a motion_correct step from bench.py's seeded movie (40 frames, 0.83 A/px, 300-10 A band):
 the whole-frame products against the middle frame and the leave-one-out products of the 1024-px patches.  Prints one
-JSON line per search: CUDA-event ms per search (median of 10), per-kernel ms of one search (library timing) and the
-live row blocks left by the coarse bound (count, total, fraction)."""
+JSON line per search: CUDA-event ms per search (median of 10), per-kernel ms of one search (library timing), the coarse
+groups the coarse bound samples (one seed group per item: count, total, fraction) and the live row blocks left by the
+row L1 norms and the seed's bound (count, total, fraction)."""
 import json
 import os
 import subprocess
@@ -36,6 +37,8 @@ offsets = torch.zeros((t + 1,), dtype=torch.int32, device=dev)
 deltas = torch.zeros((1,), dtype=torch.int32, device=dev)
 prod_p = _fourier.leave_one_out_products(spec_p, t, g, plan_p.plane_elems, offsets, deltas).view(t * g, plan_p.ky, plan_p.kx, 2)
 del movie, spec_g, spec_p
+# rows of a coarse group: the row block of rows_coarse_bound_p2<nx / 4>
+GROUP_ROWS = {1024: 128, 4096: 32, 8192: 16}
 power_limit = subprocess.run(["nvidia-smi", "--query-gpu=power.limit", "--format=csv,noheader", "-i", "0"],
                              capture_output=True, text=True).stdout.strip()
 
@@ -57,8 +60,10 @@ for name, plan, prod in (("whole_frame", plan_g, prod_g), ("patches", plan_p, pr
     kernels = {k: round(ms, 4) for k, (n, ms) in _lib.kernel_timing_report().items()}
     _lib.kernel_timing(False)
     total = prod.shape[0] * _lib.query("tmc_xc_peak_partials", plan.ny, plan.nx)
-    live = int(ws[0][:4].view(torch.int32).item()) if ws and ws[0] is not None else total
+    live, sampled = ws[0][:8].view(torch.int32).tolist()
+    all_groups = prod.shape[0] * -(-plan.ny // GROUP_ROWS[plan.nx])
     print(json.dumps({"search": name, "items": prod.shape[0], "shape": [plan.ny, plan.nx], "kx": plan.kx,
                       "ms_per_search": round(sorted(times)[len(times) // 2], 4), "kernels_ms": kernels,
+                      "coarse_groups": sampled, "groups": all_groups, "coarse_fraction": round(sampled / all_groups, 5),
                       "live_blocks": live, "row_blocks": total, "live_fraction": round(live / total, 5),
                       "gpu": torch.cuda.get_device_name(dev), "power_limit": power_limit}))

@@ -13,6 +13,7 @@
 //    instead of storing the correlation surface.
 #include "common.cuh"
 #include <stdlib.h>
+#include <cfloat>
 #include <cmath>
 #include "fft_core.cuh"
 #include "fft_core2.cuh"
@@ -650,6 +651,53 @@ rows_select_live(const float* __restrict__ hi, int nfine, const float* __restric
   }
 }
 
+// ---- seed group of the peak search (after rows_l1_bound; see rows_coarse_bound_p2's header) ------------------------
+// One CTA per item, per_group fine blocks per coarse group.  The seed: the group of the first fine block with the largest
+// hi0 (the row with the largest L1 norm), written to seeds[item]; *seed_count = items.  Every group's lo slot gets the
+// lowest finite float, a valid lower bound that rows_select_live sees as finite; the coarse bound of the seed then
+// writes the seed's.
+__global__ void __launch_bounds__(256)
+rows_l1_seeds(const float* __restrict__ hi, int nfine, int per_group, float* __restrict__ lo, int ngroups,
+              int2* __restrict__ seeds, int* __restrict__ seed_count) {
+  __shared__ float s_v[8];
+  __shared__ int s_i[8];
+  const long item = blockIdx.x;
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+  for (int g = threadIdx.x; g < ngroups; g += 256) lo[item * ngroups + g] = -FLT_MAX;
+  float best = -INFINITY;
+  int at = 0x7fffffff;
+  for (int i = threadIdx.x; i < nfine; i += 256) {
+    const float v = hi[item * nfine + i];
+    if (v > best) {
+      best = v;
+      at = i;
+    }
+  }
+#pragma unroll
+  for (int o = 16; o > 0; o >>= 1) {
+    const float ov = __shfl_xor_sync(0xffffffffu, best, o);
+    const int oi = __shfl_xor_sync(0xffffffffu, at, o);
+    if (better(ov, oi, best, at)) {
+      best = ov;
+      at = oi;
+    }
+  }
+  if (lane == 0) {
+    s_v[warp] = best;
+    s_i[warp] = at;
+  }
+  __syncthreads();
+  if (threadIdx.x == 0) {
+    for (int w = 1; w < 8; ++w)
+      if (better(s_v[w], s_i[w], best, at)) {
+        best = s_v[w];
+        at = s_i[w];
+      }
+    seeds[item] = make_int2((int)item, at < nfine ? at / per_group : 0);  // no finite hi0: any group, all stay live
+    if (item == 0) *seed_count = gridDim.x;
+  }
+}
+
 // ---- peak finalisation: argmax over CTAs, 3-point parabola, wrap ---------------------------
 
 // value of the real surface at (y, x) from the column-transformed rows (direct KX-term sum)
@@ -965,52 +1013,30 @@ int rows_inverse_ctas(int ny, int nx, int KX, bool argmax) {
 }
 
 // Workspace of the coarse bound for n items (at most kMaxGridYZ: one slice), laid out from `base`:
-//   int count, int2 list[n][fine], float hi[n][fine], float lo[n][coarse]
-// fine = row blocks of the fine kernel, coarse = CTAs of the coarse pass per item.
+//   int count, int seed_count, int unused[2], int2 list[n][fine], int2 seeds[n], float hi[n][fine], float lo[n][coarse]
+// fine = row blocks of the fine kernel, coarse = coarse groups (row blocks of the coarse pass) per item.  count: live
+// fine blocks (list); seed_count = n: the groups the coarse bound runs on (seeds).  The 8-byte entries come first.
 struct CoarseWorkspace {
   int* count;
+  int* seed_count;
   int2* list;
+  int2* seeds;
   float* hi;
   float* lo;
 };
 
-size_t coarse_workspace_bytes(int n, int fine, int coarse) { return 16 + 12ull * n * fine + 4ull * n * coarse; }
+size_t coarse_workspace_bytes(int n, int fine, int coarse) { return 16 + 8ull * n + 12ull * n * fine + 4ull * n * coarse; }
 
 CoarseWorkspace coarse_workspace(void* base, int n, int fine) {
   char* p = (char*)base;
   CoarseWorkspace w;
   w.count = (int*)p;
+  w.seed_count = w.count + 1;
   w.list = (int2*)(p + 16);
-  w.hi = (float*)(p + 16 + 8l * n * fine);
+  w.seeds = w.list + (long)n * fine;
+  w.hi = (float*)(w.seeds + n);
   w.lo = w.hi + (long)n * fine;
   return w;
-}
-
-// rows of N points: bound every row from its samples at x = 4m, select the live fine row blocks (rows_per_fine rows
-// each) of the n items into the workspace, dead ones into partial
-template <int N>
-int coarse_select(const float2* src, int n, int ny, int KX, const AxisPlan& px, int rows_per_fine, PeakCandidate* partial,
-                  void* workspace, cudaStream_t stream, CoarseWorkspace* ws) {
-  constexpr int ROWS = rows_per_cta_inverse<N / 4>();  // rows per CTA of rows_coarse_bound_p2<N / 4>
-  const int nfine = tmc_div_up(ny, rows_per_fine), ncoarse = tmc_div_up(ny, ROWS);
-  if (ROWS % rows_per_fine != 0) {
-    tmc_set_error("xc_peaks: a coarse CTA of %d rows does not cover whole row blocks of %d", ROWS, rows_per_fine);
-    return TMC_ERR_UNSUPPORTED;
-  }
-  *ws = coarse_workspace(workspace, n, nfine);
-  // eps_y = 32 eps32 (log2 N + 8) * 2 max(L1), curv = 2 (2 pi / N)^2, both rounded up
-  const float eps_rel = (float)(64.0 * 0x1p-23 * (std::log2((double)N) + 8.0) * (1.0 + 1e-6));
-  const float curv = (float)(2.0 * (2.0 * M_PI / N) * (2.0 * M_PI / N) * (1.0 + 1e-6));
-  const float2* tw = (const float2*)px.tw;
-  constexpr int M = N / 4;
-  const int rc = launch(M == 2048 ? "rows_coarse_bound_p2<2048>" : TMC_LABEL2("rows_coarse_bound_p2", M, 256, 1024),
-                        rows_coarse_bound_p2<M>, dim3(ncoarse, n), fft2::kThreads, rows_inverse_smem_bytes<M>(), stream, src,
-                        ny, KX, tw, rows_per_fine, eps_rel, curv, ws->hi, ws->lo);
-  if (rc) return rc;
-  TMC_CUDA(cudaMemsetAsync(ws->count, 0, sizeof(int), stream));
-  TMC_TIMED("rows_select_live", stream, rows_select_live<<<n, 256, 0, stream>>>(ws->hi, nfine, ws->lo, ncoarse, partial,
-                                                                                ws->list, ws->count));
-  return TMC_OK;
 }
 
 // CTAs of a fine row kernel that walks the live list: three per SM (the kernels' residency)
@@ -1018,6 +1044,39 @@ int live_list_ctas() {
   int dev = 0, sms = 148;
   if (cudaGetDevice(&dev) == cudaSuccess) cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
   return 3 * sms;
+}
+
+// rows of N points: bound every fine row block (rows_per_fine rows) by the L1 norms of its rows, bound the rows of each
+// item's seed group from their samples at x = 4m, and select the live fine row blocks of the n items into the
+// workspace, dead ones into partial
+template <int N>
+int coarse_select(const float2* src, int n, int ny, int KX, const AxisPlan& px, int rows_per_fine, PeakCandidate* partial,
+                  void* workspace, cudaStream_t stream, CoarseWorkspace* ws) {
+  constexpr int M = N / 4;
+  constexpr int ROWS = rows_per_cta_inverse<M>();  // rows per coarse group (row block of rows_coarse_bound_p2<M>)
+  const int nfine = tmc_div_up(ny, rows_per_fine), ncoarse = tmc_div_up(ny, ROWS);
+  if (ROWS % rows_per_fine != 0 || rows_per_fine % 2 != 0) {
+    tmc_set_error("xc_peaks: a coarse group of %d rows does not cover whole row blocks of %d (an even number)", ROWS,
+                  rows_per_fine);
+    return TMC_ERR_UNSUPPORTED;
+  }
+  *ws = coarse_workspace(workspace, n, nfine);
+  // eps_y = 32 eps32 (log2 N + 8) * 2 max(L1), curv = 2 (2 pi / N)^2, both rounded up
+  const float eps_rel = (float)(64.0 * 0x1p-23 * (std::log2((double)N) + 8.0) * (1.0 + 1e-6));
+  const float curv = (float)(2.0 * (2.0 * M_PI / N) * (2.0 * M_PI / N) * (1.0 + 1e-6));
+  TMC_CUDA(cudaMemsetAsync(ws->count, 0, sizeof(int), stream));
+  TMC_TIMED("rows_l1_bound", stream, rows_l1_bound<<<dim3(tmc_div_up(nfine, 8), n), 256, 0, stream>>>(
+      src, ny, KX, rows_per_fine, eps_rel, ws->hi));
+  TMC_TIMED("rows_l1_seeds", stream, rows_l1_seeds<<<n, 256, 0, stream>>>(ws->hi, nfine, ROWS / rows_per_fine, ws->lo,
+                                                                          ncoarse, ws->seeds, ws->seed_count));
+  if (int rc = launch(M == 2048 ? "rows_coarse_bound_p2<2048>" : TMC_LABEL2("rows_coarse_bound_p2", M, 256, 1024),
+                      rows_coarse_bound_p2<M>, dim3(n), fft2::kThreads, rows_inverse_smem_bytes<M>(), stream, src, ny, KX,
+                      (const float2*)px.tw, rows_per_fine, eps_rel, curv, ws->hi, ws->lo,
+                      RowBlocks{ws->seeds, ws->seed_count, ncoarse}))
+    return rc;
+  TMC_TIMED("rows_select_live", stream, rows_select_live<<<n, 256, 0, stream>>>(ws->hi, nfine, ws->lo, ncoarse, partial,
+                                                                                ws->list, ws->count));
+  return TMC_OK;
 }
 
 // c2r row pass: tmp (nitems, ny, KX) -> partial != nullptr: the maximum of each CTA's rows into partial[item][cta]

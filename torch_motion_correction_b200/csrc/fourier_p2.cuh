@@ -370,11 +370,11 @@ struct NoCoeff {
 };
 
 // Shared driver of the inverse row kernels: calls consume(ya, has_b, v) with the last-pass outputs of
-// every row pair of this CTA (v swapped: .y = row ya, .x = row ya + 1), and before that on_coeff(i, Ca, Cb) with the
-// coefficients of every packed entry i the calling thread builds.  tw: the W_N^m table, or the table of a
-// transform tw_stride times longer.
+// every row pair of row block blk (rows_per_cta_inverse<N>() rows; v swapped: .y = row ya, .x = row ya + 1), and before
+// that on_coeff(i, Ca, Cb) with the coefficients of every packed entry i the calling thread builds.  tw: the W_N^m table,
+// or the table of a transform tw_stride times longer.
 template <int N, typename Consume, typename OnCoeff = NoCoeff>
-__device__ __forceinline__ void rows_inverse_driver(const float2* __restrict__ src, int NY, int KX,
+__device__ __forceinline__ void rows_inverse_driver(const float2* __restrict__ src, int NY, int KX, int blk,
                                                     const float2* __restrict__ tw, int tw_stride, float2* smem,
                                                     Consume&& consume, OnCoeff&& on_coeff = OnCoeff{}) {
   using C = fft2::Cfg<N>;
@@ -385,7 +385,7 @@ __device__ __forceinline__ void rows_inverse_driver(const float2* __restrict__ s
   float2* myseq = sm.data + seq * C::STRIDE;
   float2* stage_a = smem + C::B * C::STRIDE + 64 + C::TW_HI;
   float2* stage_b = stage_a + C::B * N;
-  auto row_of = [&](int it) { return (int)blockIdx.x * rows_per_cta_inverse<N>() + (it * C::B + seq) * 2; };
+  auto row_of = [&](int it) { return blk * rows_per_cta_inverse<N>() + (it * C::B + seq) * 2; };
   auto prefetch = [&](int it) {
     const int ya = row_of(it);
     if (ya >= NY) return;
@@ -446,7 +446,7 @@ rows_inverse_argmax_p2(const float2* __restrict__ tmp, int NY, int KX, const flo
   const long item = blockIdx.y;
   float best = -INFINITY;
   int best_idx = 0x7fffffff;
-  rows_inverse_driver<N>(tmp + item * NY * KX, NY, KX, tw, 1, smem, [&](int ya, bool has_b, int j, const float2* v) {
+  rows_inverse_driver<N>(tmp + item * NY * KX, NY, KX, blockIdx.x, tw, 1, smem, [&](int ya, bool has_b, int j, const float2* v) {
     // the thread visits its samples in increasing index order (out_index = j + g TPS + r NS with G TPS == NS: r outer,
     // g inner; row ya, then row ya + 1; later calls have larger ya), so "strictly greater" keeps the first of equal
     // maxima: one compare and two selects per sample
@@ -667,6 +667,16 @@ rows_inverse_argmax_real2n(const float2* __restrict__ tmp, int NY, int KX, const
 // T = max_y lo_y over the surface can neither hold the fine maximum nor tie with it (rows_select_live drops it); the
 // row with the largest lo_y always stays.  Rows whose L1 norm passes 1e36 (or is not finite) get hi = NaN, which
 // keeps every block of their surface live.
+//
+// Most rows cannot hold the maximum by a margin that needs no transform to see: |r(x)| <= L1_y, so every fine value of
+// row y is at most hi0_y = L1_y + eps_y.  rows_l1_bound writes the largest hi0_y of every fine block as its hi.  The
+// coarse bound then runs on one group per surface only (a group: the rows of one rows_coarse_bound_p2 row block), the
+// seed, which holds the row with the largest L1 norm: it replaces the hi of the seed's blocks and writes the seed's lo,
+// T0 = max lo_y over the seed; the other groups' lo slots hold the lowest finite float.  rows_select_live then drops a
+// block whose hi is below T0, so it can neither hold the maximum nor tie with it.  Every slot is finite unless a row norm
+// passes 1e36 (hi0 = NaN) or a coarse bound is NaN, and then every block of the surface stays live, as above.  Sampling
+// the other groups as well was measured slower on C2 products: their hi0 already leaves almost only the blocks that
+// the coarse bound leaves (DESIGN.md 8.3).
 
 // maximum that propagates NaN from either side
 __device__ __forceinline__ float max_nan(float a, float b) { return (a > b || a != a) ? a : b; }
@@ -698,12 +708,14 @@ __device__ __forceinline__ void pair_bounds(const float (&cmax)[2], const float 
   }
 }
 
-// Bounds s_hi / s_lo of this CTA's rows [row0, row0 + ROWS) -> hi[item][fine block] (largest hi_y of the block's
-// fine_rows rows; fine_rows divides ROWS) and lo[item][cta] (largest lo_y).  Every thread calls it after a barrier.
-__device__ __forceinline__ void store_block_bounds(const float* s_hi, const float* s_lo, int ROWS, int row0, int NY,
+// Bounds s_hi / s_lo of group blk's rows [row0, row0 + ROWS) -> hi[item][fine block] (largest hi_y of the block's
+// fine_rows rows; fine_rows divides ROWS) and lo[item][blk] (largest lo_y).  Every thread calls it after a barrier.
+__device__ __forceinline__ void store_block_bounds(const float* s_hi, const float* s_lo, int ROWS, int blk, int NY,
                                                    int fine_rows, long item, float* __restrict__ hi, float* __restrict__ lo) {
+  const int row0 = blk * ROWS;
   const int rows = min(ROWS, NY - row0);
   const int nfine = (NY + fine_rows - 1) / fine_rows;
+  const int ngroups = (NY + ROWS - 1) / ROWS;
   const int fb0 = row0 / fine_rows;
   for (int b = threadIdx.x; b < ROWS / fine_rows && fb0 + b < nfine; b += blockDim.x) {
     float h = -INFINITY;
@@ -716,17 +728,18 @@ __device__ __forceinline__ void store_block_bounds(const float* s_hi, const floa
     for (int r = lane; r < rows; r += 32) l = max_nan(l, s_lo[r]);
 #pragma unroll
     for (int o = 16; o > 0; o >>= 1) l = max_nan(l, __shfl_xor_sync(0xffffffffu, l, o));
-    if (lane == 0) lo[item * gridDim.x + blockIdx.x] = l;
+    if (lane == 0) lo[item * ngroups + blk] = l;
   }
 }
 
 // tmp[item][y][kx] of N = 4M point rows -> hi[item][fine block] (largest hi_y of the block's fine_rows rows) and
-// lo[item][cta] (largest lo_y of this CTA's rows).  tw: the W_N^m table of the N-point plan.  eps_rel: the factor of
-// max(L1) in eps_y, curv: 2 (2 pi / N)^2, both rounded upward.  Smem: rows_inverse_smem_bytes<M>().
+// lo[item][group] (largest lo_y of the group's rows) for the coarse groups of `groups` (rows_per_cta_inverse<M>() rows
+// each).  tw: the W_N^m table of the N-point plan.  eps_rel: the factor of max(L1) in eps_y, curv: 2 (2 pi / N)^2, both
+// rounded upward.  Smem: rows_inverse_smem_bytes<M>().
 template <int M>
-__global__ void __launch_bounds__(fft2::kThreads)
+__global__ void __launch_bounds__(fft2::kThreads, 2)
 rows_coarse_bound_p2(const float2* __restrict__ tmp, int NY, int KX, const float2* __restrict__ tw, int fine_rows,
-                     float eps_rel, float curv, float* __restrict__ hi, float* __restrict__ lo) {
+                     float eps_rel, float curv, float* __restrict__ hi, float* __restrict__ lo, RowBlocks groups) {
   using C = fft2::Cfg<M>;
   using P = fft2::Plan<M>;
   constexpr int ROWS = rows_per_cta_inverse<M>();
@@ -736,70 +749,102 @@ rows_coarse_bound_p2(const float2* __restrict__ tmp, int NY, int KX, const float
   // per row and warp of its sequence: largest coarse sample, L1 and sum k^2 |c_k| of the warp's coefficients
   __shared__ float s_max[ROWS * NW], s_l1[ROWS * NW], s_k2[ROWS * NW];
   __shared__ float s_hi[ROWS], s_lo[ROWS];
-  const long item = blockIdx.y;
-  const int row0 = blockIdx.x * ROWS;
   const int lane = threadIdx.x & 31;
   const unsigned seq_lanes = W == 32 ? 0xffffffffu : ((1u << W) - 1) << (lane & ~(W - 1));
-  float l1a = 0.f, l1b = 0.f, k2a = 0.f, k2b = 0.f;  // this thread's share of the current row pair's sums
-  auto on_coeff = [&](int i, float2 ca, float2 cb) {
-    if (i >= KX) return;  // entries i < KX hold every k = i of the band once
-    add_coeff(i, ca, l1a, k2a);
-    add_coeff(i, cb, l1b, k2b);
-  };
-  rows_inverse_driver<M>(tmp + item * NY * KX, NY, KX, tw, 4, smem, [&](int ya, bool has_b, int j, const float2* v) {
-    float ma = -INFINITY, mb = -INFINITY;
+  // the driver's first barrier keeps the next group's writes behind every thread's store_block_bounds
+  for_each_row_block(groups, [&](long item, int blk) {
+    const int row0 = blk * ROWS;
+    float l1a = 0.f, l1b = 0.f, k2a = 0.f, k2b = 0.f;  // this thread's share of the current row pair's sums
+    auto on_coeff = [&](int i, float2 ca, float2 cb) {
+      if (i >= KX) return;  // entries i < KX hold every k = i of the band once
+      add_coeff(i, ca, l1a, k2a);
+      add_coeff(i, cb, l1b, k2b);
+    };
+    rows_inverse_driver<M>(tmp + item * NY * KX, NY, KX, blk, tw, 4, smem, [&](int ya, bool has_b, int j, const float2* v) {
+      float ma = -INFINITY, mb = -INFINITY;
 #pragma unroll
-    for (int r = 0; r < P::Last::R; ++r)
+      for (int r = 0; r < P::Last::R; ++r)
 #pragma unroll
-      for (int g = 0; g < P::Last::G; ++g) {
-        const float2 val = P::Last::result(v, g, r);  // swapped: .y = row ya, .x = row ya + 1
-        ma = max_nan(ma, val.y);
-        mb = max_nan(mb, val.x);
-      }
-#pragma unroll
-    for (int o = W / 2; o > 0; o >>= 1) {
-      ma = max_nan(ma, __shfl_xor_sync(seq_lanes, ma, o));
-      mb = max_nan(mb, __shfl_xor_sync(seq_lanes, mb, o));
-      l1a = __fadd_ru(l1a, __shfl_xor_sync(seq_lanes, l1a, o));
-      l1b = __fadd_ru(l1b, __shfl_xor_sync(seq_lanes, l1b, o));
-      k2a = __fadd_ru(k2a, __shfl_xor_sync(seq_lanes, k2a, o));
-      k2b = __fadd_ru(k2b, __shfl_xor_sync(seq_lanes, k2b, o));
-    }
-    if (j % W == 0) {
-      const int at = (ya - row0) * NW + j / W;
-      s_max[at] = ma;
-      s_l1[at] = l1a;
-      s_k2[at] = k2a;
-      if (has_b) {
-        s_max[at + NW] = mb;
-        s_l1[at + NW] = l1b;
-        s_k2[at + NW] = k2b;
-      }
-    }
-    l1a = l1b = k2a = k2b = 0.f;
-  }, on_coeff);  // ends with a barrier
-  if (threadIdx.x < ROWS / 2 && row0 + 2 * (int)threadIdx.x < NY) {
-    const int r0 = 2 * threadIdx.x;
-    float cmax[2], l1[2] = {0.f, 0.f}, k2[2] = {0.f, 0.f}, bhi[2], blo[2];
-#pragma unroll
-    for (int h = 0; h < 2; ++h) {
-      cmax[h] = -INFINITY;
-      if (row0 + r0 + h < NY)
-        for (int w = 0; w < NW; ++w) {
-          const int at = (r0 + h) * NW + w;
-          cmax[h] = max_nan(cmax[h], s_max[at]);
-          l1[h] = __fadd_ru(l1[h], s_l1[at]);
-          k2[h] = __fadd_ru(k2[h], s_k2[at]);
+        for (int g = 0; g < P::Last::G; ++g) {
+          const float2 val = P::Last::result(v, g, r);  // swapped: .y = row ya, .x = row ya + 1
+          ma = max_nan(ma, val.y);
+          mb = max_nan(mb, val.x);
         }
+#pragma unroll
+      for (int o = W / 2; o > 0; o >>= 1) {
+        ma = max_nan(ma, __shfl_xor_sync(seq_lanes, ma, o));
+        mb = max_nan(mb, __shfl_xor_sync(seq_lanes, mb, o));
+        l1a = __fadd_ru(l1a, __shfl_xor_sync(seq_lanes, l1a, o));
+        l1b = __fadd_ru(l1b, __shfl_xor_sync(seq_lanes, l1b, o));
+        k2a = __fadd_ru(k2a, __shfl_xor_sync(seq_lanes, k2a, o));
+        k2b = __fadd_ru(k2b, __shfl_xor_sync(seq_lanes, k2b, o));
+      }
+      if (j % W == 0) {
+        const int at = (ya - row0) * NW + j / W;
+        s_max[at] = ma;
+        s_l1[at] = l1a;
+        s_k2[at] = k2a;
+        if (has_b) {
+          s_max[at + NW] = mb;
+          s_l1[at + NW] = l1b;
+          s_k2[at + NW] = k2b;
+        }
+      }
+      l1a = l1b = k2a = k2b = 0.f;
+    }, on_coeff);  // ends with a barrier
+    if (threadIdx.x < ROWS / 2 && row0 + 2 * (int)threadIdx.x < NY) {
+      const int r0 = 2 * threadIdx.x;
+      float cmax[2], l1[2] = {0.f, 0.f}, k2[2] = {0.f, 0.f}, bhi[2], blo[2];
+#pragma unroll
+      for (int h = 0; h < 2; ++h) {
+        cmax[h] = -INFINITY;
+        if (row0 + r0 + h < NY)
+          for (int w = 0; w < NW; ++w) {
+            const int at = (r0 + h) * NW + w;
+            cmax[h] = max_nan(cmax[h], s_max[at]);
+            l1[h] = __fadd_ru(l1[h], s_l1[at]);
+            k2[h] = __fadd_ru(k2[h], s_k2[at]);
+          }
+      }
+      pair_bounds(cmax, l1, k2, eps_rel, curv, bhi, blo);
+      for (int h = 0; h < 2 && row0 + r0 + h < NY; ++h) {
+        s_hi[r0 + h] = bhi[h];
+        s_lo[r0 + h] = blo[h];
+      }
     }
-    pair_bounds(cmax, l1, k2, eps_rel, curv, bhi, blo);
-    for (int h = 0; h < 2 && row0 + r0 + h < NY; ++h) {
-      s_hi[r0 + h] = bhi[h];
-      s_lo[r0 + h] = blo[h];
-    }
+    __syncthreads();
+    store_block_bounds(s_hi, s_lo, ROWS, blk, NY, fine_rows, item, hi, lo);
+  });
+}
+
+// hi0 of a fine block from the largest L1 norm of its rows: L1 + eps (eps_y of that norm, rounded upward), NaN where
+// the norm passes 1e36 or is not finite
+__device__ __forceinline__ float l1_block_bound(float l1, float eps_rel) {
+  return l1 <= 1e36f ? __fadd_ru(l1, __fadd_ru(__fmul_ru(eps_rel, l1), 1e-35f)) : NAN;
+}
+
+// tmp[item][y][kx] -> hi[item][fine block] = the block's largest hi0_y (one warp per block of fine_rows rows, one row
+// per warp step; fine_rows is even, so both rows of every packed pair fall in one block).  Streams the column-pass
+// output once: grid (ceil(nfine / 8), items) of 256 threads.  (A row pair per warp step measured slower on the 1024-point
+// patch rows: 0.28 against 0.23 ms at C2.)
+__global__ void __launch_bounds__(256)
+rows_l1_bound(const float2* __restrict__ tmp, int NY, int KX, int fine_rows, float eps_rel, float* __restrict__ hi) {
+  const int nfine = (NY + fine_rows - 1) / fine_rows;
+  const int fb = blockIdx.x * 8 + (threadIdx.x >> 5), lane = threadIdx.x & 31;
+  if (fb >= nfine) return;
+  const long item = blockIdx.y;
+  const int y1 = min(NY, (fb + 1) * fine_rows);
+  float best = 0.f;
+  for (int y = fb * fine_rows; y < y1; ++y) {
+    const float2* row = tmp + (item * NY + y) * KX;
+    float l1 = 0.f, k2 = 0.f;  // k2 unused
+#pragma unroll 4
+    for (int k = lane; k < KX; k += 32) add_coeff(k, __ldg(row + k), l1, k2);
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) l1 = __fadd_ru(l1, __shfl_xor_sync(0xffffffffu, l1, o));
+    best = max_nan(best, l1);
   }
-  __syncthreads();
-  store_block_bounds(s_hi, s_lo, ROWS, row0, NY, fine_rows, item, hi, lo);
+  if (lane == 0) hi[item * nfine + fb] = l1_block_bound(best, eps_rel);
 }
 
 // ---- inverse rows + store: tmp[item][y][kx] -> out[item][y][x] real ------------------------------------
@@ -811,7 +856,7 @@ rows_inverse_store_p2(const float2* __restrict__ tmp, int NY, int KX, const floa
   extern __shared__ float2 smem[];
   const long item = blockIdx.y;
   float* dst = out + item * NY * N;
-  rows_inverse_driver<N>(tmp + item * NY * KX, NY, KX, tw, 1, smem, [&](int ya, bool has_b, int j, const float2* v) {
+  rows_inverse_driver<N>(tmp + item * NY * KX, NY, KX, blockIdx.x, tw, 1, smem, [&](int ya, bool has_b, int j, const float2* v) {
 #pragma unroll
     for (int g = 0; g < P::Last::G; ++g)
 #pragma unroll
